@@ -1,17 +1,19 @@
 #!/usr/bin/env python3
 """bench.py — the driver's measurement contract for the batched N-d radix-n FFT hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-shapes]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-shapes] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one forward C2C transform of the primary workload (BASELINE.json configs[1]:
 1-D C2C fp32, batch 100000 x 1024) through the C ABI (b200fft_exec). At N > 1 every rank
 owns its own batch of that shape (batch sharding, no data-path collective, "weak"
 scaling); the time is the max over ranks and `value` the whole-job GFLOP/s
-(5*N*log2(N) per transform, the north-star's effective-flop model). K steps last only a few
-milliseconds: they are timed exactly as the contract says (W warm-ups, then K steps between CUDA
-events), and identical blocks of K steps then continue back to back for ~0.15 s so that NVML can
-sample the clocks under the same load and a sustained figure can be reported next to the value.
+(5*N*log2(N) per transform, the usual effective-flop model of FFT benchmarks). W warm-up
+steps run first, then exactly K timed steps between CUDA events; NVML samples the clocks during them.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last step computed on rank 0: a fixed,
+seeded sample of the output rows as DIR/out.npy (see dump_outputs). The input is generated from a
+fixed seed, so two builds run with the same arguments can be compared output for output.
 
 Printed on rank 0: ONE JSON line with value / ms_per_step, `roofline` (HBM, measured
 peak from MEASURED_PEAKS.json), `cpu_baseline` (the oracle = C++ port of the
@@ -146,7 +148,7 @@ class ClockSampler:
         return {"sm_mhz": (s[len(s) // 2] if s else None), "sm_mhz_timed_region": (ts[len(ts) // 2] if ts else None),
                 "sm_max_mhz": self.max_mhz,
                 "reasons": sorted(self.reasons), "samples": len(s), "samples_in_timed_region": timed,
-                "sampled": "NVML, back to back, over the timed block and the identical blocks that follow it"}
+                "sampled": "NVML, back to back, over the timed steps"}
 
 
 def physical_gpu_index(local_index):
@@ -220,6 +222,21 @@ def time_gpu(fn, warmup, steps, torch):
     e1.record()
     torch.cuda.synchronize()
     return e0.elapsed_time(e1) / steps
+
+
+DUMP_ROWS = 4096  # 4096 transforms of 1024 complex fp32 points: 32 MB of the 819 MB output
+
+
+def dump_rows(batch):
+    """The batch items --dump-outputs writes: picked by a fixed seed, in increasing order, the same on every run."""
+    return np.sort(np.random.default_rng(0).choice(batch, size=min(DUMP_ROWS, batch), replace=False))
+
+
+def dump_outputs(dirname, out, torch):
+    """Write the dump_rows() items of `out` (batch, length, 2) to dirname/out.npy as float32 (DUMP_ROWS, length, 2)."""
+    sample = out.index_select(0, torch.from_numpy(dump_rows(out.shape[0])).to(out.device)).cpu().numpy()
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "out.npy"), sample)
 
 
 def _to_complex(x):
@@ -541,7 +558,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-shapes", action="store_true", help="skip the per-shape table vs cuFFT")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a seeded sample of the last step's output to DIR/out.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
@@ -580,42 +603,28 @@ def main():
     if dist:
         dist.barrier()
     torch.cuda.synchronize()
-    # The timed region is the FIRST block: exactly K steps after the W warm-up steps, bracketed by CUDA events on the
-    # launching stream with a synchronise on both sides -> ms_per_step / value. K = 20 steps last ~5 ms, too short for
-    # NVML (a query takes ~1 ms) to see the clocks, so identical blocks of K steps follow back to back for ~0.15 s
-    # while the sampler keeps running; their median is reported as the SUSTAINED figure (config.sustained_ms_per_step:
-    # a 1 kW part power-caps under a memory-bound kernel) and the clock record covers the first block and them.
-    est_ms = time_gpu(step, 1, 3, torch)
-    repeats = int(max(5, min(200, 150.0 / max(1e-3, est_ms * args.steps))))
-    torch.cuda.synchronize()
-    if dist:
-        dist.barrier()
-    torch.cuda.synchronize()
+    # The timed region: exactly K steps after the W warm-up steps, bracketed by CUDA events on the launching stream with
+    # a synchronise on both sides -> ms_per_step / value. An NVML query takes ~1 ms, so a short K yields few clock samples.
     sampler = ClockSampler(physical_gpu_index(local)).start()
     sampler.mark("timed_start")
     launches0 = b200fft.launch_count()
-    blocks = []
-    for _ in range(repeats):
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        for _ in range(args.steps):
-            step()
-        e1.record()
-        torch.cuda.synchronize()
-        blocks.append(e0.elapsed_time(e1) / args.steps)
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    for _ in range(args.steps):
+        step()
+    e1.record()
+    torch.cuda.synchronize()
     sampler.mark("timed_end")
-    launches = (b200fft.launch_count() - launches0) // repeats
+    launches = b200fft.launch_count() - launches0
     clocks = sampler.stop()
-    clocks["timed_blocks"] = repeats
+    ms = e0.elapsed_time(e1) / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, torch)
     if dist:
         dist.barrier()
-    torch.cuda.synchronize()
-    ms = blocks[0]
-    sustained_ms = sorted(blocks)[len(blocks) // 2]
-    if dist:
-        t = torch.tensor([ms, sustained_ms], device="cuda", dtype=torch.float64)
+        t = torch.tensor([ms], device="cuda", dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        ms, sustained_ms = (float(v) for v in t.tolist())
+        ms = float(t.item())
     gflops_total = world * flops_c2c(shape) / ms / 1e6
 
     # ---- e2e: the same transform through b200fft_exec_host with pinned HOST buffers
@@ -687,10 +696,7 @@ def main():
                    "sharding": "batch-sharded, no collective" if world > 1 else "single GPU",
                    "l2": "inputs+outputs %.0f MB per step > 126 MB L2 (no flush needed)" % (2 * ab / 2 / 1e6),
                    "flop_model": "5*N*log2(N) per transform",
-                   "timing": "exactly %d steps after %d warm-up steps (CUDA events); then %d more identical blocks for the "
-                             "clock record and the sustained figure" % (args.steps, args.warmup, repeats - 1),
-                   "sustained_ms_per_step": sustained_ms,
-                   "sustained_value": world * flops_c2c(shape) / sustained_ms / 1e6},
+                   "timing": "exactly %d steps after %d warm-up steps (CUDA events)" % (args.steps, args.warmup)},
         "roofline": roofline, "cpu_baseline": cpu, "e2e": e2e, "gpu_launches": int(launches), "clocks": clocks,
     }
     if slab is not None:

@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -32,6 +34,47 @@ def test_reference_arm_other_ranks_exit_quietly():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2"],
                          capture_output=True, text=True, env=env, timeout=120)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+def test_dump_outputs_is_refused_on_the_reference_arm(tmp_path):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", str(tmp_path / "d")],
+                         capture_output=True, text=True, timeout=120)
+    assert out.returncode != 0 and "--dump-outputs" in out.stderr and not (tmp_path / "d").exists()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_repeat_and_match_numpy(tmp_path):
+    """--dump-outputs: two runs with the same arguments write the same bits, a sample of the primary workload's output
+    that matches numpy float64 on the same seeded input; the timed region launches the plan exactly --steps times."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    import b200fft
+    batch, length = bench.PRIMARY["shape"]
+    plan = b200fft.plan_fft("float32", "float32", (batch, length, 2), (batch, length, 2))
+    launches_per_step = plan.launches
+    plan.destroy()
+    steps = 3
+    dumps = []
+    for k in range(2):
+        d = tmp_path / str(k)
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "3", "--no-shapes",
+                              "--no-cpu", "--dump-outputs", str(d)], capture_output=True, text=True, timeout=600)
+        assert out.returncode == 0, out.stderr[-2000:]
+        line = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
+        assert line["steps"] == steps and line["gpu_launches"] == steps * launches_per_step
+        assert os.listdir(d) == ["out.npy"]
+        dumps.append(np.load(d / "out.npy"))
+    assert dumps[0].dtype == np.float32 and dumps[0].shape == (bench.DUMP_ROWS, length, 2) and dumps[0].nbytes <= 64 << 20
+    assert np.array_equal(dumps[0], dumps[1])
+    g = torch.Generator(device="cuda").manual_seed(1234)            # bench.py's rank-0 input
+    x = torch.randn((batch, length, 2), generator=g, device="cuda", dtype=torch.float32)
+    rows = bench.dump_rows(batch)
+    xs = x.index_select(0, torch.from_numpy(rows).cuda()).double().cpu().numpy()
+    want = np.fft.fft(xs[..., 0] + 1j * xs[..., 1], axis=1)
+    got = dumps[0][..., 0].astype(np.float64) + 1j * dumps[0][..., 1]
+    assert np.linalg.norm(got - want) <= 2e-6 * np.linalg.norm(want)
 
 
 def test_gpu_arm_refuses_to_run_without_a_gpu():

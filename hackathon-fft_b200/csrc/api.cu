@@ -331,8 +331,12 @@ int b200fft_default_bases(uint64_t length, int gpu_target, uint32_t* out, int ca
   return copy_bases(estimate_best_bases(length, gpu_target != 0), out, cap);
 }
 
-int b200fft_jit_probe(int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in, int half,
-                      int in_dtype, int out_dtype, char* buf, size_t cap) {
+}  // extern "C"
+
+namespace {
+// b200fft_jit_probe / b200fft_jit_split_probe: validate, order the bases, run the host-only probe
+int probe_entry(bool split, int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in, int half,
+                int in_dtype, int out_dtype, char* buf, size_t cap) {
   if (in_dtype < B200FFT_U8 || in_dtype > B200FFT_F64 || (out_dtype != B200FFT_F32 && out_dtype != B200FFT_F64))
     return fail(B200FFT_ERR_INVALID_ARG, "dtypes %d -> %d", in_dtype, out_dtype);
   if (half < 0 || half > 2) return fail(B200FFT_ERR_INVALID_ARG, "half = %d (0 complex, 1 R2C, 2 C2R)", half);
@@ -345,13 +349,27 @@ int b200fft_jit_probe(int64_t n, int64_t inner, const uint32_t* bases, int nbase
   }
   if (!ordered_bases_valid((uint64_t)n, ordered)) return fail(B200FFT_ERR_BASES, "bases do not factor %lld", (long long)n);
   std::string report;
-  const int rc = jit_probe(n, inner, ordered, inverse != 0, real_in != 0, half, in_dtype, out_dtype, &report);
+  const int rc = (split ? jit_split_probe : jit_probe)(n, inner, ordered, inverse != 0, real_in != 0, half, in_dtype, out_dtype,
+                                                      &report);
   if (rc != B200FFT_OK) return rc;
   if (buf && cap) {
     strncpy(buf, report.c_str(), cap - 1);
     buf[cap - 1] = 0;
   }
   return B200FFT_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int b200fft_jit_probe(int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in, int half,
+                      int in_dtype, int out_dtype, char* buf, size_t cap) {
+  return probe_entry(false, n, inner, bases, nbases, inverse, real_in, half, in_dtype, out_dtype, buf, cap);
+}
+
+int b200fft_jit_split_probe(int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in, int half,
+                            int in_dtype, int out_dtype, char* buf, size_t cap) {
+  return probe_entry(true, n, inner, bases, nbases, inverse, real_in, half, in_dtype, out_dtype, buf, cap);
 }
 
 int b200fft_schedule_dry_run(int nphases, const int64_t* phases, int64_t batch, int64_t* segments, int cap) {

@@ -842,10 +842,11 @@ constexpr size_t cols_smem_bytes() {
 // Both are ordinary tile passes: A is a strided-axis pass with a twiddling store, B is a strided-axis
 // pass (or, for a contiguous axis, a row pass) whose destination uses a different base and stride.
 struct SplitArgs {
-  const float2* in;
+  const void* in;      // pass A: the user's array (in_scalar / in_vec2 elements); pass B: the temporary (float2)
   float2* out;
   const float2* tw;    // stage twiddles of this pass's variant
   const float2* twN;   // W_N^n, n in [0, N): pass A only
+  const float2* tw2;   // half-spectrum forms: W_n^{-+k}, k = 0..n/2, of the Hermitian unpack (R2C) / pack (C2R)
   long long inner;     // element stride of the ORIGINAL axis (1 = contiguous)
   long long nrows;     // rows pass B: outer * N1 rows of N2 points
   int tiles_per_outer; // cols passes: tiles per outer slab of THIS pass's view
@@ -867,8 +868,9 @@ struct SplitTwDst {
   }
 };
 
-// pass A: view (outer, N1 = N, inner' = n2 * inner)
-template <int N, class RL, int CW, int NT, bool INV>
+// pass A: view (outer, N1 = N, inner' = n2 * inner). REAL: the input array holds real scalars (in_scalar), read as
+// x + 0i; otherwise complex pairs (in_vec2). Both are cast to the working precision on load.
+template <int N, class RL, int CW, int NT, bool INV, bool REAL = false>
 __global__ void __launch_bounds__(NT) cols_split_a_kernel(const __grid_constant__ SplitArgs a) {
   extern __shared__ __align__(16) float2 smem_f2[];
   pdl_wait();
@@ -878,9 +880,58 @@ __global__ void __launch_bounds__(NT) cols_split_a_kernel(const __grid_constant_
   const long long c0 = (long long)(blockIdx.x - o * a.tiles_per_outer) * CW;
   const long long base = o * N * vinner + c0;
   const int valid_c = (int)min((long long)CW, vinner - c0);
-  GlobalSrc<false> src{a.in + base, 0, vinner, 1, valid_c};
+  const void* in = REAL ? (const void*)(reinterpret_cast<const in_scalar*>(a.in) + base)
+                        : (const void*)(reinterpret_cast<const in_vec2*>(a.in) + base);
+  GlobalSrc<REAL> src{in, 0, vinner, 1, valid_c};
   SplitTwDst dst{a.out + base, vinner, valid_c, a.twN, c0, a.inner};
   run_axis<RL, N, 1, CW, NT, INV, DenseLayoutN<N, CW>::template type>(src, dst, smem_f2, smem_f2 + BUF, a.tw, 1.f, false);
+}
+
+// ---- long half-spectrum axes (last axis, inner == 1) as two passes ----------------------------------------------------
+// Pass A of a long C2R: the Hermitian pack (even n = 2H) or the Hermitian extension (odd n) of the single-tile C2R
+// kernels, read straight from the rows of n/2 + 1 bins in global memory, at axis index m = n1 * N2 + n2 of the split
+// transform. The mirrored bin of an element lies in another column tile of the same transform's row (an L2 hit when
+// the tiles of one transform run close together, which the grid order gives).
+//   even: Z[m] = s + i t, s = X[m] + conj X[H-m], t = W_n^{-m} (X[m] - conj X[H-m]); H = N1 * N2, bins = H + 1
+//   odd:  Z[m] = X[m] for m <= n/2, conj X[n-m] above;                             n = N1 * N2, bins = n/2 + 1
+template <bool ODD>
+struct HermSplitSrc {
+  const in_vec2* __restrict__ xb;  // first bin of this transform's row
+  const float2* __restrict__ tw2;
+  int len;                          // H (even) or n (odd)
+  int n2;
+  long long c0;
+  int valid_c;
+  __device__ __forceinline__ float2 load(int, int i, int c) const {
+    if (c >= valid_c) return make_float2(0.f, 0.f);
+    const int m = i * n2 + (int)c0 + c;
+    if constexpr (ODD) {
+      const int bins = len / 2 + 1;
+      const in_vec2 v = __ldg(&xb[m < bins ? m : len - m]);
+      return make_float2((float)v.x, m < bins ? (float)v.y : -(float)v.y);
+    } else {
+      const in_vec2 p = __ldg(&xb[m]);
+      const in_vec2 q = __ldg(&xb[len - m]);
+      const float2 xk = make_float2((float)p.x, (float)p.y), xm = make_float2((float)q.x, -(float)q.y);
+      const float2 s = make_float2(xk.x + xm.x, xk.y + xm.y), d = make_float2(xk.x - xm.x, xk.y - xm.y);
+      const float2 t = cmulf(d, __ldg(&tw2[m]));  // W_n^{-m} * (X[m] - conj(X[H-m]))
+      return make_float2(s.x - t.y, s.y + t.x);   // s + i t
+    }
+  }
+};
+template <int N, class RL, int CW, int NT, bool ODD>
+__global__ void __launch_bounds__(NT) cols_split_a_c2r_kernel(const __grid_constant__ SplitArgs a) {
+  extern __shared__ __align__(16) float2 smem_f2[];
+  pdl_wait();
+  constexpr int BUF = max_exchange_elems<RL, 1, DenseLayoutN<N, CW>::template type>();
+  const int len = N * a.n2;
+  const long long bins = ODD ? len / 2 + 1 : len + 1;
+  const long long o = blockIdx.x / a.tiles_per_outer;
+  const long long c0 = (long long)(blockIdx.x - o * a.tiles_per_outer) * CW;
+  const int valid_c = (int)min((long long)CW, (long long)a.n2 - c0);
+  HermSplitSrc<ODD> src{reinterpret_cast<const in_vec2*>(a.in) + o * bins, a.tw2, len, a.n2, c0, valid_c};
+  SplitTwDst dst{a.out + o * len + c0, a.n2, valid_c, a.twN, c0, 1};
+  run_axis<RL, N, 1, CW, NT, true, DenseLayoutN<N, CW>::template type>(src, dst, smem_f2, smem_f2 + BUF, a.tw, 1.f, false);
 }
 
 // pass B on a strided axis: view (outer * n1, N2 = N, inner); row k2 of slab (o, k1) goes to axis index k1 + n1*k2
@@ -893,14 +944,35 @@ __global__ void __launch_bounds__(NT) cols_split_b_kernel(const __grid_constant_
   const long long c0 = (long long)(blockIdx.x - ov * a.tiles_per_outer) * CW;
   const long long o = ov / a.n1, k1 = ov - o * a.n1;
   const int valid_c = (int)min((long long)CW, a.inner - c0);
-  GlobalSrc<false> src{a.in + ov * N * a.inner + c0, 0, a.inner, 1, valid_c};
+  GlobalSrc<false> src{reinterpret_cast<const float2*>(a.in) + ov * N * a.inner + c0, 0, a.inner, 1, valid_c};
   GlobalDst dst{a.out + (o * N * a.n1 + k1) * a.inner + c0, 0, (long long)a.n1 * a.inner, 1, valid_c};
   run_axis<RL, N, 1, CW, NT, INV, DenseLayoutN<N, CW>::template type>(src, dst, smem_f2, smem_f2 + BUF, a.tw, a.scale,
                                                                       a.do_scale != 0);
 }
 
-// pass B on a contiguous axis (inner == 1): C consecutive rows k1 of one transform, N2 = N points each
-template <int N, class RL, int C, int NT, bool INV>
+// pass B of an odd-length R2C: only bins k = k1 + N1*k2 <= n/2 are stored, into rows of n/2 + 1 (GlobalHalfDst's rule)
+struct SplitHalfDst {
+  float2* __restrict__ base;  // bin k1 of this tile's transform
+  int n1, bins_left;          // bins_left = n/2 + 1 - k1
+  int valid_o;
+  __device__ __forceinline__ void store(int o, int i, int, float2 v) const {
+    const int k = o + n1 * i;
+    if (o < valid_o && k < bins_left) base[k] = v;
+  }
+};
+// pass B of an odd-length C2R: the real parts of the n-point inverse (RealDst's rule)
+struct SplitRealDst {
+  float* __restrict__ base;  // sample k1 of this tile's transform
+  int n1;
+  int valid_o;
+  __device__ __forceinline__ void store(int o, int i, int, float2 v) const {
+    if (o < valid_o) base[o + (long long)n1 * i] = v.x;
+  }
+};
+
+// pass B on a contiguous axis (inner == 1): C consecutive rows k1 of one transform, N2 = N points each.
+// STORE 0: complex natural order; 1: bins 0..n/2 of rows of n/2 + 1 (odd R2C); 2: real parts (odd C2R)
+template <int N, class RL, int C, int NT, bool INV, int STORE = 0>
 __global__ void __launch_bounds__(NT) rows_split_b_kernel(const __grid_constant__ SplitArgs a) {
   extern __shared__ __align__(16) float2 smem_f2[];
   pdl_wait();
@@ -908,10 +980,87 @@ __global__ void __launch_bounds__(NT) rows_split_b_kernel(const __grid_constant_
   const long long row0 = (long long)blockIdx.x * C;  // rows never straddle transforms: C divides n1
   const int valid = (int)min((long long)C, a.nrows - row0);
   const long long t = row0 / a.n1, k1 = row0 - t * a.n1;
-  GlobalSrc<false> src{a.in + row0 * N, N, 1, valid, 1};
-  GlobalDst dst{a.out + t * N * a.n1 + k1, 1, a.n1, valid, 1};  // element (row o, k2) -> k1 + o + n1 * k2
-  run_axis<RL, N, C, 1, NT, INV, RowLayoutN<N>::template type>(src, dst, smem_f2, smem_f2 + BUF, a.tw, a.scale,
-                                                               a.do_scale != 0);
+  GlobalSrc<false> src{reinterpret_cast<const float2*>(a.in) + row0 * N, N, 1, valid, 1};
+  const long long len = (long long)N * a.n1;
+  if constexpr (STORE == 1) {
+    const long long bins = len / 2 + 1;
+    SplitHalfDst dst{a.out + t * bins + k1, a.n1, (int)(bins - k1), valid};
+    run_axis<RL, N, C, 1, NT, INV, RowLayoutN<N>::template type>(src, dst, smem_f2, smem_f2 + BUF, a.tw, a.scale,
+                                                                 a.do_scale != 0);
+  } else if constexpr (STORE == 2) {
+    SplitRealDst dst{reinterpret_cast<float*>(a.out) + t * len + k1, a.n1, valid};
+    run_axis<RL, N, C, 1, NT, INV, RowLayoutN<N>::template type>(src, dst, smem_f2, smem_f2 + BUF, a.tw, a.scale,
+                                                                 a.do_scale != 0);
+  } else {
+    GlobalDst dst{a.out + t * len + k1, 1, a.n1, valid, 1};  // element (row o, k2) -> k1 + o + n1 * k2
+    run_axis<RL, N, C, 1, NT, INV, RowLayoutN<N>::template type>(src, dst, smem_f2, smem_f2 + BUF, a.tw, a.scale,
+                                                                 a.do_scale != 0);
+  }
+}
+
+// Pass B of a long even-length R2C (n = 2H, H = N1 * N2) with the Hermitian unpack fused into the store. Pass A has
+// transformed the real row read as H complex points; row k1 of the temporary holds Z[k1 + N1*k2] after this pass's
+// N2-point transform. The unpack of bin k needs Z[H - k]:
+//   k1 > 0: row N1 - k1, column N2 - 1 - k2          k1 = 0: row 0, column (N2 - k2) mod N2
+// so a CTA transforms C/2 consecutive rows k1 = p0 .. and their mirror rows N1 - k1 (row 0 and, for even N1, row N1/2
+// pair with themselves and are transformed twice), keeps Z of all C rows in shared memory and writes
+//   X[k] = ((Z[k] + conj Z[H-k]) - i W_n^k (Z[k] - conj Z[H-k])) / 2
+// for both rows of every pair into rows of H + 1 bins (R2CRegDst's arithmetic); row 0 also writes X[H] = Re Z[0] - Im Z[0].
+// Grid: outer * tiles_per_outer, tiles_per_outer = ceil((N1/2 + 1) / (C/2)).
+// tile slot o: slots 0 .. C/2-1 hold rows p = p0 + o, slots C/2 .. C-1 their mirror rows N1 - p (row 0 for p = 0)
+template <int N, int C>
+struct PairSrc {
+  const float2* __restrict__ z;  // row 0 of this transform in the temporary
+  int n1, p0, npairs;
+  __device__ __forceinline__ float2 load(int o, int i, int) const {
+    const int p = p0 + (o < C / 2 ? o : o - C / 2);
+    if (p >= npairs) return make_float2(0.f, 0.f);
+    const int row = o < C / 2 || p == 0 ? p : n1 - p;
+    return __ldg(&z[(long long)row * N + i]);
+  }
+};
+template <int N, class RL, int C, int NT>
+__global__ void __launch_bounds__(NT) rows_split_b_r2c_kernel(const __grid_constant__ SplitArgs a) {
+  static_assert(C % 2 == 0, "rows come in (k1, N1 - k1) pairs");
+  extern __shared__ __align__(16) float2 smem_f2[];
+  pdl_wait();
+  constexpr int PC = C / 2;
+  constexpr int EX = max_exchange_elems<RL, C, RowLayoutN<N>::template type>();
+  constexpr int BUF = EX > C * N ? EX : C * N;
+  float2* buf0 = smem_f2;
+  float2* buf1 = smem_f2 + BUF;
+  float2* zbuf = ((RL::count - 1) % 2 == 0) ? buf0 : buf1;  // the buffer the last exchange does not use
+  const int n1 = a.n1;
+  const int npairs = n1 / 2 + 1;
+  const long long t = blockIdx.x / a.tiles_per_outer;
+  const int p0 = (int)(blockIdx.x - t * a.tiles_per_outer) * PC;
+  const long long H = (long long)n1 * N;
+  PairSrc<N, C> src{reinterpret_cast<const float2*>(a.in) + t * H, n1, p0, npairs};
+  if constexpr (RL::count == 1) {
+    run_stage<RL::r[0], 1, N, C, 1, NT, false>(src, SmemDst<PlaneLayout<N>>{zbuf}, a.tw, 1.f, false);
+  } else {
+    run_axis<RL, N, C, 1, NT, false, RowLayoutN<N>::template type>(src, SmemDst<PlaneLayout<N>>{zbuf}, buf0, buf1, a.tw, 1.f,
+                                                                   false);
+  }
+  __syncthreads();
+  float2* __restrict__ out = a.out + t * (H + 1);
+  // pair fastest: consecutive threads store consecutive bins k1 (first rows) or k1 descending (mirror rows)
+  for (int idx = threadIdx.x; idx < C * N; idx += NT) {
+    const int j = idx % PC, rest = idx / PC;
+    const int k2 = rest % N, side = rest / N;
+    const int p = p0 + j;
+    if (p >= npairs || (side == 1 && (p == 0 || 2 * p == n1))) continue;  // a self-paired row is stored once
+    const int slot = side * PC + j, mslot = (1 - side) * PC + j;
+    const int mc = p == 0 ? (N - k2) % N : N - 1 - k2;
+    const float2 zk = zbuf[slot * N + k2];
+    const float2 zm = zbuf[mslot * N + mc];
+    const long long k = (side == 0 ? p : n1 - p) + (long long)n1 * k2;
+    // s = Z[k] + conj(Z[H-k]), d = Z[k] - conj(Z[H-k])
+    const float2 s = make_float2(zk.x + zm.x, zk.y - zm.y), d = make_float2(zk.x - zm.x, zk.y + zm.y);
+    const float2 tt = cmulf(d, __ldg(&a.tw2[k]));
+    out[k] = make_float2(0.5f * (s.x + tt.y), 0.5f * (s.y - tt.x));  // (s - i t) / 2
+    if (k == 0) out[H] = make_float2(zk.x - zk.y, 0.f);              // X[H] = Re Z[0] - Im Z[0]
+  }
 }
 
 }  // namespace b200fft

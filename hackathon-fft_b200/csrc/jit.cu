@@ -148,7 +148,14 @@ enum JitKind {
   // the two innermost axes in one in-place tile per (y, x) plane (plane.cuh); n = NY, n2 = NX (R2C: H), radices = y, radices2 = x
   JIT_PLANE_C2C,    // c2c_plane_ip_kernel<NY, NX, RLY, RLX, NT, INV, REAL>
   JIT_PLANE_R2C,    // r2c_plane_ip_kernel<NY, H, RLY, RLX, NT>
-  JIT_ROWS_IP       // rows_ip_kernel<N, RL, C, NT, INV, REAL>: `tile` rows per CTA, 3-5 stages in ONE shared buffer
+  JIT_ROWS_IP,      // rows_ip_kernel<N, RL, C, NT, INV, REAL>: `tile` rows per CTA, 3-5 stages in ONE shared buffer
+  // long half-spectrum rows as two passes (split length H = n/2 for even n, n for odd n); pass A of a real-input or
+  // dtype-casting axis is JIT_SPLIT_A with real_in / in_dtype
+  JIT_SPLIT_B_R2C,     // rows_split_b_r2c_kernel<N2, RL, C, NT>: even R2C, (k1, N1 - k1) row pairs, Hermitian unpack in the store
+  JIT_SPLIT_A_C2R,     // cols_split_a_c2r_kernel<N1, RL, CW, NT, false>: even C2R, Hermitian pack in the load
+  JIT_SPLIT_A_C2R_ODD, // cols_split_a_c2r_kernel<N1, RL, CW, NT, true>: odd C2R, Hermitian-extended load
+  JIT_SPLIT_B_HALF,    // rows_split_b_kernel<N2, RL, C, NT, false, 1>: odd R2C, bins 0..n/2 stored
+  JIT_SPLIT_B_REAL     // rows_split_b_kernel<N2, RL, C, NT, true, 2>: odd C2R, real parts stored
 };
 
 struct JitSpec {
@@ -172,7 +179,10 @@ struct JitSpec {
     for (int r : radices2) rx += (rx.empty() ? "" : ", ") + std::to_string(r);
     return std::to_string(n) + ", " + std::to_string(n2) + ", b200fft::Radices<" + ry + ">, b200fft::Radices<" + rx + ">";
   }
-  bool strided() const { return kind == JIT_COLS || kind == JIT_SCATTER || kind == JIT_SPLIT_A || kind == JIT_SPLIT_B_COLS; }
+  bool strided() const {
+    return kind == JIT_COLS || kind == JIT_SCATTER || kind == JIT_SPLIT_A || kind == JIT_SPLIT_B_COLS || kind == JIT_SPLIT_A_C2R ||
+           kind == JIT_SPLIT_A_C2R_ODD;
+  }
   std::string radix_list() const {
     std::string s;
     for (int r : radices) s += (s.empty() ? "" : ", ") + std::to_string(r);
@@ -197,7 +207,12 @@ struct JitSpec {
       case JIT_R2C_REG: return "b200fft::rows_r2c_reg_kernel<" + head + ">";
       case JIT_R2C_ODD: return "b200fft::rows_r2c_odd_kernel<" + head + ">";
       case JIT_C2R_ODD: return "b200fft::rows_c2r_odd_kernel<" + head + ">";
-      case JIT_SPLIT_A: return "b200fft::cols_split_a_kernel<" + head + ", " + inv + ">";
+      case JIT_SPLIT_A: return "b200fft::cols_split_a_kernel<" + head + ", " + inv + (real_in ? ", true>" : ">");
+      case JIT_SPLIT_A_C2R: return "b200fft::cols_split_a_c2r_kernel<" + head + ", false>";
+      case JIT_SPLIT_A_C2R_ODD: return "b200fft::cols_split_a_c2r_kernel<" + head + ", true>";
+      case JIT_SPLIT_B_R2C: return "b200fft::rows_split_b_r2c_kernel<" + head + ">";
+      case JIT_SPLIT_B_HALF: return "b200fft::rows_split_b_kernel<" + head + ", false, 1>";
+      case JIT_SPLIT_B_REAL: return "b200fft::rows_split_b_kernel<" + head + ", true, 2>";
       case JIT_SPLIT_B_COLS: return "b200fft::cols_split_b_kernel<" + head + ", " + inv + ">";
       case JIT_SPLIT_B_ROWS: return "b200fft::rows_split_b_kernel<" + head + ", " + inv + ">";
       default: return "b200fft::rows_c2r_kernel<" + head + ">";
@@ -214,25 +229,31 @@ struct JitSpec {
       case JIT_ROWS_IP: return "b200fft::rows_ip_smem_bytes<" + shape_args() + ">()";
       case JIT_ROWS:
       case JIT_SPLIT_B_ROWS:
+      case JIT_SPLIT_B_HALF:
+      case JIT_SPLIT_B_REAL:
       case JIT_C2R_ODD:
       case JIT_R2C_ODD: return "b200fft::rows_smem_bytes<" + shape_args() + ">()";
       case JIT_COLS:
       case JIT_SPLIT_A:
       case JIT_SPLIT_B_COLS:
+      case JIT_SPLIT_A_C2R:
+      case JIT_SPLIT_A_C2R_ODD:
       case JIT_SCATTER: return "b200fft::cols_smem_bytes<" + shape_args() + ">()";
-      case JIT_R2C: return "b200fft::rows_r2c_smem_bytes<" + shape_args() + ">()";
+      case JIT_R2C:
+      case JIT_SPLIT_B_R2C: return "b200fft::rows_r2c_smem_bytes<" + shape_args() + ">()";
       case JIT_R2C_REG: return "b200fft::rows_r2c_reg_smem_bytes<" + shape_args() + ">()";
       default: return "b200fft::rows_c2r_smem_bytes<" + shape_args() + ">()";
     }
   }
   std::string name() const {
     static const char* const tag[] = {"jitrows", "jitcols", "jitscatter", "jitr2c", "jitr2creg", "jitr2codd", "jitc2r", "jitc2rodd",
-                                      "jitsplitA", "jitsplitBcols", "jitsplitBrows", "jitplane", "jitr2cplane", "jitrowsIP"};
+                                      "jitsplitA", "jitsplitBcols", "jitsplitBrows", "jitplane", "jitr2cplane", "jitrowsIP",
+                                      "jitsplitBr2c", "jitsplitAc2r", "jitsplitAc2rodd", "jitsplitBhalf", "jitsplitBreal"};
     if (plane())
       return std::string(tag[kind]) + std::to_string(n) + "x" + std::to_string(kind == JIT_PLANE_R2C ? 2 * n2 : n2) + "(" + radix_name(radices) +
              ";" + radix_name(radices2) + ")_inplace_t" + std::to_string(threads) + (f64 ? "_f64" : "");
     return std::string(tag[kind]) + std::to_string(n) + "_" + radix_name(radices) + (strided() ? "_w" : "_c") + std::to_string(tile) +
-           "_t" + std::to_string(threads) + (f64 ? "_f64" : "") + (in_dtype == B200FFT_U8 ? "_inu8" : in_dtype == (f64 ? B200FFT_F32 : B200FFT_F64) ? (f64 ? "_inf32" : "_inf64") : "");
+           "_t" + std::to_string(threads) + (f64 ? "_f64" : "") + (kind == JIT_SPLIT_A && real_in ? "_realin" : "") + (in_dtype == B200FFT_U8 ? "_inu8" : in_dtype == (f64 ? B200FFT_F32 : B200FFT_F64) ? (f64 ? "_inf32" : "_inf64") : "");
   }
   std::string defines() const {  // rtc_prelude.cuh reads these
     std::string d;
@@ -271,7 +292,8 @@ struct JitSpec {
     }
     const size_t pingpong = radices.size() > 2 ? 2 : 1;
     switch (kind) {
-      case JIT_R2C: return esz() * (size_t)std::max<long long>(ex, (long long)tile * n) * 2;
+      case JIT_R2C:
+      case JIT_SPLIT_B_R2C: return esz() * (size_t)std::max<long long>(ex, (long long)tile * n) * 2;
       default: return esz() * (size_t)ex * pingpong;
     }
   }
@@ -572,6 +594,7 @@ bool jit_geometry(JitSpec* s, long long inner) {
     if (smem > 200 * 1024) continue;
     if (s->kind == JIT_R2C_REG && ((long long)tile * (s->n / rlast)) % 32 != 0) continue;  // r2c_reg_ok(): whole warps per row group
     if (s->tile_divides > 0 && s->tile_divides % tile != 0) continue;
+    if (s->kind == JIT_SPLIT_B_R2C && tile % 2) continue;  // whole (k1, N1 - k1) row pairs
     const long long work = tile * per;
     const double bytes = (double)tile * s->n * (double)s->esz();
     for (int rounds = 1; rounds <= 4; ++rounds) {
@@ -901,12 +924,12 @@ struct JitSplitPass : Pass {
   int n1 = 0, n2 = 0;
   bool do_scale = false;
   double scale = 1.0;
-  void *twa = nullptr, *twb = nullptr, *tmp = nullptr;
+  void *twa = nullptr, *twb = nullptr, *tw2 = nullptr, *tmp = nullptr;
   const void* twN = nullptr;
   std::string text;
 
   struct SplitArgs64 {
-    const double2* in; double2* out; const double2* tw; const double2* twN; long long inner; long long nrows;
+    const void* in; double2* out; const double2* tw; const double2* twN; const double2* tw2; long long inner; long long nrows;
     int tiles_per_outer; int n1, n2; double scale; int do_scale;
   };
   template <class A, class T2>
@@ -916,22 +939,26 @@ struct JitSplitPass : Pass {
     a.inner = view.inner;
     a.n1 = n1;
     a.n2 = n2;
-    a.in = reinterpret_cast<const T2*>(src);  // pass A: view (outer, n1, n2 * inner)
+    a.in = src;  // pass A: view (outer, n1, n2 * inner)
     a.out = reinterpret_cast<T2*>(tmp);
     a.tw = reinterpret_cast<const T2*>(twa);
     a.twN = reinterpret_cast<const T2*>(twN);
+    a.tw2 = reinterpret_cast<const T2*>(tw2);
     const long long vinner = (long long)n2 * view.inner;
     a.tiles_per_outer = (int)((vinner + sa.tile - 1) / sa.tile);
     void* params[1] = {&a};
     int rc = launch_one(*ka, sa, outer * a.tiles_per_outer, params, stream);
     if (rc != B200FFT_OK) return rc;
-    a.in = reinterpret_cast<const T2*>(tmp);  // pass B
+    a.in = tmp;  // pass B
     a.out = reinterpret_cast<T2*>(dst);
     a.tw = reinterpret_cast<const T2*>(twb);
     a.scale = scale;
     a.do_scale = do_scale;
     long long grid;
-    if (sb.kind == JIT_SPLIT_B_ROWS) {
+    if (sb.kind == JIT_SPLIT_B_R2C) {  // (n1/2 + 1) row pairs per transform, tile/2 of them per CTA
+      a.tiles_per_outer = (int)((n1 / 2 + 1 + sb.tile / 2 - 1) / (sb.tile / 2));
+      grid = outer * a.tiles_per_outer;
+    } else if (sb.kind != JIT_SPLIT_B_COLS) {
       a.nrows = outer * n1;
       grid = (a.nrows + sb.tile - 1) / sb.tile;
     } else {
@@ -983,56 +1010,121 @@ bool jit_split_stages(const std::vector<int>& radices, std::vector<int>* a, std:
   return best < 1e299;
 }
 
-std::unique_ptr<Pass> make_jit_split_pass(b200fft_plan& plan, int axis, const AxisView& view, const IoSpec& src, bool scale_inverse) {
-  const Problem& p = plan.prob;
-  const bool f64 = p.desc.out_dtype == B200FFT_F64;
-  if (src.comps != 2 || src.dtype != p.desc.out_dtype || view.n > (1 << 24) || !plan.tw[axis].ptr) return nullptr;
+// The two passes of one long axis, decided on the host alone (the plan and b200fft_jit_split_probe share it).
+//   complex / real input / cast on load: split n; pass A reads the user's array (real scalars or complex pairs)
+//   even-n R2C: split H = n/2 (the real row read as H complex); pass B unpacks mirrored row pairs into n/2+1 bins
+//   even-n C2R: split H; pass A packs the half spectrum in its load; pass B writes H complex = the n reals
+//   odd-n R2C / C2R: split n; pass B keeps bins 0..n/2 / pass A extends the half spectrum, pass B keeps real parts
+struct JitSplitChoice {
+  JitSpec sa, sb;
+  long long n1 = 0, n2 = 0;
+  long long len = 0;  // length of the complex transform the two passes run (H for even half-spectrum rows)
+};
+bool jit_split_plan(const std::vector<uint32_t>& ordered, const AxisView& view, const IoSpec& src, bool inverse, HalfMode half,
+                    bool f64, JitSplitChoice* c) {
+  const int work = f64 ? B200FFT_F64 : B200FFT_F32;
+  const bool even_half = half != HALF_NONE && view.n % 2 == 0;
+  if (half != HALF_NONE) {  // the same input rules as the single-tile half-spectrum kernels (jit_plan_axis)
+    if (view.inner != 1 || src.dtype == B200FFT_U8 || (half == HALF_C2R && src.dtype != work)) return false;
+  }
+  c->len = even_half ? view.n / 2 : view.n;
+  if (c->len > (1 << 24)) return false;
+  const std::vector<std::vector<uint32_t>> options = even_half ? drop_factor_two(ordered) : std::vector<std::vector<uint32_t>>{ordered};
   std::vector<int> all, ra, rb;
+  bool ok = false;
   // more stages than one tile takes: the cap on the stage count does not apply to the union of the two passes
-  if (!jit_group_cap(p.axes[axis].ordered, f64 ? JIT_MAX_RADIX_F64 : JIT_MAX_RADIX, &all, 8)) return nullptr;
-  if (!jit_split_stages(all, &ra, &rb)) return nullptr;
-  auto pass = std::make_unique<JitSplitPass>();
-  long long n1 = 1, n2 = 1;
-  for (int r : ra) n1 *= r;
-  for (int r : rb) n2 *= r;
-  pass->n1 = (int)n1;
-  pass->n2 = (int)n2;
-  pass->view = view;
-  for (JitSpec* s : {&pass->sa, &pass->sb}) {
-    s->inverse = p.desc.inverse != 0;
+  for (const auto& o : options)
+    if (jit_group_cap(o, f64 ? JIT_MAX_RADIX_F64 : JIT_MAX_RADIX, &all, 8) && jit_split_stages(all, &ra, &rb)) { ok = true; break; }
+  if (!ok) return false;
+  c->n1 = c->n2 = 1;
+  for (int r : ra) c->n1 *= r;
+  for (int r : rb) c->n2 *= r;
+  for (JitSpec* s : {&c->sa, &c->sb}) {
+    s->inverse = half == HALF_NONE ? inverse : half == HALF_C2R;
     s->f64 = f64;
-    s->in_dtype = src.dtype;
+    s->in_dtype = work;  // pass B reads the temporary
     s->packed = !f64;
   }
-  pass->sa.kind = JIT_SPLIT_A;
-  pass->sa.n = (int)n1;
-  pass->sa.radices = ra;
-  pass->sb.kind = view.inner == 1 ? JIT_SPLIT_B_ROWS : JIT_SPLIT_B_COLS;
-  pass->sb.n = (int)n2;
-  pass->sb.radices = rb;
-  if (view.inner == 1) pass->sb.tile_divides = (int)n1;
-  if (!jit_geometry(&pass->sa, n2 * view.inner) || !jit_geometry(&pass->sb, view.inner)) return nullptr;
+  c->sa.in_dtype = src.dtype;
+  c->sa.n = (int)c->n1;
+  c->sa.radices = ra;
+  c->sb.n = (int)c->n2;
+  c->sb.radices = rb;
+  if (half == HALF_NONE) {
+    c->sa.kind = JIT_SPLIT_A;
+    c->sa.real_in = src.comps == 1;
+    c->sb.kind = view.inner == 1 ? JIT_SPLIT_B_ROWS : JIT_SPLIT_B_COLS;
+  } else if (half == HALF_R2C) {
+    c->sa.kind = JIT_SPLIT_A;
+    c->sa.real_in = !even_half;  // even n: the real row's bytes are H complex pairs
+    c->sb.kind = even_half ? JIT_SPLIT_B_R2C : JIT_SPLIT_B_HALF;
+  } else {
+    c->sa.kind = even_half ? JIT_SPLIT_A_C2R : JIT_SPLIT_A_C2R_ODD;
+    c->sb.kind = even_half ? JIT_SPLIT_B_ROWS : JIT_SPLIT_B_REAL;
+  }
+  if (view.inner == 1 && c->sb.kind != JIT_SPLIT_B_R2C) c->sb.tile_divides = (int)c->n1;  // row tiles never straddle transforms
+  return jit_geometry(&c->sa, c->n2 * view.inner) && jit_geometry(&c->sb, view.inner);
+}
+
+std::unique_ptr<Pass> make_jit_split_pass(b200fft_plan& plan, int axis, const AxisView& view, const IoSpec& src, bool scale_inverse,
+                                          HalfMode half) {
+  const Problem& p = plan.prob;
+  const bool f64 = p.desc.out_dtype == B200FFT_F64;
+  JitSplitChoice c;
+  if (!jit_split_plan(p.axes[axis].ordered, view, src, p.desc.inverse != 0, half, f64, &c)) return nullptr;
+  const bool even_half = half != HALF_NONE && c.len != view.n;
+  if (!even_half && !plan.tw[axis].ptr) return nullptr;
+  auto pass = std::make_unique<JitSplitPass>();
+  pass->sa = c.sa;
+  pass->sb = c.sb;
+  pass->n1 = (int)c.n1;
+  pass->n2 = (int)c.n2;
+  pass->view = view;
   pass->ka = get_kernel(pass->sa, plan.device);
   pass->kb = pass->ka ? get_kernel(pass->sb, plan.device) : nullptr;
   if (!pass->ka || !pass->kb) return nullptr;
-  pass->do_scale = scale_inverse;
-  pass->scale = scale_inverse ? 1.0 / (double)view.n : 1.0;
-  pass->twN = plan.tw[axis].ptr;  // W_N^n, n in [0, N), in the working precision (api.cu: upload_twiddles)
+  // the half-spectrum inverse is always normalised (like the single-tile C2R kernels)
+  pass->do_scale = scale_inverse || half == HALF_C2R;
+  pass->scale = pass->do_scale ? 1.0 / (double)view.n : 1.0;
   auto upload = [&](const void* data, size_t bytes, void** d) {
     if (cudaMalloc(d, bytes) != cudaSuccess) { cudaGetLastError(); return false; }
     plan.owned_device.push_back(*d);
     return cudaMemcpy(*d, data, bytes, cudaMemcpyHostToDevice) == cudaSuccess;
   };
+  const bool inv = pass->sa.inverse;
   bool ok;
   if (f64) {
-    const auto ta = stage_twiddles64(ra, pass->sa.inverse), tb = stage_twiddles64(rb, pass->sa.inverse);
+    const auto ta = stage_twiddles64(c.sa.radices, inv), tb = stage_twiddles64(c.sb.radices, inv);
     ok = upload(ta.data(), ta.size() * sizeof(double2), &pass->twa) && upload(tb.data(), tb.size() * sizeof(double2), &pass->twb);
   } else {
-    const auto ta = build_twiddles(ra, pass->sa.inverse), tb = build_twiddles(rb, pass->sa.inverse);
+    const auto ta = build_twiddles(c.sa.radices, inv), tb = build_twiddles(c.sb.radices, inv);
     ok = upload(ta.data(), ta.size() * sizeof(float2), &pass->twa) && upload(tb.data(), tb.size() * sizeof(float2), &pass->twb);
   }
   if (!ok) return nullptr;
-  const size_t tmp_bytes = (size_t)p.batch * view.outer_per_batch * view.n * view.inner * pass->sa.esz();
+  if (!even_half) {
+    pass->twN = plan.tw[axis].ptr;  // W_n^m, m in [0, n), in the working precision (api.cu: upload_twiddles)
+  } else {
+    // the split runs on H = n/2 points: pass A's twiddle is W_H^m, m in [0, H), and the unpack / pack needs W_n^{-+k}, k = 0..H
+    void* d = nullptr;
+    if (f64) {
+      const std::vector<double2> th = half_twiddles64(c.len, inv);  // W_H^m for m = 0..H/2; the rest by symmetry below
+      std::vector<double2> full((size_t)c.len);
+      for (long long m = 0; m < c.len; ++m) full[(size_t)m] = m <= c.len / 2 ? th[(size_t)m] : make_double2(th[(size_t)(c.len - m)].x, -th[(size_t)(c.len - m)].y);
+      const std::vector<double2> t2 = half_twiddles64(view.n, inv);
+      ok = upload(full.data(), full.size() * sizeof(double2), &d) && upload(t2.data(), t2.size() * sizeof(double2), &pass->tw2);
+    } else {
+      std::vector<float2> full((size_t)c.len);
+      for (long long m = 0; m < c.len; ++m) {
+        const double th = 2.0 * M_PI * (double)m / (double)c.len;
+        full[(size_t)m] = make_float2((float)std::cos(th), (float)((inv ? 1.0 : -1.0) * std::sin(th)));
+      }
+      const std::vector<float2> t2 = build_half_twiddles(view.n, inv);
+      ok = upload(full.data(), full.size() * sizeof(float2), &d) && upload(t2.data(), t2.size() * sizeof(float2), &pass->tw2);
+    }
+    if (!ok) return nullptr;
+    pass->twN = d;
+  }
+  const size_t tmp_bytes = (size_t)p.batch * view.outer_per_batch * c.len * view.inner * pass->sa.esz();
   if (cudaMalloc(&pass->tmp, tmp_bytes) != cudaSuccess) {
     cudaGetLastError();
     return nullptr;
@@ -1042,10 +1134,33 @@ std::unique_ptr<Pass> make_jit_split_pass(b200fft_plan& plan, int axis, const Ax
   std::string stages;
   for (uint32_t r : p.axes[axis].ordered) stages += (stages.empty() ? "" : ",") + std::to_string(r);
   if (stages.size() > 120) stages = stages.substr(0, 117) + "...";
-  char buf[640];
-  snprintf(buf, sizeof buf, "axis %d: split n=%lld = %lld x %lld inner=%lld: %s (+W_n twiddle) -> %s (natural-order store); temp=%zuB user "
-           "stages=[%s] [NVRTC, %.0f + %.0f ms]", axis, (long long)view.n, n1, n2, (long long)view.inner, pass->sa.name().c_str(),
-           pass->sb.name().c_str(), tmp_bytes, stages.c_str(), pass->ka->compile_ms, pass->kb->compile_ms);
+  const char* form = "";
+  const char* a_note = "(+W_n twiddle)";
+  const char* b_note = "(natural-order store)";
+  if (half == HALF_R2C && even_half) {
+    form = " r2c";
+    a_note = "(+W_H twiddle)";
+    b_note = "(mirrored row pairs, unpack in the store)";
+  } else if (half == HALF_R2C) {
+    form = " r2c";
+    a_note = "(real rows, +W_n twiddle)";
+    b_note = "(bins 0..n/2 stored)";
+  } else if (half == HALF_C2R && even_half) {
+    form = " c2r";
+    a_note = "(Hermitian pack in the load, +W_H twiddle)";
+    b_note = "(natural-order store, 1/n)";
+  } else if (half == HALF_C2R) {
+    form = " c2r";
+    a_note = "(Hermitian-extended load, +W_n twiddle)";
+    b_note = "(real parts stored, 1/n)";
+  } else if (src.comps == 1) {
+    form = " real-in";
+  }
+  char buf[700];
+  snprintf(buf, sizeof buf, "axis %d: split n=%lld%s = %lld x %lld%s inner=%lld: %s %s -> %s %s; temp=%zuB user "
+           "stages=[%s] [NVRTC, %.0f + %.0f ms]", axis, (long long)view.n, form, c.n1, c.n2, even_half ? " (H points)" : "",
+           (long long)view.inner, pass->sa.name().c_str(), a_note, pass->sb.name().c_str(), b_note, tmp_bytes, stages.c_str(),
+           pass->ka->compile_ms, pass->kb->compile_ms);
   pass->text = buf;
   return pass;
 }
@@ -1061,9 +1176,9 @@ std::unique_ptr<Pass> make_jit_pass(b200fft_plan& plan, int axis, const AxisView
   const long long rows = view.inner == 1 ? (long long)p.batch * view.outer_per_batch : 0;
   if ((view.n > 16384 && view.inner != 1) || view.n > 32768 ||
       !jit_plan_axis(p.axes[axis], view, src, p.desc.inverse != 0, half, f64, &spec, rows)) {
-    // too long (or too many stages) for one tile: two passes, if the axis is a plain complex one
-    if (half != HALF_NONE || view.n < 1024) return nullptr;
-    return make_jit_split_pass(plan, axis, view, src, scale_inverse);
+    // too long (or too many stages) for one tile: two passes
+    if (view.n < 1024) return nullptr;
+    return make_jit_split_pass(plan, axis, view, src, scale_inverse, half);
   }
   std::shared_ptr<JitKernel> k = get_kernel(spec, plan.device);
   if (!k) return nullptr;
@@ -1226,6 +1341,27 @@ std::unique_ptr<Pass> make_jit_plane_pass(b200fft_plan& plan) {
   return pass;
 }
 
+namespace {
+// compile `spec` (or load it from the on-disk cache) and describe the result; no CUDA device involved
+int probe_compile(const JitSpec& spec, std::string* report) {
+  std::vector<char> cubin;
+  std::string lowered, log;
+  double ms = 0;
+  const std::string on_disk = disk_cache_path(spec);
+  const bool from_disk = disk_cache_load(on_disk, &cubin, &lowered);
+  if (!from_disk) {
+    const int rc = compile(spec, &cubin, &lowered, &log, &ms);
+    if (rc != B200FFT_OK) return rc;
+    disk_cache_store(on_disk, cubin, lowered);
+  }
+  char buf[700];
+  snprintf(buf, sizeof buf, "%s: %s, smem=%zuB, cubin=%zuB, %.0f ms%s, symbol %s", spec.name().c_str(), spec.expression().c_str(), spec.smem(),
+           cubin.size(), ms, from_disk ? " (disk cache)" : "", lowered.c_str());
+  *report = buf;
+  return B200FFT_OK;
+}
+}  // namespace
+
 // Host-only probe (no CUDA device needed): compile the kernel the planner would pick for one axis and report it.
 // half: 0 = complex / real-input full spectrum, 1 = R2C rows, 2 = C2R rows
 int jit_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bool inverse, bool real_in, int half,
@@ -1242,20 +1378,27 @@ int jit_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bo
   JitSpec spec;
   if (!jit_plan_axis(ax, view, src, inverse, (HalfMode)half, out_dtype == B200FFT_F64, &spec))
     return fail(B200FFT_ERR_UNSUPPORTED, "the specialisation tier does not serve this axis (radix above %d, or no tile fits)", JIT_MAX_PRIME);
-  std::vector<char> cubin;
-  std::string lowered, log;
-  double ms = 0;
-  const std::string on_disk = disk_cache_path(spec);
-  const bool from_disk = disk_cache_load(on_disk, &cubin, &lowered);
-  if (!from_disk) {
-    const int rc = compile(spec, &cubin, &lowered, &log, &ms);
-    if (rc != B200FFT_OK) return rc;
-    disk_cache_store(on_disk, cubin, lowered);
-  }
-  char buf[700];
-  snprintf(buf, sizeof buf, "%s: %s, smem=%zuB, cubin=%zuB, %.0f ms%s, symbol %s", spec.name().c_str(), spec.expression().c_str(), spec.smem(),
-           cubin.size(), ms, from_disk ? " (disk cache)" : "", lowered.c_str());
-  *report = buf;
+  return probe_compile(spec, report);
+}
+
+// The same for the two passes the planner builds for a long axis (make_jit_split_pass): "<pass A report>; <pass B report>"
+int jit_split_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bool inverse, bool real_in, int half,
+                    int in_dtype, int out_dtype, std::string* report) {
+  AxisView view;
+  view.n = n;
+  view.inner = inner;
+  IoSpec src;
+  src.comps = real_in ? 1 : 2;
+  src.dtype = in_dtype;
+  JitSplitChoice c;
+  if (!jit_split_plan(ordered, view, src, inverse, (HalfMode)half, out_dtype == B200FFT_F64, &c))
+    return fail(B200FFT_ERR_UNSUPPORTED, "no two-pass split of this axis (a radix above %d, more than 2^24 points, or no tile fits)",
+                JIT_MAX_PRIME);
+  std::string ra, rb;
+  int rc = probe_compile(c.sa, &ra);
+  if (rc == B200FFT_OK) rc = probe_compile(c.sb, &rb);
+  if (rc != B200FFT_OK) return rc;
+  *report = ra + "; " + rb;
   return B200FFT_OK;
 }
 

@@ -133,6 +133,9 @@ std::unique_ptr<Pass> make_jit_pass(b200fft_plan& plan, int axis, const AxisView
                                     HalfMode half);
 int jit_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bool inverse, bool real_in, int half,
               int in_dtype, int out_dtype, std::string* report);
+// the two passes the plan-time tier builds for an axis too long for one tile (same arguments)
+int jit_split_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bool inverse, bool real_in, int half,
+                    int in_dtype, int out_dtype, std::string* report);
 // number of registered kernel variants per tier (host-only; triggers the one-time registration)
 size_t fast_variant_count();
 size_t fused_variant_count();

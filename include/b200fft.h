@@ -251,6 +251,12 @@ B200FFT_API int b200fft_plan_dry_run(const b200fft_desc* desc, char* buf, size_t
 B200FFT_API int b200fft_jit_probe(int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in,
                                   int half /* 0 complex, 1 half-spectrum R2C rows, 2 C2R rows */, int in_dtype, int out_dtype,
                                   char* buf, size_t cap);
+/* The same for an axis too long for one tile: compiles the two passes (pass A: N1-point strided transforms with the
+ * twiddle fused into the store; pass B: N2-point rows with the natural-order, half-spectrum or real store) the
+ * planner builds for it, and writes "<pass A report>; <pass B report>". Serves complex, real-input and half-spectrum
+ * (R2C / C2R, even and odd n) axes; B200FFT_ERR_UNSUPPORTED when the stage list has no such split. No GPU needed. */
+B200FFT_API int b200fft_jit_split_probe(int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in,
+                                        int half, int in_dtype, int out_dtype, char* buf, size_t cap);
 
 /* Tile schedule of the fused N-d kernel (host logic, no CUDA): phases[p] = {tiles_per_transform,
  * tiles_per_group, dep_div, quota}; writes up to `cap` segments as {phase, first_item, first_tile, count}

@@ -229,56 +229,6 @@ int build_passes(b200fft_plan* plan, bool dry, std::string* text) {
   return add(last, rows, any ? work_spec : in_spec, HALF_C2R, any ? BUF_WORK : BUF_INPUT, BUF_OUTPUT);
 }
 
-// ---- L2-resident pass groups -------------------------------------------------------------------------------------
-// Every per-axis pass streams its whole operand: k axes = k HBM round trips. The innermost axes a..k-1 are independent
-// across the outer index o in [0, batch * prod(dims[:a])), so their passes can run chunk by chunk — pass(axis k-1) on
-// chunk c, pass(axis k-2) on chunk c, ... — with a chunk sized to stay in the 126 MB L2 between passes: the group then
-// costs ONE read of the input and ONE write of the output in HBM, whatever the number of axes in it (2-D images:
-// 2 passes -> 1; 512^3: x and y per z-plane chunk -> 2 passes instead of 3). The outer axes (< a) run as whole-array
-// passes afterwards. The grouped passes were built with views whose outer extent is counted per group unit, so the
-// same Pass::launch serves a chunk (nbatch = units in the chunk) and the whole range.
-//   B200FFT_PASS_CHUNK_MB=<n>  chunk budget in MB of output; unset or 0 = no grouping (the default)
-// MEASURED (profiles/r2_chunk_sweep.jsonl): on B200 this loses at every chunk size — 100 x 640 x 480: 0.174 ms as two
-// whole-array passes, 0.194 ms in 64 MB chunks (8 launches), 0.267 ms in 24 MB chunks (20 launches); 512^3: 1.03 ms vs
-// 1.18 / 1.39 ms. Each extra launch costs 4-5 us of ramp and tail, and a pass over L2-resident data is hardly faster
-// than one over HBM-resident data (~8 vs ~6.5 TB/s read+write, tools/micro/warp_cols.cu). Kept as an opt-in knob.
-void plan_pass_group(b200fft_plan* plan) {
-  const Problem& p = plan->prob;
-  plan->group_passes = 0;
-  plan->group_mult = 1;
-  if (plan->passes.size() < 2 || plan->workspace) return;
-  for (auto& ax : p.axes)
-    if (!ax.transformed) return;
-  long long budget_mb = 0;
-  if (const char* e = getenv("B200FFT_PASS_CHUNK_MB")) budget_mb = atoll(e);
-  if (budget_mb <= 0) return;
-  const size_t budget = (size_t)budget_mb << 20;
-  const int last = p.rank - 1;
-  // complex extents of the output array (half spectrum: n/2+1 bins on the last axis)
-  std::vector<int64_t> cd;
-  for (auto& ax : p.axes) cd.push_back(ax.n);
-  if (p.half) cd[last] = cd[last] / 2 + 1;
-  const size_t out_total = (size_t)p.batch * p.out_scalars_per_batch * p.out_elem;
-  if (out_total <= 2 * budget) return;  // the whole array already lives in L2 between passes
-  // passes run right to left: passes[i] transforms axis last - i. Smallest a whose unit fits the budget twice over.
-  for (int a = 0; a + 1 <= last; ++a) {
-    size_t unit_out = 2 * p.out_elem;
-    for (int i = a; i <= last; ++i) unit_out *= (size_t)cd[i];
-    if (unit_out * 2 > budget) continue;
-    int64_t mult = 1;
-    for (int i = 0; i < a; ++i) mult *= p.axes[i].n;
-    size_t unit_in = (size_t)p.desc.in_components * p.in_elem;
-    for (int i = a; i <= last; ++i) unit_in *= (size_t)p.axes[i].n;
-    if (p.half && p.desc.inverse) return;
-    plan->group_passes = last - a + 1;
-    plan->group_mult = mult;
-    plan->group_in_stride = unit_in;
-    plan->group_out_stride = unit_out;
-    plan->group_chunk_units = std::max<int64_t>(1, (int64_t)(budget / unit_out));
-    return;
-  }
-}
-
 int copy_bases(const std::vector<uint32_t>& v, uint32_t* out, int cap) {
   if (!out || (int)v.size() > cap) return -1;
   for (size_t i = 0; i < v.size(); ++i) out[i] = v[i];
@@ -434,21 +384,6 @@ int b200fft_plan_create(b200fft_plan** out, const b200fft_desc* desc) {
   }
   rc = build_passes(plan.get(), /*dry=*/false, nullptr);
   if (rc != B200FFT_OK) { b200fft_plan_destroy(plan.release()); return rc; }
-  plan_pass_group(plan.get());
-  for (int i = 0; i < plan->group_passes; ++i)
-    if (!plan->passes[(size_t)i]->supports_units()) plan->group_passes = 0;  // a pass kind without unit launches: no grouping
-  if (plan->group_passes >= 2) {
-    const char* e = getenv("B200FFT_PASS_PIPELINE");  // 0 = run the group's chunks serially on the caller's stream
-    plan->group_pipeline = !(e && atoi(e) == 0);
-    if (plan->group_pipeline) {
-      bool ok = cudaStreamCreateWithFlags(&plan->group_stream, cudaStreamNonBlocking) == cudaSuccess;
-      for (auto& ev : plan->group_ev) ok = ok && cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) == cudaSuccess;
-      if (!ok) {
-        cudaGetLastError();
-        plan->group_pipeline = false;
-      }
-    }
-  }
   // The tables were uploaded with cudaMemcpy from pageable memory on the legacy stream: make sure they have landed
   // before the caller launches on a non-blocking stream of its own (which is not ordered after the legacy stream).
   if (cudaError_t e = cudaDeviceSynchronize(); e != cudaSuccess) {
@@ -475,9 +410,6 @@ int b200fft_plan_destroy(b200fft_plan* plan) {
     if (plan->hs[i]) cudaStreamDestroy(plan->hs[i]);
   for (auto& e : plan->h_ev)
     if (e) cudaEventDestroy(e);
-  for (auto& e : plan->group_ev)
-    if (e) cudaEventDestroy(e);
-  if (plan->group_stream) cudaStreamDestroy(plan->group_stream);
   delete plan;
   return B200FFT_OK;
 }
@@ -486,50 +418,7 @@ int b200fft_plan_destroy(b200fft_plan* plan) {
 static int run_passes(b200fft_plan* plan, void* d_out, const void* d_in, int64_t nbatch, cudaStream_t st,
                       int64_t work_batch0 = 0) {
   char* work = (char*)plan->workspace + (size_t)work_batch0 * plan->work_stride;
-  size_t first = 0;
-  if (plan->group_passes >= 2) {
-    // the L2-resident group (see plan_pass_group): all its passes per chunk of units, input -> output then in place
-    first = (size_t)plan->group_passes;
-    const int64_t units = nbatch * plan->group_mult;
-    auto launch_chunk = [&](size_t i, int64_t u0, cudaStream_t s) -> int {
-      const int64_t nu = std::min<int64_t>(plan->group_chunk_units, units - u0);
-      char* out_c = (char*)d_out + (size_t)u0 * plan->group_out_stride;
-      const char* in_c = (const char*)d_in + (size_t)u0 * plan->group_in_stride;
-      Pass& pass = *plan->passes[i];
-      return pass.launch_units(pass.src_sel == BUF_INPUT ? (const void*)in_c : (const void*)out_c, out_c, nu, plan->group_mult, s);
-    };
-    if (plan->group_pipeline && plan->group_stream) {
-      // Two streams: pass 0 of chunk k on the caller's stream, passes 1.. of chunk k on the side stream as soon as it is
-      // done, while pass 0 of chunk k+1 already runs: the kernels' ramps and tails overlap, and pass 0 may run at most
-      // two chunks ahead so that what sits between the streams stays L2-resident.
-      cudaStream_t s2 = plan->group_stream;
-      cudaEvent_t ev_fork = plan->group_ev[0], ev_first = plan->group_ev[1];
-      cudaEvent_t* ev_tail = &plan->group_ev[2];
-      B200_CUDA_CHECK(cudaEventRecord(ev_fork, st));
-      B200_CUDA_CHECK(cudaStreamWaitEvent(s2, ev_fork, 0));
-      int64_t k = 0;
-      for (int64_t u0 = 0; u0 < units; u0 += plan->group_chunk_units, ++k) {
-        if (k >= 2) B200_CUDA_CHECK(cudaStreamWaitEvent(st, ev_tail[k & 1], 0));
-        int rc = launch_chunk(0, u0, st);
-        if (rc != B200FFT_OK) return rc;
-        B200_CUDA_CHECK(cudaEventRecord(ev_first, st));
-        B200_CUDA_CHECK(cudaStreamWaitEvent(s2, ev_first, 0));
-        for (size_t i = 1; i < first; ++i)
-          if ((rc = launch_chunk(i, u0, s2)) != B200FFT_OK) return rc;
-        B200_CUDA_CHECK(cudaEventRecord(ev_tail[k & 1], s2));
-      }
-      B200_CUDA_CHECK(cudaStreamWaitEvent(st, ev_tail[(k - 1) & 1], 0));  // join: everything after this sees the group's result
-      if (k >= 2) B200_CUDA_CHECK(cudaStreamWaitEvent(st, ev_tail[k & 1], 0));
-    } else {
-      for (int64_t u0 = 0; u0 < units; u0 += plan->group_chunk_units)
-        for (size_t i = 0; i < first; ++i) {
-          int rc = launch_chunk(i, u0, st);
-          if (rc != B200FFT_OK) return rc;
-        }
-    }
-  }
-  for (size_t i = first; i < plan->passes.size(); ++i) {
-    auto& pass = plan->passes[i];
+  for (auto& pass : plan->passes) {
     const void* src = pass->src_sel == BUF_INPUT ? d_in : pass->src_sel == BUF_WORK ? (const void*)work : (const void*)d_out;
     void* dst = pass->dst_sel == BUF_WORK ? (void*)work : d_out;
     int rc = pass->launch(src, dst, nbatch, st);
@@ -697,13 +586,6 @@ size_t b200fft_plan_describe(const b200fft_plan* plan, char* buf, size_t cap) {
   if (!plan) return 0;
   std::string text;
   for (auto& pass : plan->passes) text += pass->describe() + "\n";
-  if (plan->group_passes >= 2) {
-    char buf[200];
-    snprintf(buf, sizeof buf, "L2-resident group: the first %d passes run per chunk of %lld units (%zu KB out each) of %lld\n",
-             plan->group_passes, (long long)plan->group_chunk_units, plan->group_out_stride >> 10,
-             (long long)(plan->prob.batch * plan->group_mult));
-    text += buf;
-  }
   if (buf && cap) {
     strncpy(buf, text.c_str(), cap - 1);
     buf[cap - 1] = 0;
@@ -714,14 +596,7 @@ size_t b200fft_plan_describe(const b200fft_plan* plan, char* buf, size_t cap) {
 int b200fft_plan_launches(const b200fft_plan* plan) {
   if (!plan) return 0;
   int n = 0;
-  for (size_t i = 0; i < plan->passes.size(); ++i) {
-    int reps = 1;
-    if ((int)i < plan->group_passes) {
-      const int64_t units = plan->prob.batch * plan->group_mult;
-      reps = (int)((units + plan->group_chunk_units - 1) / plan->group_chunk_units);
-    }
-    n += plan->passes[i]->launches() * reps;
-  }
+  for (auto& pass : plan->passes) n += pass->launches();
   return n;
 }
 

@@ -56,7 +56,6 @@ struct NdArgs {
   unsigned* err;                  // mapped HOST word: set to 1 when a dependency wait gave up (checked by the next exec)
   int cnt_off[ND_MAX_PHASES];     // offset of each phase's counters inside ctrl
   int nwords;                     // words to clear at the end (header + counters)
-  int prefetch_ahead;             // v2: L2-prefetch the input of the phase-0 tile this many of the CTA's own items ahead (0 = off)
 };
 
 __device__ __forceinline__ unsigned ld_acquire_gpu(const unsigned* p) {

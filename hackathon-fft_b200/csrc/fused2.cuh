@@ -37,10 +37,6 @@ __device__ __forceinline__ void load_1d(void* smem_dst, const void* gsrc, uint32
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
-// bring [gsrc, gsrc + bytes) into L2 ahead of the copy that will stage it (no shared memory, no completion to wait for)
-__device__ __forceinline__ void prefetch_l2(const void* gsrc, uint32_t bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(gsrc), "r"(bytes) : "memory");
-}
 // order earlier generic-proxy accesses (the acquire that observed other SMs' st.global) before later
 // async-proxy reads of global memory (the bulk copies)
 __device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async;" ::: "memory"); }
@@ -67,7 +63,6 @@ struct ANone {
   static constexpr int tw_elems = 0, tw2_elems = 0;
   static __device__ __forceinline__ void load(const NdPhase&, const CUtensorMap*, const void*, long long, int, void*,
                                               uint64_t*) {}
-  static __device__ __forceinline__ void prefetch(const NdPhase&, const void*, int) {}
   template <int NT, class Rel>
   static __device__ __forceinline__ void run(const NdPhase&, const float2*, const float2*, const void*, float2*, int,
                                              float2*, Rel) {}
@@ -90,11 +85,6 @@ struct ARows {
     const uint32_t bytes = (uint32_t)valid * N * ELEM;
     tma::mbar_arrive_expect_tx(full, bytes);
     tma::load_1d(in_buf, reinterpret_cast<const char*>(src_t) + row0 * N * ELEM, bytes, full);
-  }
-  static __device__ __forceinline__ void prefetch(const NdPhase& p, const void* src_t, int tile) {
-    const long long row0 = (long long)tile * C;
-    const int valid = (int)min((long long)C, p.units_per_transform - row0);
-    tma::prefetch_l2(reinterpret_cast<const char*>(src_t) + row0 * N * ELEM, (uint32_t)valid * N * ELEM);
   }
   template <int NT, class Rel>
   static __device__ __forceinline__ void run(const NdPhase& p, const float2* tw, const float2*, const void* in_buf,
@@ -140,7 +130,6 @@ struct ACols {
     for (int b = 0; b < N / BR; ++b)
       tma::load_3d(reinterpret_cast<float2*>(in_buf) + b * BR * CW, map, c0, b * BR, outer, full);
   }
-  static __device__ __forceinline__ void prefetch(const NdPhase&, const void*, int) {}  // reads the L2-resident intermediate
   template <int NT, class Rel>
   static __device__ __forceinline__ void run(const NdPhase& p, const float2* tw, const float2*, const void* in_buf,
                                              float2* dst_t, int tile, float2* ex, Rel release) {
@@ -183,11 +172,6 @@ struct AR2C {
     tma::mbar_arrive_expect_tx(full, bytes);
     tma::load_1d(in_buf, reinterpret_cast<const char*>(src_t) + row0 * H * 8, bytes, full);
   }
-  static __device__ __forceinline__ void prefetch(const NdPhase& p, const void* src_t, int tile) {
-    const long long row0 = (long long)tile * C;
-    const int valid = (int)min((long long)C, p.units_per_transform - row0);
-    tma::prefetch_l2(reinterpret_cast<const char*>(src_t) + row0 * H * 8, (uint32_t)valid * H * 8);
-  }
   template <int NT, class Rel>
   static __device__ __forceinline__ void run(const NdPhase& p, const float2* tw, const float2*, const void* in_buf,
                                              float2* dst_t, int tile, float2* ex, Rel release) {
@@ -217,9 +201,6 @@ struct APlane {
                                               void* in_buf, uint64_t* full) {
     tma::mbar_arrive_expect_tx(full, (uint32_t)in_bytes);
     tma::load_1d(in_buf, reinterpret_cast<const float2*>(src_t) + (long long)tile * NY * NX, (uint32_t)in_bytes, full);
-  }
-  static __device__ __forceinline__ void prefetch(const NdPhase&, const void* src_t, int tile) {
-    tma::prefetch_l2(reinterpret_cast<const float2*>(src_t) + (long long)tile * NY * NX, (uint32_t)in_bytes);
   }
   template <int NT, class Rel>
   static __device__ __forceinline__ void run(const NdPhase& p, const float2* tw, const float2* tw2, const void* in_buf,
@@ -289,9 +270,6 @@ struct AR2CPlane {
                                               void* in_buf, uint64_t* full) {
     tma::mbar_arrive_expect_tx(full, (uint32_t)in_bytes);
     tma::load_1d(in_buf, reinterpret_cast<const float2*>(src_t) + (long long)tile * NY * H, (uint32_t)in_bytes, full);
-  }
-  static __device__ __forceinline__ void prefetch(const NdPhase&, const void* src_t, int tile) {
-    tma::prefetch_l2(reinterpret_cast<const float2*>(src_t) + (long long)tile * NY * H, (uint32_t)in_bytes);
   }
   template <int NT, class Rel>
   static __device__ __forceinline__ void run(const NdPhase& p, const float2* tw, const float2* tw2, const void* in_buf,
@@ -486,22 +464,6 @@ __global__ void __launch_bounds__(NT + 32, MINB)
         else if constexpr (!P2::none) nd_issue<2, P2>(a, &map2, r, in_buf, &full[slot], &ring[slot]);
         item += gridDim.x;
         resolve(item, &rn);  // look one tile ahead
-        // ... and pull the input of the phase-0 tile `a.prefetch_ahead` items further on from HBM into L2 now: the copy
-        // that stages it then finds it in L2, so fewer bytes have to be in flight per SM to cover the HBM latency
-        if (a.prefetch_ahead > 0) {
-          const unsigned pit = item + (unsigned)(a.prefetch_ahead - 1) * gridDim.x;
-          if (pit < a.total_items) {
-            NdLocate pl{loc.seg};
-            int pphase;
-            long long pg;
-            pl.find(a, pit, &pphase, &pg);
-            if (pphase == 0) {
-              const long long pt = pg / a.ph[0].tiles_per_transform;
-              P0::prefetch(a.ph[0], reinterpret_cast<const char*>(a.in) + pt * a.in_stride_bytes,
-                           (int)(pg - pt * a.ph[0].tiles_per_transform));
-            }
-          }
-        }
       }
     }
     return;

@@ -105,7 +105,6 @@ struct FusedPass : Pass {
     return B200FFT_OK;
   }
 
-  int prefetch_ahead = 0;     // (measured: no gain at 1-2, loses from 4 on; profiles/r2_prefetch_sweep.log) B200FFT_PREFETCH_AHEAD: L2 prefetch distance of the v2 producer, in items of its own CTA
   unsigned* h_err = nullptr;  // mapped host word the kernels raise when a dependency wait gives up
   unsigned* d_err = nullptr;
   bool use_fallback = false;  // a cooperative launch was refused once: stay on the per-axis kernels
@@ -141,7 +140,6 @@ struct FusedPass : Pass {
     a.total_items = pb->total_items;
     a.ctrl = pb->d_ctrl;
     a.err = d_err;
-    a.prefetch_ahead = prefetch_ahead;
     for (int p = 0; p < ND_MAX_PHASES; ++p) a.cnt_off[p] = pb->cnt_off[p];
     a.nwords = pb->nwords;
     const unsigned grid = (unsigned)std::min<long long>(pb->total_items, max_grid);
@@ -381,7 +379,6 @@ std::unique_ptr<Pass> make_fused_pass(b200fft_plan& plan) {
     return nullptr;
   }
   pass->max_grid = occ * plan.sm_count;
-  if (const char* e = getenv("B200FFT_PREFETCH_AHEAD")) pass->prefetch_ahead = std::max(0, atoi(e));
   if (v.async) {
     int coop = 0;
     if (cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, plan.device) != cudaSuccess || !coop) {

@@ -44,12 +44,6 @@ struct Slot {
   b200fft_plan* planz = nullptr; // SLAB: Z pass over the received [Z][Y/G][X] slab
   cudaStream_t stream = nullptr;
   cudaEvent_t scattered = nullptr, done = nullptr;
-  // SLAB with chunks > 1: the slot's planes in `chunks` pieces; X pass of piece c+1 (stream) overlaps the NVLink-bound
-  // scattering Y pass of piece c (stream2)
-  b200fft_plan* planx = nullptr;  // X rows of one piece (axis 1 only)
-  b200fft_plan* plany = nullptr;  // Y pass of one piece (axis 0 only): its single pass is the scattering one
-  cudaStream_t stream2 = nullptr;
-  std::vector<cudaEvent_t> xdone;
   void* work = nullptr;          // SLAB: [Z/G][Y][X] intermediate of step 1
   void* h_in = nullptr;          // SLAB exec_host: device staging, allocated on first use
   void* h_out = nullptr;
@@ -81,7 +75,6 @@ struct b200fft_mgpu_plan {
   int64_t Z = 0, Y = 0, X = 0;
   size_t in_item = 0, out_item = 0;  // BATCH_SHARD: bytes per batch item
   bool executed = false;             // SLAB: `done` events have been recorded at least once
-  int chunks = 1;                    // SLAB: pieces per slot (B200FFT_MGPU_SLAB_CHUNKS)
   std::vector<Slot> slots;
   std::string text;
 };
@@ -155,17 +148,11 @@ int b200fft_mgpu_plan_destroy(b200fft_mgpu_plan* m) {
   for (Slot& s : m->slots) {
     cudaSetDevice(s.device);
     if (s.stream) cudaStreamSynchronize(s.stream);
-    if (s.stream2) cudaStreamSynchronize(s.stream2);
   }
   for (Slot& s : m->slots) {
     cudaSetDevice(s.device);
     if (s.plan) b200fft_plan_destroy(s.plan);
     if (s.planz) b200fft_plan_destroy(s.planz);
-    if (s.planx) b200fft_plan_destroy(s.planx);
-    if (s.plany) b200fft_plan_destroy(s.plany);
-    for (cudaEvent_t e : s.xdone)
-      if (e) cudaEventDestroy(e);
-    if (s.stream2) cudaStreamDestroy(s.stream2);
     for (void* p : {s.work, s.h_in, s.h_out})
       if (p) cudaFree(p);
     if (s.scattered) cudaEventDestroy(s.scattered);
@@ -237,12 +224,6 @@ int b200fft_mgpu_plan_create(b200fft_mgpu_plan** out, const b200fft_desc* desc, 
     const int64_t zl = m->Z / ngpu, yl = m->Y / ngpu;
     if (yl < 2 && ngpu > 1) return bail(fail(B200FFT_ERR_INVALID_ARG, "fewer than 2 y rows per device"));
     if (int rc = enable_peers(m->slots)) return bail(rc);
-    // Pieces per slot: measured on 8 B200 (profiles/r2_slab.md). The Y pass is bound by its NVLink stores, so the SMs have
-    // room for the next piece's X pass while it runs.
-    int chunks = 1;
-    if (const char* e = getenv("B200FFT_MGPU_SLAB_CHUNKS")) chunks = std::max(1, atoi(e));
-    while (chunks > 1 && zl % chunks) --chunks;
-    m->chunks = chunks;
     std::vector<uint32_t> b_yx, b_z;
     std::vector<int32_t> c_yx, c_z;
     slice_bases(*desc, 1, 3, &b_yx, &c_yx);
@@ -276,14 +257,6 @@ int b200fft_mgpu_plan_create(b200fft_mgpu_plan** out, const b200fft_desc* desc, 
       dz.bases = cz3.empty() ? nullptr : b_z.data();
       dz.bases_count = cz3.empty() ? nullptr : cz3.data();
       if (int rc = b200fft_plan_create(&s.planz, &dz)) return bail(rc);
-      if (m->chunks > 1) {
-        b200fft_desc dx = d2, dy = d2;
-        dx.batch = dy.batch = zl / m->chunks;
-        dx.axis_mask = 2;  // axis 1 = X
-        dy.axis_mask = 1;  // axis 0 = Y
-        if (int rc = b200fft_plan_create(&s.planx, &dx)) return bail(rc);
-        if (int rc = b200fft_plan_create(&s.plany, &dy)) return bail(rc);
-      }
       if (cudaSetDevice(s.device) != cudaSuccess || cudaMalloc(&s.work, s.in_bytes) != cudaSuccess) {
         cudaGetLastError();
         return bail(fail(B200FFT_ERR_ALLOC, "cannot allocate %zu B of slab workspace on device %d", s.in_bytes, s.device));
@@ -293,30 +266,18 @@ int b200fft_mgpu_plan_create(b200fft_mgpu_plan** out, const b200fft_desc* desc, 
   for (Slot& s : m->slots) {
     if (cudaSetDevice(s.device) != cudaSuccess || cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking) != cudaSuccess ||
         cudaEventCreateWithFlags(&s.scattered, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming) != cudaSuccess ||
-        (m->chunks > 1 && cudaStreamCreateWithFlags(&s.stream2, cudaStreamNonBlocking) != cudaSuccess)) {
+        cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming) != cudaSuccess) {
       cudaError_t e = cudaGetLastError();
       return bail(fail(B200FFT_ERR_CUDA, "stream / event creation on device %d: %s", s.device, cudaGetErrorString(e)));
     }
   }
-  if (m->chunks > 1)
-    for (Slot& s : m->slots) {
-      cudaSetDevice(s.device);
-      s.xdone.assign((size_t)m->chunks, nullptr);
-      for (auto& e : s.xdone)
-        if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) {
-          cudaGetLastError();
-          return bail(fail(B200FFT_ERR_CUDA, "event creation on device %d", s.device));
-        }
-    }
   char head[320];
   if (mode == B200FFT_MGPU_BATCH_SHARD)
     snprintf(head, sizeof head, "mgpu batch-shard over %d devices, batch %lld, no communication\n", ngpu, (long long)m->batch);
   else
     snprintf(head, sizeof head,
-             "mgpu slab %lldx%lldx%lld over %d devices: local (Y,X) + peer-to-peer scattering Y stores -> event barrier -> Z pass%s\n",
-             (long long)m->Z, (long long)m->Y, (long long)m->X, ngpu,
-             m->chunks > 1 ? (" [" + std::to_string(m->chunks) + " pieces per device: X of piece c+1 overlaps the scattering Y pass of piece c]").c_str() : "");
+             "mgpu slab %lldx%lldx%lld over %d devices: local (Y,X) + peer-to-peer scattering Y stores -> event barrier -> Z pass\n",
+             (long long)m->Z, (long long)m->Y, (long long)m->X, ngpu);
   m->text = head;
   for (int g = 0; g < ngpu; ++g) {
     const Slot& s = m->slots[(size_t)g];
@@ -385,28 +346,13 @@ static int slot_enqueue(b200fft_mgpu_plan* m, int g, int phase, void* const* d_o
     if (m->executed)
       for (int h = 0; h < G; ++h)
         if (h != g) B200_CUDA_CHECK(cudaStreamWaitEvent(s.stream, m->slots[(size_t)h].done, 0));
-    if (m->chunks <= 1) {
-      if (int rc = b200fft_exec_scatter(s.plan, d_out, G, g, d_in[g], s.work, s.stream)) return rc;
-      B200_CUDA_CHECK(cudaSetDevice(s.device));
-      B200_CUDA_CHECK(cudaEventRecord(s.scattered, s.stream));
-    } else {
-      const int64_t zc = s.count / m->chunks;
-      const size_t piece = (size_t)zc * (size_t)m->Y * (size_t)m->X * 8;
-      for (int c = 0; c < m->chunks; ++c) {
-        char* work_c = (char*)s.work + (size_t)c * piece;
-        if (int rc = b200fft_exec(s.planx, work_c, (const char*)d_in[g] + (size_t)c * piece, s.stream)) return rc;
-        B200_CUDA_CHECK(cudaSetDevice(s.device));
-        B200_CUDA_CHECK(cudaEventRecord(s.xdone[(size_t)c], s.stream));
-        B200_CUDA_CHECK(cudaStreamWaitEvent(s.stream2, s.xdone[(size_t)c], 0));
-        if (int rc = b200fft_exec_scatter_at(s.plany, d_out, G, s.first + c * zc, work_c, work_c, s.stream2)) return rc;
-        B200_CUDA_CHECK(cudaSetDevice(s.device));
-      }
-      B200_CUDA_CHECK(cudaEventRecord(s.scattered, s.stream2));
-    }
+    if (int rc = b200fft_exec_scatter(s.plan, d_out, G, g, d_in[g], s.work, s.stream)) return rc;
+    B200_CUDA_CHECK(cudaSetDevice(s.device));
+    B200_CUDA_CHECK(cudaEventRecord(s.scattered, s.stream));
     return B200FFT_OK;
   }
   for (int h = 0; h < G; ++h)
-    if (h != g || m->chunks > 1) B200_CUDA_CHECK(cudaStreamWaitEvent(s.stream, m->slots[(size_t)h].scattered, 0));
+    if (h != g) B200_CUDA_CHECK(cudaStreamWaitEvent(s.stream, m->slots[(size_t)h].scattered, 0));
   if (int rc = b200fft_exec(s.planz, d_out[g], d_out[g], s.stream)) return rc;
   B200_CUDA_CHECK(cudaSetDevice(s.device));
   B200_CUDA_CHECK(cudaEventRecord(s.done, s.stream));

@@ -46,12 +46,6 @@ struct Pass {
   virtual int launch(const void* src, void* dst, int64_t nbatch, cudaStream_t stream) = 0;
   virtual std::string describe() const = 0;
   virtual int launches() const { return 1; }
-  // The same pass over `nunits` consecutive group units, a unit being 1 / units_per_batch of a batch item along the
-  // outermost dimensions (L2-resident pass groups, api.cu: plan_pass_group). src/dst point at the first unit.
-  virtual bool supports_units() const { return false; }
-  virtual int launch_units(const void*, void*, int64_t, int64_t, cudaStream_t) {
-    return fail(B200FFT_ERR_UNSUPPORTED, "this pass cannot run on a sub-range of a batch item (%s)", describe().c_str());
-  }
   // Same pass, but output row i of the transformed axis goes to sc.peer_out[i / rows_per_peer]
   // (slab exchange fused into the store). Only strided fast passes implement it.
   virtual int launch_scatter(const void*, const Scatter&, int64_t, cudaStream_t) {
@@ -82,16 +76,6 @@ struct b200fft_plan {
   std::vector<std::unique_ptr<b200fft::Pass>> passes;
   std::vector<void*> owned_device;          // misc device allocations freed at destroy
   bool building_fallback = false;           // build_passes is collecting the per-axis passes behind a fused pass
-  // L2-resident pass group (api.cu: plan_pass_group): passes[0 .. group_passes) run chunk by chunk
-  int group_passes = 0;
-  int64_t group_mult = 1;         // group units per batch item = prod(dims outside the group)
-  int64_t group_chunk_units = 0;
-  size_t group_in_stride = 0, group_out_stride = 0;  // bytes per unit
-  // pipelined group execution (api.cu: run_passes): the group's first pass runs on the caller's stream, the others on
-  // this side stream one chunk behind, so the two kernels overlap and the chunk between them never leaves L2
-  cudaStream_t group_stream = nullptr;
-  cudaEvent_t group_ev[4] = {};  // fork, first-pass-done, tail[2]
-  bool group_pipeline = false;
   void* workspace = nullptr;
   size_t workspace_bytes = 0;
   size_t work_stride = 0;     // workspace bytes per batch item

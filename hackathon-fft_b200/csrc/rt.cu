@@ -66,12 +66,6 @@ struct RtPass : Pass {
   int launch(const void* src, void* dst, int64_t nbatch, cudaStream_t stream) override {
     return launch_outer(src, dst, nbatch * view.outer_per_batch, stream);
   }
-  bool supports_units() const override { return true; }
-  int launch_units(const void* src, void* dst, int64_t nunits, int64_t units_per_batch, cudaStream_t stream) override {
-    if (units_per_batch < 1 || view.outer_per_batch % units_per_batch)
-      return fail(B200FFT_ERR_INVALID_ARG, "%s: outer slabs do not split into %lld units", text.c_str(), (long long)units_per_batch);
-    return launch_outer(src, dst, nunits * (view.outer_per_batch / units_per_batch), stream);
-  }
   int launch_outer(const void* src, void* dst, long long outer, cudaStream_t stream) {
     RtArgs a = base;
     a.in = src;

@@ -150,7 +150,7 @@ B200FFT_API int b200fft_exec_scatter(b200fft_plan* plan, void* const* peer_out, 
 
 /* The same for a SUB-RANGE of a rank's planes: the plan's `batch` planes are planes [z_first, z_first + batch) of the
  * global volume (exec_scatter is the case z_first = my_rank * batch). Lets a caller cut its slab into chunks and overlap
- * the X pass of one chunk with the NVLink-bound scattering Y pass of the previous one (b200fft_mgpu_* does). */
+ * the X pass of one chunk with the NVLink-bound scattering Y pass of the previous one. */
 B200FFT_API int b200fft_exec_scatter_at(b200fft_plan* plan, void* const* peer_out, int npeers, int64_t z_first,
                                         const void* d_in, void* d_work, void* cu_stream);
 

@@ -96,39 +96,6 @@ def test_slab_device_and_host(dims, ngpu, inverse, monkeypatch):
     plan.destroy()
 
 
-@pytest.mark.parametrize("dims,ngpu,chunks", [((64, 64, 64), 2, 4), ((128, 128, 64), 4, 2), ((64, 128, 256), 8, 8), ((96, 64, 64), 1, 3)])
-def test_slab_in_pieces(dims, ngpu, chunks, monkeypatch):
-    """B200FFT_MGPU_SLAB_CHUNKS: every slot's planes in pieces, X pass of piece c+1 on one stream overlapping the scattering
-    Y pass of piece c on another (b200fft_exec_scatter_at). Same result as the one-piece plan, bit for bit."""
-    import torch
-    devs, real = _devices(ngpu)
-    if not real:
-        monkeypatch.setenv("B200FFT_MGPU_ALLOW_SAME_DEVICE", "1")
-    Z, Y, X = dims
-    zl, yl = Z // ngpu, Y // ngpu
-    layout = (1, Z, Y, X, 2)
-    rng = np.random.default_rng(13)
-    x = rng.standard_normal((Z, Y, X, 2)).astype(np.float32)
-    res = []
-    for k in (1, chunks):
-        monkeypatch.setenv("B200FFT_MGPU_SLAB_CHUNKS", str(k))
-        plan = b200fft.MgpuPlan("float32", "float32", layout, layout, devices=devs, mode=b200fft.MGPU_SLAB)
-        assert ("pieces per device" in plan.describe()) == (k > 1), plan.describe()
-        ins = [torch.from_numpy(x[g * zl:(g + 1) * zl]).to(torch.device("cuda", devs[g])) for g in range(ngpu)]
-        outs = [torch.full((Z, yl, X, 2), float("nan"), device=torch.device("cuda", devs[g])) for g in range(ngpu)]
-        torch.cuda.synchronize()
-        for _ in range(3):
-            plan.exec(outs, ins)
-        plan.synchronize()
-        res.append([o.cpu() for o in outs])
-        plan.destroy()
-    want = np.fft.fftn(x[..., 0].astype(np.float64) + 1j * x[..., 1])
-    for h in range(ngpu):
-        assert torch.equal(res[0][h], res[1][h])
-        got = res[1][h].numpy().astype(np.float64)
-        assert _rel(got[..., 0] + 1j * got[..., 1], want[:, h * yl:(h + 1) * yl, :]) < TOL
-
-
 def test_mgpu_user_bases_reach_every_axis():
     devs, real = _devices(2)
     if not real:

@@ -1,6 +1,8 @@
 """Slab decomposition on ONE GPU: G virtual ranks emulated in one process (their slabs all live on
 cuda:0), exercising b200fft_exec_scatter's peer indexing for G > 1 and the Z pass, against numpy.
 The real multi-process / multi-GPU run is tools/slab_check.py (torchrun, NCCL + CUDA IPC)."""
+import ctypes
+
 import numpy as np
 import pytest
 
@@ -37,6 +39,51 @@ def test_exec_scatter_virtual_ranks(dims, G):
         ref = want[:, r * yl:(r + 1) * yl, :]
         assert torch.isfinite(recv[r]).all()
         assert float((got - ref).norm() / ref.norm()) < 2e-6
+
+
+def _scatter_at(plan, recv, z_first, x, work, st):
+    arr = (ctypes.c_void_p * len(recv))(*[t.data_ptr() for t in recv])
+    return b200fft.lib().b200fft_exec_scatter_at(plan._h, arr, len(recv), z_first, x.data_ptr(), work.data_ptr(), st)
+
+
+@pytest.mark.parametrize("dims,G,pieces", [((64, 64, 64), 2, 4), ((128, 128, 64), 4, 2), ((64, 128, 256), 8, 8),
+                                           ((96, 64, 64), 1, 3)])
+@pytest.mark.parametrize("axis_mask", [0, 1])  # 1: only the split axis Y, a one-pass plan that scatters from its input
+def test_exec_scatter_at_virtual_ranks(dims, G, pieces, axis_mask):
+    """b200fft_exec_scatter_at with z_first = r * zl stores bit for bit what exec_scatter with my_rank = r stores, and
+    so does the same rank's slab cut into `pieces` sub-ranges of planes, each scattered at its own z_first."""
+    import torch
+    Z, Y, X = dims
+    zl, yl, zc = Z // G, Y // G, Z // G // pieces
+    g = torch.Generator(device="cuda").manual_seed(5)
+    full = torch.randn((Z, Y, X, 2), generator=g, device="cuda")
+    flags = b200fft.FLAG_NO_FUSED
+    plan = b200fft.plan_fft("float32", "float32", (zl, Y, X, 2), (zl, Y, X, 2), axis_mask=axis_mask, flags=flags)
+    plan_c = b200fft.plan_fft("float32", "float32", (zc, Y, X, 2), (zc, Y, X, 2), axis_mask=axis_mask, flags=flags)
+    work = torch.empty((zl, Y, X, 2), device="cuda")
+    st = torch.cuda.current_stream().cuda_stream
+    recv = {k: [torch.full((Z, yl, X, 2), float("nan"), device="cuda") for _ in range(G)] for k in ("rank", "at", "pieces")}
+    for r in range(G):
+        x_local = full[r * zl:(r + 1) * zl].contiguous()
+        keep = x_local.clone()
+        plan.exec_scatter(recv["rank"], r, x_local, work, st)
+        assert _scatter_at(plan, recv["at"], r * zl, x_local, work, st) == 0
+        for c in range(pieces):
+            x_c = x_local[c * zc:(c + 1) * zc]
+            assert _scatter_at(plan_c, recv["pieces"], r * zl + c * zc, x_c, work[c * zc:(c + 1) * zc], st) == 0
+        assert torch.equal(x_local, keep)
+    torch.cuda.synchronize()
+    xc = torch.view_as_complex(full.double().contiguous())
+    want = torch.fft.fft(xc, dim=1) if axis_mask == 1 else torch.fft.fftn(xc, dim=(1, 2))
+    for h in range(G):
+        assert torch.equal(recv["at"][h], recv["rank"][h])
+        assert torch.equal(recv["pieces"][h], recv["rank"][h])
+        got = torch.view_as_complex(recv["rank"][h].double().contiguous())
+        ref = want[:, h * yl:(h + 1) * yl, :]
+        assert float((got - ref).norm() / ref.norm()) < 2e-6
+    assert _scatter_at(plan, recv["at"], -1, full[:zl].contiguous(), work, st) == 1  # B200FFT_ERR_INVALID_ARG
+    plan.destroy()
+    plan_c.destroy()
 
 
 def test_exec_scatter_errors():

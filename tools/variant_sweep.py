@@ -12,7 +12,7 @@ import torch
 import b200fft
 from bench import time_gpu
 
-KNOBS = ("B200FFT_PDL", "B200FFT_PLANE_PREFER", "B200FFT_PLANE", "B200FFT_PLANE_C2R", "B200FFT_PASS_PIPELINE", "B200FFT_SERPENTINE", "B200FFT_JIT", "B200FFT_JIT_MAX_RADIX", "B200FFT_PREFETCH_AHEAD", "B200FFT_FUSED", "B200FFT_CHUNK_MB", "B200FFT_FUSED_PREFER", "B200FFT_PREFER", "B200FFT_PASS_CHUNK_MB")
+KNOBS = ("B200FFT_PDL", "B200FFT_PLANE_PREFER", "B200FFT_PLANE", "B200FFT_PLANE_C2R", "B200FFT_SERPENTINE", "B200FFT_JIT", "B200FFT_JIT_MAX_RADIX", "B200FFT_FUSED", "B200FFT_CHUNK_MB", "B200FFT_FUSED_PREFER", "B200FFT_PREFER")
 
 
 def main():

@@ -65,18 +65,27 @@ AxisView view_of(const Problem& p, int axis) {
   return v;
 }
 
-std::unique_ptr<Pass> make_pass(b200fft_plan* plan, int axis, const AxisView& view, const IoSpec& src, HalfMode half) {
+// nullptr with *status = why no kernel family serves the axis (B200FFT_ERR_UNSUPPORTED or B200FFT_ERR_ALLOC)
+std::unique_ptr<Pass> make_pass(b200fft_plan* plan, int axis, const AxisView& view, const IoSpec& src, HalfMode half, int* status) {
   const Problem& p = plan->prob;
+  *status = B200FFT_ERR_UNSUPPORTED;
+  // an axis longer than SPLIT2_MAX_N points: only the three-pass split of the specialisation tier can serve it, so its
+  // reason for refusing is the one reported (the runtime-length and generic kernels refuse any such axis)
+  std::string long_why = "FORCE_GENERIC and FORCE_RT leave out the plan-time three-pass split that axes longer than 2^24 "
+                         "points need";
   std::unique_ptr<Pass> pass;
   if (!(p.desc.flags & B200FFT_FLAG_FORCE_GENERIC)) {
     if (!(p.desc.flags & B200FFT_FLAG_FORCE_RT)) {
       pass = make_fast_pass(*plan, axis, view, src, p.desc.inverse != 0, half);
       if (!pass) pass = make_split_pass(*plan, axis, view, src, p.desc.inverse != 0, half);
-      if (!pass) pass = make_jit_pass(*plan, axis, view, src, p.desc.inverse != 0, half);
+      if (!pass) pass = make_jit_pass(*plan, axis, view, src, p.desc.inverse != 0, half, status);
+      if (!pass && *status != B200FFT_ERR_UNSUPPORTED) return nullptr;
+      if (!pass) long_why = last_error();
     }
     if (!pass) pass = make_rt_pass(*plan, axis, view, src, p.desc.inverse != 0, half);
   }
   if (!pass) pass = make_generic_pass(*plan, axis, view, src, p.desc.inverse != 0, half);
+  if (!pass && view.n > SPLIT2_MAX_N) fail(B200FFT_ERR_UNSUPPORTED, "axis %d: %s", axis, long_why.c_str());
   return pass;
 }
 
@@ -109,8 +118,9 @@ int build_passes(b200fft_plan* plan, bool dry, std::string* text) {
       *text += buf;
       return B200FFT_OK;
     }
-    std::unique_ptr<Pass> pass = make_pass(plan, axis, view, src, half);
-    if (!pass) return B200FFT_ERR_UNSUPPORTED;
+    int status;
+    std::unique_ptr<Pass> pass = make_pass(plan, axis, view, src, half, &status);
+    if (!pass) return status;
     pass->src_sel = ssel;
     pass->dst_sel = dsel;
     pass->axis = axis;
@@ -284,8 +294,9 @@ int b200fft_default_bases(uint64_t length, int gpu_target, uint32_t* out, int ca
 }  // extern "C"
 
 namespace {
-// b200fft_jit_probe / b200fft_jit_split_probe: validate, order the bases, run the host-only probe
-int probe_entry(bool split, int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in, int half,
+// b200fft_jit_probe / b200fft_jit_split_probe / b200fft_jit_split3_probe: validate, order the bases, run the host-only probe
+using ProbeFn = int (*)(int64_t, int64_t, const std::vector<uint32_t>&, bool, bool, int, int, int, std::string*);
+int probe_entry(ProbeFn probe, int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in, int half,
                 int in_dtype, int out_dtype, char* buf, size_t cap) {
   if (in_dtype < B200FFT_U8 || in_dtype > B200FFT_F64 || (out_dtype != B200FFT_F32 && out_dtype != B200FFT_F64))
     return fail(B200FFT_ERR_INVALID_ARG, "dtypes %d -> %d", in_dtype, out_dtype);
@@ -299,8 +310,7 @@ int probe_entry(bool split, int64_t n, int64_t inner, const uint32_t* bases, int
   }
   if (!ordered_bases_valid((uint64_t)n, ordered)) return fail(B200FFT_ERR_BASES, "bases do not factor %lld", (long long)n);
   std::string report;
-  const int rc = (split ? jit_split_probe : jit_probe)(n, inner, ordered, inverse != 0, real_in != 0, half, in_dtype, out_dtype,
-                                                      &report);
+  const int rc = probe(n, inner, ordered, inverse != 0, real_in != 0, half, in_dtype, out_dtype, &report);
   if (rc != B200FFT_OK) return rc;
   if (buf && cap) {
     strncpy(buf, report.c_str(), cap - 1);
@@ -314,12 +324,17 @@ extern "C" {
 
 int b200fft_jit_probe(int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in, int half,
                       int in_dtype, int out_dtype, char* buf, size_t cap) {
-  return probe_entry(false, n, inner, bases, nbases, inverse, real_in, half, in_dtype, out_dtype, buf, cap);
+  return probe_entry(jit_probe, n, inner, bases, nbases, inverse, real_in, half, in_dtype, out_dtype, buf, cap);
 }
 
 int b200fft_jit_split_probe(int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in, int half,
                             int in_dtype, int out_dtype, char* buf, size_t cap) {
-  return probe_entry(true, n, inner, bases, nbases, inverse, real_in, half, in_dtype, out_dtype, buf, cap);
+  return probe_entry(jit_split_probe, n, inner, bases, nbases, inverse, real_in, half, in_dtype, out_dtype, buf, cap);
+}
+
+int b200fft_jit_split3_probe(int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in, int half,
+                             int in_dtype, int out_dtype, char* buf, size_t cap) {
+  return probe_entry(jit_split3_probe, n, inner, bases, nbases, inverse, real_in, half, in_dtype, out_dtype, buf, cap);
 }
 
 int b200fft_schedule_dry_run(int nphases, const int64_t* phases, int64_t batch, int64_t* segments, int cap) {
@@ -378,7 +393,8 @@ int b200fft_plan_create(b200fft_plan** out, const b200fft_desc* desc) {
   const bool f64 = desc->out_dtype == B200FFT_F64;
   plan->tw.resize(plan->prob.rank);
   for (int a = 0; a < plan->prob.rank; ++a) {
-    if (!plan->prob.axes[a].transformed) continue;
+    // the n-entry W_n table serves passes of at most SPLIT2_MAX_N points; a longer axis has twiddle tables of its own
+    if (!plan->prob.axes[a].transformed || plan->prob.axes[a].n > SPLIT2_MAX_N) continue;
     rc = upload_twiddles(plan->prob.axes[a].n, desc->inverse != 0, f64, &plan->tw[a]);
     if (rc != B200FFT_OK) { b200fft_plan_destroy(plan.release()); return rc; }
   }

@@ -845,8 +845,9 @@ struct SplitArgs {
   const void* in;      // pass A: the user's array (in_scalar / in_vec2 elements); pass B: the temporary (float2)
   float2* out;
   const float2* tw;    // stage twiddles of this pass's variant
-  const float2* twN;   // W_N^n, n in [0, N): pass A only
+  const float2* twN;   // W_N^n, n in [0, N): pass A only (three-pass split: T_hi of SplitTw2Dst)
   const float2* tw2;   // half-spectrum forms: W_n^{-+k}, k = 0..n/2, of the Hermitian unpack (R2C) / pack (C2R)
+                       // (three-pass split: T_lo of SplitTw2Dst)
   long long inner;     // element stride of the ORIGINAL axis (1 = contiguous)
   long long nrows;     // rows pass B: outer * N1 rows of N2 points
   int tiles_per_outer; // cols passes: tiles per outer slab of THIS pass's view
@@ -868,9 +869,36 @@ struct SplitTwDst {
   }
 };
 
+// The twiddle of SplitTwDst for a contiguous axis (inner == 1) too long for a table of L entries: W_L^e, e = k * r,
+// as T_hi[e >> s] * T_lo[e & (2^s - 1)], two tables of about sqrt(L) entries (split_tw_shift). k < N and r < L / N,
+// so e < L needs no reduction; it reaches 2^31 and is formed in 64 bits.
+struct SplitTw2Dst {
+  float2* __restrict__ base;
+  long long si;
+  int valid_c;
+  const float2* __restrict__ thi;
+  const float2* __restrict__ tlo;
+  long long c0;
+  int s;
+  __device__ __forceinline__ void store(int, int i, int c, float2 v) const {
+    if (c >= valid_c) return;
+    const long long e = (long long)i * (c0 + c);
+    const float2 w = cmulf(__ldg(&thi[e >> s]), __ldg(&tlo[e & ((1LL << s) - 1)]));
+    base[i * si + c] = cmulf(v, w);
+  }
+};
+// s = ceil(bits(L - 1) / 2): T_lo holds 2^s entries, T_hi ceil(L / 2^s) (the host builds them with the same rule)
+__host__ __device__ __forceinline__ int split_tw_shift(long long L) {
+  int bits = 0;
+  while (bits < 62 && (1LL << bits) < L) ++bits;
+  return (bits + 1) / 2;
+}
+
 // pass A: view (outer, N1 = N, inner' = n2 * inner). REAL: the input array holds real scalars (in_scalar), read as
 // x + 0i; otherwise complex pairs (in_vec2). Both are cast to the working precision on load.
-template <int N, class RL, int CW, int NT, bool INV, bool REAL = false>
+// TW2: the contiguous axis of a three-pass split (inner == 1, L = N * n2): the twiddle from the two tables twN = T_hi
+// and tw2 = T_lo (SplitTw2Dst) instead of the L-entry table twN.
+template <int N, class RL, int CW, int NT, bool INV, bool REAL = false, bool TW2 = false>
 __global__ void __launch_bounds__(NT) cols_split_a_kernel(const __grid_constant__ SplitArgs a) {
   extern __shared__ __align__(16) float2 smem_f2[];
   pdl_wait();
@@ -883,8 +911,13 @@ __global__ void __launch_bounds__(NT) cols_split_a_kernel(const __grid_constant_
   const void* in = REAL ? (const void*)(reinterpret_cast<const in_scalar*>(a.in) + base)
                         : (const void*)(reinterpret_cast<const in_vec2*>(a.in) + base);
   GlobalSrc<REAL> src{in, 0, vinner, 1, valid_c};
-  SplitTwDst dst{a.out + base, vinner, valid_c, a.twN, c0, a.inner};
-  run_axis<RL, N, 1, CW, NT, INV, DenseLayoutN<N, CW>::template type>(src, dst, smem_f2, smem_f2 + BUF, a.tw, 1.f, false);
+  if constexpr (TW2) {
+    SplitTw2Dst dst{a.out + base, vinner, valid_c, a.twN, a.tw2, c0, split_tw_shift(N * vinner)};
+    run_axis<RL, N, 1, CW, NT, INV, DenseLayoutN<N, CW>::template type>(src, dst, smem_f2, smem_f2 + BUF, a.tw, 1.f, false);
+  } else {
+    SplitTwDst dst{a.out + base, vinner, valid_c, a.twN, c0, a.inner};
+    run_axis<RL, N, 1, CW, NT, INV, DenseLayoutN<N, CW>::template type>(src, dst, smem_f2, smem_f2 + BUF, a.tw, 1.f, false);
+  }
 }
 
 // ---- long half-spectrum axes (last axis, inner == 1) as two passes ----------------------------------------------------
@@ -996,6 +1029,30 @@ __global__ void __launch_bounds__(NT) rows_split_b_kernel(const __grid_constant_
     run_axis<RL, N, C, 1, NT, INV, RowLayoutN<N>::template type>(src, dst, smem_f2, smem_f2 + BUF, a.tw, a.scale,
                                                                  a.do_scale != 0);
   }
+}
+
+// ---- contiguous axes longer than 2^24 points as three passes, n = N1 * N2 * N3, M = N2 * N3 -----------------------
+//   1: cols_split_a_kernel<TW2> on the view (outer, N1, M): user array -> temporary, W_n^{k1 (n2 N3 + n3)} in the store
+//   2: the same on the view (outer N1, N2, N3), in place on the temporary, W_M^{k2 n3} in the store
+//   3: this kernel: the contiguous N3-point rows (k1, k2) of the temporary (row k1 * M + k2 * N3 of transform t),
+//      output k3 stored at k1 + N1 * k2 + N1 * N2 * k3, which is natural order
+// A CTA takes C rows of consecutive k1 and one k2 (C divides N1), so every store is a run of C elements.
+// Args: n1 = N1, n2 = N2, nrows = outer * N1 * N2.
+template <int N, class RL, int C, int NT, bool INV>
+__global__ void __launch_bounds__(NT) rows_split_c_kernel(const __grid_constant__ SplitArgs a) {
+  extern __shared__ __align__(16) float2 smem_f2[];
+  pdl_wait();
+  constexpr int BUF = max_exchange_elems<RL, C, RowLayoutN<N>::template type>();
+  const long long row0 = (long long)blockIdx.x * C;  // row = (t * N2 + k2) * N1 + k1
+  const int valid = (int)min((long long)C, a.nrows - row0);
+  const long long tk2 = row0 / a.n1, k1 = row0 - tk2 * a.n1;
+  const long long t = tk2 / a.n2, k2 = tk2 - t * a.n2;
+  const long long m = (long long)a.n2 * N;
+  const long long len = (long long)a.n1 * m;
+  GlobalSrc<false> src{reinterpret_cast<const float2*>(a.in) + t * len + k1 * m + k2 * N, m, 1, valid, 1};
+  GlobalDst dst{a.out + t * len + k1 + (long long)a.n1 * k2, 1, (long long)a.n1 * a.n2, valid, 1};
+  run_axis<RL, N, C, 1, NT, INV, RowLayoutN<N>::template type>(src, dst, smem_f2, smem_f2 + BUF, a.tw, a.scale,
+                                                               a.do_scale != 0);
 }
 
 // Pass B of a long even-length R2C (n = 2H, H = N1 * N2) with the Hermitian unpack fused into the store. Pass A has

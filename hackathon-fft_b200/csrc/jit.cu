@@ -155,7 +155,10 @@ enum JitKind {
   JIT_SPLIT_A_C2R,     // cols_split_a_c2r_kernel<N1, RL, CW, NT, false>: even C2R, Hermitian pack in the load
   JIT_SPLIT_A_C2R_ODD, // cols_split_a_c2r_kernel<N1, RL, CW, NT, true>: odd C2R, Hermitian-extended load
   JIT_SPLIT_B_HALF,    // rows_split_b_kernel<N2, RL, C, NT, false, 1>: odd R2C, bins 0..n/2 stored
-  JIT_SPLIT_B_REAL     // rows_split_b_kernel<N2, RL, C, NT, true, 2>: odd C2R, real parts stored
+  JIT_SPLIT_B_REAL,    // rows_split_b_kernel<N2, RL, C, NT, true, 2>: odd C2R, real parts stored
+  // contiguous axes longer than 2^24 points as three passes, n = N1 * N2 * N3 (fast.cuh):
+  JIT_SPLIT3_A,        // cols_split_a_kernel<N, RL, CW, NT, INV, REAL, true>: passes 1 and 2, the twiddle from two tables
+  JIT_SPLIT3_C         // rows_split_c_kernel<N3, RL, C, NT, INV>: pass 3, rows (k1, k2), natural-order store
 };
 
 struct JitSpec {
@@ -181,7 +184,7 @@ struct JitSpec {
   }
   bool strided() const {
     return kind == JIT_COLS || kind == JIT_SCATTER || kind == JIT_SPLIT_A || kind == JIT_SPLIT_B_COLS || kind == JIT_SPLIT_A_C2R ||
-           kind == JIT_SPLIT_A_C2R_ODD;
+           kind == JIT_SPLIT_A_C2R_ODD || kind == JIT_SPLIT3_A;
   }
   std::string radix_list() const {
     std::string s;
@@ -215,6 +218,8 @@ struct JitSpec {
       case JIT_SPLIT_B_REAL: return "b200fft::rows_split_b_kernel<" + head + ", true, 2>";
       case JIT_SPLIT_B_COLS: return "b200fft::cols_split_b_kernel<" + head + ", " + inv + ">";
       case JIT_SPLIT_B_ROWS: return "b200fft::rows_split_b_kernel<" + head + ", " + inv + ">";
+      case JIT_SPLIT3_A: return "b200fft::cols_split_a_kernel<" + head + ", " + inv + ", " + real + ", true>";
+      case JIT_SPLIT3_C: return "b200fft::rows_split_c_kernel<" + head + ", " + inv + ">";
       default: return "b200fft::rows_c2r_kernel<" + head + ">";
     }
   }
@@ -231,6 +236,7 @@ struct JitSpec {
       case JIT_SPLIT_B_ROWS:
       case JIT_SPLIT_B_HALF:
       case JIT_SPLIT_B_REAL:
+      case JIT_SPLIT3_C:
       case JIT_C2R_ODD:
       case JIT_R2C_ODD: return "b200fft::rows_smem_bytes<" + shape_args() + ">()";
       case JIT_COLS:
@@ -238,6 +244,7 @@ struct JitSpec {
       case JIT_SPLIT_B_COLS:
       case JIT_SPLIT_A_C2R:
       case JIT_SPLIT_A_C2R_ODD:
+      case JIT_SPLIT3_A:
       case JIT_SCATTER: return "b200fft::cols_smem_bytes<" + shape_args() + ">()";
       case JIT_R2C:
       case JIT_SPLIT_B_R2C: return "b200fft::rows_r2c_smem_bytes<" + shape_args() + ">()";
@@ -248,12 +255,13 @@ struct JitSpec {
   std::string name() const {
     static const char* const tag[] = {"jitrows", "jitcols", "jitscatter", "jitr2c", "jitr2creg", "jitr2codd", "jitc2r", "jitc2rodd",
                                       "jitsplitA", "jitsplitBcols", "jitsplitBrows", "jitplane", "jitr2cplane", "jitrowsIP",
-                                      "jitsplitBr2c", "jitsplitAc2r", "jitsplitAc2rodd", "jitsplitBhalf", "jitsplitBreal"};
+                                      "jitsplitBr2c", "jitsplitAc2r", "jitsplitAc2rodd", "jitsplitBhalf", "jitsplitBreal",
+                                      "jitsplit3A", "jitsplit3C"};
     if (plane())
       return std::string(tag[kind]) + std::to_string(n) + "x" + std::to_string(kind == JIT_PLANE_R2C ? 2 * n2 : n2) + "(" + radix_name(radices) +
              ";" + radix_name(radices2) + ")_inplace_t" + std::to_string(threads) + (f64 ? "_f64" : "");
     return std::string(tag[kind]) + std::to_string(n) + "_" + radix_name(radices) + (strided() ? "_w" : "_c") + std::to_string(tile) +
-           "_t" + std::to_string(threads) + (f64 ? "_f64" : "") + (kind == JIT_SPLIT_A && real_in ? "_realin" : "") + (in_dtype == B200FFT_U8 ? "_inu8" : in_dtype == (f64 ? B200FFT_F32 : B200FFT_F64) ? (f64 ? "_inf32" : "_inf64") : "");
+           "_t" + std::to_string(threads) + (f64 ? "_f64" : "") + ((kind == JIT_SPLIT_A || kind == JIT_SPLIT3_A) && real_in ? "_realin" : "") + (in_dtype == B200FFT_U8 ? "_inu8" : in_dtype == (f64 ? B200FFT_F32 : B200FFT_F64) ? (f64 ? "_inf32" : "_inf64") : "");
   }
   std::string defines() const {  // rtc_prelude.cuh reads these
     std::string d;
@@ -961,7 +969,7 @@ struct JitSplitPass : Pass {
     }
     return launch_one(*kb, sb, grid, params, stream);
   }
-  int launch_one(const JitKernel& kern, const JitSpec& sp, long long grid, void** params, cudaStream_t stream) {
+  static int launch_one(const JitKernel& kern, const JitSpec& sp, long long grid, void** params, cudaStream_t stream) {
     if (grid <= 0) return B200FFT_OK;
     if (grid > 0x7fffffffLL) return fail(B200FFT_ERR_UNSUPPORTED, "too many tiles");
     const CUresult r = driver().LaunchKernel(kern.fn, (unsigned)grid, 1, 1, (unsigned)sp.threads, 1, 1, (unsigned)sp.smem(),
@@ -1022,7 +1030,7 @@ bool jit_split_plan(const std::vector<uint32_t>& ordered, const AxisView& view, 
     if (view.inner != 1 || src.dtype == B200FFT_U8 || (half == HALF_C2R && src.dtype != work)) return false;
   }
   c->len = even_half ? view.n / 2 : view.n;
-  if (c->len > (1 << 24)) return false;
+  if (c->len > SPLIT2_MAX_N) return false;
   const std::vector<std::vector<uint32_t>> options = even_half ? drop_factor_two(ordered) : std::vector<std::vector<uint32_t>>{ordered};
   std::vector<int> all, ra, rb;
   bool ok = false;
@@ -1159,20 +1167,261 @@ std::unique_ptr<Pass> make_jit_split_pass(b200fft_plan& plan, int axis, const Ax
   return pass;
 }
 
+// ---- contiguous axes longer than 2^24 points: n = N1 * N2 * N3 as three specialised passes and one plan-owned temporary
+// (fast.cuh: rows_split_c_kernel). Both twiddles come from two tables of about sqrt(L) entries (SplitTw2Dst), so nothing
+// the plan holds grows like n except the temporary.
+struct JitSplit3Pass : Pass {
+  JitSpec s[3];
+  std::shared_ptr<JitKernel> k[3];
+  AxisView view;
+  int n1 = 0, n2 = 0, n3 = 0;
+  bool do_scale = false;
+  double scale = 1.0;
+  void* tw[3] = {};               // stage twiddles of each pass
+  void *hi[2] = {}, *lo[2] = {};  // T_hi / T_lo of W_n (pass 1) and W_M (pass 2)
+  void* tmp = nullptr;
+  std::string text;
+
+  template <class A, class T2>
+  int go(const void* src, void* dst, long long outer, cudaStream_t stream) {
+    A a;
+    memset(&a, 0, sizeof a);
+    void* params[1] = {&a};
+    a.inner = 1;
+    a.n1 = n1;
+    for (int p = 0; p < 2; ++p) {  // 1: view (outer, N1, M), input -> temporary; 2: view (outer N1, N2, N3) in place
+      const long long cols = p == 0 ? (long long)n2 * n3 : n3;
+      a.in = p == 0 ? src : tmp;
+      a.out = reinterpret_cast<T2*>(tmp);
+      a.tw = reinterpret_cast<const T2*>(tw[p]);
+      a.twN = reinterpret_cast<const T2*>(hi[p]);
+      a.tw2 = reinterpret_cast<const T2*>(lo[p]);
+      a.n2 = (int)cols;
+      a.tiles_per_outer = (int)((cols + s[p].tile - 1) / s[p].tile);
+      const int rc = JitSplitPass::launch_one(*k[p], s[p], (p == 0 ? outer : outer * n1) * a.tiles_per_outer, params, stream);
+      if (rc != B200FFT_OK) return rc;
+    }
+    a.in = tmp;  // 3: rows (k1, k2) of the temporary -> natural order
+    a.out = reinterpret_cast<T2*>(dst);
+    a.tw = reinterpret_cast<const T2*>(tw[2]);
+    a.twN = a.tw2 = nullptr;
+    a.n2 = n2;
+    a.nrows = outer * n1 * n2;
+    a.scale = scale;
+    a.do_scale = do_scale;
+    return JitSplitPass::launch_one(*k[2], s[2], (a.nrows + s[2].tile - 1) / s[2].tile, params, stream);
+  }
+  int launch(const void* src, void* dst, int64_t nbatch, cudaStream_t stream) override {
+    const long long outer = nbatch * view.outer_per_batch;
+    if (outer <= 0) return B200FFT_OK;
+    return s[0].f64 ? go<JitSplitPass::SplitArgs64, double2>(src, dst, outer, stream) : go<SplitArgs, float2>(src, dst, outer, stream);
+  }
+  std::string describe() const override { return text; }
+  int launches() const override { return 3; }
+};
+
+// Every split of the grouped super-stage list into three sets (products N1, N2, N3) of at most 8192 points and 4 stages,
+// most balanced first (the measure jit_split_stages applies to two): each assignment of the m <= 12 groups is scored.
+// The strided passes 1 and 2 hold fewer points per tile than the row pass 3, so the caller takes the first split whose
+// three tiles fit. Each split is returned as its assignment in base 3 (digit i: the set of group i).
+std::vector<long long> jit_split3_stages(const std::vector<int>& radices) {
+  const size_t m = radices.size();
+  std::vector<std::pair<double, long long>> scored;  // (score, assignment)
+  if (m < 3 || m > 12) return {};
+  long long total = 1;
+  for (size_t i = 0; i < m; ++i) total *= 3;
+  for (long long code = 0; code < total; ++code) {
+    long long p[3] = {1, 1, 1};
+    int cnt[3] = {0, 0, 0};
+    long long rest = code;
+    for (size_t i = 0; i < m; ++i, rest /= 3) {
+      p[rest % 3] *= radices[i];
+      ++cnt[rest % 3];
+    }
+    bool ok = true;
+    for (int j = 0; j < 3; ++j) ok = ok && cnt[j] > 0 && cnt[j] <= 4 && p[j] <= 8192;
+    if (!ok) continue;
+    const long long pmax = std::max({p[0], p[1], p[2]}), pmin = std::min({p[0], p[1], p[2]});
+    const int cmax = std::max({cnt[0], cnt[1], cnt[2]}), cmin = std::min({cnt[0], cnt[1], cnt[2]});
+    scored.emplace_back(std::log2((double)pmax / (double)pmin) + 0.25 * (cmax - cmin), code);
+  }
+  std::stable_sort(scored.begin(), scored.end(), [](const auto& x, const auto& y) { return x.first < y.first; });
+  std::vector<long long> out(scored.size());
+  for (size_t k = 0; k < scored.size(); ++k) out[k] = scored[k].second;
+  return out;
+}
+
+// The three passes of a contiguous axis longer than SPLIT2_MAX_N points, decided on the host alone (the plan and
+// b200fft_jit_split3_probe share it). Complex input, or real input with the full spectrum, of any input dtype (cast on
+// load in pass 1). False, with the reason in last_error(), for every axis it does not serve.
+struct JitSplit3Choice {
+  JitSpec s[3];
+  long long n[3] = {0, 0, 0};
+};
+bool jit_split3_plan(const std::vector<uint32_t>& ordered, const AxisView& view, const IoSpec& src, bool inverse, HalfMode half,
+                     bool f64, JitSplit3Choice* c) {
+  const long long n = view.n;
+  const char* why = nullptr;
+  char radix_why[64];
+  if (n <= SPLIT2_MAX_N) why = "axes up to 2^24 points take the two-pass split";
+  else if (half != HALF_NONE)
+    why = "half-spectrum rows whose split length is above 2^24 points are not served (B200FFT_REAL_FULL serves real input with "
+          "the full spectrum)";
+  else if (view.inner != 1) why = "strided axes (inner > 1) longer than 2^24 points are not served; the three-pass split takes contiguous axes";
+  for (uint32_t r : ordered)
+    if (!why && r > (uint32_t)JIT_MAX_PRIME) {
+      snprintf(radix_why, sizeof radix_why, "radix %u is above %d", r, JIT_MAX_PRIME);
+      why = radix_why;
+    }
+  std::vector<int> all;
+  std::vector<long long> splits;
+  if (!why && jit_group_cap(ordered, f64 ? JIT_MAX_RADIX_F64 : JIT_MAX_RADIX, &all, 12)) splits = jit_split3_stages(all);
+  if (!why && splits.empty()) why = "the stage list does not split into three tiles of at most 8192 points and 4 stages each";
+  if (why) {
+    fail(B200FFT_ERR_UNSUPPORTED, "%lld points: %s", n, why);
+    return false;
+  }
+  const int work = f64 ? B200FFT_F64 : B200FFT_F32;
+  for (long long code : splits) {
+    std::vector<int> sets[3];
+    for (size_t i = 0; i < all.size(); ++i, code /= 3) sets[code % 3].push_back(all[i]);
+    for (int j = 0; j < 3; ++j) {
+      JitSpec& s = c->s[j];
+      s = JitSpec();
+      c->n[j] = 1;
+      for (int r : sets[j]) c->n[j] *= r;
+      s.kind = j < 2 ? JIT_SPLIT3_A : JIT_SPLIT3_C;
+      s.n = (int)c->n[j];
+      s.radices = sets[j];
+      s.inverse = inverse;
+      s.f64 = f64;
+      s.in_dtype = work;  // passes 2 and 3 read the temporary
+      s.packed = !f64;
+    }
+    c->s[0].in_dtype = src.dtype;
+    c->s[0].real_in = src.comps == 1;
+    c->s[2].tile_divides = (int)c->n[0];  // a CTA's rows share k2
+    if (jit_geometry(&c->s[0], c->n[1] * c->n[2]) && jit_geometry(&c->s[1], c->n[2]) && jit_geometry(&c->s[2], 1)) return true;
+  }
+  fail(B200FFT_ERR_UNSUPPORTED, "%lld points: no split into three tiles fits shared memory", n);
+  return false;
+}
+
+// W_L^e = T_hi[e >> s] * T_lo[e & (2^s - 1)] (fast.cuh: SplitTw2Dst): T_hi[h] = W_L^{h 2^s}, h < ceil(L / 2^s), and
+// T_lo[j] = W_L^j, j < 2^s; evaluated in double, stored in the working precision T2
+template <class T2>
+void split_tw2_tables(long long L, bool inverse, std::vector<T2>* thi, std::vector<T2>* tlo) {
+  const int s = split_tw_shift(L);
+  const long long lo = 1LL << s, hi = (L + lo - 1) / lo;
+  auto w = [&](long long e) {
+    const double th = 2.0 * M_PI * ((double)e / (double)L);
+    T2 v;
+    v.x = std::cos(th);
+    v.y = (inverse ? 1.0 : -1.0) * std::sin(th);
+    return v;
+  };
+  thi->resize((size_t)hi);
+  tlo->resize((size_t)lo);
+  for (long long h = 0; h < hi; ++h) (*thi)[(size_t)h] = w(h * lo);
+  for (long long j = 0; j < lo; ++j) (*tlo)[(size_t)j] = w(j);
+}
+
+// nullptr when the three-pass split does not serve the axis; *status = B200FFT_ERR_ALLOC (not 4) when it would but its
+// device memory cannot be allocated
+std::unique_ptr<Pass> make_jit_split3_pass(b200fft_plan& plan, int axis, const AxisView& view, const IoSpec& src, bool scale_inverse,
+                                           HalfMode half, int* status) {
+  const Problem& p = plan.prob;
+  const bool f64 = p.desc.out_dtype == B200FFT_F64;
+  JitSplit3Choice c;
+  if (!jit_split3_plan(p.axes[axis].ordered, view, src, p.desc.inverse != 0, half, f64, &c)) return nullptr;
+  auto pass = std::make_unique<JitSplit3Pass>();
+  pass->view = view;
+  pass->n1 = (int)c.n[0];
+  pass->n2 = (int)c.n[1];
+  pass->n3 = (int)c.n[2];
+  for (int j = 0; j < 3; ++j) {
+    pass->s[j] = c.s[j];
+    pass->k[j] = get_kernel(c.s[j], plan.device);
+    if (!pass->k[j]) return nullptr;
+  }
+  pass->do_scale = scale_inverse;
+  pass->scale = scale_inverse ? 1.0 / (double)view.n : 1.0;
+  auto upload = [&](const void* data, size_t bytes, void** d) {
+    if (cudaMalloc(d, bytes) != cudaSuccess) {
+      cudaGetLastError();
+      *status = fail(B200FFT_ERR_ALLOC, "axis %d: cannot allocate %zu B of three-pass split tables", axis, bytes);
+      return false;
+    }
+    plan.owned_device.push_back(*d);
+    return cudaMemcpy(*d, data, bytes, cudaMemcpyHostToDevice) == cudaSuccess;
+  };
+  const bool inv = p.desc.inverse != 0;
+  const long long L[2] = {view.n, c.n[1] * c.n[2]};
+  bool ok = true;
+  if (f64) {
+    std::vector<double2> hi, lo;
+    for (int j = 0; j < 3 && ok; ++j) {
+      const auto t = stage_twiddles64(c.s[j].radices, inv);
+      ok = upload(t.data(), t.size() * sizeof(double2), &pass->tw[j]);
+    }
+    for (int j = 0; j < 2 && ok; ++j) {
+      split_tw2_tables(L[j], inv, &hi, &lo);
+      ok = upload(hi.data(), hi.size() * sizeof(double2), &pass->hi[j]) && upload(lo.data(), lo.size() * sizeof(double2), &pass->lo[j]);
+    }
+  } else {
+    std::vector<float2> hi, lo;
+    for (int j = 0; j < 3 && ok; ++j) {
+      const auto t = build_twiddles(c.s[j].radices, inv);
+      ok = upload(t.data(), t.size() * sizeof(float2), &pass->tw[j]);
+    }
+    for (int j = 0; j < 2 && ok; ++j) {
+      split_tw2_tables(L[j], inv, &hi, &lo);
+      ok = upload(hi.data(), hi.size() * sizeof(float2), &pass->hi[j]) && upload(lo.data(), lo.size() * sizeof(float2), &pass->lo[j]);
+    }
+  }
+  if (!ok) return nullptr;
+  const size_t tmp_bytes = (size_t)p.batch * (size_t)view.outer_per_batch * (size_t)view.n * c.s[1].esz();
+  if (cudaMalloc(&pass->tmp, tmp_bytes) != cudaSuccess) {
+    cudaGetLastError();
+    *status = fail(B200FFT_ERR_ALLOC, "axis %d: cannot allocate the %zu B temporary of the three-pass split", axis, tmp_bytes);
+    return nullptr;
+  }
+  plan.owned_device.push_back(pass->tmp);
+  plan.workspace_bytes += tmp_bytes;
+  std::string stages;
+  for (uint32_t r : p.axes[axis].ordered) stages += (stages.empty() ? "" : ",") + std::to_string(r);
+  if (stages.size() > 120) stages = stages.substr(0, 117) + "...";
+  char buf[800];
+  snprintf(buf, sizeof buf, "axis %d: split3 n=%lld%s = %lld x %lld x %lld inner=1: %s (+W_n twiddle, two tables) -> %s (in place, "
+           "+W_M twiddle, two tables) -> %s (natural-order store%s); temp=%zuB user stages=[%s] [NVRTC, %.0f + %.0f + %.0f ms]",
+           axis, (long long)view.n, src.comps == 1 ? " real-in" : "", c.n[0], c.n[1], c.n[2], c.s[0].name().c_str(),
+           c.s[1].name().c_str(), c.s[2].name().c_str(), scale_inverse ? ", 1/n" : "", tmp_bytes, stages.c_str(),
+           pass->k[0]->compile_ms, pass->k[1]->compile_ms, pass->k[2]->compile_ms);
+  pass->text = buf;
+  return pass;
+}
+
 }  // namespace
 
 std::unique_ptr<Pass> make_jit_pass(b200fft_plan& plan, int axis, const AxisView& view, const IoSpec& src, bool scale_inverse,
-                                    HalfMode half) {
+                                    HalfMode half, int* status) {
   const Problem& p = plan.prob;
-  if (!jit_enabled() || view.n < 2) return nullptr;
+  if (!jit_enabled() || view.n < 2) {
+    if (view.n > SPLIT2_MAX_N)
+      fail(B200FFT_ERR_UNSUPPORTED, "%lld points: axes longer than 2^24 points need the plan-time specialisation tier, which "
+           "B200FFT_JIT=0 turns off", (long long)view.n);
+    return nullptr;
+  }
   const bool f64 = p.desc.out_dtype == B200FFT_F64;
   JitSpec spec;
   const long long rows = view.inner == 1 ? (long long)p.batch * view.outer_per_batch : 0;
   if ((view.n > 16384 && view.inner != 1) || view.n > 32768 ||
       !jit_plan_axis(p.axes[axis], view, src, p.desc.inverse != 0, half, f64, &spec, rows)) {
-    // too long (or too many stages) for one tile: two passes
+    // too long (or too many stages) for one tile: two passes, or three beyond what two serve
     if (view.n < 1024) return nullptr;
-    return make_jit_split_pass(plan, axis, view, src, scale_inverse, half);
+    std::unique_ptr<Pass> pass = make_jit_split_pass(plan, axis, view, src, scale_inverse, half);
+    if (!pass && view.n > SPLIT2_MAX_N) pass = make_jit_split3_pass(plan, axis, view, src, scale_inverse, half, status);
+    return pass;
   }
   std::shared_ptr<JitKernel> k = get_kernel(spec, plan.device);
   if (!k) return nullptr;
@@ -1393,6 +1642,26 @@ int jit_split_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& order
   if (rc == B200FFT_OK) rc = probe_compile(c.sb, &rb);
   if (rc != B200FFT_OK) return rc;
   *report = ra + "; " + rb;
+  return B200FFT_OK;
+}
+
+// The same for the three passes of an axis longer than 2^24 points (make_jit_split3_pass): "<pass 1>; <pass 2>; <pass 3>"
+int jit_split3_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bool inverse, bool real_in, int half,
+                     int in_dtype, int out_dtype, std::string* report) {
+  AxisView view;
+  view.n = n;
+  view.inner = inner;
+  IoSpec src;
+  src.comps = real_in ? 1 : 2;
+  src.dtype = in_dtype;
+  JitSplit3Choice c;
+  if (!jit_split3_plan(ordered, view, src, inverse, (HalfMode)half, out_dtype == B200FFT_F64, &c)) return B200FFT_ERR_UNSUPPORTED;
+  std::string r[3];
+  for (int j = 0; j < 3; ++j) {
+    const int rc = probe_compile(c.s[j], &r[j]);
+    if (rc != B200FFT_OK) return rc;
+  }
+  *report = r[0] + "; " + r[1] + "; " + r[2];
   return B200FFT_OK;
 }
 

@@ -61,6 +61,11 @@ struct Pass {
   std::vector<std::unique_ptr<Pass>> fallback;
 };
 
+// The longest axis the two-pass split serves (two tiles of at most 8192 points would reach 2^26; its W_n table of n
+// entries is the limit). api.cu uploads that table only for axes up to this length; longer contiguous axes take the
+// three-pass split (jit.cu), whose twiddles are two tables of about sqrt(n) entries.
+constexpr int64_t SPLIT2_MAX_N = 1 << 24;
+
 struct DeviceTwiddles {
   void* ptr = nullptr;  // out-dtype complex W_N^n, n in [0, N)
   int64_t n = 0;
@@ -113,13 +118,17 @@ std::unique_ptr<Pass> make_plane_fwd_pass(b200fft_plan& plan);
 // ... the same for plane sizes without a registered variant, specialised at plan time (jit.cu)
 std::unique_ptr<Pass> make_jit_plane_pass(b200fft_plan& plan);
 // plan-time specialisation (jit.cu): the compile-time kernels instantiated through NVRTC for unregistered lengths
+// *status becomes B200FFT_ERR_ALLOC when an axis it would serve cannot get its device memory (stays as given otherwise)
 std::unique_ptr<Pass> make_jit_pass(b200fft_plan& plan, int axis, const AxisView& view, const IoSpec& src, bool scale_inverse,
-                                    HalfMode half);
+                                    HalfMode half, int* status);
 int jit_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bool inverse, bool real_in, int half,
               int in_dtype, int out_dtype, std::string* report);
 // the two passes the plan-time tier builds for an axis too long for one tile (same arguments)
 int jit_split_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bool inverse, bool real_in, int half,
                     int in_dtype, int out_dtype, std::string* report);
+// the three passes it builds for a contiguous axis longer than SPLIT2_MAX_N points (same arguments)
+int jit_split3_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bool inverse, bool real_in, int half,
+                     int in_dtype, int out_dtype, std::string* report);
 // number of registered kernel variants per tier (host-only; triggers the one-time registration)
 size_t fast_variant_count();
 size_t fused_variant_count();

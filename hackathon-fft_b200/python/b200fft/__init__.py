@@ -119,6 +119,8 @@ SYMBOLS = [
                                           ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_char_p, ctypes.c_size_t]),
     ("b200fft_jit_split_probe", ctypes.c_int, [ctypes.c_int64, ctypes.c_int64, _u32p, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                                 ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_char_p, ctypes.c_size_t]),
+    ("b200fft_jit_split3_probe", ctypes.c_int, [ctypes.c_int64, ctypes.c_int64, _u32p, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                                 ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_char_p, ctypes.c_size_t]),
     ("b200fft_schedule_dry_run", ctypes.c_int, [ctypes.c_int, ctypes.POINTER(ctypes.c_int64), ctypes.c_int64,
                                                  ctypes.POINTER(ctypes.c_int64), ctypes.c_int]),
     ("b200fft_strerror", ctypes.c_char_p, [ctypes.c_int]),
@@ -249,6 +251,16 @@ def jit_split_probe(n, inner=1, bases=None, inverse=False, real_in=False, half=0
     buf = ctypes.create_string_buffer(2048)
     _check(lib().b200fft_jit_split_probe(n, inner, arr, len(bases) if bases else 0, 1 if inverse else 0, 1 if real_in else 0,
                                          half, _dtype_code(in_dtype), _dtype_code(out_dtype), buf, len(buf)))
+    return buf.value.decode()
+
+
+def jit_split3_probe(n, inner=1, bases=None, inverse=False, real_in=False, half=0, in_dtype="float32", out_dtype="float32"):
+    """Compile (NVRTC, no GPU needed) the three passes the planner builds for a contiguous axis longer than 2^24 points;
+    returns "<pass 1 report>; <pass 2 report>; <pass 3 report>"."""
+    arr = (ctypes.c_uint32 * len(bases))(*bases) if bases else None
+    buf = ctypes.create_string_buffer(4096)
+    _check(lib().b200fft_jit_split3_probe(n, inner, arr, len(bases) if bases else 0, 1 if inverse else 0, 1 if real_in else 0,
+                                          half, _dtype_code(in_dtype), _dtype_code(out_dtype), buf, len(buf)))
     return buf.value.decode()
 
 

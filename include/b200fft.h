@@ -257,6 +257,14 @@ B200FFT_API int b200fft_jit_probe(int64_t n, int64_t inner, const uint32_t* base
  * (R2C / C2R, even and odd n) axes; B200FFT_ERR_UNSUPPORTED when the stage list has no such split. No GPU needed. */
 B200FFT_API int b200fft_jit_split_probe(int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in,
                                         int half, int in_dtype, int out_dtype, char* buf, size_t cap);
+/* The same for a contiguous axis longer than 2^24 points: compiles the three passes (1: N1-point strided transforms of
+ * the user's array, W_n twiddle from two tables of about sqrt(n) entries; 2: N2-point strided transforms in place on
+ * the temporary, W_M twiddle likewise; 3: N3-point rows with the natural-order store) the planner builds for it, and
+ * writes "<pass 1 report>; <pass 2 report>; <pass 3 report>". Complex input, or real input with the full spectrum;
+ * B200FFT_ERR_UNSUPPORTED for n <= 2^24, half-spectrum rows, strided axes (inner > 1), a radix above 127, or a stage
+ * list with no such split. No GPU needed. */
+B200FFT_API int b200fft_jit_split3_probe(int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in,
+                                         int half, int in_dtype, int out_dtype, char* buf, size_t cap);
 
 /* Tile schedule of the fused N-d kernel (host logic, no CUDA): phases[p] = {tiles_per_transform,
  * tiles_per_group, dep_div, quota}; writes up to `cap` segments as {phase, first_item, first_tile, count}

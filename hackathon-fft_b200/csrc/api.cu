@@ -2,7 +2,9 @@
 // kernel selection, execution on device or host buffers.
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <cmath>
+#include <cstdint>
 #include <cstdlib>
 #include <cstring>
 #include <memory>
@@ -239,6 +241,34 @@ int build_passes(b200fft_plan* plan, bool dry, std::string* text) {
   return add(last, rows, any ? work_spec : in_spec, HALF_C2R, any ? BUF_WORK : BUF_INPUT, BUF_OUTPUT);
 }
 
+// The alignment b200fft_exec requires of the input and output pointers: one element of each buffer, raised to what the
+// kernels of every pass that touches it need (Pass::min_align), fallback passes included.
+void record_alignment(b200fft_plan* plan) {
+  const Problem& p = plan->prob;
+  const bool real_out = p.half && p.desc.inverse;
+  plan->in_align = p.in_elem * (p.desc.in_components == 2 ? 2 : 1);
+  plan->out_align = p.out_elem * (real_out ? 1 : 2);
+  auto user_buffer = [&](BufSel sel) -> size_t* {  // the plan-owned workspace is cudaMalloc'ed: no requirement to record
+    return sel == BUF_INPUT ? &plan->in_align : sel == BUF_OUTPUT ? &plan->out_align : nullptr;
+  };
+  auto visit = [&](const Pass& pass, auto& self) -> void {
+    if (size_t* a = user_buffer(pass.src_sel)) *a = std::max(*a, pass.min_align(true));
+    if (size_t* a = user_buffer(pass.dst_sel)) *a = std::max(*a, pass.min_align(false));
+    for (const auto& f : pass.fallback) self(*f, self);
+  };
+  for (const auto& pass : plan->passes) visit(*pass, visit);
+}
+
+int check_alignment(const b200fft_plan* plan, const void* in, const char* in_name, const void* out, const char* out_name) {
+  if ((uintptr_t)in % plan->in_align)
+    return fail(B200FFT_ERR_INVALID_ARG, "%s %p is not aligned to %zu bytes, which this plan's kernels need", in_name, in,
+                plan->in_align);
+  if ((uintptr_t)out % plan->out_align)
+    return fail(B200FFT_ERR_INVALID_ARG, "%s %p is not aligned to %zu bytes, which this plan's kernels need", out_name, out,
+                plan->out_align);
+  return B200FFT_OK;
+}
+
 int copy_bases(const std::vector<uint32_t>& v, uint32_t* out, int cap) {
   if (!out || (int)v.size() > cap) return -1;
   for (size_t i = 0; i < v.size(); ++i) out[i] = v[i];
@@ -260,6 +290,23 @@ int b200fft_variant_count(int tier) {
     case 2: return (int)split_variant_count();
     default: return -1;
   }
+}
+
+int b200fft_variant_info(int tier, int index, char* buf, size_t cap) {
+  if (index < 0) return -1;
+  std::string line;
+  switch (tier) {
+    case 0: line = fast_variant_info((size_t)index); break;
+    case 1: line = fused_variant_info((size_t)index); break;
+    case 2: line = split_variant_info((size_t)index); break;
+    default: return -1;
+  }
+  if (line.empty()) return -1;
+  if (buf && cap) {
+    strncpy(buf, line.c_str(), cap - 1);
+    buf[cap - 1] = 0;
+  }
+  return (int)line.size() + 1;
 }
 
 const char* b200fft_last_error(void) { return last_error().c_str(); }
@@ -400,6 +447,7 @@ int b200fft_plan_create(b200fft_plan** out, const b200fft_desc* desc) {
   }
   rc = build_passes(plan.get(), /*dry=*/false, nullptr);
   if (rc != B200FFT_OK) { b200fft_plan_destroy(plan.release()); return rc; }
+  record_alignment(plan.get());
   // The tables were uploaded with cudaMemcpy from pageable memory on the legacy stream: make sure they have landed
   // before the caller launches on a non-blocking stream of its own (which is not ordered after the legacy stream).
   if (cudaError_t e = cudaDeviceSynchronize(); e != cudaSuccess) {
@@ -445,6 +493,7 @@ static int run_passes(b200fft_plan* plan, void* d_out, const void* d_in, int64_t
 
 int b200fft_exec(b200fft_plan* plan, void* d_out, const void* d_in, void* cu_stream) {
   if (!plan || !d_out || !d_in) return fail(B200FFT_ERR_INVALID_ARG, "null plan or buffer");
+  if (int rc = check_alignment(plan, d_in, "d_in", d_out, "d_out")) return rc;
   DeviceGuard guard(plan->device);
   return run_passes(plan, d_out, d_in, plan->prob.batch, (cudaStream_t)cu_stream);
 }
@@ -457,6 +506,10 @@ static int exec_scatter_impl(b200fft_plan* plan, void* const* peer_out, int npee
   if (plan->passes.empty() || plan->passes.back()->axis != 0)
     return fail(B200FFT_ERR_INVALID_ARG, "exec_scatter: the plan's last pass must transform axis 0 (the split axis); "
                                          "create the plan with B200FFT_FLAG_NO_FUSED");
+  if (int rc = check_alignment(plan, d_in, "d_in", d_work, "d_work")) return rc;
+  for (int i = 0; i < npeers && i < 16; ++i)
+    if (!peer_out[i] || (uintptr_t)peer_out[i] % plan->out_align)
+      return fail(B200FFT_ERR_INVALID_ARG, "peer_out[%d] %p is null or not aligned to %zu bytes", i, peer_out[i], plan->out_align);
   DeviceGuard guard(plan->device);
   cudaStream_t st = (cudaStream_t)cu_stream;
   const size_t n = plan->passes.size();

@@ -262,6 +262,14 @@ struct FastPass : Pass {
     return B200FFT_OK;
   }
   std::string describe() const override { return text; }
+  size_t min_align(bool src) const override {
+    if (v->kind == COLS_TMA) return 16;  // tensor maps need 16-byte global addresses
+    // rowsV: complex-input instantiations load and store through float4 (GlobalSrcV4 / GlobalDstV4)
+    if (half == HALF_NONE && v->kind == ROWS && !real_in && v->name.compare(0, 5, "rowsV") == 0) return 16;
+    // even half spectrum: R2C reads the real row as float2 pairs, C2R stores it as float2 pairs
+    if (r2c_mode != R2C_ODD && half == (src ? HALF_R2C : HALF_C2R)) return 8;
+    return 0;
+  }
 };
 
 }  // namespace
@@ -269,6 +277,36 @@ struct FastPass : Pass {
 size_t fast_variant_count() {
   register_all();
   return registry().size();
+}
+
+std::string fast_variant_info(size_t i) {
+  register_all();
+  if (i >= registry().size()) return "";
+  const Variant& v = registry()[i];
+  std::string kind, forms;
+  auto add = [&](const char* f) { forms += (forms.empty() ? "" : ",") + std::string(f); };
+  if (v.kind == ROWS) {
+    kind = v.inv_ok ? "rowsIP" : "rows";
+    add("fwd");
+    if (v.full || v.inv_ok) { add("inv"); add("real"); }
+    if (v.launch_half) { add("r2c"); add("c2r"); }
+    if (v.launch_r2c_reg) add("r2c-reg");
+    if (v.launch_r2c_odd) add("r2c-odd");
+    if (v.launch_c2r_odd) add("c2r-odd");
+  } else if (v.kind == COLS) {
+    kind = "cols";
+    add("fwd");
+    if (v.full) { add("inv"); add("real"); }
+    if (v.launch_scatter) add("scatter");
+  } else {
+    kind = "colsT";  // complex input only: the tensor maps describe complex64 elements
+    add("fwd");
+    add("inv");
+  }
+  return "name=" + v.name + " kind=" + kind + " n=" + std::to_string(v.n) + " radices=" + radix_name(v.radices) +
+         " tile=" + std::to_string(v.tile) + " threads=" + std::to_string(v.threads) + " full=" + (v.full ? "1" : "0") +
+         " smem=" + std::to_string(v.smem) + " smem_r2c=" + std::to_string(v.smem_r2c) +
+         " smem_c2r=" + std::to_string(v.smem_c2r) + " forms=" + forms;
 }
 
 std::unique_ptr<Pass> make_fast_pass(b200fft_plan& plan, int axis, const AxisView& view, const IoSpec& src,

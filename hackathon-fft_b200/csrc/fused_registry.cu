@@ -172,6 +172,12 @@ struct FusedPass : Pass {
     if (h_err) cudaFreeHost(h_err);
   }
   std::string describe() const override { return text; }
+  size_t min_align(bool src) const override {
+    if (v->async) return 16;  // bulk-async copies of the input tiles, tensor maps over the output
+    // half spectrum: the real rows are read as float2 pairs
+    if (src && v->mode == 2) return 8;
+    return 0;
+  }
 };
 
 }  // namespace
@@ -179,6 +185,21 @@ struct FusedPass : Pass {
 size_t fused_variant_count() {
   register_all_fused();
   return fused_registry().size();
+}
+
+std::string fused_variant_info(size_t i) {
+  register_all_fused();
+  if (i >= fused_registry().size()) return "";
+  const FusedVariant& v = fused_registry()[i];
+  std::string dims, radices;
+  for (size_t a = 0; a < v.dims.size(); ++a) dims += (a ? "x" : "") + std::to_string(v.dims[a]);
+  for (int q = 0; q < v.nphases; ++q) {  // phases in order; a plane phase lists its y stages, then ';', then its x stages
+    const FusedPhaseInfo& ph = v.ph[q];
+    radices += (q ? "|" : "") + (ph.radices2.empty() ? "" : radix_name(ph.radices2) + ";") + radix_name(ph.radices);
+  }
+  return "name=" + v.name + " kind=fused n=" + dims + " radices=" + radices + " tile=" + std::to_string(v.ph[0].tile) +
+         " threads=" + std::to_string(v.threads) + " smem=" + std::to_string(v.smem) + " async=" + (v.async ? "1" : "0") +
+         " mode=" + (v.mode == 0 ? "c2c" : v.mode == 1 ? "real" : "r2c") + " forms=" + (v.inverse ? "inv" : "fwd");
 }
 
 std::unique_ptr<Pass> make_fused_pass(b200fft_plan& plan) {

@@ -668,6 +668,8 @@ bool jit_rows_ip_geometry(JitSpec* s) {
   return s->smem() <= 200 * 1024;
 }
 
+size_t in_scalar_bytes(int dtype) { return dtype == B200FFT_U8 ? 1 : dtype == B200FFT_F64 ? 8 : 4; }
+
 // rows_r2c_reg_kernel's precondition (fast.cuh: r2c_reg_ok) apart from the tile, which jit_geometry picks
 bool r2c_reg_shape_ok(const JitSpec& s) {
   const int P = s.n / s.radices.back();
@@ -807,6 +809,11 @@ struct JitPass : Pass {
     return run(*k_scatter, sp, outer * ca.tiles_per_outer, params, stream);
   }
   std::string describe() const override { return text; }
+  size_t min_align(bool src) const override {
+    // even half spectrum: R2C reads the real row as complex pairs, C2R stores it as complex pairs
+    if (src) return spec.kind == JIT_R2C || spec.kind == JIT_R2C_REG ? 2 * in_scalar_bytes(spec.in_dtype) : 0;
+    return spec.kind == JIT_C2R ? spec.esz() : 0;
+  }
 };
 
 // fp64 forms of build_twiddles / build_half_twiddles (fast_registry.cu): tw[(j-1)*P + p] = W_{P*R}^{j*p} per stage s >= 1
@@ -984,6 +991,11 @@ struct JitSplitPass : Pass {
     return sa.f64 ? go<SplitArgs64, double2>(src, dst, outer, stream) : go<SplitArgs, float2>(src, dst, outer, stream);
   }
   std::string describe() const override { return text; }
+  size_t min_align(bool src) const override {
+    // even half spectrum: R2C pass A reads the real row as H complex pairs, C2R pass B stores it as H complex pairs
+    if (src) return sb.kind == JIT_SPLIT_B_R2C ? 2 * in_scalar_bytes(sa.in_dtype) : 0;
+    return sa.kind == JIT_SPLIT_A_C2R ? sb.esz() : 0;
+  }
   int launches() const override { return 2; }
 };
 
@@ -1499,6 +1511,10 @@ struct JitPlanePass : Pass {
     return B200FFT_OK;
   }
   std::string describe() const override { return text; }
+  size_t min_align(bool src) const override {
+    // R2C planes read the real rows as complex pairs of the input element type
+    return src && spec.kind == JIT_PLANE_R2C ? 2 * in_scalar_bytes(spec.in_dtype) : 0;
+  }
 };
 
 // exactly two register stages of at most 32 for one axis, or false

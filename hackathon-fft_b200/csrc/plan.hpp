@@ -46,6 +46,11 @@ struct Pass {
   virtual int launch(const void* src, void* dst, int64_t nbatch, cudaStream_t stream) = 0;
   virtual std::string describe() const = 0;
   virtual int launches() const { return 1; }
+  // Byte alignment the pass's kernels need of the buffer they read (src) or write (!src). 0 = the alignment of one
+  // element of that buffer, which any access needs; passes whose kernels move wider units (128-bit, TMA or bulk-async
+  // copies, real rows read or written as pairs) return it. b200fft_exec refuses user pointers less aligned than the
+  // maximum over the plan's passes (b200fft_plan::in_align / out_align).
+  virtual size_t min_align(bool /*src*/) const { return 0; }
   // Same pass, but output row i of the transformed axis goes to sc.peer_out[i / rows_per_peer]
   // (slab exchange fused into the store). Only strided fast passes implement it.
   virtual int launch_scatter(const void*, const Scatter&, int64_t, cudaStream_t) {
@@ -84,6 +89,7 @@ struct b200fft_plan {
   void* workspace = nullptr;
   size_t workspace_bytes = 0;
   size_t work_stride = 0;     // workspace bytes per batch item
+  size_t in_align = 1, out_align = 1;  // least byte alignment of the input / output pointers the passes accept
   // exec_host resources (lazily created)
   cudaStream_t hs[3] = {nullptr, nullptr, nullptr};
   void* h_dev_in[2] = {nullptr, nullptr};
@@ -133,5 +139,9 @@ int jit_split3_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& orde
 size_t fast_variant_count();
 size_t fused_variant_count();
 size_t split_variant_count();
+// one line per variant for b200fft_variant_info (host-only); empty for an index past the end
+std::string fast_variant_info(size_t index);
+std::string fused_variant_info(size_t index);
+std::string split_variant_info(size_t index);
 
 }  // namespace b200fft

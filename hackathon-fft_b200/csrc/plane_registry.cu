@@ -107,6 +107,7 @@ struct PlaneC2RPass : Pass {
     return B200FFT_OK;
   }
   std::string describe() const override { return text; }
+  size_t min_align(bool src) const override { return src ? 0 : 8; }  // the real rows are stored as float2 pairs
 };
 
 // ---- forward / complex plane kernels
@@ -281,6 +282,7 @@ struct PlaneFwdPass : Pass {
     return B200FFT_OK;
   }
   std::string describe() const override { return text; }
+  size_t min_align(bool src) const override { return src && v->r2c ? 8 : 0; }  // R2C: real rows read as float2 pairs
 };
 
 }  // namespace

@@ -99,6 +99,16 @@ size_t split_variant_count() {
   return split_registry().size();
 }
 
+std::string split_variant_info(size_t i) {
+  register_split();
+  if (i >= split_registry().size()) return "";
+  const SplitKernel& k = split_registry()[i];
+  const char* kind = k.role == SPLIT_A ? "splitA" : k.role == SPLIT_B_COLS ? "splitB_cols" : "splitB_rows";
+  return "name=" + k.name + " kind=" + kind + " n=" + std::to_string(k.n) + " radices=" + radix_name(k.radices) +
+         " tile=" + std::to_string(k.tile) + " threads=" + std::to_string(k.threads) + " smem=" + std::to_string(k.smem) +
+         " forms=fwd,inv";
+}
+
 std::unique_ptr<Pass> make_split_pass(b200fft_plan& plan, int axis, const AxisView& view, const IoSpec& src,
                                       bool scale_inverse, HalfMode half) {
   register_split();

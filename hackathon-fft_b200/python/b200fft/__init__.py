@@ -17,7 +17,7 @@ import ctypes
 import os
 
 __all__ = ["plan_fft", "fft", "Plan", "SlabPlan", "B200FFTError", "ordered_bases", "default_bases", "dry_run",
-           "launch_count", "lib_path", "REAL_FULL", "REAL_HALF", "FLAG_FORCE_GENERIC", "FLAG_NO_FUSED", "FLAG_PREFER_FUSED",
+           "launch_count", "variant_info", "lib_path", "REAL_FULL", "REAL_HALF", "FLAG_FORCE_GENERIC", "FLAG_NO_FUSED", "FLAG_PREFER_FUSED",
            "FLAG_FORCE_RT", "GPUTest", "stream_synchronize", "host_register", "host_unregister", "MgpuPlan", "mgpu_split",
            "MGPU_BATCH_SHARD", "MGPU_SLAB"]
 
@@ -128,6 +128,7 @@ SYMBOLS = [
     ("b200fft_version", ctypes.c_int, []),
     ("b200fft_launch_count", ctypes.c_uint64, []),
     ("b200fft_variant_count", ctypes.c_int, [ctypes.c_int]),
+    ("b200fft_variant_info", ctypes.c_int, [ctypes.c_int, ctypes.c_int, ctypes.c_char_p, ctypes.c_size_t]),
 ]
 
 
@@ -266,6 +267,30 @@ def jit_split3_probe(n, inner=1, bases=None, inverse=False, real_in=False, half=
 
 def launch_count():
     return int(lib().b200fft_launch_count())
+
+
+def variant_info(tier):
+    """The compiled-in kernel variants of `tier` (0 row / column, 1 fused N-d, 2 two-pass split), in registration
+    order, as dicts of the fields b200fft_variant_info writes. `forms` is a list; `n` and `radices` are ints / a list
+    of ints except for fused variants, whose `n` is the dims text ("64x64x64") and `radices` the phases' stage lists
+    ("8x8;8x8|8x8"). Host-only."""
+    out = []
+    for i in range(lib().b200fft_variant_count(tier)):
+        need = lib().b200fft_variant_info(tier, i, None, 0)
+        if need < 0:
+            raise B200FFTError(1, "variant %d of tier %d" % (i, tier))
+        buf = ctypes.create_string_buffer(need)
+        lib().b200fft_variant_info(tier, i, buf, len(buf))
+        d = dict(tok.split("=", 1) for tok in buf.value.decode().split())
+        d["forms"] = d["forms"].split(",")
+        for k in ("tile", "threads", "smem", "smem_r2c", "smem_c2r", "full", "async"):
+            if k in d:
+                d[k] = int(d[k])
+        if d["kind"] != "fused":
+            d["n"] = int(d["n"])
+            d["radices"] = [int(r) for r in d["radices"].split("x")]
+        out.append(d)
+    return out
 
 
 def _make_desc(in_dtype, out_dtype, in_layout, out_layout, bases, inverse, real_mode, axis_mask, device, flags):

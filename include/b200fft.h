@@ -115,7 +115,15 @@ B200FFT_API int b200fft_plan_create(b200fft_plan** plan, const b200fft_desc* des
  * Asynchronous on `cu_stream` (a CUstream / cudaStream_t; NULL = default stream);
  * the caller synchronises, as bench.mojo:51-52 does. `d_out` and `d_in` are device
  * pointers; out-of-place, or in-place (d_out == d_in) when input and output have the
- * same element type and component count. */
+ * same element type and component count.
+ * Alignment: each pointer must be aligned to one element of its buffer (1 B uint8, 4 B fp32 real, 8 B fp32 complex
+ * or fp64 real, 16 B fp64 complex) and to what the plan's kernels need beyond that: 16 B where they use 128-bit,
+ * TMA or bulk-async global accesses (the default plans of 64-, 128- and 256-point complex rows among them), two
+ * scalars where they read or write real rows as pairs (half-spectrum transforms of even length). Any pointer that
+ * cudaMalloc or a torch allocation returns satisfies all of these; a view at an element offset may not. A less
+ * aligned pointer returns B200FFT_ERR_INVALID_ARG before anything is launched, and b200fft_last_error() names the
+ * pointer and the alignment. b200fft_exec_scatter(_at) check d_in, d_work and the peers the same way;
+ * b200fft_exec_host stages through its own buffers and has no requirement. */
 B200FFT_API int b200fft_exec(b200fft_plan* plan, void* d_out, const void* d_in, void* cu_stream);
 
 /* Blocks until everything enqueued on `cu_stream` has finished (NULL = the legacy default stream, which is
@@ -283,6 +291,17 @@ B200FFT_API uint64_t b200fft_launch_count(void);
  * 2 = two-pass split kernels; -1 for an unknown tier. Host-only (no CUDA call); safe to call from several threads at
  * once, like plan creation: the variant tables are built exactly once. */
 B200FFT_API int b200fft_variant_count(int tier);
+/* One line describing variant `index` of `tier` (same tiers and order as b200fft_variant_count), fields separated
+ * by spaces:
+ *   name=<name> kind=<rows|rowsIP|cols|colsT|splitA|splitB_cols|splitB_rows|fused> n=<length> (fused: dims, "64x64x64")
+ *   radices=<16x8> (fused: the phases' stage lists, "8x8;8x8|8x8") tile=<rows or columns per CTA> threads=<count>
+ *   forms=<comma list> of what the variant instantiates: fwd, inv (complex input), real (real input, full spectrum),
+ *   r2c, c2r (half spectrum of 2n points on this n-point variant), r2c-reg (R2C with the register unpack), r2c-odd,
+ *   c2r-odd (half spectrum of odd n itself), scatter (slab exchange in the store); fused: mode=<c2c|real|r2c> and
+ *   direction fwd or inv.
+ * Writes at most `cap` bytes including the terminating NUL and returns the length of the whole line plus one, or
+ * -1 for an unknown tier or index. Host-only (no CUDA call). */
+B200FFT_API int b200fft_variant_info(int tier, int index, char* buf, size_t cap);
 
 #ifdef __cplusplus
 }

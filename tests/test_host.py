@@ -335,3 +335,66 @@ def test_jit_disk_cache(tmp_path):
     off = subprocess.run([sys.executable, "-c", code % 1000], env=dict(env, B200FFT_JIT_CACHE="0"), capture_output=True, text=True,
                          check=True).stdout
     assert "disk cache" not in off
+
+
+@pytest.mark.parametrize("tier", [0, 1, 2])
+def test_variant_info_describes_every_registered_variant(tier):
+    """b200fft_variant_info lists each tier's registry (what tests/test_gpu_variants.py forces one variant at a time),
+    and the lines agree with what the planner relies on: unique names, radices that multiply to n, and the forms
+    a variant instantiates."""
+    info = b200fft.variant_info(tier)
+    assert len(info) == b200fft.lib().b200fft_variant_count(tier)
+    names = [v["name"] for v in info]
+    assert len(set(names)) == len(names)
+    L = b200fft.lib()
+    assert L.b200fft_variant_info(tier, len(info), None, 0) == -1
+    assert L.b200fft_variant_info(tier, -1, None, 0) == -1
+    assert L.b200fft_variant_info(3, 0, None, 0) == -1
+    small = ctypes.create_string_buffer(8)  # a short buffer is truncated, the return value is the full length
+    need = L.b200fft_variant_info(tier, 0, small, len(small))
+    assert need > len(small) and small.value.decode() == ("name=" + names[0])[:7]
+    for v in info:
+        if tier == 1:
+            assert v["kind"] == "fused" and v["mode"] in ("c2c", "real", "r2c") and v["forms"] in (["fwd"], ["inv"])
+            assert v["async"] == v["name"].startswith("ndA")
+            dims = [int(d) for d in v["n"].split("x")]
+            assert v["name"].startswith(("ndA" if v["async"] else "nd") + v["n"] + ("_inv" if v["forms"] == ["inv"] else ""))
+            # one stage list per axis (a plane phase carries two: y; x), together the whole transform (R2C: n/2 on x)
+            stages = [s for ph in v["radices"].split("|") for s in ph.split(";")]
+            assert len(stages) == len(dims), v["name"]
+            prod = int(np.prod([int(r) for s in stages for r in s.split("x")]))
+            assert prod == int(np.prod(dims)) // (2 if v["mode"] == "r2c" else 1), v["name"]
+            continue
+        assert int(np.prod(v["radices"])) == v["n"], v["name"]
+        assert v["tile"] >= 1 and v["threads"] >= 32
+        if tier == 2:
+            assert v["kind"] in ("splitA", "splitB_cols", "splitB_rows") and v["forms"] == ["fwd", "inv"]
+            assert v["name"].startswith({"splitA": "splitA_cols", "splitB_cols": "splitB_cols", "splitB_rows": "splitB_rows"}
+                                        [v["kind"]] + str(v["n"]) + "_")
+            continue
+        assert v["kind"] in ("rows", "rowsIP", "cols", "colsT")
+        assert v["name"].startswith({"rows": "rows", "rowsIP": "rowsIP", "cols": "cols", "colsT": "colsT"}[v["kind"]])
+        forms = v["forms"]
+        assert forms[0] == "fwd"
+        if v["kind"] == "rowsIP":  # one-buffer rows: every direction and input, no half-spectrum forms
+            assert forms == ["fwd", "inv", "real"] and v["full"] == 0
+        elif v["kind"] == "colsT":
+            assert forms == ["fwd", "inv"]
+        elif not v["full"]:  # tuning candidates: forward complex only
+            assert forms == ["fwd"]
+        else:
+            assert forms[:3] == ["fwd", "inv", "real"]
+        if v["kind"] == "rows" and v["full"]:
+            fits = v["smem_r2c"] <= 227 * 1024 and v["smem_c2r"] <= 227 * 1024
+            assert ("r2c" in forms) == fits and ("c2r" in forms) == fits, v
+            assert ("r2c-reg" not in forms) or fits
+            assert ("r2c-odd" in forms) == ("c2r-odd" in forms) == (v["n"] % 2 == 1)
+        else:
+            assert not {"r2c", "c2r", "r2c-reg", "r2c-odd", "c2r-odd"} & set(forms)
+        assert ("scatter" in forms) == (v["kind"] == "cols" and bool(v["full"]))
+    if tier == 0:
+        # B200FFT_PREFER matches substrings: each name must select exactly one variant
+        clash = [(a, b) for a in names for b in names if a != b and a in b]
+        assert not clash, clash
+        kinds = {v["kind"] for v in info}
+        assert kinds == {"rows", "rowsIP", "cols", "colsT"}

@@ -361,7 +361,7 @@ constexpr int max_exchange_elems() {
 
 // ---- programmatic dependent launch -----------------------------------------------------------------
 // A pass that FOLLOWS another pass of a plan is launched with cudaLaunchAttributeProgrammaticStreamSerialization
-// (fast_registry.hpp: launch_dependent): the driver may set its grid up while the previous pass is still running, and its
+// (tile.cu: launch_tile): the driver may set its grid up while the previous pass is still running, and its
 // CTAs block in pdl_wait until that grid has completed and its writes are visible. For a kernel launched the ordinary way
 // pdl_wait is a no-op, so every tile kernel calls it first thing. The previous pass does NOT signal early
 // (griddepcontrol.launch_dependents at CTA start was measured: the same gain on most shapes, but the waiting CTAs it lets

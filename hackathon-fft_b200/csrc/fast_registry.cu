@@ -82,36 +82,6 @@ bool can_group(std::vector<uint32_t> ordered, std::vector<int> target) {
   return rec(0, 1, rest);
 }
 
-// per-stage twiddle table: stage s >= 1 holds tw[(j-1)*P + p] = W_{P*R}^{j*p}
-std::vector<float2> build_twiddles(const std::vector<int>& radices, bool inverse) {
-  std::vector<float2> t;
-  long long P = 1;
-  for (size_t s = 0; s < radices.size(); ++s) {
-    const int R = radices[s];
-    if (s > 0) {
-      const long long Q = P * R;
-      for (int j = 1; j < R; ++j)
-        for (long long p = 0; p < P; ++p) {
-          const double th = 2.0 * M_PI * (double)((j * p) % Q) / (double)Q;
-          t.push_back(make_float2((float)std::cos(th), (float)((inverse ? 1.0 : -1.0) * std::sin(th))));
-        }
-    }
-    P *= R;
-  }
-  if (t.empty()) t.push_back(make_float2(1.f, 0.f));
-  return t;
-}
-
-// W_n^{+-k}, k = 0..n/2, for the R2C unpack / C2R pack
-std::vector<float2> build_half_twiddles(long long n, bool inverse) {
-  std::vector<float2> t;
-  for (long long k = 0; k <= n / 2; ++k) {
-    const double th = 2.0 * M_PI * (double)k / (double)n;
-    t.push_back(make_float2((float)std::cos(th), (float)((inverse ? 1.0 : -1.0) * std::sin(th))));
-  }
-  return t;
-}
-
 // stage list of length n with one factor 2 removed (the even/odd split the real transform uses)
 std::vector<std::vector<uint32_t>> drop_factor_two(const std::vector<uint32_t>& ordered) {
   std::vector<std::vector<uint32_t>> out;
@@ -155,125 +125,6 @@ bool encode_axis_map(CUtensorMap* map, const void* base, long long inner, long l
              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-namespace {
-
-struct FastPass : Pass {
-  const Variant* v = nullptr;
-  HalfMode half = HALF_NONE;
-  enum R2CMode { R2C_SMEM = 0, R2C_REG = 1, R2C_ODD = 2 } r2c_mode = R2C_SMEM;  // which R2C kernel (fast.cuh); R2C_ODD also
-                                                                                // marks the odd-length C2R
-  float2* d_tw2 = nullptr;
-  AxisView view;
-  bool inverse = false, real_in = false, do_scale = false;
-  float scale = 1.f;
-  float2* d_tw = nullptr;
-  std::string text;
-
-  int launch(const void* src, void* dst, int64_t nbatch, cudaStream_t stream) override {
-    return launch_outer(src, dst, nbatch * view.outer_per_batch, stream);
-  }
-  // `outer` consecutive outer slabs (rows passes: rows) starting at src / dst
-  int launch_outer(const void* src, void* dst, int64_t outer, cudaStream_t stream) {
-    if (half != HALF_NONE) {
-      HalfArgs a;
-      a.in = src;
-      a.out = dst;
-      a.tw = d_tw;
-      a.tw2 = d_tw2;
-      a.nrows = outer;
-      a.scale = scale;
-      const long long grid = (a.nrows + v->tile - 1) / v->tile;
-      if (grid <= 0) return B200FFT_OK;
-      if (grid > 0x7fffffffLL) return fail(B200FFT_ERR_UNSUPPORTED, "too many row tiles");
-      if (half == HALF_R2C && r2c_mode == R2C_REG) v->launch_r2c_reg(a, (unsigned)grid, stream);
-      else if (half == HALF_R2C && r2c_mode == R2C_ODD) v->launch_r2c_odd(a, (unsigned)grid, v->smem, stream);
-      else if (half == HALF_C2R && r2c_mode == R2C_ODD) v->launch_c2r_odd(a, (unsigned)grid, v->smem, stream);
-      else v->launch_half(half == HALF_C2R, a, (unsigned)grid, stream);
-    } else if (v->kind == ROWS) {
-      RowsArgs a;
-      a.in = src;
-      a.out = reinterpret_cast<float2*>(dst);
-      a.tw = d_tw;
-      a.nrows = outer;
-      a.scale = scale;
-      a.do_scale = do_scale;
-      const long long grid = (a.nrows + v->tile - 1) / v->tile;
-      if (grid <= 0) return B200FFT_OK;
-      if (grid > 0x7fffffffLL) return fail(B200FFT_ERR_UNSUPPORTED, "too many row tiles");
-      v->launch_rows(inverse, real_in, a, (unsigned)grid, v->smem, stream);
-    } else if (v->kind == COLS_TMA) {
-      CUtensorMap mi, mo;
-      if (!encode_axis_map(&mi, src, view.inner, view.n, outer, v->tile, v->box_rows) ||
-          !encode_axis_map(&mo, dst, view.inner, view.n, outer, v->tile, v->box_rows))
-        return fail(B200FFT_ERR_CUDA, "cuTensorMapEncodeTiled failed for the strided-axis pass");
-      ColsTmaArgs a;
-      a.tw = d_tw;
-      a.tiles_per_outer = (int)((view.inner + v->tile - 1) / v->tile);
-      a.scale = scale;
-      a.do_scale = do_scale;
-      const long long grid = outer * a.tiles_per_outer;
-      if (grid <= 0) return B200FFT_OK;
-      if (grid > 0x7fffffffLL) return fail(B200FFT_ERR_UNSUPPORTED, "too many column tiles");
-      v->launch_cols_tma(inverse, mi, mo, a, (unsigned)grid, v->smem, stream);
-    } else {
-      ColsArgs a;
-      a.in = src;
-      a.out = reinterpret_cast<float2*>(dst);
-      a.tw = d_tw;
-      a.inner = view.inner;
-      a.tiles_per_outer = (int)((view.inner + v->tile - 1) / v->tile);
-      a.scale = scale;
-      a.do_scale = do_scale;
-      a.reverse = reverse_order ? 1 : 0;
-      const long long grid = outer * a.tiles_per_outer;
-      if (grid <= 0) return B200FFT_OK;
-      if (grid > 0x7fffffffLL) return fail(B200FFT_ERR_UNSUPPORTED, "too many column tiles");
-      v->launch_cols(inverse, real_in, a, (unsigned)grid, v->smem, stream);
-    }
-    g_launch_count.fetch_add(1, std::memory_order_relaxed);
-    B200_CUDA_CHECK(cudaGetLastError());
-    return B200FFT_OK;
-  }
-  int launch_scatter(const void* src, const Scatter& sc, int64_t nbatch, cudaStream_t stream) override {
-    if (v->kind != COLS || !v->launch_scatter || half != HALF_NONE || real_in)
-      return fail(B200FFT_ERR_UNSUPPORTED, "no scattering store for %s", text.c_str());
-    if (sc.npeers < 1 || sc.npeers > 16 || view.n % sc.npeers)
-      return fail(B200FFT_ERR_INVALID_ARG, "split axis length %lld is not divisible by %d peers", (long long)view.n, sc.npeers);
-    ColsArgs a;
-    a.in = src;
-    a.out = nullptr;
-    a.tw = d_tw;
-    a.inner = view.inner;
-    a.tiles_per_outer = (int)((view.inner + v->tile - 1) / v->tile);
-    a.scale = scale;
-    a.do_scale = do_scale;
-    a.reverse = reverse_order ? 1 : 0;
-    ScatterArgs sa;
-    for (int i = 0; i < 16; ++i) sa.peer[i] = i < sc.npeers ? reinterpret_cast<float2*>(sc.peer_out[i]) : nullptr;
-    sa.yl = (int)(view.n / sc.npeers);
-    const long long outer = nbatch * view.outer_per_batch;
-    sa.zbase = sc.zbase >= 0 ? sc.zbase : (long long)sc.my_rank * outer;
-    const long long grid = outer * a.tiles_per_outer;
-    if (grid <= 0) return B200FFT_OK;
-    if (grid > 0x7fffffffLL) return fail(B200FFT_ERR_UNSUPPORTED, "too many column tiles");
-    v->launch_scatter(inverse, a, sa, (unsigned)grid, v->smem, stream);
-    g_launch_count.fetch_add(1, std::memory_order_relaxed);
-    B200_CUDA_CHECK(cudaGetLastError());
-    return B200FFT_OK;
-  }
-  std::string describe() const override { return text; }
-  size_t min_align(bool src) const override {
-    if (v->kind == COLS_TMA) return 16;  // tensor maps need 16-byte global addresses
-    // rowsV: complex-input instantiations load and store through float4 (GlobalSrcV4 / GlobalDstV4)
-    if (half == HALF_NONE && v->kind == ROWS && !real_in && v->name.compare(0, 5, "rowsV") == 0) return 16;
-    // even half spectrum: R2C reads the real row as float2 pairs, C2R stores it as float2 pairs
-    if (r2c_mode != R2C_ODD && half == (src ? HALF_R2C : HALF_C2R)) return 8;
-    return 0;
-  }
-};
-
-}  // namespace
-
 size_t fast_variant_count() {
   register_all();
   return registry().size();
@@ -283,30 +134,17 @@ std::string fast_variant_info(size_t i) {
   register_all();
   if (i >= registry().size()) return "";
   const Variant& v = registry()[i];
-  std::string kind, forms;
-  auto add = [&](const char* f) { forms += (forms.empty() ? "" : ",") + std::string(f); };
-  if (v.kind == ROWS) {
-    kind = v.inv_ok ? "rowsIP" : "rows";
-    add("fwd");
-    if (v.full || v.inv_ok) { add("inv"); add("real"); }
-    if (v.launch_half) { add("r2c"); add("c2r"); }
-    if (v.launch_r2c_reg) add("r2c-reg");
-    if (v.launch_r2c_odd) add("r2c-odd");
-    if (v.launch_c2r_odd) add("c2r-odd");
-  } else if (v.kind == COLS) {
-    kind = "cols";
-    add("fwd");
-    if (v.full) { add("inv"); add("real"); }
-    if (v.launch_scatter) add("scatter");
-  } else {
-    kind = "colsT";  // complex input only: the tensor maps describe complex64 elements
-    add("fwd");
-    add("inv");
-  }
+  static const struct { Form form; const char* name; } forms[] = {
+      {FORM_FWD, "fwd"}, {FORM_INV, "inv"}, {FORM_FWD_REAL, "real"}, {FORM_R2C, "r2c"}, {FORM_C2R, "c2r"},
+      {FORM_R2C_REG, "r2c-reg"}, {FORM_R2C_ODD, "r2c-odd"}, {FORM_C2R_ODD, "c2r-odd"}, {FORM_SCATTER_FWD, "scatter"}};
+  std::string list;
+  for (const auto& f : forms)
+    if (v.sym[f.form]) list += (list.empty() ? "" : ",") + std::string(f.name);
+  const char* kind = v.kind == TILE_ROWS ? "rows" : v.kind == TILE_ROWS_IP ? "rowsIP" : v.kind == TILE_COLS ? "cols" : "colsT";
   return "name=" + v.name + " kind=" + kind + " n=" + std::to_string(v.n) + " radices=" + radix_name(v.radices) +
          " tile=" + std::to_string(v.tile) + " threads=" + std::to_string(v.threads) + " full=" + (v.full ? "1" : "0") +
          " smem=" + std::to_string(v.smem) + " smem_r2c=" + std::to_string(v.smem_r2c) +
-         " smem_c2r=" + std::to_string(v.smem_c2r) + " forms=" + forms;
+         " smem_c2r=" + std::to_string(v.smem_c2r) + " forms=" + list;
 }
 
 std::unique_ptr<Pass> make_fast_pass(b200fft_plan& plan, int axis, const AxisView& view, const IoSpec& src,
@@ -315,40 +153,41 @@ std::unique_ptr<Pass> make_fast_pass(b200fft_plan& plan, int axis, const AxisVie
   const Problem& p = plan.prob;
   if (p.desc.out_dtype != B200FFT_F32 || src.dtype != B200FFT_F32) return nullptr;
   if (view.n > 0x7fffffff) return nullptr;
-  const Kind kind = view.inner == 1 ? ROWS : COLS;
+  const TileKind kind = view.inner == 1 ? TILE_ROWS : TILE_COLS;
   const AxisSpec& ax = p.axes[axis];
 
   std::vector<const Variant*> cands;
-  const bool odd_r2c = half != HALF_NONE && kind == ROWS && view.n % 2 == 1;  // (both directions of an odd half-spectrum axis)
+  const bool odd_r2c = half != HALF_NONE && kind == TILE_ROWS && view.n % 2 == 1;  // (both directions of an odd half-spectrum axis)
   if (odd_r2c) {
     // odd n: the n-point row variant itself — R2C on real input storing bins 0..n/2, C2R on the Hermitian-extended row
     if (src.dtype != B200FFT_F32) return nullptr;
     for (const Variant& v : registry())
-      if (v.kind == ROWS && v.n == (int)view.n && v.launch_r2c_odd && v.launch_c2r_odd && can_group(ax.ordered, v.radices))
+      if (v.kind == TILE_ROWS && v.n == (int)view.n && v.sym[FORM_R2C_ODD] && v.sym[FORM_C2R_ODD] && can_group(ax.ordered, v.radices))
         cands.push_back(&v);
   } else if (half != HALF_NONE) {
-    if (kind != ROWS || view.n % 2) return nullptr;
+    if (kind != TILE_ROWS || view.n % 2) return nullptr;
     const auto reduced = drop_factor_two(ax.ordered);
     for (const Variant& v : registry()) {
-      if (v.kind != ROWS || v.n != (int)(view.n / 2) || !v.launch_half) continue;
+      if (v.kind != TILE_ROWS || v.n != (int)(view.n / 2) || !v.sym[FORM_R2C]) continue;
       for (const auto& o : reduced)
         if (can_group(o, v.radices)) { cands.push_back(&v); break; }
     }
   } else {
     // TMA tiles need 16-byte global strides (even inner), complex fp32 source, a usable encoder
-    const bool tma_ok = kind == COLS && src.comps == 2 && view.inner % 2 == 0 && tensor_map_encoder() != nullptr &&
+    const bool tma_ok = kind == TILE_COLS && src.comps == 2 && view.inner % 2 == 0 && tensor_map_encoder() != nullptr &&
                         (unsigned long long)view.inner * view.n * 8 < (1ull << 40);
     const char* ip_env = std::getenv("B200FFT_ROWS_INPLACE");  // =0: long rows as two split passes again (A/B, tests)
     const bool ip_ok = !(ip_env && ip_env[0] == '0');
+    const Form form = p.desc.inverse ? (src.comps == 1 ? FORM_INV_REAL : FORM_INV) : (src.comps == 1 ? FORM_FWD_REAL : FORM_FWD);
     for (const Variant& v : registry()) {
-      const bool kind_ok = (v.kind == kind || (v.kind == COLS_TMA && tma_ok)) && (ip_ok || !v.inv_ok);
-      if (kind_ok && v.n == (int)view.n && (v.full || v.inv_ok || (!p.desc.inverse && src.comps == 2)) &&
-          can_group(ax.ordered, v.radices))
+      const bool kind_ok =
+          v.kind == kind || (v.kind == TILE_ROWS_IP && kind == TILE_ROWS && ip_ok) || (v.kind == TILE_COLS_TMA && tma_ok);
+      if (kind_ok && v.n == (int)view.n && v.sym[form] && can_group(ax.ordered, v.radices))
         cands.push_back(&v);
     }
   }
   if (cands.empty()) return nullptr;
-  if (kind == COLS && half == HALF_NONE) {
+  if (kind == TILE_COLS && half == HALF_NONE) {
     // a tile wider than the axis's inner extent would leave lanes idle: prefer variants that fit
     std::vector<const Variant*> fit;
     for (const Variant* v : cands)
@@ -377,35 +216,47 @@ std::unique_ptr<Pass> make_fast_pass(b200fft_plan& plan, int axis, const AxisVie
   const Variant* v = cands[0];
   // B200FFT_R2C_SMEM=1: keep the shared-memory Hermitian unpack (A/B knob for the register unpack)
   const char* r2c_env = getenv("B200FFT_R2C_SMEM");
-  const bool r2c_reg = half == HALF_R2C && !odd_r2c && v->launch_r2c_reg && !(r2c_env && atoi(r2c_env) != 0);
-  cudaError_t prep = odd_r2c ? v->prepare_r2c_odd(v->smem) : half != HALF_NONE ? v->prepare_half() : v->prepare(v->smem);
-  if (prep == cudaSuccess && r2c_reg) prep = v->prepare_r2c_reg();
+  const bool r2c_reg = half == HALF_R2C && !odd_r2c && v->sym[FORM_R2C_REG] && !(r2c_env && atoi(r2c_env) != 0);
+  auto pass = std::make_unique<TilePass>();
+  TileSpec& s = pass->spec;
+  s.n = v->n;
+  s.radices = v->radices;
+  s.tile = v->tile;
+  s.threads = v->threads;
+  s.vec = v->vec;
+  s.inverse = half == HALF_NONE ? p.desc.inverse != 0 : half == HALF_C2R;  // (C2R: inverse tables)
+  s.real_in = half == HALF_NONE && src.comps == 1;
+  Form form;
+  pass->smem = v->smem;
+  if (odd_r2c) {
+    s.kind = half == HALF_R2C ? TILE_R2C_ODD : TILE_C2R_ODD;
+    form = half == HALF_R2C ? FORM_R2C_ODD : FORM_C2R_ODD;
+  } else if (half == HALF_R2C) {
+    s.kind = r2c_reg ? TILE_R2C_REG : TILE_R2C;
+    form = r2c_reg ? FORM_R2C_REG : FORM_R2C;
+    pass->smem = r2c_reg ? v->smem_r2c_reg : v->smem_r2c;
+  } else if (half == HALF_C2R) {
+    s.kind = TILE_C2R;
+    form = FORM_C2R;
+    pass->smem = v->smem_c2r;
+  } else {
+    s.kind = v->kind;
+    form = s.inverse ? (s.real_in ? FORM_INV_REAL : FORM_INV) : (s.real_in ? FORM_FWD_REAL : FORM_FWD);
+  }
+  pass->k = {v->sym[form], nullptr, v->name};
+  if (s.kind == TILE_COLS) pass->k_scatter = {v->sym[s.inverse ? FORM_SCATTER_INV : FORM_SCATTER_FWD], nullptr, v->name};
+  cudaError_t prep = prepare_tile(pass->k.sym, pass->smem);
+  if (prep == cudaSuccess && pass->k_scatter.sym) prep = prepare_tile(pass->k_scatter.sym, pass->smem);
   if (prep != cudaSuccess) {
     cudaGetLastError();
     return nullptr;
   }
-  auto pass = std::make_unique<FastPass>();
-  pass->v = v;
   pass->view = view;
-  pass->inverse = p.desc.inverse != 0;
-  pass->real_in = src.comps == 1;
+  pass->device = plan.device;
   pass->do_scale = scale_inverse;
-  pass->scale = scale_inverse ? (float)(1.0 / (double)view.n) : 1.f;
-  pass->half = half;
-  pass->r2c_mode = odd_r2c ? FastPass::R2C_ODD : r2c_reg ? FastPass::R2C_REG : FastPass::R2C_SMEM;
-  if (odd_r2c) pass->real_in = half == HALF_R2C;
-  if (odd_r2c && half == HALF_C2R) pass->scale = (float)(1.0 / (double)view.n);
-  if (half != HALF_NONE && !odd_r2c) {
-    if (half == HALF_C2R) pass->scale = (float)(1.0 / (double)view.n);  // 1/(2H): the inverse is always normalised
-    std::vector<float2> tw2 = build_half_twiddles(view.n, half == HALF_C2R);
-    if (cudaMalloc(&pass->d_tw2, tw2.size() * sizeof(float2)) != cudaSuccess) return nullptr;
-    plan.owned_device.push_back(pass->d_tw2);
-    if (cudaMemcpy(pass->d_tw2, tw2.data(), tw2.size() * sizeof(float2), cudaMemcpyHostToDevice) != cudaSuccess) return nullptr;
-  }
-  std::vector<float2> tw = build_twiddles(v->radices, half == HALF_NONE ? pass->inverse : half == HALF_C2R);  // (C2R: inverse tables)
-  if (cudaMalloc(&pass->d_tw, tw.size() * sizeof(float2)) != cudaSuccess) return nullptr;
-  plan.owned_device.push_back(pass->d_tw);  // owned by the plan BEFORE the copy: a failed copy must not leak it
-  if (cudaMemcpy(pass->d_tw, tw.data(), tw.size() * sizeof(float2), cudaMemcpyHostToDevice) != cudaSuccess) return nullptr;
+  pass->scale = (scale_inverse || half == HALF_C2R) ? 1.0 / (double)view.n : 1.0;  // the half-spectrum inverse is always normalised
+  if (half != HALF_NONE && !odd_r2c && !(pass->tw2 = plan_upload(plan, build_half_twiddles(view.n, half == HALF_C2R)))) return nullptr;
+  if (!(pass->tw = plan_upload(plan, build_twiddles(v->radices, s.inverse)))) return nullptr;
   std::string stages;
   for (uint32_t r : ax.ordered) stages += (stages.empty() ? "" : ",") + std::to_string(r);
   char buf[320];
@@ -422,7 +273,7 @@ std::unique_ptr<Pass> make_fast_pass(b200fft_plan& plan, int axis, const AxisVie
   else
     snprintf(buf, sizeof buf, "axis %d: %s n=%lld inner=%lld smem=%zuB user stages=[%s] fused as (%s)%s", axis,
              v->name.c_str(), (long long)view.n, (long long)view.inner, v->smem, stages.c_str(),
-             radix_name(v->radices).c_str(), pass->real_in ? " real-in" : "");
+             radix_name(v->radices).c_str(), s.real_in ? " real-in" : "");
   pass->text = buf;
   return pass;
 }

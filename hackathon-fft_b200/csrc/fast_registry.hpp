@@ -2,221 +2,47 @@
 #pragma once
 #include <cuda_runtime.h>
 
-#include <cstdlib>
 #include <string>
-#include <utility>
 #include <vector>
 
 #include "fast.cuh"
+#include "tile.hpp"
 
 namespace b200fft {
 
-enum Kind { ROWS = 0, COLS = 1, COLS_TMA = 2 };
+// Instantiations a variant may have, one kernel each (null where the variant has none)
+enum Form {
+  FORM_FWD = 0, FORM_INV, FORM_FWD_REAL, FORM_INV_REAL,  // rows / rowsIP / cols; colsT: FWD and INV only
+  FORM_R2C, FORM_C2R, FORM_R2C_REG, FORM_R2C_ODD, FORM_C2R_ODD,  // half-spectrum forms of a row variant
+  FORM_SCATTER_FWD, FORM_SCATTER_INV,  // cols: the slab exchange fused into the store
+  FORM_COUNT
+};
 
 struct Variant {
   std::string name;
-  Kind kind;
+  TileKind kind;  // TILE_ROWS, TILE_ROWS_IP, TILE_COLS or TILE_COLS_TMA
   int n;
   std::vector<int> radices;
   int tile, threads;
   size_t smem;
-  // inv, real_in
-  void (*launch_rows)(bool, bool, const RowsArgs&, unsigned, size_t, cudaStream_t);
-  void (*launch_cols)(bool, bool, const ColsArgs&, unsigned, size_t, cudaStream_t);
-  cudaError_t (*prepare)(size_t);
-  void (*launch_cols_tma)(bool, const CUtensorMap&, const CUtensorMap&, const ColsTmaArgs&, unsigned, size_t,
-                          cudaStream_t) = nullptr;
-  int box_rows = 0;  // TMA box extent along the transform axis
-  void (*launch_scatter)(bool, const ColsArgs&, const ScatterArgs&, unsigned, size_t, cudaStream_t) = nullptr;
-  bool full;  // has inverse and real-input instantiations
-  bool inv_ok = false;  // not FULL (no R2C / C2R forms), but inverse and real-input instantiations exist (one-buffer rows)
+  bool full;   // has inverse and real-input instantiations
+  bool vec = false;  // complex-input rows move data with 128-bit accesses ("rowsV")
   // half-spectrum real transforms of length 2*n on top of this n-point row variant (FULL only)
-  void (*launch_half)(bool c2r, const HalfArgs&, unsigned, cudaStream_t) = nullptr;
-  cudaError_t (*prepare_half)() = nullptr;
   size_t smem_r2c = 0, smem_c2r = 0;
-  // R2C with the Hermitian unpack in registers (fast.cuh, R2CRegDst): when the last stage keeps a row inside a warp
-  void (*launch_r2c_reg)(const HalfArgs&, unsigned, cudaStream_t) = nullptr;
-  cudaError_t (*prepare_r2c_reg)() = nullptr;
-  size_t smem_r2c_reg = 0;
-  // odd n: half-spectrum R2C of length n itself (real rows in, bins 0..n/2 out) on this n-point variant
-  void (*launch_r2c_odd)(const HalfArgs&, unsigned, size_t, cudaStream_t) = nullptr;
-  cudaError_t (*prepare_r2c_odd)(size_t) = nullptr;
-  // ... and its inverse: rows of n/2+1 bins in, Hermitian-extended on load, real rows out
-  void (*launch_c2r_odd)(const HalfArgs&, unsigned, size_t, cudaStream_t) = nullptr;
+  size_t smem_r2c_reg = 0;  // R2C with the Hermitian unpack in registers (fast.cuh, R2CRegDst)
+  const void* sym[FORM_COUNT] = {};
 };
 
 std::vector<Variant>& registry();
 
 // shared with the fused N-d registry (fused_registry.cu)
 bool can_group(std::vector<uint32_t> ordered, std::vector<int> target);
-std::vector<float2> build_twiddles(const std::vector<int>& radices, bool inverse);
-std::vector<float2> build_half_twiddles(long long n, bool inverse);
 std::vector<std::vector<uint32_t>> drop_factor_two(const std::vector<uint32_t>& ordered);
 // tensor map over the (inner, n, outer) view of a dense complex64 array, box = (cw, box_rows, 1); false
 // when the driver entry point is unavailable or the encode fails
 bool encode_axis_map(CUtensorMap* map, const void* base, long long inner, long long n, long long outer, int cw,
                      int box_rows);
 bool tensor_maps_available();
-
-
-// Launch a pass whose grid may be set up while the previous pass of the same stream is still running (fast.cuh: pdl_wait).
-// Used for the passes that FOLLOW another pass of a plan (strided passes, the C2R row pass). Measured (profiles/r2_pdl.md):
-// 256^3 0.126 -> 0.122 ms, its R2C 0.071 -> 0.066, 2-D 640 x 480 0.161 -> 0.158, 100 x 64^3 0.149 -> 0.146.
-inline bool pdl_enabled() {
-  const char* e = getenv("B200FFT_PDL");  // read per launch (~50 ns): lets one process A/B the two launch modes
-  return !(e && atoi(e) == 0);
-}
-template <class... KArgs, class... Args>
-void launch_dependent(void (*kernel)(KArgs...), unsigned grid, unsigned block, size_t smem, cudaStream_t st, Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(block);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
-}
-
-// FULL variants instantiate forward/inverse x complex/real-input; tuning candidates only
-// forward complex (they are skipped for other requests).
-// VEC: complex-input instantiations use 128-bit global accesses + shuffle exchange (real input keeps 32-bit loads)
-template <int N, class RL, int C, int NT, bool FULL, bool VEC = false>
-struct RowsV {
-  static void launch(bool inv, bool real, const RowsArgs& a, unsigned grid, size_t smem, cudaStream_t st) {
-    if constexpr (FULL) {
-      if (!inv && real) return (void)rows_kernel<N, RL, C, NT, false, true><<<grid, NT, smem, st>>>(a);
-      if (inv && !real) return (void)rows_kernel<N, RL, C, NT, true, false, VEC><<<grid, NT, smem, st>>>(a);
-      if (inv && real) return (void)rows_kernel<N, RL, C, NT, true, true><<<grid, NT, smem, st>>>(a);
-    }
-    rows_kernel<N, RL, C, NT, false, false, VEC><<<grid, NT, smem, st>>>(a);
-  }
-  static cudaError_t prepare(size_t smem) {
-    if (smem <= 48 * 1024) return cudaSuccess;
-    const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;
-    cudaError_t e = cudaFuncSetAttribute(rows_kernel<N, RL, C, NT, false, false, VEC>, attr, (int)smem);
-    if constexpr (FULL) {
-      if (!e) e = cudaFuncSetAttribute(rows_kernel<N, RL, C, NT, false, true>, attr, (int)smem);
-      if (!e) e = cudaFuncSetAttribute(rows_kernel<N, RL, C, NT, true, false, VEC>, attr, (int)smem);
-      if (!e) e = cudaFuncSetAttribute(rows_kernel<N, RL, C, NT, true, true>, attr, (int)smem);
-    }
-    return e;
-  }
-};
-
-template <int N, class RL, int NT>
-struct RowsIpV {
-  static void launch(bool inv, bool real, const RowsArgs& a, unsigned grid, size_t smem, cudaStream_t st) {
-    if (inv && real) rows_ip_kernel<N, RL, 1, NT, true, true><<<grid, NT, smem, st>>>(a);
-    else if (inv) rows_ip_kernel<N, RL, 1, NT, true, false><<<grid, NT, smem, st>>>(a);
-    else if (real) rows_ip_kernel<N, RL, 1, NT, false, true><<<grid, NT, smem, st>>>(a);
-    else rows_ip_kernel<N, RL, 1, NT, false, false><<<grid, NT, smem, st>>>(a);
-  }
-  static cudaError_t prepare(size_t smem) {
-    const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;
-    cudaError_t e = cudaFuncSetAttribute(rows_ip_kernel<N, RL, 1, NT, false, false>, attr, (int)smem);
-    if (!e) e = cudaFuncSetAttribute(rows_ip_kernel<N, RL, 1, NT, true, false>, attr, (int)smem);
-    if (!e) e = cudaFuncSetAttribute(rows_ip_kernel<N, RL, 1, NT, false, true>, attr, (int)smem);
-    if (!e) e = cudaFuncSetAttribute(rows_ip_kernel<N, RL, 1, NT, true, true>, attr, (int)smem);
-    return e;
-  }
-};
-
-template <int H, class RL, int C, int NT>
-struct HalfV {
-  static void launch(bool c2r, const HalfArgs& a, unsigned grid, cudaStream_t st) {
-    if (c2r) launch_dependent(rows_c2r_kernel<H, RL, C, NT>, grid, NT, rows_c2r_smem_bytes<H, RL, C>(), st, a);  // last pass of a C2R plan
-    else rows_r2c_kernel<H, RL, C, NT><<<grid, NT, rows_r2c_smem_bytes<H, RL, C>(), st>>>(a);
-  }
-  static cudaError_t prepare() {
-    const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;
-    cudaError_t e = cudaFuncSetAttribute(rows_r2c_kernel<H, RL, C, NT>, attr, (int)rows_r2c_smem_bytes<H, RL, C>());
-    if (!e) e = cudaFuncSetAttribute(rows_c2r_kernel<H, RL, C, NT>, attr, (int)rows_c2r_smem_bytes<H, RL, C>());
-    return e;
-  }
-};
-
-template <int H, class RL, int C, int NT>
-struct HalfRegV {
-  static void launch(const HalfArgs& a, unsigned grid, cudaStream_t st) {
-    rows_r2c_reg_kernel<H, RL, C, NT><<<grid, NT, rows_r2c_reg_smem_bytes<H, RL, C>(), st>>>(a);
-  }
-  static cudaError_t prepare() {
-    if (rows_r2c_reg_smem_bytes<H, RL, C>() <= 48 * 1024) return cudaSuccess;
-    return cudaFuncSetAttribute(rows_r2c_reg_kernel<H, RL, C, NT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)rows_r2c_reg_smem_bytes<H, RL, C>());
-  }
-};
-template <int N, class RL, int C, int NT>
-struct HalfOddV {
-  static void launch(const HalfArgs& a, unsigned grid, size_t smem, cudaStream_t st) {
-    rows_r2c_odd_kernel<N, RL, C, NT><<<grid, NT, smem, st>>>(a);
-  }
-  static void launch_c2r(const HalfArgs& a, unsigned grid, size_t smem, cudaStream_t st) {
-    launch_dependent(rows_c2r_odd_kernel<N, RL, C, NT>, grid, NT, smem, st, a);  // last pass of a C2R plan
-  }
-  static cudaError_t prepare(size_t smem) {
-    if (smem <= 48 * 1024) return cudaSuccess;
-    cudaError_t e = cudaFuncSetAttribute(rows_r2c_odd_kernel<N, RL, C, NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (!e) e = cudaFuncSetAttribute(rows_c2r_odd_kernel<N, RL, C, NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    return e;
-  }
-};
-
-template <int N, class RL, int CW, int NT, bool FULL>
-struct ColsV {
-  static void launch(bool inv, bool real, const ColsArgs& a, unsigned grid, size_t smem, cudaStream_t st) {
-    if constexpr (FULL) {
-      if (!inv && real) return launch_dependent(cols_kernel<N, RL, CW, NT, false, true>, grid, NT, smem, st, a);
-      if (inv && !real) return launch_dependent(cols_kernel<N, RL, CW, NT, true, false>, grid, NT, smem, st, a);
-      if (inv && real) return launch_dependent(cols_kernel<N, RL, CW, NT, true, true>, grid, NT, smem, st, a);
-    }
-    launch_dependent(cols_kernel<N, RL, CW, NT, false, false>, grid, NT, smem, st, a);
-  }
-  static cudaError_t prepare(size_t smem) {
-    if (smem <= 48 * 1024) return cudaSuccess;
-    const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;
-    cudaError_t e = cudaFuncSetAttribute(cols_kernel<N, RL, CW, NT, false, false>, attr, (int)smem);
-    if constexpr (FULL) {
-      if (!e) e = cudaFuncSetAttribute(cols_kernel<N, RL, CW, NT, false, true>, attr, (int)smem);
-      if (!e) e = cudaFuncSetAttribute(cols_kernel<N, RL, CW, NT, true, false>, attr, (int)smem);
-      if (!e) e = cudaFuncSetAttribute(cols_kernel<N, RL, CW, NT, true, true>, attr, (int)smem);
-    }
-    return e;
-  }
-};
-
-template <int N, class RL, int CW, int NT>
-struct ColsScatterV {
-  static void launch(bool inv, const ColsArgs& a, const ScatterArgs& sa, unsigned grid, size_t smem, cudaStream_t st) {
-    const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;
-    if (inv) {
-      if (smem > 48 * 1024) cudaFuncSetAttribute(cols_scatter_kernel<N, RL, CW, NT, true>, attr, (int)smem);
-      cols_scatter_kernel<N, RL, CW, NT, true><<<grid, NT, smem, st>>>(a, sa);
-    } else {
-      if (smem > 48 * 1024) cudaFuncSetAttribute(cols_scatter_kernel<N, RL, CW, NT, false>, attr, (int)smem);
-      cols_scatter_kernel<N, RL, CW, NT, false><<<grid, NT, smem, st>>>(a, sa);
-    }
-  }
-};
-
-template <int N, class RL, int CW, int NT>
-struct ColsTmaV {
-  static void launch(bool inv, const CUtensorMap& mi, const CUtensorMap& mo, const ColsTmaArgs& a, unsigned grid,
-                     size_t smem, cudaStream_t st) {
-    if (inv) cols_tma_kernel<N, RL, CW, NT, true><<<grid, NT, smem, st>>>(mi, mo, a);
-    else cols_tma_kernel<N, RL, CW, NT, false><<<grid, NT, smem, st>>>(mi, mo, a);
-  }
-  static cudaError_t prepare(size_t smem) {
-    const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;
-    cudaError_t e = cudaFuncSetAttribute(cols_tma_kernel<N, RL, CW, NT, false>, attr, (int)smem);
-    if (!e) e = cudaFuncSetAttribute(cols_tma_kernel<N, RL, CW, NT, true>, attr, (int)smem);
-    return e;
-  }
-};
 
 template <class RL>
 std::vector<int> radix_vec() {
@@ -233,29 +59,31 @@ void reg_rows_impl() {
   using RL = Radices<Rs...>;
   static_assert(RL::product() == N, "radices must multiply to N");
   Variant v;
-  v.kind = ROWS; v.n = N; v.radices = radix_vec<RL>(); v.tile = C; v.threads = NT;
+  v.kind = TILE_ROWS; v.n = N; v.radices = radix_vec<RL>(); v.tile = C; v.threads = NT;
   v.smem = rows_smem_bytes<N, RL, C>();
   v.name = std::string(VEC ? "rowsV" : "rows") + std::to_string(N) + "_" + radix_name(v.radices) + "_c" + std::to_string(C) +
            "_t" + std::to_string(NT);
-  v.launch_rows = &RowsV<N, RL, C, NT, FULL, VEC>::launch;
-  v.launch_cols = nullptr;
-  v.prepare = &RowsV<N, RL, C, NT, FULL, VEC>::prepare;
+  v.vec = VEC;
+  // FULL variants instantiate forward/inverse x complex/real-input; tuning candidates only forward complex (they are
+  // skipped for other requests). Real input keeps the 32-bit loads.
+  v.sym[FORM_FWD] = (const void*)rows_kernel<N, RL, C, NT, false, false, VEC>;
   if constexpr (FULL) {
+    v.sym[FORM_INV] = (const void*)rows_kernel<N, RL, C, NT, true, false, VEC>;
+    v.sym[FORM_FWD_REAL] = (const void*)rows_kernel<N, RL, C, NT, false, true>;
+    v.sym[FORM_INV_REAL] = (const void*)rows_kernel<N, RL, C, NT, true, true>;
     v.smem_r2c = rows_r2c_smem_bytes<N, RL, C>();
     v.smem_c2r = rows_c2r_smem_bytes<N, RL, C>();
     if (v.smem_r2c <= 227 * 1024 && v.smem_c2r <= 227 * 1024) {
-      v.launch_half = &HalfV<N, RL, C, NT>::launch;
-      v.prepare_half = &HalfV<N, RL, C, NT>::prepare;
+      v.sym[FORM_R2C] = (const void*)rows_r2c_kernel<N, RL, C, NT>;
+      v.sym[FORM_C2R] = (const void*)rows_c2r_kernel<N, RL, C, NT>;
       if constexpr (r2c_reg_ok<N, RL, C, NT>()) {
-        v.launch_r2c_reg = &HalfRegV<N, RL, C, NT>::launch;
-        v.prepare_r2c_reg = &HalfRegV<N, RL, C, NT>::prepare;
+        v.sym[FORM_R2C_REG] = (const void*)rows_r2c_reg_kernel<N, RL, C, NT>;
         v.smem_r2c_reg = rows_r2c_reg_smem_bytes<N, RL, C>();
       }
     }
-    if constexpr (N % 2 == 1) {
-      v.launch_r2c_odd = &HalfOddV<N, RL, C, NT>::launch;
-      v.launch_c2r_odd = &HalfOddV<N, RL, C, NT>::launch_c2r;
-      v.prepare_r2c_odd = &HalfOddV<N, RL, C, NT>::prepare;
+    if constexpr (N % 2 == 1) {  // odd n: half-spectrum R2C of length n itself and its inverse on this n-point variant
+      v.sym[FORM_R2C_ODD] = (const void*)rows_r2c_odd_kernel<N, RL, C, NT>;
+      v.sym[FORM_C2R_ODD] = (const void*)rows_c2r_odd_kernel<N, RL, C, NT>;
     }
   }
   v.full = FULL;
@@ -276,14 +104,14 @@ void reg_rows_inplace() {
   using RL = Radices<Rs...>;
   static_assert(RL::product() == N, "radices must multiply to N");
   Variant v;
-  v.kind = ROWS; v.n = N; v.radices = radix_vec<RL>(); v.tile = 1; v.threads = NT;
+  v.kind = TILE_ROWS_IP; v.n = N; v.radices = radix_vec<RL>(); v.tile = 1; v.threads = NT;
   v.smem = rows_ip_smem_bytes<N, RL>();
   v.name = "rowsIP" + std::to_string(N) + "_" + radix_name(v.radices) + "_c1_t" + std::to_string(NT);
-  v.launch_rows = &RowsIpV<N, RL, NT>::launch;
-  v.launch_cols = nullptr;
-  v.prepare = &RowsIpV<N, RL, NT>::prepare;
+  v.sym[FORM_FWD] = (const void*)rows_ip_kernel<N, RL, 1, NT, false, false>;
+  v.sym[FORM_INV] = (const void*)rows_ip_kernel<N, RL, 1, NT, true, false>;
+  v.sym[FORM_FWD_REAL] = (const void*)rows_ip_kernel<N, RL, 1, NT, false, true>;
+  v.sym[FORM_INV_REAL] = (const void*)rows_ip_kernel<N, RL, 1, NT, true, true>;
   v.full = false;
-  v.inv_ok = true;
   registry().push_back(v);
 }
 template <int N, int CW, int NT, bool FULL, int... Rs>
@@ -291,31 +119,32 @@ void reg_cols() {
   using RL = Radices<Rs...>;
   static_assert(RL::product() == N, "radices must multiply to N");
   Variant v;
-  v.kind = COLS; v.n = N; v.radices = radix_vec<RL>(); v.tile = CW; v.threads = NT;
+  v.kind = TILE_COLS; v.n = N; v.radices = radix_vec<RL>(); v.tile = CW; v.threads = NT;
   v.smem = cols_smem_bytes<N, RL, CW>();
   v.name = "cols" + std::to_string(N) + "_" + radix_name(v.radices) + "_w" + std::to_string(CW) + "_t" + std::to_string(NT);
-  v.launch_rows = nullptr;
-  v.launch_cols = &ColsV<N, RL, CW, NT, FULL>::launch;
-  v.prepare = &ColsV<N, RL, CW, NT, FULL>::prepare;
-  if constexpr (FULL) v.launch_scatter = &ColsScatterV<N, RL, CW, NT>::launch;
+  v.sym[FORM_FWD] = (const void*)cols_kernel<N, RL, CW, NT, false, false>;
+  if constexpr (FULL) {
+    v.sym[FORM_INV] = (const void*)cols_kernel<N, RL, CW, NT, true, false>;
+    v.sym[FORM_FWD_REAL] = (const void*)cols_kernel<N, RL, CW, NT, false, true>;
+    v.sym[FORM_INV_REAL] = (const void*)cols_kernel<N, RL, CW, NT, true, true>;
+    v.sym[FORM_SCATTER_FWD] = (const void*)cols_scatter_kernel<N, RL, CW, NT, false>;
+    v.sym[FORM_SCATTER_INV] = (const void*)cols_scatter_kernel<N, RL, CW, NT, true>;
+  }
   v.full = FULL;
   registry().push_back(v);
 }
 
-
+// complex input only: the tensor maps describe complex64 elements
 template <int N, int CW, int NT, int... Rs>
 void reg_cols_tma() {
   using RL = Radices<Rs...>;
   static_assert(RL::product() == N, "radices must multiply to N");
   Variant v;
-  v.kind = COLS_TMA; v.n = N; v.radices = radix_vec<RL>(); v.tile = CW; v.threads = NT;
+  v.kind = TILE_COLS_TMA; v.n = N; v.radices = radix_vec<RL>(); v.tile = CW; v.threads = NT;
   v.smem = cols_tma_smem_bytes<N, CW>();
   v.name = "colsT" + std::to_string(N) + "_" + radix_name(v.radices) + "_w" + std::to_string(CW) + "_t" + std::to_string(NT);
-  v.launch_rows = nullptr;
-  v.launch_cols = nullptr;
-  v.launch_cols_tma = &ColsTmaV<N, RL, CW, NT>::launch;
-  v.prepare = &ColsTmaV<N, RL, CW, NT>::prepare;
-  v.box_rows = tma_box_rows(N);
+  v.sym[FORM_FWD] = (const void*)cols_tma_kernel<N, RL, CW, NT, false>;
+  v.sym[FORM_INV] = (const void*)cols_tma_kernel<N, RL, CW, NT, true>;
   v.full = true;
   registry().push_back(v);
 }

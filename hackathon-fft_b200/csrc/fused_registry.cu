@@ -301,15 +301,6 @@ std::unique_ptr<Pass> make_fused_pass(b200fft_plan& plan) {
   A.in_stride_bytes = in_scalars * (p.desc.in_components == 1 ? 4 : 8);
   A.out_stride = out_pts;
 
-  auto upload = [&](const std::vector<float2>& t, const float2** out) -> bool {
-    float2* d = nullptr;
-    if (cudaMalloc(&d, t.size() * sizeof(float2)) != cudaSuccess) return false;
-    plan.owned_device.push_back(d);
-    if (cudaMemcpy(d, t.data(), t.size() * sizeof(float2), cudaMemcpyHostToDevice) != cudaSuccess) return false;
-    *out = d;
-    return true;
-  };
-
   const bool inv = p.desc.inverse != 0;
   double total_scale = 1.0;
   for (int a = 0; a < p.rank; ++a) total_scale *= (double)dims[a];
@@ -330,7 +321,7 @@ std::unique_ptr<Pass> make_fused_pass(b200fft_plan& plan) {
         const std::vector<float2> half = build_half_twiddles(dims[last], false);
         table.insert(table.end(), half.begin(), half.end());
       }
-      if (!upload(table, &P.tw)) return nullptr;
+      if (!(P.tw = plan_upload(plan, table))) return nullptr;
     }
     P.scale = 1.f;
     P.do_scale = 0;
@@ -339,13 +330,13 @@ std::unique_ptr<Pass> make_fused_pass(b200fft_plan& plan) {
       P.units_per_transform = prod(dims, 0, last);
       P.tiles_per_transform = (int)((P.units_per_transform + ph.tile - 1) / ph.tile);
       P.tiles_per_outer = 1;
-      if (ph.kind == ND_R2C && !upload(build_half_twiddles(dims[last], false), &P.tw2)) return nullptr;
+      if (ph.kind == ND_R2C && !(P.tw2 = plan_upload(plan, build_half_twiddles(dims[last], false)))) return nullptr;
       tile_bytes = (long long)ph.tile * cdims[last] * 8;
     } else if (ph.kind == ND_PLANE || ph.kind == ND_R2C_PLANE) {
       P.units_per_transform = prod(dims, 0, last - 1);
       P.tiles_per_transform = (int)P.units_per_transform;
       P.tiles_per_outer = 1;
-      if (!upload(build_twiddles(ph.radices2, inv), &P.tw2)) return nullptr;
+      if (!(P.tw2 = plan_upload(plan, build_twiddles(ph.radices2, inv)))) return nullptr;
       tile_bytes = cdims[last] * dims[last - 1] * 8;
     } else {  // ND_COLS on axis a
       P.inner = prod(cdims, a + 1, cdims.size());

@@ -34,6 +34,7 @@
 #include "fast_registry.hpp"
 #include "plan.hpp"
 #include "plane.cuh"
+#include "tile.hpp"
 
 namespace b200fft {
 
@@ -91,20 +92,9 @@ const Nvrtc& nvrtc() {
   return api;
 }
 
-// ---- driver entry points through the runtime (no link against libcuda, like the tensor-map encoder) ----------------
-struct Driver {
-  CUresult (*ModuleLoadData)(CUmodule*, const void*) = nullptr;
-  CUresult (*ModuleUnload)(CUmodule) = nullptr;
-  CUresult (*ModuleGetFunction)(CUfunction*, CUmodule, const char*) = nullptr;
-  CUresult (*ModuleGetGlobal)(CUdeviceptr*, size_t*, CUmodule, const char*) = nullptr;
-  CUresult (*FuncSetAttribute)(CUfunction, CUfunction_attribute, int) = nullptr;
-  CUresult (*FuncGetAttribute)(int*, CUfunction_attribute, CUfunction) = nullptr;
-  CUresult (*LaunchKernel)(CUfunction, unsigned, unsigned, unsigned, unsigned, unsigned, unsigned, unsigned, CUstream, void**,
-                           void**) = nullptr;
-  CUresult (*LaunchKernelEx)(const CUlaunchConfig*, CUfunction, void**, void**) = nullptr;  // optional (dependent launches)
-  bool ok = false;
-};
+}  // namespace
 
+// ---- driver entry points through the runtime (no link against libcuda, like the tensor-map encoder) ----------------
 const Driver& driver() {
   static const Driver api = [] {
     Driver d;
@@ -123,189 +113,107 @@ const Driver& driver() {
     d.ModuleGetGlobal = reinterpret_cast<decltype(d.ModuleGetGlobal)>(get("cuModuleGetGlobal"));
     d.FuncSetAttribute = reinterpret_cast<decltype(d.FuncSetAttribute)>(get("cuFuncSetAttribute"));
     d.FuncGetAttribute = reinterpret_cast<decltype(d.FuncGetAttribute)>(get("cuFuncGetAttribute"));
-    d.LaunchKernel = reinterpret_cast<decltype(d.LaunchKernel)>(get("cuLaunchKernel"));
     d.LaunchKernelEx = reinterpret_cast<decltype(d.LaunchKernelEx)>(get("cuLaunchKernelEx"));
-    d.ok = d.ModuleLoadData && d.ModuleUnload && d.ModuleGetFunction && d.ModuleGetGlobal && d.FuncSetAttribute && d.FuncGetAttribute && d.LaunchKernel;
+    d.ok = d.ModuleLoadData && d.ModuleUnload && d.ModuleGetFunction && d.ModuleGetGlobal && d.FuncSetAttribute && d.FuncGetAttribute && d.LaunchKernelEx;
     return d;
   }();
   return api;
 }
 
-// ---- what to compile ------------------------------------------------------------------------------------------------
-enum JitKind {
-  JIT_ROWS = 0,     // rows_kernel<N, RL, C, NT, INV, REAL>: `tile` contiguous transforms per CTA
-  JIT_COLS,         // cols_kernel<N, RL, CW, NT, INV, REAL>: all N points of `tile` adjacent columns of a strided axis
-  JIT_SCATTER,      // cols_scatter_kernel<N, RL, CW, NT, INV>: the same with the slab exchange in its stores
-  JIT_R2C,          // rows_r2c_kernel<H, RL, C, NT>: n = 2H real points as an H-point complex row + shared-memory unpack
-  JIT_R2C_REG,      // rows_r2c_reg_kernel<H, RL, C, NT>: Hermitian unpack in registers (warp shuffles)
-  JIT_R2C_ODD,      // rows_r2c_odd_kernel<N, RL, C, NT>: odd n, the n-point row kernel on real rows, bins 0..n/2 stored
-  JIT_C2R,          // rows_c2r_kernel<H, RL, C, NT>: Hermitian pack fused into stage 0 of the H-point inverse
-  JIT_C2R_ODD,      // rows_c2r_odd_kernel<N, RL, C, NT>: odd n, Hermitian-extended load, real rows stored
-  // long axes as two passes, N = N1 * N2 (fast.cuh, "four-step"):
-  JIT_SPLIT_A,      // cols_split_a_kernel<N1, RL, CW, NT, INV>: N1-point strided transforms, W_N^{k1 n2} fused into the store
-  JIT_SPLIT_B_COLS, // cols_split_b_kernel<N2, RL, CW, NT, INV>: N2-point strided transforms, natural-order store
-  JIT_SPLIT_B_ROWS, // rows_split_b_kernel<N2, RL, C, NT, INV>: the same for a contiguous axis
-  // the two innermost axes in one in-place tile per (y, x) plane (plane.cuh); n = NY, n2 = NX (R2C: H), radices = y, radices2 = x
-  JIT_PLANE_C2C,    // c2c_plane_ip_kernel<NY, NX, RLY, RLX, NT, INV, REAL>
-  JIT_PLANE_R2C,    // r2c_plane_ip_kernel<NY, H, RLY, RLX, NT>
-  JIT_ROWS_IP,      // rows_ip_kernel<N, RL, C, NT, INV, REAL>: `tile` rows per CTA, 3-5 stages in ONE shared buffer
-  // long half-spectrum rows as two passes (split length H = n/2 for even n, n for odd n); pass A of a real-input or
-  // dtype-casting axis is JIT_SPLIT_A with real_in / in_dtype
-  JIT_SPLIT_B_R2C,     // rows_split_b_r2c_kernel<N2, RL, C, NT>: even R2C, (k1, N1 - k1) row pairs, Hermitian unpack in the store
-  JIT_SPLIT_A_C2R,     // cols_split_a_c2r_kernel<N1, RL, CW, NT, false>: even C2R, Hermitian pack in the load
-  JIT_SPLIT_A_C2R_ODD, // cols_split_a_c2r_kernel<N1, RL, CW, NT, true>: odd C2R, Hermitian-extended load
-  JIT_SPLIT_B_HALF,    // rows_split_b_kernel<N2, RL, C, NT, false, 1>: odd R2C, bins 0..n/2 stored
-  JIT_SPLIT_B_REAL,    // rows_split_b_kernel<N2, RL, C, NT, true, 2>: odd C2R, real parts stored
-  // contiguous axes longer than 2^24 points as three passes, n = N1 * N2 * N3 (fast.cuh):
-  JIT_SPLIT3_A,        // cols_split_a_kernel<N, RL, CW, NT, INV, REAL, true>: passes 1 and 2, the twiddle from two tables
-  JIT_SPLIT3_C         // rows_split_c_kernel<N3, RL, C, NT, INV>: pass 3, rows (k1, k2), natural-order store
-};
+namespace {
 
-struct JitSpec {
-  JitKind kind = JIT_ROWS;
-  int n = 0;  // length of the complex transform the kernel runs (H = n_real / 2 for R2C / R2C_REG / C2R)
-  std::vector<int> radices;
-  int n2 = 0;                  // plane kinds: the x extent (R2C: H)
-  std::vector<int> radices2;   // plane kinds: the x stages
-  int tile = 0, threads = 0;
-  bool inverse = false, real_in = false, packed = false;
-  bool f64 = false;            // working precision (the plan's out_dtype): fp64 = the same kernels with the scalar type swapped
-  int in_dtype = B200FFT_F32;  // element type of the array the kernel READS (cast on load)
-
-  size_t esz() const { return f64 ? sizeof(double2) : sizeof(float2); }
-  int tile_divides = 0;        // geometry only: the tile must divide this (split pass B rows never straddle transforms)
-  long long rows_hint = 0;     // geometry only: transforms per call when the planner knows it (few rows: more threads per row)
-  bool plane() const { return kind == JIT_PLANE_C2C || kind == JIT_PLANE_R2C; }
-  std::string plane_args() const {  // "<NY, NX, Radices<y...>, Radices<x...>"
-    std::string ry, rx;
-    for (int r : radices) ry += (ry.empty() ? "" : ", ") + std::to_string(r);
-    for (int r : radices2) rx += (rx.empty() ? "" : ", ") + std::to_string(r);
-    return std::to_string(n) + ", " + std::to_string(n2) + ", b200fft::Radices<" + ry + ">, b200fft::Radices<" + rx + ">";
+// ---- what to compile: the NVRTC source of a TileSpec (tile.hpp) ----------------------------------------------------
+std::string radix_list(const std::vector<int>& radices) {
+  std::string s;
+  for (int r : radices) s += (s.empty() ? "" : ", ") + std::to_string(r);
+  return s;
+}
+std::string plane_args(const TileSpec& s) {  // "<NY, NX, Radices<y...>, Radices<x...>"
+  return std::to_string(s.n) + ", " + std::to_string(s.n2) + ", b200fft::Radices<" + radix_list(s.radices) + ">, b200fft::Radices<" +
+         radix_list(s.radices2) + ">";
+}
+std::string shape_args(const TileSpec& s) {  // "<N, Radices<...>, tile" shared by every kernel and smem-size template
+  return std::to_string(s.n) + ", b200fft::Radices<" + radix_list(s.radices) + ">, " + std::to_string(s.tile);
+}
+std::string expression(const TileSpec& s) {  // the template-id NVRTC instantiates
+  const std::string head = shape_args(s) + ", " + std::to_string(s.threads);
+  const char* inv = s.inverse ? "true" : "false";
+  const char* real = s.real_in ? "true" : "false";
+  switch (s.kind) {
+    case TILE_PLANE_C2C: return "b200fft::c2c_plane_ip_kernel<" + plane_args(s) + ", " + std::to_string(s.threads) + ", " + inv + ", " + real + ">";
+    case TILE_PLANE_R2C: return "b200fft::r2c_plane_ip_kernel<" + plane_args(s) + ", " + std::to_string(s.threads) + ">";
+    case TILE_ROWS: return "b200fft::rows_kernel<" + head + ", " + inv + ", " + real + ">";
+    case TILE_ROWS_IP:
+      return "b200fft::rows_ip_kernel<" + head + ", " + inv + ", " + real + ">";
+    case TILE_COLS: return "b200fft::cols_kernel<" + head + ", " + inv + ", " + real + ">";
+    case TILE_SCATTER: return "b200fft::cols_scatter_kernel<" + head + ", " + inv + ">";
+    case TILE_R2C: return "b200fft::rows_r2c_kernel<" + head + ">";
+    case TILE_R2C_REG: return "b200fft::rows_r2c_reg_kernel<" + head + ">";
+    case TILE_R2C_ODD: return "b200fft::rows_r2c_odd_kernel<" + head + ">";
+    case TILE_C2R_ODD: return "b200fft::rows_c2r_odd_kernel<" + head + ">";
+    case TILE_SPLIT_A: return "b200fft::cols_split_a_kernel<" + head + ", " + inv + (s.real_in ? ", true>" : ">");
+    case TILE_SPLIT_A_C2R: return "b200fft::cols_split_a_c2r_kernel<" + head + ", false>";
+    case TILE_SPLIT_A_C2R_ODD: return "b200fft::cols_split_a_c2r_kernel<" + head + ", true>";
+    case TILE_SPLIT_B_R2C: return "b200fft::rows_split_b_r2c_kernel<" + head + ">";
+    case TILE_SPLIT_B_HALF: return "b200fft::rows_split_b_kernel<" + head + ", false, 1>";
+    case TILE_SPLIT_B_REAL: return "b200fft::rows_split_b_kernel<" + head + ", true, 2>";
+    case TILE_SPLIT_B_COLS: return "b200fft::cols_split_b_kernel<" + head + ", " + inv + ">";
+    case TILE_SPLIT_B_ROWS: return "b200fft::rows_split_b_kernel<" + head + ", " + inv + ">";
+    case TILE_SPLIT3_A: return "b200fft::cols_split_a_kernel<" + head + ", " + inv + ", " + real + ", true>";
+    case TILE_SPLIT3_C: return "b200fft::rows_split_c_kernel<" + head + ", " + inv + ">";
+    default: return "b200fft::rows_c2r_kernel<" + head + ">";
   }
-  bool strided() const {
-    return kind == JIT_COLS || kind == JIT_SCATTER || kind == JIT_SPLIT_A || kind == JIT_SPLIT_B_COLS || kind == JIT_SPLIT_A_C2R ||
-           kind == JIT_SPLIT_A_C2R_ODD || kind == JIT_SPLIT3_A;
+}
+std::string smem_expression(const TileSpec& s) {  // fast.cuh's own constexpr for the instantiation's dynamic shared memory
+  switch (s.kind) {
+    case TILE_PLANE_C2C:
+      return "b200fft::c2c_plane_ip_smem_bytes<" + std::to_string(s.n) + ", " + std::to_string(s.n2) + ", b200fft::Radices<" +
+             std::to_string(s.radices2[0]) + ", " + std::to_string(s.radices2[1]) + ">>()";
+    case TILE_PLANE_R2C:
+      return "b200fft::r2c_plane_ip_smem_bytes<" + std::to_string(s.n) + ", " + std::to_string(s.n2) + ", b200fft::Radices<" +
+             std::to_string(s.radices2[0]) + ", " + std::to_string(s.radices2[1]) + ">>()";
+    case TILE_ROWS_IP: return "b200fft::rows_ip_smem_bytes<" + shape_args(s) + ">()";
+    case TILE_ROWS:
+    case TILE_SPLIT_B_ROWS:
+    case TILE_SPLIT_B_HALF:
+    case TILE_SPLIT_B_REAL:
+    case TILE_SPLIT3_C:
+    case TILE_C2R_ODD:
+    case TILE_R2C_ODD: return "b200fft::rows_smem_bytes<" + shape_args(s) + ">()";
+    case TILE_COLS:
+    case TILE_SPLIT_A:
+    case TILE_SPLIT_B_COLS:
+    case TILE_SPLIT_A_C2R:
+    case TILE_SPLIT_A_C2R_ODD:
+    case TILE_SPLIT3_A:
+    case TILE_SCATTER: return "b200fft::cols_smem_bytes<" + shape_args(s) + ">()";
+    case TILE_R2C:
+    case TILE_SPLIT_B_R2C: return "b200fft::rows_r2c_smem_bytes<" + shape_args(s) + ">()";
+    case TILE_R2C_REG: return "b200fft::rows_r2c_reg_smem_bytes<" + shape_args(s) + ">()";
+    default: return "b200fft::rows_c2r_smem_bytes<" + shape_args(s) + ">()";
   }
-  std::string radix_list() const {
-    std::string s;
-    for (int r : radices) s += (s.empty() ? "" : ", ") + std::to_string(r);
-    return s;
-  }
-  std::string shape_args() const {  // "<N, Radices<...>, tile" shared by every kernel and smem-size template
-    return std::to_string(n) + ", b200fft::Radices<" + radix_list() + ">, " + std::to_string(tile);
-  }
-  std::string expression() const {  // the template-id NVRTC instantiates
-    const std::string head = shape_args() + ", " + std::to_string(threads);
-    const char* inv = inverse ? "true" : "false";
-    const char* real = real_in ? "true" : "false";
-    switch (kind) {
-      case JIT_PLANE_C2C: return "b200fft::c2c_plane_ip_kernel<" + plane_args() + ", " + std::to_string(threads) + ", " + inv + ", " + real + ">";
-      case JIT_PLANE_R2C: return "b200fft::r2c_plane_ip_kernel<" + plane_args() + ", " + std::to_string(threads) + ">";
-      case JIT_ROWS: return "b200fft::rows_kernel<" + head + ", " + inv + ", " + real + ">";
-      case JIT_ROWS_IP:
-        return "b200fft::rows_ip_kernel<" + head + ", " + inv + ", " + real + ">";
-      case JIT_COLS: return "b200fft::cols_kernel<" + head + ", " + inv + ", " + real + ">";
-      case JIT_SCATTER: return "b200fft::cols_scatter_kernel<" + head + ", " + inv + ">";
-      case JIT_R2C: return "b200fft::rows_r2c_kernel<" + head + ">";
-      case JIT_R2C_REG: return "b200fft::rows_r2c_reg_kernel<" + head + ">";
-      case JIT_R2C_ODD: return "b200fft::rows_r2c_odd_kernel<" + head + ">";
-      case JIT_C2R_ODD: return "b200fft::rows_c2r_odd_kernel<" + head + ">";
-      case JIT_SPLIT_A: return "b200fft::cols_split_a_kernel<" + head + ", " + inv + (real_in ? ", true>" : ">");
-      case JIT_SPLIT_A_C2R: return "b200fft::cols_split_a_c2r_kernel<" + head + ", false>";
-      case JIT_SPLIT_A_C2R_ODD: return "b200fft::cols_split_a_c2r_kernel<" + head + ", true>";
-      case JIT_SPLIT_B_R2C: return "b200fft::rows_split_b_r2c_kernel<" + head + ">";
-      case JIT_SPLIT_B_HALF: return "b200fft::rows_split_b_kernel<" + head + ", false, 1>";
-      case JIT_SPLIT_B_REAL: return "b200fft::rows_split_b_kernel<" + head + ", true, 2>";
-      case JIT_SPLIT_B_COLS: return "b200fft::cols_split_b_kernel<" + head + ", " + inv + ">";
-      case JIT_SPLIT_B_ROWS: return "b200fft::rows_split_b_kernel<" + head + ", " + inv + ">";
-      case JIT_SPLIT3_A: return "b200fft::cols_split_a_kernel<" + head + ", " + inv + ", " + real + ", true>";
-      case JIT_SPLIT3_C: return "b200fft::rows_split_c_kernel<" + head + ", " + inv + ">";
-      default: return "b200fft::rows_c2r_kernel<" + head + ">";
-    }
-  }
-  std::string smem_expression() const {  // fast.cuh's own constexpr for the instantiation's dynamic shared memory
-    switch (kind) {
-      case JIT_PLANE_C2C:
-        return "b200fft::c2c_plane_ip_smem_bytes<" + std::to_string(n) + ", " + std::to_string(n2) + ", b200fft::Radices<" +
-               std::to_string(radices2[0]) + ", " + std::to_string(radices2[1]) + ">>()";
-      case JIT_PLANE_R2C:
-        return "b200fft::r2c_plane_ip_smem_bytes<" + std::to_string(n) + ", " + std::to_string(n2) + ", b200fft::Radices<" +
-               std::to_string(radices2[0]) + ", " + std::to_string(radices2[1]) + ">>()";
-      case JIT_ROWS_IP: return "b200fft::rows_ip_smem_bytes<" + shape_args() + ">()";
-      case JIT_ROWS:
-      case JIT_SPLIT_B_ROWS:
-      case JIT_SPLIT_B_HALF:
-      case JIT_SPLIT_B_REAL:
-      case JIT_SPLIT3_C:
-      case JIT_C2R_ODD:
-      case JIT_R2C_ODD: return "b200fft::rows_smem_bytes<" + shape_args() + ">()";
-      case JIT_COLS:
-      case JIT_SPLIT_A:
-      case JIT_SPLIT_B_COLS:
-      case JIT_SPLIT_A_C2R:
-      case JIT_SPLIT_A_C2R_ODD:
-      case JIT_SPLIT3_A:
-      case JIT_SCATTER: return "b200fft::cols_smem_bytes<" + shape_args() + ">()";
-      case JIT_R2C:
-      case JIT_SPLIT_B_R2C: return "b200fft::rows_r2c_smem_bytes<" + shape_args() + ">()";
-      case JIT_R2C_REG: return "b200fft::rows_r2c_reg_smem_bytes<" + shape_args() + ">()";
-      default: return "b200fft::rows_c2r_smem_bytes<" + shape_args() + ">()";
-    }
-  }
-  std::string name() const {
-    static const char* const tag[] = {"jitrows", "jitcols", "jitscatter", "jitr2c", "jitr2creg", "jitr2codd", "jitc2r", "jitc2rodd",
-                                      "jitsplitA", "jitsplitBcols", "jitsplitBrows", "jitplane", "jitr2cplane", "jitrowsIP",
-                                      "jitsplitBr2c", "jitsplitAc2r", "jitsplitAc2rodd", "jitsplitBhalf", "jitsplitBreal",
-                                      "jitsplit3A", "jitsplit3C"};
-    if (plane())
-      return std::string(tag[kind]) + std::to_string(n) + "x" + std::to_string(kind == JIT_PLANE_R2C ? 2 * n2 : n2) + "(" + radix_name(radices) +
-             ";" + radix_name(radices2) + ")_inplace_t" + std::to_string(threads) + (f64 ? "_f64" : "");
-    return std::string(tag[kind]) + std::to_string(n) + "_" + radix_name(radices) + (strided() ? "_w" : "_c") + std::to_string(tile) +
-           "_t" + std::to_string(threads) + (f64 ? "_f64" : "") + ((kind == JIT_SPLIT_A || kind == JIT_SPLIT3_A) && real_in ? "_realin" : "") + (in_dtype == B200FFT_U8 ? "_inu8" : in_dtype == (f64 ? B200FFT_F32 : B200FFT_F64) ? (f64 ? "_inf32" : "_inf64") : "");
-  }
-  std::string defines() const {  // rtc_prelude.cuh reads these
-    std::string d;
-    if (in_dtype == B200FFT_U8) d += "#define B200FFT_JIT_IN_U8 1\n";
-    if (in_dtype == B200FFT_F64) d += "#define B200FFT_JIT_IN_F64 1\n";
-    if (f64) d += "#define B200FFT_JIT_F64 1\n";
-    if (packed && !f64) d += "#define B200FFT_PACKED 1\n";
-    return d;
-  }
-  std::string key() const { return expression() + "|" + defines(); }
-  // Host mirror of the smem_expression() formulas (fast.cuh): used to choose the tile before anything is compiled, and
-  // checked against the value the compiled module reports (b200fft_jit_smem_bytes) when it is loaded.
-  // RowLayout pads a Q-block by P elements when P < 16, Q even and Q < N; DenseLayout is N x CW.
-  size_t smem() const {
-    if (plane()) return esz() * (size_t)n * (size_t)(n2 + n2 / radices2[0]);  // one buffer of NY rows, pitch NX + NX / r0
-    long long P = 1, ex = 0;
-    if (kind == JIT_ROWS_IP) {  // rows_ip_smem_bytes: the largest exchange layout, once
-      for (size_t s = 0; s + 1 < radices.size(); ++s) {
-        const long long Q = P * radices[s];
-        ex = std::max(ex, (P < 16 && Q % 2 == 0 && Q < n) ? n + n / Q * P : (long long)n);
-        P = Q;
-      }
-      return esz() * (size_t)ex * (size_t)tile;
-    }
-    for (size_t s = 0; s + 1 < radices.size(); ++s) {
-      const long long Q = P * radices[s];
-      long long elems;
-      if (strided()) {
-        elems = (long long)n * tile;
-      } else {
-        const bool padded = P < 16 && Q % 2 == 0 && Q < n;
-        elems = (long long)tile * (padded ? n + n / Q * P : n);
-      }
-      ex = std::max(ex, elems);
-      P = Q;
-    }
-    const size_t pingpong = radices.size() > 2 ? 2 : 1;
-    switch (kind) {
-      case JIT_R2C:
-      case JIT_SPLIT_B_R2C: return esz() * (size_t)std::max<long long>(ex, (long long)tile * n) * 2;
-      default: return esz() * (size_t)ex * pingpong;
-    }
-  }
-};
+}
+std::string jit_name(const TileSpec& s) {
+  static const char* const tag[] = {"jitrows", "jitcols", "jitscatter", "jitr2c", "jitr2creg", "jitr2codd", "jitc2r", "jitc2rodd",
+                                    "jitsplitA", "jitsplitBcols", "jitsplitBrows", "jitplane", "jitr2cplane", "jitrowsIP",
+                                    "jitsplitBr2c", "jitsplitAc2r", "jitsplitAc2rodd", "jitsplitBhalf", "jitsplitBreal",
+                                    "jitsplit3A", "jitsplit3C"};
+  if (s.plane())
+    return std::string(tag[s.kind]) + std::to_string(s.n) + "x" + std::to_string(s.kind == TILE_PLANE_R2C ? 2 * s.n2 : s.n2) + "(" +
+           radix_name(s.radices) + ";" + radix_name(s.radices2) + ")_inplace_t" + std::to_string(s.threads) + (s.f64 ? "_f64" : "");
+  return std::string(tag[s.kind]) + std::to_string(s.n) + "_" + radix_name(s.radices) + (s.strided() ? "_w" : "_c") + std::to_string(s.tile) +
+         "_t" + std::to_string(s.threads) + (s.f64 ? "_f64" : "") + ((s.kind == TILE_SPLIT_A || s.kind == TILE_SPLIT3_A) && s.real_in ? "_realin" : "") +
+         (s.in_dtype == B200FFT_U8 ? "_inu8" : s.in_dtype == (s.f64 ? B200FFT_F32 : B200FFT_F64) ? (s.f64 ? "_inf32" : "_inf64") : "");
+}
+std::string defines(const TileSpec& s) {  // rtc_prelude.cuh reads these
+  std::string d;
+  if (s.in_dtype == B200FFT_U8) d += "#define B200FFT_JIT_IN_U8 1\n";
+  if (s.in_dtype == B200FFT_F64) d += "#define B200FFT_JIT_IN_F64 1\n";
+  if (s.f64) d += "#define B200FFT_JIT_F64 1\n";
+  if (s.packed && !s.f64) d += "#define B200FFT_PACKED 1\n";
+  return d;
+}
+std::string spec_key(const TileSpec& s) { return expression(s) + "|" + defines(s); }
 
 struct JitKernel {
   CUmodule module = nullptr;
@@ -316,19 +224,19 @@ struct JitKernel {
 };
 
 // compile `spec` to a cubin for sm_100a; `lowered` receives the kernel's mangled name
-int compile(const JitSpec& spec, std::vector<char>* cubin, std::string* lowered, std::string* log, double* ms) {
+int compile(const TileSpec& spec, std::vector<char>* cubin, std::string* lowered, std::string* log, double* ms) {
   const Nvrtc& rtc = nvrtc();
   if (!rtc.ok) return fail(B200FFT_ERR_UNSUPPORTED, "run-time compilation unavailable: %s", rtc.why.c_str());
   const auto t0 = std::chrono::steady_clock::now();
-  std::string src = spec.defines();
+  std::string src = defines(spec);
   src += "#include \"fast.cuh\"\n#include \"plane.cuh\"\n";
-  src += "extern \"C\" __device__ unsigned long long b200fft_jit_smem_bytes = (unsigned long long)" + spec.smem_expression() + ";\n";
+  src += "extern \"C\" __device__ unsigned long long b200fft_jit_smem_bytes = (unsigned long long)" + smem_expression(spec) + ";\n";
   const char* headers[] = {k_src_rtc_prelude, k_src_dft, k_src_tma, k_src_fast, k_src_plane};
   const char* names[] = {"rtc_prelude.cuh", "dft.cuh", "tma.cuh", "fast.cuh", "plane.cuh"};
   Nvrtc::Program prog = nullptr;
   int rc = rtc.CreateProgram(&prog, src.c_str(), "b200fft_jit.cu", 5, headers, names);
   if (rc) return fail(B200FFT_ERR_CUDA, "nvrtcCreateProgram: %s", rtc.GetErrorString(rc));
-  const std::string expr = spec.expression();
+  const std::string expr = expression(spec);
   rc = rtc.AddNameExpression(prog, expr.c_str());
   // -default-device: the headers' plain constexpr helpers (index arithmetic, compile-time trigonometry) are device
   // functions here, which is what --expt-relaxed-constexpr gives them under nvcc
@@ -356,7 +264,7 @@ int compile(const JitSpec& spec, std::vector<char>* cubin, std::string* lowered,
   if (rc) return fail(B200FFT_ERR_CUDA, "nvrtcGetCUBIN: %s", rtc.GetErrorString(rc));
   *ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
   if (const char* dir = getenv("B200FFT_JIT_DUMP_DIR")) {  // keep the cubin (cuobjdump -sass <file>: profiles/sass/)
-    const std::string path = std::string(dir) + "/" + spec.name() + ".cubin";
+    const std::string path = std::string(dir) + "/" + jit_name(spec) + ".cubin";
     if (FILE* f = fopen(path.c_str(), "wb")) {
       fwrite(cubin->data(), 1, cubin->size(), f);
       fclose(f);
@@ -389,7 +297,7 @@ std::string disk_cache_dir() {
     }
   return dir;
 }
-std::string disk_cache_path(const JitSpec& spec) {
+std::string disk_cache_path(const TileSpec& spec) {
   static const uint64_t src_hash = [] {
     uint64_t h = fnv1a(k_src_rtc_prelude, strlen(k_src_rtc_prelude));
     h = fnv1a(k_src_dft, strlen(k_src_dft), h);
@@ -399,7 +307,7 @@ std::string disk_cache_path(const JitSpec& spec) {
   }();
   static const std::string dir = disk_cache_dir();
   if (dir.empty()) return "";
-  const std::string key = spec.key() + "|" + spec.smem_expression();
+  const std::string key = spec_key(spec) + "|" + smem_expression(spec);
   char name[64];
   snprintf(name, sizeof name, "/%016llx.cubin", (unsigned long long)fnv1a(key.data(), key.size(), src_hash));
   return dir + name;
@@ -449,13 +357,13 @@ std::map<std::string, std::shared_ptr<JitKernel>>& cache() {
 }
 
 // compiled + loaded kernel for `spec` on `device` (the current device), from the cache when it was built before
-std::shared_ptr<JitKernel> get_kernel(const JitSpec& spec, int device) {
+std::shared_ptr<JitKernel> get_kernel(const TileSpec& spec, int device) {
   const Driver& drv = driver();
   if (!drv.ok) {
     fail(B200FFT_ERR_UNSUPPORTED, "driver entry points for module loading are unavailable");
     return nullptr;
   }
-  const std::string key = std::to_string(device) + "|" + spec.key();
+  const std::string key = std::to_string(device) + "|" + spec_key(spec);
   std::lock_guard<std::mutex> lock(g_jit_mutex);
   auto it = cache().find(key);
   if (it != cache().end()) return it->second;
@@ -477,7 +385,7 @@ std::shared_ptr<JitKernel> get_kernel(const JitSpec& spec, int device) {
   k->compile_ms = ms;
   cudaFree(0);  // make sure the primary context of the current device exists and is current
   if (drv.ModuleLoadData(&k->module, cubin.data()) != CUDA_SUCCESS || drv.ModuleGetFunction(&k->fn, k->module, lowered.c_str()) != CUDA_SUCCESS) {
-    fail(B200FFT_ERR_CUDA, "cannot load the compiled module for %s", spec.expression().c_str());
+    fail(B200FFT_ERR_CUDA, "cannot load the compiled module for %s", expression(spec).c_str());
     if (k->module) drv.ModuleUnload(k->module);
     if (from_disk) remove(on_disk.c_str());  // a damaged cache file: the next plan compiles afresh
     cache()[key] = nullptr;
@@ -491,7 +399,7 @@ std::shared_ptr<JitKernel> get_kernel(const JitSpec& spec, int device) {
         cudaMemcpy(&reported, reinterpret_cast<const void*>(gp), sizeof reported, cudaMemcpyDeviceToHost) != cudaSuccess ||
         reported != (unsigned long long)spec.smem()) {
       cudaGetLastError();
-      fail(B200FFT_ERR_CUDA, "%s: module reports %llu B of shared memory, the planner computed %zu", spec.name().c_str(), reported,
+      fail(B200FFT_ERR_CUDA, "%s: module reports %llu B of shared memory, the planner computed %zu", jit_name(spec).c_str(), reported,
            spec.smem());
       if (getenv("B200FFT_JIT_VERBOSE")) fprintf(stderr, "[b200fft jit] %s\n", last_error().c_str());
       drv.ModuleUnload(k->module);
@@ -503,17 +411,26 @@ std::shared_ptr<JitKernel> get_kernel(const JitSpec& spec, int device) {
   drv.FuncGetAttribute(&k->local_bytes, CU_FUNC_ATTRIBUTE_LOCAL_SIZE_BYTES, k->fn);
   const size_t smem = spec.smem();
   if (smem > 48 * 1024 && drv.FuncSetAttribute(k->fn, CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES, (int)smem) != CUDA_SUCCESS) {
-    fail(B200FFT_ERR_CUDA, "cannot reserve %zu B of shared memory for %s", smem, spec.name().c_str());
+    fail(B200FFT_ERR_CUDA, "cannot reserve %zu B of shared memory for %s", smem, jit_name(spec).c_str());
     drv.ModuleUnload(k->module);
     cache()[key] = nullptr;
     return nullptr;
   }
   if (getenv("B200FFT_JIT_VERBOSE"))
-    fprintf(stderr, "[b200fft jit] %s: %.0f ms, cubin %zu B, %d registers, %d B local\n", spec.expression().c_str(), ms, cubin.size(),
+    fprintf(stderr, "[b200fft jit] %s: %.0f ms, cubin %zu B, %d registers, %d B local\n", expression(spec).c_str(), ms, cubin.size(),
             k->regs, k->local_bytes);
   cache()[key] = k;
   return k;
 }
+
+}  // namespace
+
+TileKernel jit_tile_kernel(const TileSpec& spec, int device) {
+  const std::shared_ptr<JitKernel> k = get_kernel(spec, device);
+  return {nullptr, k ? k->fn : nullptr, jit_name(spec)};
+}
+
+namespace {
 
 // Group the user's ordered stage list into super-stages (register codelets): products <= 32, fewest stages, balanced
 // (the longest-processing-time rule rt.cu uses); a prime base above 32 (the reference allows any prime, fft.mojo:83-104
@@ -582,7 +499,7 @@ bool jit_group(const std::vector<uint32_t>& ordered, std::vector<int>* out, bool
 // stage with the LARGEST radix (fewest butterflies; up to four rounds when that would be too many threads), tiles of
 // 16-48 KB so several CTAs share an SM, strided tiles 16 columns wide (128 contiguous bytes per axis step) unless the
 // axis is so long that only 8 fit. Every candidate (tile, rounds) is scored; the cheapest wins.
-bool jit_geometry(JitSpec* s, long long inner) {
+bool jit_geometry(TileSpec* s, long long inner) {
   const int rmax = *std::max_element(s->radices.begin(), s->radices.end());
   const int rlast = s->radices.back();
   const long long per = (long long)s->n / rmax;  // butterflies of the widest stage per sub-transform
@@ -600,9 +517,9 @@ bool jit_geometry(JitSpec* s, long long inner) {
     s->tile = tile;
     const size_t smem = s->smem();
     if (smem > 200 * 1024) continue;
-    if (s->kind == JIT_R2C_REG && ((long long)tile * (s->n / rlast)) % 32 != 0) continue;  // r2c_reg_ok(): whole warps per row group
+    if (s->kind == TILE_R2C_REG && ((long long)tile * (s->n / rlast)) % 32 != 0) continue;  // r2c_reg_ok(): whole warps per row group
     if (s->tile_divides > 0 && s->tile_divides % tile != 0) continue;
-    if (s->kind == JIT_SPLIT_B_R2C && tile % 2) continue;  // whole (k1, N1 - k1) row pairs
+    if (s->kind == TILE_SPLIT_B_R2C && tile % 2) continue;  // whole (k1, N1 - k1) row pairs
     const long long work = tile * per;
     const double bytes = (double)tile * s->n * (double)s->esz();
     for (int rounds = 1; rounds <= 4; ++rounds) {
@@ -627,7 +544,7 @@ bool jit_geometry(JitSpec* s, long long inner) {
 }
 
 // rows_ip_kernel (fast.cuh): one row per CTA; the in-place middle stage holds rounds * r1 points per thread in registers
-bool jit_rows_ip_geometry(JitSpec* s) {
+bool jit_rows_ip_geometry(TileSpec* s) {
   if (s->radices.size() < 3 || s->radices.size() > 5) return false;
   const char* env = getenv("B200FFT_ROWS_INPLACE");
   if (env && env[0] == '0') return false;
@@ -668,180 +585,10 @@ bool jit_rows_ip_geometry(JitSpec* s) {
   return s->smem() <= 200 * 1024;
 }
 
-size_t in_scalar_bytes(int dtype) { return dtype == B200FFT_U8 ? 1 : dtype == B200FFT_F64 ? 8 : 4; }
-
 // rows_r2c_reg_kernel's precondition (fast.cuh: r2c_reg_ok) apart from the tile, which jit_geometry picks
-bool r2c_reg_shape_ok(const JitSpec& s) {
+bool r2c_reg_shape_ok(const TileSpec& s) {
   const int P = s.n / s.radices.back();
   return s.radices.size() >= 1 && P >= 8 && P <= 32 && 32 % P == 0;
-}
-
-struct JitPass : Pass {
-  JitSpec spec;
-  std::shared_ptr<JitKernel> k;
-  std::shared_ptr<JitKernel> k_scatter;  // compiled on the first launch_scatter
-  AxisView view;
-  int device = 0;
-  bool do_scale = false;
-  double scale = 1.0;
-  void* d_tw = nullptr;   // stage twiddles, float2 or double2
-  void* d_tw2 = nullptr;  // W_n^{+-k} of the Hermitian unpack / pack
-  size_t smem = 0;
-  std::string text;
-
-  int launch(const void* src, void* dst, int64_t nbatch, cudaStream_t stream) override {
-    return launch_outer(src, dst, nbatch * view.outer_per_batch, stream);
-  }
-  int run(const JitKernel& kern, const JitSpec& sp, long long grid, void** params, cudaStream_t stream) {
-    if (grid <= 0) return B200FFT_OK;
-    if (grid > 0x7fffffffLL) return fail(B200FFT_ERR_UNSUPPORTED, "too many tiles");
-    // a pass that follows another pass of the plan: programmatic dependent launch (fast.cuh: pdl_wait; profiles/r2_pdl.md)
-    const bool dependent = (sp.kind == JIT_COLS || sp.kind == JIT_C2R || sp.kind == JIT_C2R_ODD) && driver().LaunchKernelEx && pdl_enabled();
-    CUresult r;
-    if (dependent) {
-      CUlaunchConfig cfg;
-      memset(&cfg, 0, sizeof cfg);
-      cfg.gridDimX = (unsigned)grid;
-      cfg.gridDimY = cfg.gridDimZ = 1;
-      cfg.blockDimX = (unsigned)sp.threads;
-      cfg.blockDimY = cfg.blockDimZ = 1;
-      cfg.sharedMemBytes = (unsigned)sp.smem();
-      cfg.hStream = (CUstream)stream;
-      CUlaunchAttribute attr;
-      memset(&attr, 0, sizeof attr);
-      attr.id = CU_LAUNCH_ATTRIBUTE_PROGRAMMATIC_STREAM_SERIALIZATION;
-      attr.value.programmaticStreamSerializationAllowed = 1;
-      cfg.attrs = &attr;
-      cfg.numAttrs = 1;
-      r = driver().LaunchKernelEx(&cfg, kern.fn, params, nullptr);
-    } else {
-      r = driver().LaunchKernel(kern.fn, (unsigned)grid, 1, 1, (unsigned)sp.threads, 1, 1, (unsigned)sp.smem(), (CUstream)stream, params,
-                                nullptr);
-    }
-    if (r != CUDA_SUCCESS) return fail(B200FFT_ERR_CUDA, "launch of %s failed (CUresult %d)", sp.name().c_str(), (int)r);
-    g_launch_count.fetch_add(1, std::memory_order_relaxed);
-    return B200FFT_OK;
-  }
-  // Kernel argument blocks. The fp64 build of a kernel sees the same structs with float -> double (rtc_prelude.cuh), so
-  // the host fills a struct of that layout.
-  struct RowsArgs64 { const void* in; double2* out; const double2* tw; long long nrows; double scale; int do_scale; };
-  struct ColsArgs64 { const void* in; double2* out; const double2* tw; long long inner; int tiles_per_outer; double scale; int do_scale; int reverse; };
-  struct HalfArgs64 { const void* in; void* out; const double2* tw; const double2* tw2; long long nrows; double scale; };
-  template <class A, class T2>
-  A cols_args(const void* src, void* dst) const {
-    A ca;
-    ca.in = src;
-    ca.out = reinterpret_cast<T2*>(dst);
-    ca.tw = reinterpret_cast<const T2*>(d_tw);
-    ca.inner = view.inner;
-    ca.tiles_per_outer = (int)((view.inner + spec.tile - 1) / spec.tile);
-    ca.scale = scale;
-    ca.do_scale = do_scale;
-    ca.reverse = reverse_order ? 1 : 0;
-    return ca;
-  }
-  template <class A, class T2>
-  int launch_rows(const void* src, void* dst, int64_t outer, cudaStream_t stream) {
-    A ra;
-    ra.in = src;
-    ra.out = reinterpret_cast<T2*>(dst);
-    ra.tw = reinterpret_cast<const T2*>(d_tw);
-    ra.nrows = outer;
-    ra.scale = scale;
-    ra.do_scale = do_scale;
-    void* params[1] = {&ra};
-    return run(*k, spec, (outer + spec.tile - 1) / spec.tile, params, stream);
-  }
-  template <class A, class T2>
-  int launch_half(const void* src, void* dst, int64_t outer, cudaStream_t stream) {
-    A ha;
-    ha.in = src;
-    ha.out = dst;
-    ha.tw = reinterpret_cast<const T2*>(d_tw);
-    ha.tw2 = reinterpret_cast<const T2*>(d_tw2);
-    ha.nrows = outer;
-    ha.scale = scale;
-    void* params[1] = {&ha};
-    return run(*k, spec, (outer + spec.tile - 1) / spec.tile, params, stream);
-  }
-  int launch_outer(const void* src, void* dst, int64_t outer, cudaStream_t stream) {
-    if (spec.kind == JIT_ROWS || spec.kind == JIT_ROWS_IP)
-      return spec.f64 ? launch_rows<RowsArgs64, double2>(src, dst, outer, stream) : launch_rows<RowsArgs, float2>(src, dst, outer, stream);
-    if (spec.kind == JIT_COLS) {
-      void* params[1];
-      if (spec.f64) {
-        ColsArgs64 ca = cols_args<ColsArgs64, double2>(src, dst);
-        params[0] = &ca;
-        return run(*k, spec, outer * ca.tiles_per_outer, params, stream);
-      }
-      ColsArgs ca = cols_args<ColsArgs, float2>(src, dst);
-      params[0] = &ca;
-      return run(*k, spec, outer * ca.tiles_per_outer, params, stream);
-    }
-    return spec.f64 ? launch_half<HalfArgs64, double2>(src, dst, outer, stream) : launch_half<HalfArgs, float2>(src, dst, outer, stream);
-  }
-  int launch_scatter(const void* src, const Scatter& sc, int64_t nbatch, cudaStream_t stream) override {
-    if (spec.kind != JIT_COLS || spec.real_in || spec.in_dtype != (spec.f64 ? B200FFT_F64 : B200FFT_F32)) return fail(B200FFT_ERR_UNSUPPORTED, "no scattering store for %s", text.c_str());
-    if (sc.npeers < 1 || sc.npeers > 16 || view.n % sc.npeers)
-      return fail(B200FFT_ERR_INVALID_ARG, "split axis length %lld is not divisible by %d peers", (long long)view.n, sc.npeers);
-    JitSpec sp = spec;
-    sp.kind = JIT_SCATTER;
-    if (!k_scatter) {
-      int cur = -1;
-      cudaGetDevice(&cur);
-      if (cur != device) cudaSetDevice(device);
-      k_scatter = get_kernel(sp, device);
-      if (cur != device && cur >= 0) cudaSetDevice(cur);
-      if (!k_scatter) return fail(B200FFT_ERR_UNSUPPORTED, "could not specialise the scattering store for %s", text.c_str());
-    }
-    ScatterArgs sa;  // pointers and integers only: the same block for both precisions
-    for (int i = 0; i < 16; ++i) sa.peer[i] = i < sc.npeers ? reinterpret_cast<float2*>(sc.peer_out[i]) : nullptr;
-    sa.yl = (int)(view.n / sc.npeers);
-    const long long outer = nbatch * view.outer_per_batch;
-    sa.zbase = sc.zbase >= 0 ? sc.zbase : (long long)sc.my_rank * outer;
-    if (spec.f64) {
-      ColsArgs64 ca = cols_args<ColsArgs64, double2>(src, nullptr);
-      void* params[2] = {&ca, &sa};
-      return run(*k_scatter, sp, outer * ca.tiles_per_outer, params, stream);
-    }
-    ColsArgs ca = cols_args<ColsArgs, float2>(src, nullptr);
-    void* params[2] = {&ca, &sa};
-    return run(*k_scatter, sp, outer * ca.tiles_per_outer, params, stream);
-  }
-  std::string describe() const override { return text; }
-  size_t min_align(bool src) const override {
-    // even half spectrum: R2C reads the real row as complex pairs, C2R stores it as complex pairs
-    if (src) return spec.kind == JIT_R2C || spec.kind == JIT_R2C_REG ? 2 * in_scalar_bytes(spec.in_dtype) : 0;
-    return spec.kind == JIT_C2R ? spec.esz() : 0;
-  }
-};
-
-// fp64 forms of build_twiddles / build_half_twiddles (fast_registry.cu): tw[(j-1)*P + p] = W_{P*R}^{j*p} per stage s >= 1
-std::vector<double2> stage_twiddles64(const std::vector<int>& radices, bool inverse) {
-  std::vector<double2> t;
-  long long P = 1;
-  for (size_t s = 0; s < radices.size(); ++s) {
-    const int R = radices[s];
-    if (s > 0) {
-      const long long Q = P * R;
-      for (int j = 1; j < R; ++j)
-        for (long long p = 0; p < P; ++p) {
-          const long double th = 2.0L * 3.14159265358979323846264338327950288L * (long double)((j * p) % Q) / (long double)Q;
-          t.push_back(make_double2((double)cosl(th), (double)((inverse ? 1.0L : -1.0L) * sinl(th))));
-        }
-    }
-    P *= R;
-  }
-  if (t.empty()) t.push_back(make_double2(1.0, 0.0));
-  return t;
-}
-std::vector<double2> half_twiddles64(long long n, bool inverse) {
-  std::vector<double2> t;
-  for (long long k = 0; k <= n / 2; ++k) {
-    const long double th = 2.0L * 3.14159265358979323846264338327950288L * (long double)k / (long double)n;
-    t.push_back(make_double2((double)cosl(th), (double)((inverse ? 1.0L : -1.0L) * sinl(th))));
-  }
-  return t;
 }
 
 bool jit_enabled() {
@@ -851,7 +598,7 @@ bool jit_enabled() {
 
 // kind + transform length + stage list for one axis; false when this tier does not serve it
 bool jit_plan_axis(const AxisSpec& ax, const AxisView& view, const IoSpec& src, bool inverse, HalfMode half, bool f64,
-                   JitSpec* spec, long long rows_hint = 0) {
+                   TileSpec* spec, long long rows_hint = 0) {
   spec->rows_hint = rows_hint;
   spec->inverse = inverse;
   spec->real_in = src.comps == 1;
@@ -860,13 +607,13 @@ bool jit_plan_axis(const AxisSpec& ax, const AxisView& view, const IoSpec& src, 
   if (half == HALF_C2R && src.dtype != (f64 ? B200FFT_F64 : B200FFT_F32)) return false;  // the staged half spectrum is read as is
   if (half != HALF_NONE && src.dtype == B200FFT_U8) return false;
   if (half == HALF_NONE) {
-    spec->kind = view.inner != 1 ? JIT_COLS : JIT_ROWS;
+    spec->kind = view.inner != 1 ? TILE_COLS : TILE_ROWS;
     spec->n = (int)view.n;
     if (!jit_group(ax.ordered, &spec->radices, f64)) return false;
   } else {
     if (view.inner != 1) return false;  // half-spectrum handling is a row pass
     if (view.n % 2) {
-      spec->kind = half == HALF_R2C ? JIT_R2C_ODD : JIT_C2R_ODD;
+      spec->kind = half == HALF_R2C ? TILE_R2C_ODD : TILE_C2R_ODD;
       spec->n = (int)view.n;
       if (!jit_group(ax.ordered, &spec->radices, f64)) return false;
     } else {
@@ -877,8 +624,8 @@ bool jit_plan_axis(const AxisSpec& ax, const AxisView& view, const IoSpec& src, 
         if (jit_group(o, &spec->radices, f64)) { ok = true; break; }
       if (!ok) return false;
       if (spec->n == 1) return false;
-      spec->kind = half == HALF_C2R ? JIT_C2R : JIT_R2C;
-      if (half == HALF_R2C && r2c_reg_shape_ok(*spec) && !getenv("B200FFT_R2C_SMEM")) spec->kind = JIT_R2C_REG;
+      spec->kind = half == HALF_C2R ? TILE_C2R : TILE_R2C;
+      if (half == HALF_R2C && r2c_reg_shape_ok(*spec) && !getenv("B200FFT_R2C_SMEM")) spec->kind = TILE_R2C_REG;
     }
     spec->inverse = half == HALF_C2R;
     spec->real_in = false;
@@ -899,26 +646,26 @@ bool jit_plan_axis(const AxisSpec& ax, const AxisView& view, const IoSpec& src, 
   const bool few_rows = rows_hint > 0 && rows_hint <= 2 * 148;
   // two wide stages containing a radix-40 / 50 codelet lose to three narrow stages in one buffer (26214 x 1000: 40x25
   // 0.097 ms, 10x10x10 in place 0.082; 13107 x 2000: 50x40 0.104, 20x10x10 0.084; 40x40, 36x36 and 48x32 do not)
-  if (spec->kind == JIT_ROWS && !f64 && !few_rows && spec->n >= 1000 && spec->radices.size() == 2 && !getenv("B200FFT_JIT_MAX_RADIX")) {
+  if (spec->kind == TILE_ROWS && !f64 && !few_rows && spec->n >= 1000 && spec->radices.size() == 2 && !getenv("B200FFT_JIT_MAX_RADIX")) {
     const int n40 = (int)std::count(spec->radices.begin(), spec->radices.end(), 40);
     const int n50 = (int)std::count(spec->radices.begin(), spec->radices.end(), 50);
-    JitSpec narrow = *spec;
+    TileSpec narrow = *spec;
     if ((n50 > 0 || n40 == 1) && jit_group_cap(ax.ordered, JIT_MAX_RADIX, &narrow.radices) && narrow.radices.size() == 3) {
-      narrow.kind = JIT_ROWS_IP;
+      narrow.kind = TILE_ROWS_IP;
       if (jit_rows_ip_geometry(&narrow)) {
         *spec = narrow;
         return true;
       }
     }
   }
-  if (spec->kind == JIT_ROWS && row_bytes >= ip_min_bytes && (row_bytes >= 32768 || !few_rows)) {
-    spec->kind = JIT_ROWS_IP;
+  if (spec->kind == TILE_ROWS && row_bytes >= ip_min_bytes && (row_bytes >= 32768 || !few_rows)) {
+    spec->kind = TILE_ROWS_IP;
     if (jit_rows_ip_geometry(spec)) return true;
-    spec->kind = JIT_ROWS;
+    spec->kind = TILE_ROWS;
   }
   if (!jit_geometry(spec, view.inner)) {
-    if (spec->kind != JIT_R2C_REG) return false;
-    spec->kind = JIT_R2C;  // no tile keeps whole warps per row group: the shared-memory unpack
+    if (spec->kind != TILE_R2C_REG) return false;
+    spec->kind = TILE_R2C;  // no tile keeps whole warps per row group: the shared-memory unpack
     if (!jit_geometry(spec, view.inner)) return false;
   }
   return true;
@@ -926,79 +673,6 @@ bool jit_plan_axis(const AxisSpec& ax, const AxisView& view, const IoSpec& src, 
 
 // ---- long axes: N = N1 * N2 as two specialised passes and one plan-owned temporary (split_registry.cu does this for a
 // fixed list of (N1, N2); here any factorisation the stage list allows) ---------------------------------------------------
-struct JitSplitPass : Pass {
-  JitSpec sa, sb;
-  std::shared_ptr<JitKernel> ka, kb;
-  AxisView view;
-  int n1 = 0, n2 = 0;
-  bool do_scale = false;
-  double scale = 1.0;
-  void *twa = nullptr, *twb = nullptr, *tw2 = nullptr, *tmp = nullptr;
-  const void* twN = nullptr;
-  std::string text;
-
-  struct SplitArgs64 {
-    const void* in; double2* out; const double2* tw; const double2* twN; const double2* tw2; long long inner; long long nrows;
-    int tiles_per_outer; int n1, n2; double scale; int do_scale;
-  };
-  template <class A, class T2>
-  int go(const void* src, void* dst, long long outer, cudaStream_t stream) {
-    A a;
-    memset(&a, 0, sizeof a);
-    a.inner = view.inner;
-    a.n1 = n1;
-    a.n2 = n2;
-    a.in = src;  // pass A: view (outer, n1, n2 * inner)
-    a.out = reinterpret_cast<T2*>(tmp);
-    a.tw = reinterpret_cast<const T2*>(twa);
-    a.twN = reinterpret_cast<const T2*>(twN);
-    a.tw2 = reinterpret_cast<const T2*>(tw2);
-    const long long vinner = (long long)n2 * view.inner;
-    a.tiles_per_outer = (int)((vinner + sa.tile - 1) / sa.tile);
-    void* params[1] = {&a};
-    int rc = launch_one(*ka, sa, outer * a.tiles_per_outer, params, stream);
-    if (rc != B200FFT_OK) return rc;
-    a.in = tmp;  // pass B
-    a.out = reinterpret_cast<T2*>(dst);
-    a.tw = reinterpret_cast<const T2*>(twb);
-    a.scale = scale;
-    a.do_scale = do_scale;
-    long long grid;
-    if (sb.kind == JIT_SPLIT_B_R2C) {  // (n1/2 + 1) row pairs per transform, tile/2 of them per CTA
-      a.tiles_per_outer = (int)((n1 / 2 + 1 + sb.tile / 2 - 1) / (sb.tile / 2));
-      grid = outer * a.tiles_per_outer;
-    } else if (sb.kind != JIT_SPLIT_B_COLS) {
-      a.nrows = outer * n1;
-      grid = (a.nrows + sb.tile - 1) / sb.tile;
-    } else {
-      a.tiles_per_outer = (int)((view.inner + sb.tile - 1) / sb.tile);
-      grid = outer * n1 * a.tiles_per_outer;
-    }
-    return launch_one(*kb, sb, grid, params, stream);
-  }
-  static int launch_one(const JitKernel& kern, const JitSpec& sp, long long grid, void** params, cudaStream_t stream) {
-    if (grid <= 0) return B200FFT_OK;
-    if (grid > 0x7fffffffLL) return fail(B200FFT_ERR_UNSUPPORTED, "too many tiles");
-    const CUresult r = driver().LaunchKernel(kern.fn, (unsigned)grid, 1, 1, (unsigned)sp.threads, 1, 1, (unsigned)sp.smem(),
-                                             (CUstream)stream, params, nullptr);
-    if (r != CUDA_SUCCESS) return fail(B200FFT_ERR_CUDA, "launch of %s failed (CUresult %d)", sp.name().c_str(), (int)r);
-    g_launch_count.fetch_add(1, std::memory_order_relaxed);
-    return B200FFT_OK;
-  }
-  int launch(const void* src, void* dst, int64_t nbatch, cudaStream_t stream) override {
-    const long long outer = nbatch * view.outer_per_batch;
-    if (outer <= 0) return B200FFT_OK;
-    return sa.f64 ? go<SplitArgs64, double2>(src, dst, outer, stream) : go<SplitArgs, float2>(src, dst, outer, stream);
-  }
-  std::string describe() const override { return text; }
-  size_t min_align(bool src) const override {
-    // even half spectrum: R2C pass A reads the real row as H complex pairs, C2R pass B stores it as H complex pairs
-    if (src) return sb.kind == JIT_SPLIT_B_R2C ? 2 * in_scalar_bytes(sa.in_dtype) : 0;
-    return sa.kind == JIT_SPLIT_A_C2R ? sb.esz() : 0;
-  }
-  int launches() const override { return 2; }
-};
-
 // Split the grouped super-stage list into the stages of pass A (product N1) and pass B (product N2): both as close to
 // sqrt(N) as the radices allow, each short enough for one tile.
 bool jit_split_stages(const std::vector<int>& radices, std::vector<int>* a, std::vector<int>* b) {
@@ -1030,7 +704,7 @@ bool jit_split_stages(const std::vector<int>& radices, std::vector<int>* a, std:
 //   even-n C2R: split H; pass A packs the half spectrum in its load; pass B writes H complex = the n reals
 //   odd-n R2C / C2R: split n; pass B keeps bins 0..n/2 / pass A extends the half spectrum, pass B keeps real parts
 struct JitSplitChoice {
-  JitSpec sa, sb;
+  TileSpec sa, sb;
   long long n1 = 0, n2 = 0;
   long long len = 0;  // length of the complex transform the two passes run (H for even half-spectrum rows)
 };
@@ -1053,7 +727,7 @@ bool jit_split_plan(const std::vector<uint32_t>& ordered, const AxisView& view, 
   c->n1 = c->n2 = 1;
   for (int r : ra) c->n1 *= r;
   for (int r : rb) c->n2 *= r;
-  for (JitSpec* s : {&c->sa, &c->sb}) {
+  for (TileSpec* s : {&c->sa, &c->sb}) {
     s->inverse = half == HALF_NONE ? inverse : half == HALF_C2R;
     s->f64 = f64;
     s->in_dtype = work;  // pass B reads the temporary
@@ -1065,18 +739,18 @@ bool jit_split_plan(const std::vector<uint32_t>& ordered, const AxisView& view, 
   c->sb.n = (int)c->n2;
   c->sb.radices = rb;
   if (half == HALF_NONE) {
-    c->sa.kind = JIT_SPLIT_A;
+    c->sa.kind = TILE_SPLIT_A;
     c->sa.real_in = src.comps == 1;
-    c->sb.kind = view.inner == 1 ? JIT_SPLIT_B_ROWS : JIT_SPLIT_B_COLS;
+    c->sb.kind = view.inner == 1 ? TILE_SPLIT_B_ROWS : TILE_SPLIT_B_COLS;
   } else if (half == HALF_R2C) {
-    c->sa.kind = JIT_SPLIT_A;
+    c->sa.kind = TILE_SPLIT_A;
     c->sa.real_in = !even_half;  // even n: the real row's bytes are H complex pairs
-    c->sb.kind = even_half ? JIT_SPLIT_B_R2C : JIT_SPLIT_B_HALF;
+    c->sb.kind = even_half ? TILE_SPLIT_B_R2C : TILE_SPLIT_B_HALF;
   } else {
-    c->sa.kind = even_half ? JIT_SPLIT_A_C2R : JIT_SPLIT_A_C2R_ODD;
-    c->sb.kind = even_half ? JIT_SPLIT_B_ROWS : JIT_SPLIT_B_REAL;
+    c->sa.kind = even_half ? TILE_SPLIT_A_C2R : TILE_SPLIT_A_C2R_ODD;
+    c->sb.kind = even_half ? TILE_SPLIT_B_ROWS : TILE_SPLIT_B_REAL;
   }
-  if (view.inner == 1 && c->sb.kind != JIT_SPLIT_B_R2C) c->sb.tile_divides = (int)c->n1;  // row tiles never straddle transforms
+  if (view.inner == 1 && c->sb.kind != TILE_SPLIT_B_R2C) c->sb.tile_divides = (int)c->n1;  // row tiles never straddle transforms
   return jit_geometry(&c->sa, c->n2 * view.inner) && jit_geometry(&c->sb, view.inner);
 }
 
@@ -1088,57 +762,49 @@ std::unique_ptr<Pass> make_jit_split_pass(b200fft_plan& plan, int axis, const Ax
   if (!jit_split_plan(p.axes[axis].ordered, view, src, p.desc.inverse != 0, half, f64, &c)) return nullptr;
   const bool even_half = half != HALF_NONE && c.len != view.n;
   if (!even_half && !plan.tw[axis].ptr) return nullptr;
-  auto pass = std::make_unique<JitSplitPass>();
-  pass->sa = c.sa;
-  pass->sb = c.sb;
-  pass->n1 = (int)c.n1;
-  pass->n2 = (int)c.n2;
+  auto pass = std::make_unique<SplitPass>();
+  pass->len[0] = c.n1;
+  pass->len[1] = c.n2;
   pass->view = view;
-  pass->ka = get_kernel(pass->sa, plan.device);
-  pass->kb = pass->ka ? get_kernel(pass->sb, plan.device) : nullptr;
-  if (!pass->ka || !pass->kb) return nullptr;
+  const TileSpec* spec[2] = {&c.sa, &c.sb};
+  std::shared_ptr<JitKernel> k[2];
+  for (int i = 0; i < 2; ++i) {
+    if (!(k[i] = get_kernel(*spec[i], plan.device))) return nullptr;
+    SplitPass::Stage& st = pass->st[i];
+    st.spec = *spec[i];
+    st.k = {nullptr, k[i]->fn, jit_name(st.spec)};
+    st.smem = st.spec.smem();
+    st.n2 = (int)c.n2;
+  }
   // the half-spectrum inverse is always normalised (like the single-tile C2R kernels)
   pass->do_scale = scale_inverse || half == HALF_C2R;
   pass->scale = pass->do_scale ? 1.0 / (double)view.n : 1.0;
-  auto upload = [&](const void* data, size_t bytes, void** d) {
-    if (cudaMalloc(d, bytes) != cudaSuccess) { cudaGetLastError(); return false; }
-    plan.owned_device.push_back(*d);
-    return cudaMemcpy(*d, data, bytes, cudaMemcpyHostToDevice) == cudaSuccess;
-  };
-  const bool inv = pass->sa.inverse;
-  bool ok;
-  if (f64) {
-    const auto ta = stage_twiddles64(c.sa.radices, inv), tb = stage_twiddles64(c.sb.radices, inv);
-    ok = upload(ta.data(), ta.size() * sizeof(double2), &pass->twa) && upload(tb.data(), tb.size() * sizeof(double2), &pass->twb);
-  } else {
-    const auto ta = build_twiddles(c.sa.radices, inv), tb = build_twiddles(c.sb.radices, inv);
-    ok = upload(ta.data(), ta.size() * sizeof(float2), &pass->twa) && upload(tb.data(), tb.size() * sizeof(float2), &pass->twb);
-  }
-  if (!ok) return nullptr;
-  if (!even_half) {
-    pass->twN = plan.tw[axis].ptr;  // W_n^m, m in [0, n), in the working precision (api.cu: upload_twiddles)
-  } else {
+  const bool inv = c.sa.inverse;
+  const void *twN = plan.tw[axis].ptr, *tw2 = nullptr;  // W_n^m, m in [0, n), in the working precision (api.cu: upload_twiddles)
+  auto tables = [&](auto zero) {
+    using T2 = decltype(zero);
+    for (int i = 0; i < 2; ++i)
+      if (!(pass->st[i].tw = plan_upload(plan, build_twiddles<T2>(spec[i]->radices, inv)))) return false;
+    if (!even_half) return true;
     // the split runs on H = n/2 points: pass A's twiddle is W_H^m, m in [0, H), and the unpack / pack needs W_n^{-+k}, k = 0..H
-    void* d = nullptr;
-    if (f64) {
-      const std::vector<double2> th = half_twiddles64(c.len, inv);  // W_H^m for m = 0..H/2; the rest by symmetry below
-      std::vector<double2> full((size_t)c.len);
+    std::vector<T2> full((size_t)c.len);
+    if constexpr (std::is_same<T2, double2>::value) {
+      const std::vector<double2> th = build_half_twiddles<double2>(c.len, inv);  // W_H^m for m = 0..H/2; the rest by symmetry
       for (long long m = 0; m < c.len; ++m) full[(size_t)m] = m <= c.len / 2 ? th[(size_t)m] : make_double2(th[(size_t)(c.len - m)].x, -th[(size_t)(c.len - m)].y);
-      const std::vector<double2> t2 = half_twiddles64(view.n, inv);
-      ok = upload(full.data(), full.size() * sizeof(double2), &d) && upload(t2.data(), t2.size() * sizeof(double2), &pass->tw2);
     } else {
-      std::vector<float2> full((size_t)c.len);
       for (long long m = 0; m < c.len; ++m) {
         const double th = 2.0 * M_PI * (double)m / (double)c.len;
         full[(size_t)m] = make_float2((float)std::cos(th), (float)((inv ? 1.0 : -1.0) * std::sin(th)));
       }
-      const std::vector<float2> t2 = build_half_twiddles(view.n, inv);
-      ok = upload(full.data(), full.size() * sizeof(float2), &d) && upload(t2.data(), t2.size() * sizeof(float2), &pass->tw2);
     }
-    if (!ok) return nullptr;
-    pass->twN = d;
+    return (twN = plan_upload(plan, full)) && (tw2 = plan_upload(plan, build_half_twiddles<T2>(view.n, inv)));
+  };
+  if (!(f64 ? tables(double2()) : tables(float2()))) return nullptr;
+  for (SplitPass::Stage& st : pass->st) {
+    st.twN = twN;
+    st.tw2 = tw2;
   }
-  const size_t tmp_bytes = (size_t)p.batch * view.outer_per_batch * c.len * view.inner * pass->sa.esz();
+  const size_t tmp_bytes = (size_t)p.batch * view.outer_per_batch * c.len * view.inner * c.sa.esz();
   if (cudaMalloc(&pass->tmp, tmp_bytes) != cudaSuccess) {
     cudaGetLastError();
     return nullptr;
@@ -1173,8 +839,8 @@ std::unique_ptr<Pass> make_jit_split_pass(b200fft_plan& plan, int axis, const Ax
   char buf[700];
   snprintf(buf, sizeof buf, "axis %d: split n=%lld%s = %lld x %lld%s inner=%lld: %s %s -> %s %s; temp=%zuB user "
            "stages=[%s] [NVRTC, %.0f + %.0f ms]", axis, (long long)view.n, form, c.n1, c.n2, even_half ? " (H points)" : "",
-           (long long)view.inner, pass->sa.name().c_str(), a_note, pass->sb.name().c_str(), b_note, tmp_bytes, stages.c_str(),
-           pass->ka->compile_ms, pass->kb->compile_ms);
+           (long long)view.inner, jit_name(c.sa).c_str(), a_note, jit_name(c.sb).c_str(), b_note, tmp_bytes, stages.c_str(),
+           k[0]->compile_ms, k[1]->compile_ms);
   pass->text = buf;
   return pass;
 }
@@ -1182,56 +848,6 @@ std::unique_ptr<Pass> make_jit_split_pass(b200fft_plan& plan, int axis, const Ax
 // ---- contiguous axes longer than 2^24 points: n = N1 * N2 * N3 as three specialised passes and one plan-owned temporary
 // (fast.cuh: rows_split_c_kernel). Both twiddles come from two tables of about sqrt(L) entries (SplitTw2Dst), so nothing
 // the plan holds grows like n except the temporary.
-struct JitSplit3Pass : Pass {
-  JitSpec s[3];
-  std::shared_ptr<JitKernel> k[3];
-  AxisView view;
-  int n1 = 0, n2 = 0, n3 = 0;
-  bool do_scale = false;
-  double scale = 1.0;
-  void* tw[3] = {};               // stage twiddles of each pass
-  void *hi[2] = {}, *lo[2] = {};  // T_hi / T_lo of W_n (pass 1) and W_M (pass 2)
-  void* tmp = nullptr;
-  std::string text;
-
-  template <class A, class T2>
-  int go(const void* src, void* dst, long long outer, cudaStream_t stream) {
-    A a;
-    memset(&a, 0, sizeof a);
-    void* params[1] = {&a};
-    a.inner = 1;
-    a.n1 = n1;
-    for (int p = 0; p < 2; ++p) {  // 1: view (outer, N1, M), input -> temporary; 2: view (outer N1, N2, N3) in place
-      const long long cols = p == 0 ? (long long)n2 * n3 : n3;
-      a.in = p == 0 ? src : tmp;
-      a.out = reinterpret_cast<T2*>(tmp);
-      a.tw = reinterpret_cast<const T2*>(tw[p]);
-      a.twN = reinterpret_cast<const T2*>(hi[p]);
-      a.tw2 = reinterpret_cast<const T2*>(lo[p]);
-      a.n2 = (int)cols;
-      a.tiles_per_outer = (int)((cols + s[p].tile - 1) / s[p].tile);
-      const int rc = JitSplitPass::launch_one(*k[p], s[p], (p == 0 ? outer : outer * n1) * a.tiles_per_outer, params, stream);
-      if (rc != B200FFT_OK) return rc;
-    }
-    a.in = tmp;  // 3: rows (k1, k2) of the temporary -> natural order
-    a.out = reinterpret_cast<T2*>(dst);
-    a.tw = reinterpret_cast<const T2*>(tw[2]);
-    a.twN = a.tw2 = nullptr;
-    a.n2 = n2;
-    a.nrows = outer * n1 * n2;
-    a.scale = scale;
-    a.do_scale = do_scale;
-    return JitSplitPass::launch_one(*k[2], s[2], (a.nrows + s[2].tile - 1) / s[2].tile, params, stream);
-  }
-  int launch(const void* src, void* dst, int64_t nbatch, cudaStream_t stream) override {
-    const long long outer = nbatch * view.outer_per_batch;
-    if (outer <= 0) return B200FFT_OK;
-    return s[0].f64 ? go<JitSplitPass::SplitArgs64, double2>(src, dst, outer, stream) : go<SplitArgs, float2>(src, dst, outer, stream);
-  }
-  std::string describe() const override { return text; }
-  int launches() const override { return 3; }
-};
-
 // Every split of the grouped super-stage list into three sets (products N1, N2, N3) of at most 8192 points and 4 stages,
 // most balanced first (the measure jit_split_stages applies to two): each assignment of the m <= 12 groups is scored.
 // The strided passes 1 and 2 hold fewer points per tile than the row pass 3, so the caller takes the first split whose
@@ -1267,7 +883,7 @@ std::vector<long long> jit_split3_stages(const std::vector<int>& radices) {
 // b200fft_jit_split3_probe share it). Complex input, or real input with the full spectrum, of any input dtype (cast on
 // load in pass 1). False, with the reason in last_error(), for every axis it does not serve.
 struct JitSplit3Choice {
-  JitSpec s[3];
+  TileSpec s[3];
   long long n[3] = {0, 0, 0};
 };
 bool jit_split3_plan(const std::vector<uint32_t>& ordered, const AxisView& view, const IoSpec& src, bool inverse, HalfMode half,
@@ -1298,11 +914,11 @@ bool jit_split3_plan(const std::vector<uint32_t>& ordered, const AxisView& view,
     std::vector<int> sets[3];
     for (size_t i = 0; i < all.size(); ++i, code /= 3) sets[code % 3].push_back(all[i]);
     for (int j = 0; j < 3; ++j) {
-      JitSpec& s = c->s[j];
-      s = JitSpec();
+      TileSpec& s = c->s[j];
+      s = TileSpec();
       c->n[j] = 1;
       for (int r : sets[j]) c->n[j] *= r;
-      s.kind = j < 2 ? JIT_SPLIT3_A : JIT_SPLIT3_C;
+      s.kind = j < 2 ? TILE_SPLIT3_A : TILE_SPLIT3_C;
       s.n = (int)c->n[j];
       s.radices = sets[j];
       s.inverse = inverse;
@@ -1346,52 +962,42 @@ std::unique_ptr<Pass> make_jit_split3_pass(b200fft_plan& plan, int axis, const A
   const bool f64 = p.desc.out_dtype == B200FFT_F64;
   JitSplit3Choice c;
   if (!jit_split3_plan(p.axes[axis].ordered, view, src, p.desc.inverse != 0, half, f64, &c)) return nullptr;
-  auto pass = std::make_unique<JitSplit3Pass>();
+  auto pass = std::make_unique<SplitPass>();
+  pass->count = 3;
   pass->view = view;
-  pass->n1 = (int)c.n[0];
-  pass->n2 = (int)c.n[1];
-  pass->n3 = (int)c.n[2];
+  std::shared_ptr<JitKernel> k[3];
   for (int j = 0; j < 3; ++j) {
-    pass->s[j] = c.s[j];
-    pass->k[j] = get_kernel(c.s[j], plan.device);
-    if (!pass->k[j]) return nullptr;
+    if (!(k[j] = get_kernel(c.s[j], plan.device))) return nullptr;
+    SplitPass::Stage& st = pass->st[j];
+    st.spec = c.s[j];
+    st.k = {nullptr, k[j]->fn, jit_name(st.spec)};
+    st.smem = st.spec.smem();
+    pass->len[j] = c.n[j];
   }
+  pass->st[0].n2 = (int)(c.n[1] * c.n[2]);  // passes 1 and 2: the columns of their view; pass 3: N2 of the natural-order store
+  pass->st[1].n2 = (int)c.n[2];
+  pass->st[2].n2 = (int)c.n[1];
   pass->do_scale = scale_inverse;
   pass->scale = scale_inverse ? 1.0 / (double)view.n : 1.0;
-  auto upload = [&](const void* data, size_t bytes, void** d) {
-    if (cudaMalloc(d, bytes) != cudaSuccess) {
-      cudaGetLastError();
-      *status = fail(B200FFT_ERR_ALLOC, "axis %d: cannot allocate %zu B of three-pass split tables", axis, bytes);
-      return false;
-    }
-    plan.owned_device.push_back(*d);
-    return cudaMemcpy(*d, data, bytes, cudaMemcpyHostToDevice) == cudaSuccess;
-  };
   const bool inv = p.desc.inverse != 0;
   const long long L[2] = {view.n, c.n[1] * c.n[2]};
-  bool ok = true;
-  if (f64) {
-    std::vector<double2> hi, lo;
-    for (int j = 0; j < 3 && ok; ++j) {
-      const auto t = stage_twiddles64(c.s[j].radices, inv);
-      ok = upload(t.data(), t.size() * sizeof(double2), &pass->tw[j]);
-    }
-    for (int j = 0; j < 2 && ok; ++j) {
+  auto tables = [&](auto zero) {
+    using T2 = decltype(zero);
+    auto upload = [&](const std::vector<T2>& t, const void** d) {
+      if ((*d = plan_upload(plan, t))) return true;
+      *status = fail(B200FFT_ERR_ALLOC, "axis %d: cannot allocate %zu B of three-pass split tables", axis, t.size() * sizeof(T2));
+      return false;
+    };
+    std::vector<T2> hi, lo;
+    for (int j = 0; j < 3; ++j)
+      if (!upload(build_twiddles<T2>(c.s[j].radices, inv), &pass->st[j].tw)) return false;
+    for (int j = 0; j < 2; ++j) {  // T_hi / T_lo of W_n (pass 1) and W_M (pass 2)
       split_tw2_tables(L[j], inv, &hi, &lo);
-      ok = upload(hi.data(), hi.size() * sizeof(double2), &pass->hi[j]) && upload(lo.data(), lo.size() * sizeof(double2), &pass->lo[j]);
+      if (!upload(hi, &pass->st[j].twN) || !upload(lo, &pass->st[j].tw2)) return false;
     }
-  } else {
-    std::vector<float2> hi, lo;
-    for (int j = 0; j < 3 && ok; ++j) {
-      const auto t = build_twiddles(c.s[j].radices, inv);
-      ok = upload(t.data(), t.size() * sizeof(float2), &pass->tw[j]);
-    }
-    for (int j = 0; j < 2 && ok; ++j) {
-      split_tw2_tables(L[j], inv, &hi, &lo);
-      ok = upload(hi.data(), hi.size() * sizeof(float2), &pass->hi[j]) && upload(lo.data(), lo.size() * sizeof(float2), &pass->lo[j]);
-    }
-  }
-  if (!ok) return nullptr;
+    return true;
+  };
+  if (!(f64 ? tables(double2()) : tables(float2()))) return nullptr;
   const size_t tmp_bytes = (size_t)p.batch * (size_t)view.outer_per_batch * (size_t)view.n * c.s[1].esz();
   if (cudaMalloc(&pass->tmp, tmp_bytes) != cudaSuccess) {
     cudaGetLastError();
@@ -1406,9 +1012,9 @@ std::unique_ptr<Pass> make_jit_split3_pass(b200fft_plan& plan, int axis, const A
   char buf[800];
   snprintf(buf, sizeof buf, "axis %d: split3 n=%lld%s = %lld x %lld x %lld inner=1: %s (+W_n twiddle, two tables) -> %s (in place, "
            "+W_M twiddle, two tables) -> %s (natural-order store%s); temp=%zuB user stages=[%s] [NVRTC, %.0f + %.0f + %.0f ms]",
-           axis, (long long)view.n, src.comps == 1 ? " real-in" : "", c.n[0], c.n[1], c.n[2], c.s[0].name().c_str(),
-           c.s[1].name().c_str(), c.s[2].name().c_str(), scale_inverse ? ", 1/n" : "", tmp_bytes, stages.c_str(),
-           pass->k[0]->compile_ms, pass->k[1]->compile_ms, pass->k[2]->compile_ms);
+           axis, (long long)view.n, src.comps == 1 ? " real-in" : "", c.n[0], c.n[1], c.n[2], jit_name(c.s[0]).c_str(),
+           jit_name(c.s[1]).c_str(), jit_name(c.s[2]).c_str(), scale_inverse ? ", 1/n" : "", tmp_bytes, stages.c_str(),
+           k[0]->compile_ms, k[1]->compile_ms, k[2]->compile_ms);
   pass->text = buf;
   return pass;
 }
@@ -1425,7 +1031,7 @@ std::unique_ptr<Pass> make_jit_pass(b200fft_plan& plan, int axis, const AxisView
     return nullptr;
   }
   const bool f64 = p.desc.out_dtype == B200FFT_F64;
-  JitSpec spec;
+  TileSpec spec;
   const long long rows = view.inner == 1 ? (long long)p.batch * view.outer_per_batch : 0;
   if ((view.n > 16384 && view.inner != 1) || view.n > 32768 ||
       !jit_plan_axis(p.axes[axis], view, src, p.desc.inverse != 0, half, f64, &spec, rows)) {
@@ -1437,44 +1043,30 @@ std::unique_ptr<Pass> make_jit_pass(b200fft_plan& plan, int axis, const AxisView
   }
   std::shared_ptr<JitKernel> k = get_kernel(spec, plan.device);
   if (!k) return nullptr;
-  auto pass = std::make_unique<JitPass>();
+  auto pass = std::make_unique<TilePass>();
   pass->spec = spec;
-  pass->k = k;
+  pass->k = {nullptr, k->fn, jit_name(spec)};
   pass->view = view;
   pass->device = plan.device;
   pass->do_scale = scale_inverse;
   pass->scale = (scale_inverse || half == HALF_C2R) ? 1.0 / (double)view.n : 1.0;  // the half-spectrum inverse is always normalised
   pass->smem = spec.smem();
-  auto upload = [&](const void* data, size_t bytes, void** d) {
-    if (cudaMalloc(d, bytes) != cudaSuccess) { cudaGetLastError(); return false; }
-    plan.owned_device.push_back(*d);  // owned by the plan before the copy: a failed copy must not leak it
-    return cudaMemcpy(*d, data, bytes, cudaMemcpyHostToDevice) == cudaSuccess;
+  const bool need_tw2 = half != HALF_NONE && spec.kind != TILE_R2C_ODD && spec.kind != TILE_C2R_ODD;
+  auto tables = [&](auto zero) {
+    using T2 = decltype(zero);
+    return (pass->tw = plan_upload(plan, build_twiddles<T2>(spec.radices, spec.inverse))) &&
+           (!need_tw2 || (pass->tw2 = plan_upload(plan, build_half_twiddles<T2>(view.n, half == HALF_C2R))));
   };
-  const bool need_tw2 = half != HALF_NONE && spec.kind != JIT_R2C_ODD && spec.kind != JIT_C2R_ODD;
-  if (f64) {
-    const std::vector<double2> tw = stage_twiddles64(spec.radices, spec.inverse);
-    if (!upload(tw.data(), tw.size() * sizeof(double2), &pass->d_tw)) return nullptr;
-    if (need_tw2) {
-      const std::vector<double2> t2 = half_twiddles64(view.n, half == HALF_C2R);
-      if (!upload(t2.data(), t2.size() * sizeof(double2), &pass->d_tw2)) return nullptr;
-    }
-  } else {
-    const std::vector<float2> tw = build_twiddles(spec.radices, spec.inverse);
-    if (!upload(tw.data(), tw.size() * sizeof(float2), &pass->d_tw)) return nullptr;
-    if (need_tw2) {
-      const std::vector<float2> t2 = build_half_twiddles(view.n, half == HALF_C2R);
-      if (!upload(t2.data(), t2.size() * sizeof(float2), &pass->d_tw2)) return nullptr;
-    }
-  }
+  if (!(f64 ? tables(double2()) : tables(float2()))) return nullptr;
   std::string stages;
   for (uint32_t r : p.axes[axis].ordered) stages += (stages.empty() ? "" : ",") + std::to_string(r);
   char buf[400];
   snprintf(buf, sizeof buf, "axis %d: %s n=%lld inner=%lld smem=%zuB regs=%d%s user stages=[%s] fused as %s(%s)%s [NVRTC, %.0f ms]", axis,
-           spec.name().c_str(), (long long)view.n, (long long)view.inner, pass->smem, k->regs,
+           jit_name(spec).c_str(), (long long)view.n, (long long)view.inner, pass->smem, k->regs,
            k->local_bytes ? (" local=" + std::to_string(k->local_bytes) + "B").c_str() : "", stages.c_str(),
            need_tw2 ? "(2)" : "", radix_name(spec.radices).c_str(),
-           half == HALF_R2C ? (spec.kind == JIT_R2C_ODD ? " r2c (real rows, bins 0..n/2 stored)" : " r2c")
-           : half == HALF_C2R ? (spec.kind == JIT_C2R_ODD ? " c2r (Hermitian-extended load)" : " c2r") : spec.real_in ? " real-in" : "",
+           half == HALF_R2C ? (spec.kind == TILE_R2C_ODD ? " r2c (real rows, bins 0..n/2 stored)" : " r2c")
+           : half == HALF_C2R ? (spec.kind == TILE_C2R_ODD ? " c2r (Hermitian-extended load)" : " c2r") : spec.real_in ? " real-in" : "",
            k->compile_ms);
   pass->text = buf;
   return pass;
@@ -1485,36 +1077,27 @@ std::unique_ptr<Pass> make_jit_pass(b200fft_plan& plan, int axis, const AxisView
 namespace {
 
 struct JitPlanePass : Pass {
-  JitSpec spec;
-  std::shared_ptr<JitKernel> k;
+  TileSpec spec;
+  TileKernel k;
   long long planes_per_batch = 1;
   float scale = 1.f;
-  void *twx = nullptr, *twy = nullptr, *tw2 = nullptr;
+  const float2 *twx = nullptr, *twy = nullptr, *tw2 = nullptr;
   std::string text;
   int launch(const void* src, void* dst, int64_t nbatch, cudaStream_t stream) override {
     PlaneFwdArgs a;
     a.in = src;
     a.out = reinterpret_cast<float2*>(dst);
-    a.twx = reinterpret_cast<const float2*>(twx);
-    a.twy = reinterpret_cast<const float2*>(twy);
-    a.tw2 = reinterpret_cast<const float2*>(tw2);
+    a.twx = twx;
+    a.twy = twy;
+    a.tw2 = tw2;
     a.planes = nbatch * planes_per_batch;
     a.scale = scale;
     a.do_scale = spec.inverse ? 1 : 0;
-    if (a.planes <= 0) return B200FFT_OK;
-    if (a.planes > 0x7fffffffLL) return fail(B200FFT_ERR_UNSUPPORTED, "too many planes");
     void* params[1] = {&a};
-    const CUresult r = driver().LaunchKernel(k->fn, (unsigned)a.planes, 1, 1, (unsigned)spec.threads, 1, 1, (unsigned)spec.smem(),
-                                             (CUstream)stream, params, nullptr);
-    if (r != CUDA_SUCCESS) return fail(B200FFT_ERR_CUDA, "launch of %s failed (CUresult %d)", spec.name().c_str(), (int)r);
-    g_launch_count.fetch_add(1, std::memory_order_relaxed);
-    return B200FFT_OK;
+    return launch_tile(k, a.planes, spec.threads, spec.smem(), false, params, stream);
   }
   std::string describe() const override { return text; }
-  size_t min_align(bool src) const override {
-    // R2C planes read the real rows as complex pairs of the input element type
-    return src && spec.kind == JIT_PLANE_R2C ? 2 * in_scalar_bytes(spec.in_dtype) : 0;
-  }
+  size_t min_align(bool src) const override { return tile_min_align({&spec}, src); }
 };
 
 // exactly two register stages of at most 32 for one axis, or false
@@ -1546,8 +1129,8 @@ std::unique_ptr<Pass> make_jit_plane_pass(b200fft_plan& plan) {
   const bool real_in = !p.half && p.desc.in_components == 1;
   if (real_in && p.desc.inverse) return nullptr;
   if (p.half && p.axes[last].n % 2) return nullptr;
-  JitSpec spec;
-  spec.kind = p.half ? JIT_PLANE_R2C : JIT_PLANE_C2C;
+  TileSpec spec;
+  spec.kind = p.half ? TILE_PLANE_R2C : TILE_PLANE_C2C;
   spec.n = (int)p.axes[last - 1].n;
   spec.n2 = (int)(p.half ? p.axes[last].n / 2 : p.axes[last].n);
   spec.inverse = p.desc.inverse != 0;
@@ -1581,28 +1164,24 @@ std::unique_ptr<Pass> make_jit_plane_pass(b200fft_plan& plan) {
   if (!k) return nullptr;
   auto pass = std::make_unique<JitPlanePass>();
   pass->spec = spec;
-  pass->k = k;
+  pass->k = {nullptr, k->fn, jit_name(spec)};
   pass->planes_per_batch = 1;
   for (int a = 0; a < last - 1; ++a) pass->planes_per_batch *= p.axes[a].n;
   pass->scale = spec.inverse ? (float)(1.0 / ((double)spec.n * spec.n2)) : 1.f;
-  auto upload = [&](const std::vector<float2>& t, void** d) {
-    if (cudaMalloc(d, t.size() * sizeof(float2)) != cudaSuccess) { cudaGetLastError(); return false; }
-    plan.owned_device.push_back(*d);
-    return cudaMemcpy(*d, t.data(), t.size() * sizeof(float2), cudaMemcpyHostToDevice) == cudaSuccess;
-  };
-  if (!upload(build_twiddles(spec.radices, spec.inverse), &pass->twy) || !upload(build_twiddles(spec.radices2, spec.inverse), &pass->twx))
+  if (!(pass->twy = plan_upload(plan, build_twiddles(spec.radices, spec.inverse))) ||
+      !(pass->twx = plan_upload(plan, build_twiddles(spec.radices2, spec.inverse))))
     return nullptr;
-  if (p.half && !upload(build_half_twiddles(p.axes[last].n, false), &pass->tw2)) return nullptr;
+  if (p.half && !(pass->tw2 = plan_upload(plan, build_half_twiddles(p.axes[last].n, false)))) return nullptr;
   char buf[360];
   snprintf(buf, sizeof buf, "axes %d,%d: %s: one in-place tile per (y, x) plane%s, smem=%zuB regs=%d [NVRTC, %.0f ms]", last - 1, last,
-           spec.name().c_str(), real_in ? " real-in" : "", spec.smem(), k->regs, k->compile_ms);
+           jit_name(spec).c_str(), real_in ? " real-in" : "", spec.smem(), k->regs, k->compile_ms);
   pass->text = buf;
   return pass;
 }
 
 namespace {
 // compile `spec` (or load it from the on-disk cache) and describe the result; no CUDA device involved
-int probe_compile(const JitSpec& spec, std::string* report) {
+int probe_compile(const TileSpec& spec, std::string* report) {
   std::vector<char> cubin;
   std::string lowered, log;
   double ms = 0;
@@ -1614,7 +1193,7 @@ int probe_compile(const JitSpec& spec, std::string* report) {
     disk_cache_store(on_disk, cubin, lowered);
   }
   char buf[700];
-  snprintf(buf, sizeof buf, "%s: %s, smem=%zuB, cubin=%zuB, %.0f ms%s, symbol %s", spec.name().c_str(), spec.expression().c_str(), spec.smem(),
+  snprintf(buf, sizeof buf, "%s: %s, smem=%zuB, cubin=%zuB, %.0f ms%s, symbol %s", jit_name(spec).c_str(), expression(spec).c_str(), spec.smem(),
            cubin.size(), ms, from_disk ? " (disk cache)" : "", lowered.c_str());
   *report = buf;
   return B200FFT_OK;
@@ -1634,7 +1213,7 @@ int jit_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bo
   IoSpec src;
   src.comps = real_in ? 1 : 2;
   src.dtype = in_dtype;
-  JitSpec spec;
+  TileSpec spec;
   if (!jit_plan_axis(ax, view, src, inverse, (HalfMode)half, out_dtype == B200FFT_F64, &spec))
     return fail(B200FFT_ERR_UNSUPPORTED, "the specialisation tier does not serve this axis (radix above %d, or no tile fits)", JIT_MAX_PRIME);
   return probe_compile(spec, report);

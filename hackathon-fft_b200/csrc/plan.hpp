@@ -101,11 +101,28 @@ struct b200fft_plan {
 
 namespace b200fft {
 
+// Copies `t` into a new device allocation that the plan owns from before the copy (so a failed copy does not leak it).
+// nullptr, with the CUDA error cleared, when the allocation or the copy fails.
+template <class T>
+T* plan_upload(b200fft_plan& plan, const std::vector<T>& t) {
+  void* d = nullptr;
+  if (cudaMalloc(&d, t.size() * sizeof(T)) != cudaSuccess) {
+    cudaGetLastError();
+    return nullptr;
+  }
+  plan.owned_device.push_back(d);
+  if (cudaMemcpy(d, t.data(), t.size() * sizeof(T), cudaMemcpyHostToDevice) != cudaSuccess) {
+    cudaGetLastError();
+    return nullptr;
+  }
+  return static_cast<T*>(d);
+}
+
 // kernel families (each returns nullptr when it does not cover the request)
 // `half`: HALF_R2C = rows of n reals -> n/2+1 complex bins; HALF_C2R = the inverse (rows only).
 std::unique_ptr<Pass> make_generic_pass(const b200fft_plan& plan, int axis, const AxisView& view,
                                         const IoSpec& src, bool scale_inverse, HalfMode half = HALF_NONE);
-// compile-time kernels (fast_registry.cu); allocates its stage twiddle table into plan.owned_device
+// compile-time kernels (fast_registry.cu); uploads its twiddle tables with plan_upload
 std::unique_ptr<Pass> make_fast_pass(b200fft_plan& plan, int axis, const AxisView& view, const IoSpec& src,
                                      bool scale_inverse, HalfMode half = HALF_NONE);
 

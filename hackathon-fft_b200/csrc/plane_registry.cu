@@ -331,13 +331,10 @@ std::unique_ptr<Pass> make_plane_fwd_pass(b200fft_plan& plan) {
     pass->planes_per_batch = 1;
     for (int a = 0; a < last - 1; ++a) pass->planes_per_batch *= p.axes[a].n;
     pass->scale = pass->inverse ? (float)(1.0 / ((double)v.ny * v.nx)) : 1.f;
-    auto upload = [&](const std::vector<float2>& t, float2** d) {
-      if (cudaMalloc(d, t.size() * sizeof(float2)) != cudaSuccess) { cudaGetLastError(); return false; }
-      plan.owned_device.push_back(*d);
-      return cudaMemcpy(*d, t.data(), t.size() * sizeof(float2), cudaMemcpyHostToDevice) == cudaSuccess;
-    };
-    if (!upload(build_twiddles(v.ry, pass->inverse), &pass->twy) || !upload(build_twiddles(v.rx, pass->inverse), &pass->twx)) return nullptr;
-    if (v.r2c && !upload(build_half_twiddles(2 * v.nx, false), &pass->tw2)) return nullptr;
+    if (!(pass->twy = plan_upload(plan, build_twiddles(v.ry, pass->inverse))) ||
+        !(pass->twx = plan_upload(plan, build_twiddles(v.rx, pass->inverse))))
+      return nullptr;
+    if (v.r2c && !(pass->tw2 = plan_upload(plan, build_half_twiddles(2 * v.nx, false)))) return nullptr;
     char buf[320];
     snprintf(buf, sizeof buf, "axes %d,%d: %s: one tile per (y, x) plane (x transform%s, y transform in shared memory)%s, smem=%zuB", last - 1,
              last, v.name.c_str(), v.r2c ? " of the real rows, Hermitian unpack on the fly" : "", real_in ? " real-in" : "", v.smem);
@@ -376,13 +373,8 @@ std::unique_ptr<Pass> make_plane_c2r_pass(b200fft_plan& plan) {
     pass->planes_per_batch = 1;
     for (int a = 0; a < last - 1; ++a) pass->planes_per_batch *= p.axes[a].n;
     pass->scale = (float)(1.0 / ((double)v.ny * 2.0 * v.h));
-    auto upload = [&](const std::vector<float2>& t, float2** d) {
-      if (cudaMalloc(d, t.size() * sizeof(float2)) != cudaSuccess) { cudaGetLastError(); return false; }
-      plan.owned_device.push_back(*d);
-      return cudaMemcpy(*d, t.data(), t.size() * sizeof(float2), cudaMemcpyHostToDevice) == cudaSuccess;
-    };
-    if (!upload(build_twiddles(v.ry, true), &pass->twy) || !upload(build_twiddles(v.rx, true), &pass->twx) ||
-        !upload(build_half_twiddles(2 * v.h, true), &pass->tw2))
+    if (!(pass->twy = plan_upload(plan, build_twiddles(v.ry, true))) || !(pass->twx = plan_upload(plan, build_twiddles(v.rx, true))) ||
+        !(pass->tw2 = plan_upload(plan, build_half_twiddles(2 * v.h, true))))
       return nullptr;
     char buf[320];
     snprintf(buf, sizeof buf, "axes %d,%d: %s: (y, x) plane of %d x %d bins -> %d x %d reals in one tile (y inverse, Hermitian pack, "

@@ -167,12 +167,7 @@ std::unique_ptr<Pass> make_rt_pass(b200fft_plan& plan, int axis, const AxisView&
     cudaGetLastError();
     return nullptr;
   }
-  std::vector<float2> tw = build_twiddles(radices, pass->inverse);
-  float2* d_tw = nullptr;
-  if (cudaMalloc(&d_tw, tw.size() * sizeof(float2)) != cudaSuccess) { cudaGetLastError(); return nullptr; }
-  plan.owned_device.push_back(d_tw);
-  if (cudaMemcpy(d_tw, tw.data(), tw.size() * sizeof(float2), cudaMemcpyHostToDevice) != cudaSuccess) return nullptr;
-  a.tw = d_tw;
+  if (!(a.tw = plan_upload(plan, build_twiddles(radices, pass->inverse)))) return nullptr;
   std::string stages;
   for (uint32_t r : ax.ordered) stages += (stages.empty() ? "" : ",") + std::to_string(r);
   char buf[320];

@@ -24,73 +24,22 @@ namespace {
 void register_split() {
   static const bool done = [] {  // thread-safe one-time initialisation (see register_all, fast_registry.cu)
     // pass A candidates (N1): <role, N, columns per tile, threads, super-stages...>
-    reg_split<SPLIT_A, 128, 16, 128, 16, 8>();
-    reg_split<SPLIT_A, 256, 16, 256, 16, 16>();
-    reg_split<SPLIT_A, 512, 16, 256, 32, 16>();
-    reg_split<SPLIT_A, 512, 16, 256, 8, 8, 8>();  // the reference's default bases for 7680 are [15, 8, 8, 8]
-    reg_split<SPLIT_A, 64, 16, 128, 8, 8>();
+    reg_split<TILE_SPLIT_A, 128, 16, 128, 16, 8>();
+    reg_split<TILE_SPLIT_A, 256, 16, 256, 16, 16>();
+    reg_split<TILE_SPLIT_A, 512, 16, 256, 32, 16>();
+    reg_split<TILE_SPLIT_A, 512, 16, 256, 8, 8, 8>();  // the reference's default bases for 7680 are [15, 8, 8, 8]
+    reg_split<TILE_SPLIT_A, 64, 16, 128, 8, 8>();
     // pass B candidates (N2)
-    reg_split<SPLIT_B_COLS, 15, 128, 128, 15>();
-    reg_split<SPLIT_B_COLS, 30, 64, 64, 30>();
-    reg_split<SPLIT_B_COLS, 16, 128, 128, 16>();
-    reg_split<SPLIT_B_ROWS, 128, 32, 256, 16, 8>();
-    reg_split<SPLIT_B_ROWS, 64, 32, 256, 8, 8>();
-    reg_split<SPLIT_B_ROWS, 256, 16, 256, 16, 16>();
+    reg_split<TILE_SPLIT_B_COLS, 15, 128, 128, 15>();
+    reg_split<TILE_SPLIT_B_COLS, 30, 64, 64, 30>();
+    reg_split<TILE_SPLIT_B_COLS, 16, 128, 128, 16>();
+    reg_split<TILE_SPLIT_B_ROWS, 128, 32, 256, 16, 8>();
+    reg_split<TILE_SPLIT_B_ROWS, 64, 32, 256, 8, 8>();
+    reg_split<TILE_SPLIT_B_ROWS, 256, 16, 256, 16, 16>();
     return true;
   }();
   (void)done;
 }
-
-struct SplitPass : Pass {
-  const SplitKernel *ka = nullptr, *kb = nullptr;
-  AxisView view;
-  bool inverse = false;
-  float scale = 1.f;
-  int do_scale = 0;
-  float2 *twa = nullptr, *twb = nullptr, *tmp = nullptr;
-  const float2* twN = nullptr;
-  std::string text;
-
-  int launch(const void* src, void* dst, int64_t nbatch, cudaStream_t stream) override {
-    const long long outer = nbatch * view.outer_per_batch;
-    if (outer <= 0) return B200FFT_OK;
-    SplitArgs a;
-    memset(&a, 0, sizeof a);
-    a.inner = view.inner;
-    a.n1 = ka->n;
-    a.n2 = kb->n;
-    // pass A: view (outer, n1, n2 * inner)
-    a.in = reinterpret_cast<const float2*>(src);
-    a.out = tmp;
-    a.tw = twa;
-    a.twN = twN;
-    const long long vinner = (long long)a.n2 * view.inner;
-    a.tiles_per_outer = (int)((vinner + ka->tile - 1) / ka->tile);
-    long long grid = outer * a.tiles_per_outer;
-    if (grid > 0x7fffffffLL) return fail(B200FFT_ERR_UNSUPPORTED, "too many tiles");
-    ka->launch(inverse, a, (unsigned)grid, ka->smem, stream);
-    // pass B
-    a.in = tmp;
-    a.out = reinterpret_cast<float2*>(dst);
-    a.tw = twb;
-    a.scale = scale;
-    a.do_scale = do_scale;
-    if (kb->role == SPLIT_B_ROWS) {
-      a.nrows = outer * a.n1;
-      grid = (a.nrows + kb->tile - 1) / kb->tile;
-    } else {
-      a.tiles_per_outer = (int)((view.inner + kb->tile - 1) / kb->tile);
-      grid = outer * a.n1 * a.tiles_per_outer;
-    }
-    if (grid > 0x7fffffffLL) return fail(B200FFT_ERR_UNSUPPORTED, "too many tiles");
-    kb->launch(inverse, a, (unsigned)grid, kb->smem, stream);
-    g_launch_count.fetch_add(2, std::memory_order_relaxed);
-    B200_CUDA_CHECK(cudaGetLastError());
-    return B200FFT_OK;
-  }
-  std::string describe() const override { return text; }
-  int launches() const override { return 2; }
-};
 
 }  // namespace
 
@@ -103,7 +52,7 @@ std::string split_variant_info(size_t i) {
   register_split();
   if (i >= split_registry().size()) return "";
   const SplitKernel& k = split_registry()[i];
-  const char* kind = k.role == SPLIT_A ? "splitA" : k.role == SPLIT_B_COLS ? "splitB_cols" : "splitB_rows";
+  const char* kind = k.kind == TILE_SPLIT_A ? "splitA" : k.kind == TILE_SPLIT_B_COLS ? "splitB_cols" : "splitB_rows";
   return "name=" + k.name + " kind=" + kind + " n=" + std::to_string(k.n) + " radices=" + radix_name(k.radices) +
          " tile=" + std::to_string(k.tile) + " threads=" + std::to_string(k.threads) + " smem=" + std::to_string(k.smem) +
          " forms=fwd,inv";
@@ -118,12 +67,12 @@ std::unique_ptr<Pass> make_split_pass(b200fft_plan& plan, int axis, const AxisVi
   const AxisSpec& ax = p.axes[axis];
   const SplitKernel *best_a = nullptr, *best_b = nullptr;
   for (const SplitKernel& ka : split_registry()) {
-    if (ka.role != SPLIT_A || view.n % ka.n) continue;
+    if (ka.kind != TILE_SPLIT_A || view.n % ka.n) continue;
     const long long n2 = view.n / ka.n;
     for (const SplitKernel& kb : split_registry()) {
       if (kb.n != n2) continue;
-      if (view.inner == 1 ? kb.role != SPLIT_B_ROWS : kb.role != SPLIT_B_COLS) continue;
-      if (kb.role == SPLIT_B_ROWS && ka.n % kb.tile) continue;  // row tiles must not straddle transforms
+      if (kb.kind != (view.inner == 1 ? TILE_SPLIT_B_ROWS : TILE_SPLIT_B_COLS)) continue;
+      if (kb.kind == TILE_SPLIT_B_ROWS && ka.n % kb.tile) continue;  // row tiles must not straddle transforms
       std::vector<int> all(ka.radices);
       all.insert(all.end(), kb.radices.begin(), kb.radices.end());
       if (!can_group(ax.ordered, all)) continue;
@@ -131,28 +80,34 @@ std::unique_ptr<Pass> make_split_pass(b200fft_plan& plan, int axis, const AxisVi
     }
   }
   if (!best_a) return nullptr;
-  if (best_a->prepare(best_a->smem) != cudaSuccess || best_b->prepare(best_b->smem) != cudaSuccess) {
-    cudaGetLastError();
-    return nullptr;
-  }
+  const bool inv = p.desc.inverse != 0;
   auto pass = std::make_unique<SplitPass>();
-  pass->ka = best_a;
-  pass->kb = best_b;
-  pass->view = view;
-  pass->inverse = p.desc.inverse != 0;
-  pass->do_scale = scale_inverse ? 1 : 0;
-  pass->scale = scale_inverse ? (float)(1.0 / (double)view.n) : 1.f;
-  pass->twN = reinterpret_cast<const float2*>(plan.tw[axis].ptr);
-  auto upload = [&](const std::vector<float2>& t, float2** out) {
-    if (cudaMalloc(out, t.size() * sizeof(float2)) != cudaSuccess) return false;
-    plan.owned_device.push_back(*out);
-    return cudaMemcpy(*out, t.data(), t.size() * sizeof(float2), cudaMemcpyHostToDevice) == cudaSuccess;
-  };
-  if (!upload(build_twiddles(best_a->radices, pass->inverse), &pass->twa) ||
-      !upload(build_twiddles(best_b->radices, pass->inverse), &pass->twb)) {
-    cudaGetLastError();
-    return nullptr;
+  const void* twN = plan.tw[axis].ptr;
+  int i = 0;
+  for (const SplitKernel* k : {best_a, best_b}) {
+    SplitPass::Stage& st = pass->st[i];
+    st.spec.kind = k->kind;
+    st.spec.n = k->n;
+    st.spec.radices = k->radices;
+    st.spec.tile = k->tile;
+    st.spec.threads = k->threads;
+    st.spec.inverse = inv;
+    st.k = {k->sym[inv], nullptr, k->name};
+    st.smem = k->smem;
+    st.twN = twN;
+    st.n2 = best_b->n;
+    pass->len[i++] = k->n;
+    if (prepare_tile(st.k.sym, st.smem) != cudaSuccess) {
+      cudaGetLastError();
+      return nullptr;
+    }
   }
+  pass->view = view;
+  pass->do_scale = scale_inverse;
+  pass->scale = scale_inverse ? 1.0 / (double)view.n : 1.0;
+  if (!(pass->st[0].tw = plan_upload(plan, build_twiddles(best_a->radices, inv))) ||
+      !(pass->st[1].tw = plan_upload(plan, build_twiddles(best_b->radices, inv))))
+    return nullptr;
   const size_t tmp_bytes = (size_t)p.batch * view.outer_per_batch * view.n * view.inner * sizeof(float2);
   if (cudaMalloc(&pass->tmp, tmp_bytes) != cudaSuccess) {
     cudaGetLastError();

@@ -9,66 +9,43 @@
 
 namespace b200fft {
 
-enum SplitRole { SPLIT_A = 0, SPLIT_B_COLS = 1, SPLIT_B_ROWS = 2 };
-
 struct SplitKernel {
   std::string name;
-  SplitRole role;
+  TileKind kind;  // TILE_SPLIT_A, TILE_SPLIT_B_COLS or TILE_SPLIT_B_ROWS
   int n;
   std::vector<int> radices;
   int tile, threads;
   size_t smem;
-  void (*launch)(bool inv, const SplitArgs&, unsigned grid, size_t smem, cudaStream_t) = nullptr;
-  cudaError_t (*prepare)(size_t) = nullptr;
+  const void* sym[2] = {};  // forward, inverse
 };
 
 std::vector<SplitKernel>& split_registry();
 
-#define B200_SPLIT_V(NAME, KERNEL)                                                                         \
-  template <int N, class RL, int T, int NT>                                                                \
-  struct NAME {                                                                                            \
-    static void launch(bool inv, const SplitArgs& a, unsigned grid, size_t smem, cudaStream_t st) {        \
-      if (inv) KERNEL<N, RL, T, NT, true><<<grid, NT, smem, st>>>(a);                                      \
-      else KERNEL<N, RL, T, NT, false><<<grid, NT, smem, st>>>(a);                                         \
-    }                                                                                                      \
-    static cudaError_t prepare(size_t smem) {                                                              \
-      if (smem <= 48 * 1024) return cudaSuccess;                                                           \
-      const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;                                       \
-      cudaError_t e = cudaFuncSetAttribute(KERNEL<N, RL, T, NT, false>, attr, (int)smem);                  \
-      if (!e) e = cudaFuncSetAttribute(KERNEL<N, RL, T, NT, true>, attr, (int)smem);                       \
-      return e;                                                                                            \
-    }                                                                                                      \
-  };
-B200_SPLIT_V(SplitAV, cols_split_a_kernel)
-B200_SPLIT_V(SplitBColsV, cols_split_b_kernel)
-B200_SPLIT_V(SplitBRowsV, rows_split_b_kernel)
-#undef B200_SPLIT_V
-
-template <SplitRole ROLE, int N, int T, int NT, int... Rs>
+template <TileKind KIND, int N, int T, int NT, int... Rs>
 void reg_split() {
   using RL = Radices<Rs...>;
   static_assert(RL::product() == N, "radices must multiply to N");
   SplitKernel k;
-  k.role = ROLE;
+  k.kind = KIND;
   k.n = N;
   k.radices = radix_vec<RL>();
   k.tile = T;
   k.threads = NT;
-  const char* tag = ROLE == SPLIT_A ? "splitA_cols" : ROLE == SPLIT_B_COLS ? "splitB_cols" : "splitB_rows";
-  k.name = std::string(tag) + std::to_string(N) + "_" + radix_name(k.radices) + (ROLE == SPLIT_B_ROWS ? "_c" : "_w") +
+  const char* tag = KIND == TILE_SPLIT_A ? "splitA_cols" : KIND == TILE_SPLIT_B_COLS ? "splitB_cols" : "splitB_rows";
+  k.name = std::string(tag) + std::to_string(N) + "_" + radix_name(k.radices) + (KIND == TILE_SPLIT_B_ROWS ? "_c" : "_w") +
            std::to_string(T) + "_t" + std::to_string(NT);
-  if constexpr (ROLE == SPLIT_A) {
+  if constexpr (KIND == TILE_SPLIT_A) {
     k.smem = cols_smem_bytes<N, RL, T>();
-    k.launch = &SplitAV<N, RL, T, NT>::launch;
-    k.prepare = &SplitAV<N, RL, T, NT>::prepare;
-  } else if constexpr (ROLE == SPLIT_B_COLS) {
+    k.sym[0] = (const void*)cols_split_a_kernel<N, RL, T, NT, false>;
+    k.sym[1] = (const void*)cols_split_a_kernel<N, RL, T, NT, true>;
+  } else if constexpr (KIND == TILE_SPLIT_B_COLS) {
     k.smem = cols_smem_bytes<N, RL, T>();
-    k.launch = &SplitBColsV<N, RL, T, NT>::launch;
-    k.prepare = &SplitBColsV<N, RL, T, NT>::prepare;
+    k.sym[0] = (const void*)cols_split_b_kernel<N, RL, T, NT, false>;
+    k.sym[1] = (const void*)cols_split_b_kernel<N, RL, T, NT, true>;
   } else {
     k.smem = rows_smem_bytes<N, RL, T>();
-    k.launch = &SplitBRowsV<N, RL, T, NT>::launch;
-    k.prepare = &SplitBRowsV<N, RL, T, NT>::prepare;
+    k.sym[0] = (const void*)rows_split_b_kernel<N, RL, T, NT, false>;
+    k.sym[1] = (const void*)rows_split_b_kernel<N, RL, T, NT, true>;
   }
   split_registry().push_back(k);
 }

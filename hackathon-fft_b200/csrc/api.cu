@@ -374,6 +374,11 @@ int b200fft_jit_probe(int64_t n, int64_t inner, const uint32_t* bases, int nbase
   return probe_entry(jit_probe, n, inner, bases, nbases, inverse, real_in, half, in_dtype, out_dtype, buf, cap);
 }
 
+int b200fft_jit_probe_strided(int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in, int half,
+                              int in_dtype, int out_dtype, char* buf, size_t cap) {
+  return probe_entry(jit_probe_strided, n, inner, bases, nbases, inverse, real_in, half, in_dtype, out_dtype, buf, cap);
+}
+
 int b200fft_jit_split_probe(int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in, int half,
                             int in_dtype, int out_dtype, char* buf, size_t cap) {
   return probe_entry(jit_split_probe, n, inner, bases, nbases, inverse, real_in, half, in_dtype, out_dtype, buf, cap);
@@ -419,13 +424,11 @@ int b200fft_plan_dry_run(const b200fft_desc* desc, char* buf, size_t cap) {
   return B200FFT_OK;
 }
 
-int b200fft_plan_create(b200fft_plan** out, const b200fft_desc* desc) {
-  if (!out) return fail(B200FFT_ERR_INVALID_ARG, "null plan pointer");
-  *out = nullptr;
-  std::unique_ptr<b200fft_plan> plan(new b200fft_plan());
-  int rc = validate(desc, &plan->prob);
-  if (rc != B200FFT_OK) return rc;
+}  // extern "C"
 
+// the device part of plan creation: twiddle tables (dense plans), passes, alignment; *out only on success
+static int finish_plan(std::unique_ptr<b200fft_plan> plan, const b200fft_desc* desc, b200fft_plan** out) {
+  int rc;
   int dev = desc->device;
   if (dev < 0) B200_CUDA_CHECK(cudaGetDevice(&dev));
   cudaDeviceProp prop;
@@ -440,12 +443,13 @@ int b200fft_plan_create(b200fft_plan** out, const b200fft_desc* desc) {
   const bool f64 = desc->out_dtype == B200FFT_F64;
   plan->tw.resize(plan->prob.rank);
   for (int a = 0; a < plan->prob.rank; ++a) {
-    // the n-entry W_n table serves passes of at most SPLIT2_MAX_N points; a longer axis has twiddle tables of its own
-    if (!plan->prob.axes[a].transformed || plan->prob.axes[a].n > SPLIT2_MAX_N) continue;
+    // the n-entry W_n table serves passes of at most SPLIT2_MAX_N points; a longer axis has twiddle tables of its own, and
+    // the single-tile passes of a strided plan upload their own stage tables
+    if (plan->strided || !plan->prob.axes[a].transformed || plan->prob.axes[a].n > SPLIT2_MAX_N) continue;
     rc = upload_twiddles(plan->prob.axes[a].n, desc->inverse != 0, f64, &plan->tw[a]);
     if (rc != B200FFT_OK) { b200fft_plan_destroy(plan.release()); return rc; }
   }
-  rc = build_passes(plan.get(), /*dry=*/false, nullptr);
+  rc = plan->strided ? build_strided_passes(plan.get()) : build_passes(plan.get(), /*dry=*/false, nullptr);
   if (rc != B200FFT_OK) { b200fft_plan_destroy(plan.release()); return rc; }
   record_alignment(plan.get());
   // The tables were uploaded with cudaMemcpy from pageable memory on the legacy stream: make sure they have landed
@@ -456,6 +460,29 @@ int b200fft_plan_create(b200fft_plan** out, const b200fft_desc* desc) {
   }
   *out = plan.release();
   return B200FFT_OK;
+}
+
+extern "C" {
+
+int b200fft_plan_create(b200fft_plan** out, const b200fft_desc* desc) {
+  if (!out) return fail(B200FFT_ERR_INVALID_ARG, "null plan pointer");
+  *out = nullptr;
+  std::unique_ptr<b200fft_plan> plan(new b200fft_plan());
+  int rc = validate(desc, &plan->prob);
+  if (rc != B200FFT_OK) return rc;
+  return finish_plan(std::move(plan), desc, out);
+}
+
+int b200fft_plan_create_strided(b200fft_plan** out, const b200fft_desc* desc, const int64_t* in_strides, const int64_t* out_strides) {
+  if (!out) return fail(B200FFT_ERR_INVALID_ARG, "null plan pointer");
+  *out = nullptr;
+  std::unique_ptr<b200fft_plan> plan(new b200fft_plan());
+  int rc = validate(desc, &plan->prob);
+  if (rc != B200FFT_OK) return rc;
+  bool dense = false;
+  if ((rc = strided_check(plan.get(), in_strides, out_strides, &dense)) != B200FFT_OK) return rc;
+  if (dense) return b200fft_plan_create(out, desc);
+  return finish_plan(std::move(plan), desc, out);
 }
 
 int b200fft_plan_destroy(b200fft_plan* plan) {
@@ -494,6 +521,10 @@ static int run_passes(b200fft_plan* plan, void* d_out, const void* d_in, int64_t
 int b200fft_exec(b200fft_plan* plan, void* d_out, const void* d_in, void* cu_stream) {
   if (!plan || !d_out || !d_in) return fail(B200FFT_ERR_INVALID_ARG, "null plan or buffer");
   if (int rc = check_alignment(plan, d_in, "d_in", d_out, "d_out")) return rc;
+  if (plan->strided && d_out == d_in && !plan->inplace_exact)
+    return fail(B200FFT_ERR_INVALID_ARG, "this strided plan cannot run in place: its input and output layouts do not map every "
+                                         "element onto itself (equal strides and element types, or the padded real layout of "
+                                         "twice the complex strides)");
   DeviceGuard guard(plan->device);
   return run_passes(plan, d_out, d_in, plan->prob.batch, (cudaStream_t)cu_stream);
 }
@@ -502,6 +533,7 @@ static int exec_scatter_impl(b200fft_plan* plan, void* const* peer_out, int npee
                              void* d_work, void* cu_stream) {
   if (!plan || !peer_out || !d_in || !d_work) return fail(B200FFT_ERR_INVALID_ARG, "null plan or buffer");
   if (plan->prob.half) return fail(B200FFT_ERR_UNSUPPORTED, "exec_scatter takes a complex plan");
+  if (plan->strided) return fail(B200FFT_ERR_UNSUPPORTED, "exec_scatter takes dense layouts; this plan is strided");
   if (my_rank < 0 || my_rank >= npeers) return fail(B200FFT_ERR_INVALID_ARG, "my_rank %d outside 0..%d", my_rank, npeers);
   if (plan->passes.empty() || plan->passes.back()->axis != 0)
     return fail(B200FFT_ERR_INVALID_ARG, "exec_scatter: the plan's last pass must transform axis 0 (the split axis); "
@@ -586,6 +618,7 @@ int b200fft_ipc_close(void* d_ptr) {
 // per direction, so PCIe transfers in both directions overlap the kernels.
 int b200fft_exec_host(b200fft_plan* plan, void* h_out, const void* h_in) {
   if (!plan || !h_out || !h_in) return fail(B200FFT_ERR_INVALID_ARG, "null plan or buffer");
+  if (plan->strided) return fail(B200FFT_ERR_UNSUPPORTED, "exec_host takes dense layouts; this plan is strided");
   DeviceGuard guard(plan->device);
   const Problem& p = plan->prob;
   const size_t in_stride = (size_t)p.in_scalars_per_batch * p.in_elem;
@@ -670,9 +703,11 @@ int b200fft_plan_launches(const b200fft_plan* plan) {
 }
 
 size_t b200fft_plan_in_bytes(const b200fft_plan* plan) {
+  if (plan && plan->strided) return plan->in_span;
   return plan ? (size_t)plan->prob.batch * plan->prob.in_scalars_per_batch * plan->prob.in_elem : 0;
 }
 size_t b200fft_plan_out_bytes(const b200fft_plan* plan) {
+  if (plan && plan->strided) return plan->out_span;
   return plan ? (size_t)plan->prob.batch * plan->prob.out_scalars_per_batch * plan->prob.out_elem : 0;
 }
 

@@ -134,6 +134,80 @@ struct GlobalDstV4 {
     *reinterpret_cast<float4*>(base + o * so + i_even) = v;
   }
 };
+// ---- strided layouts (b200fft_plan_create_strided) ----------------------------------------------------------------
+// A pass over strided buffers walks its tiles over the pass's OUTER dimensions: every dimension of the buffer except the
+// transformed axis (and, for a column tile, the dimension its columns run along), each an (extent, src stride, dst stride)
+// triple in elements of the two buffers, fastest-varying first. A CTA decomposes its tile index over them once
+// (str_origin); row kernels keep the row bases of their tile in shared memory (str_rows), so no element access divides.
+constexpr int STR_MAX_OUTER = 1 + 8;  // batch + up to 8 axes
+struct StrGeo {
+  long long ext[STR_MAX_OUTER], ss[STR_MAX_OUTER], ds[STR_MAX_OUTER];
+  long long s_ax, d_ax;    // element stride along the transformed axis in the source / destination
+  long long s_col, d_col;  // column tiles: stride of the dimension the tile's columns run along
+  int nouter;
+};
+// Addressing policy of a tile kernel, its last template parameter: DenseLay = the dense row-major addressing, the argument
+// block as is; StrLay = the same block followed by the pass's StrGeo.
+struct DenseLay {
+  static constexpr bool strided = false;
+  template <class A>
+  using Args = A;
+};
+struct StrLay {
+  static constexpr bool strided = true;
+  template <class A>
+  struct Args : A {
+    StrGeo g;
+  };
+};
+__device__ __forceinline__ void str_origin(const StrGeo& g, long long t, long long* so, long long* dso) {
+  long long s = 0, d = 0;
+  for (int k = 0; k < g.nouter; ++k) {
+    const long long q = t / g.ext[k], x = t - q * g.ext[k];
+    s += x * g.ss[k];
+    d += x * g.ds[k];
+    t = q;
+  }
+  *so = s;
+  *dso = d;
+}
+// source / destination offsets of the `valid` rows from row0 on, then a barrier
+template <int NT>
+__device__ __forceinline__ void str_rows(const StrGeo& g, long long row0, int valid, long long* rs, long long* rd) {
+  for (int o = threadIdx.x; o < valid; o += NT) str_origin(g, row0 + o, &rs[o], &rd[o]);
+  __syncthreads();
+}
+// element (o, i, c) of a strided tile lives at base[row(o) + i*si + c*sc]: row(o) = rows[o] for row tiles (ROWS), 0 for a
+// column tile, whose origin is already in `base`
+template <bool REAL, bool ROWS>
+struct StrSrc {
+  const void* __restrict__ base;
+  const long long* rows;
+  long long si, sc;
+  int valid_o, valid_c;
+  __device__ __forceinline__ float2 load(int o, int i, int c) const {
+    if (o >= valid_o || c >= valid_c) return make_float2(0.f, 0.f);
+    const long long idx = (ROWS ? rows[o] : 0) + i * si + c * sc;
+    if constexpr (REAL) {
+      return make_float2((float)__ldg(reinterpret_cast<const in_scalar*>(base) + idx), 0.f);
+    } else {
+      const in_vec2 v = __ldg(reinterpret_cast<const in_vec2*>(base) + idx);
+      return make_float2((float)v.x, (float)v.y);
+    }
+  }
+};
+template <bool ROWS>
+struct StrDst {
+  float2* __restrict__ base;
+  const long long* rows;
+  long long si, sc;
+  int valid_o, valid_c;
+  __device__ __forceinline__ void store(int o, int i, int c, float2 v) const {
+    if (o >= valid_o || c >= valid_c) return;
+    base[(ROWS ? rows[o] : 0) + i * si + c * sc] = v;
+  }
+};
+
 template <class T, class = void>
 struct is_pairwise : std::false_type {};
 template <class T>
@@ -150,6 +224,8 @@ template <class T>
 struct is_real_src : std::false_type {};
 template <bool COHERENT>
 struct is_real_src<GlobalSrc<true, COHERENT>> : std::true_type {};
+template <bool ROWS>
+struct is_real_src<StrSrc<true, ROWS>> : std::true_type {};
 
 template <class Layout>
 struct SmemSrc {
@@ -382,8 +458,9 @@ struct RowsArgs {
 // contiguous rows: tile = C consecutive transforms of length N, one tile per CTA
 // VEC: 128-bit global accesses with an intra-warp shuffle exchange (GlobalSrcV4 / GlobalDstV4); needs complex
 // input, at least two stages and even N / R_0, R_last, P_last
-template <int N, class RL, int C, int NT, bool INV, bool REAL, bool VEC = false>
-__global__ void __launch_bounds__(NT) rows_kernel(const __grid_constant__ RowsArgs a) {
+// Lay = StrLay: rows of a strided buffer (element stride g.s_ax / g.d_ax along the axis, row bases from the geometry)
+template <int N, class RL, int C, int NT, bool INV, bool REAL, bool VEC = false, class Lay = DenseLay>
+__global__ void __launch_bounds__(NT) rows_kernel(const __grid_constant__ typename Lay::template Args<RowsArgs> a) {
   extern __shared__ __align__(16) float2 smem_f2[];
   constexpr int BUF = max_exchange_elems<RL, C, RowLayoutN<N>::template type>();
   float2* buf0 = smem_f2;
@@ -391,6 +468,14 @@ __global__ void __launch_bounds__(NT) rows_kernel(const __grid_constant__ RowsAr
   pdl_wait();
   const long long row0 = (long long)blockIdx.x * C;
   const int valid = (int)min((long long)C, a.nrows - row0);
+  if constexpr (Lay::strided) {
+    __shared__ long long rs[C], rd[C];
+    str_rows<NT>(a.g, row0, valid, rs, rd);
+    StrSrc<REAL, true> src{a.in, rs, a.g.s_ax, 0, valid, 1};
+    StrDst<true> dst{a.out, rd, a.g.d_ax, 0, valid, 1};
+    run_axis<RL, N, C, 1, NT, INV, RowLayoutN<N>::template type>(src, dst, buf0, buf1, a.tw, a.scale, a.do_scale != 0);
+    return;
+  }
   const void* in = REAL ? (const void*)(reinterpret_cast<const in_scalar*>(a.in) + row0 * N)
                         : (const void*)(reinterpret_cast<const in_vec2*>(a.in) + row0 * N);
   if constexpr (VEC && !REAL) {
@@ -433,8 +518,8 @@ __device__ __forceinline__ void rows_ip_middle(float2* buf, const float2* __rest
     rows_ip_middle<N, RL, C, NT, INV, S + 1>(buf, tw);
   }
 }
-template <int N, class RL, int C, int NT, bool INV, bool REAL = false>
-__global__ void __launch_bounds__(NT) rows_ip_kernel(const __grid_constant__ RowsArgs a) {
+template <int N, class RL, int C, int NT, bool INV, bool REAL = false, class Lay = DenseLay>
+__global__ void __launch_bounds__(NT) rows_ip_kernel(const __grid_constant__ typename Lay::template Args<RowsArgs> a) {
   static_assert(RL::count >= 3 && RL::product() == N, "three or more stages that multiply to N");
   extern __shared__ __align__(16) float2 smem_f2[];
   pdl_wait();
@@ -444,6 +529,17 @@ __global__ void __launch_bounds__(NT) rows_ip_kernel(const __grid_constant__ Row
   constexpr int L = RL::count - 1;
   using L0 = RowLayout<N, RL::r[0], 1>;
   using LL = RowLayout<N, RL::processed(L), RL::processed(L - 1)>;
+  if constexpr (Lay::strided) {
+    __shared__ long long rs[C], rd[C];
+    str_rows<NT>(a.g, row0, valid, rs, rd);
+    StrSrc<REAL, true> src{a.in, rs, a.g.s_ax, 0, valid, 1};
+    run_stage<RL::r[0], 1, N, C, 1, NT, INV>(src, SmemDst<L0>{smem_f2}, a.tw, 1.f, false);
+    __syncthreads();
+    rows_ip_middle<N, RL, C, NT, INV, 1>(smem_f2, a.tw);
+    StrDst<true> dst{a.out, rd, a.g.d_ax, 0, valid, 1};
+    run_stage<RL::r[L], RL::processed(L), N, C, 1, NT, INV>(SmemSrc<LL>{smem_f2}, dst, a.tw + RL::tw_offset(L), a.scale, a.do_scale != 0);
+    return;
+  }
   const void* in = REAL ? (const void*)(reinterpret_cast<const in_scalar*>(a.in) + row0 * N)
                         : (const void*)(reinterpret_cast<const in_vec2*>(a.in) + row0 * N);
   GlobalSrc<REAL> src{in, N, 1, valid, 1};
@@ -535,9 +631,11 @@ struct HalfArgs {
 
 // one tile of C rows: `src` yields the real rows viewed as H complex each, `out` = first output row.
 // `after_stage0` runs once the input has been consumed (async kernels release their input buffer there).
+// `out_rows`: offsets of the tile's output rows from `out` (strided layouts); null = rows of H + 1 bins back to back.
 template <int H, class RL, int C, int NT, bool NB = false, bool TWS = false, class Src, class Hook>
 __device__ __forceinline__ void r2c_tile_from(const Src& src, float2* __restrict__ out, const float2* __restrict__ tw,
-                                              const float2* __restrict__ tw2, int valid, float2* smem_f2, Hook after_stage0) {
+                                              const float2* __restrict__ tw2, int valid, float2* smem_f2, Hook after_stage0,
+                                              const long long* out_rows = nullptr) {
   constexpr int EX = max_exchange_elems<RL, C, RowLayoutN<H>::template type>();
   constexpr int BUF = EX > C * H ? EX : C * H;
   float2* buf0 = smem_f2;
@@ -567,7 +665,9 @@ __device__ __forceinline__ void r2c_tile_from(const Src& src, float2* __restrict
     const float2 w = __ldg(&tw2[k]);
     const float2 t = cmulf(d, w);  // W * (Z[k] - conj(Z[H-k]))
     // X = (s - i t) / 2
-    out[idx] = make_float2(0.5f * (s.x + t.y), 0.5f * (s.y - t.x));
+    const float2 x = make_float2(0.5f * (s.x + t.y), 0.5f * (s.y - t.x));
+    if (out_rows) out[out_rows[o] + k] = x;
+    else out[idx] = x;
   }
 }
 template <int H, class RL, int C, int NT, bool COHERENT = false>
@@ -577,12 +677,20 @@ __device__ __forceinline__ void r2c_tile(const in_vec2* in, float2* __restrict__
   r2c_tile_from<H, RL, C, NT, false>(src, out, tw, tw2, valid, smem_f2, [] {});
 }
 
-template <int H, class RL, int C, int NT>
-__global__ void __launch_bounds__(NT) rows_r2c_kernel(const __grid_constant__ HalfArgs a) {
+// Lay = StrLay: the geometry's source strides count real PAIRS (every real-side stride is even)
+template <int H, class RL, int C, int NT, class Lay = DenseLay>
+__global__ void __launch_bounds__(NT) rows_r2c_kernel(const __grid_constant__ typename Lay::template Args<HalfArgs> a) {
   extern __shared__ __align__(16) float2 smem_f2[];
   pdl_wait();
   const long long row0 = (long long)blockIdx.x * C;
   const int valid = (int)min((long long)C, a.nrows - row0);
+  if constexpr (Lay::strided) {
+    __shared__ long long rs[C], rd[C];
+    str_rows<NT>(a.g, row0, valid, rs, rd);
+    StrSrc<false, true> src{a.in, rs, 1, 0, valid, 1};
+    r2c_tile_from<H, RL, C, NT>(src, reinterpret_cast<float2*>(a.out), a.tw, a.tw2, valid, smem_f2, [] {}, rd);
+    return;
+  }
   r2c_tile<H, RL, C, NT>(reinterpret_cast<const in_vec2*>(a.in) + row0 * H,
                          reinterpret_cast<float2*>(a.out) + row0 * (H + 1), a.tw, a.tw2, valid, smem_f2);
 }
@@ -595,19 +703,21 @@ __global__ void __launch_bounds__(NT) rows_r2c_kernel(const __grid_constant__ Ha
 // consecutive lanes of one warp, so the partner's value arrives with one __shfl_sync per component and the
 // unpacked bins go straight from registers to global memory: no Z buffer, no extra barrier, and the kernel
 // needs only the exchange buffer(s) of the H-point transform (none at all for a single-stage H).
-template <int H>
+// TAB: the tile's rows start at out + rows[o] (strided layouts) instead of back to back
+template <int H, bool TAB = false>
 struct R2CRegDst {
   static constexpr bool whole = true;
   float2* __restrict__ out;          // first output row of the tile; rows of H + 1 bins
   const float2* __restrict__ tw2;    // W_n^k, k = 0..H
   int valid_o;
+  const long long* rows;             // TAB: offsets of the tile's rows from `out`
   template <int R, int P>
   __device__ __forceinline__ void store_all(int o, int g, int p, const float2 (&x)[R]) const {
     static_assert(P * R == H && P <= 32 && 32 % P == 0, "last stage of an H-point transform, rows inside a warp");
     (void)g;  // always 0 in the last stage
     const int lane = (int)threadIdx.x & 31;
     const int partner = (lane & ~(P - 1)) | ((P - p) & (P - 1));
-    float2* __restrict__ row = out + (long long)o * (H + 1);
+    float2* __restrict__ row = out + (TAB ? rows[o] : (long long)o * (H + 1));
     const bool live = o < valid_o;
 #pragma unroll
     for (int k = 0; k < R; ++k) {
@@ -637,13 +747,21 @@ template <int H, class RL, int C>
 constexpr size_t rows_r2c_reg_smem_bytes() {
   return sizeof(float2) * (size_t)max_exchange_elems<RL, C, RowLayoutN<H>::template type>() * (RL::count > 2 ? 2 : 1);
 }
-template <int H, class RL, int C, int NT>
-__global__ void __launch_bounds__(NT) rows_r2c_reg_kernel(const __grid_constant__ HalfArgs a) {
+template <int H, class RL, int C, int NT, class Lay = DenseLay>
+__global__ void __launch_bounds__(NT) rows_r2c_reg_kernel(const __grid_constant__ typename Lay::template Args<HalfArgs> a) {
   extern __shared__ __align__(16) float2 smem_f2[];
   constexpr int EX = max_exchange_elems<RL, C, RowLayoutN<H>::template type>();
   pdl_wait();
   const long long row0 = (long long)blockIdx.x * C;
   const int valid = (int)min((long long)C, a.nrows - row0);
+  if constexpr (Lay::strided) {
+    __shared__ long long rs[C], rd[C];
+    str_rows<NT>(a.g, row0, valid, rs, rd);
+    StrSrc<false, true> src{a.in, rs, 1, 0, valid, 1};
+    R2CRegDst<H, true> dst{reinterpret_cast<float2*>(a.out), a.tw2, valid, rd};
+    run_axis<RL, H, C, 1, NT, false, RowLayoutN<H>::template type>(src, dst, smem_f2, smem_f2 + EX, a.tw, 1.f, false);
+    return;
+  }
   GlobalSrc<false> src{reinterpret_cast<const in_vec2*>(a.in) + row0 * H, H, 1, valid, 1};
   R2CRegDst<H> dst{reinterpret_cast<float2*>(a.out) + row0 * (H + 1), a.tw2, valid};
   run_axis<RL, H, C, 1, NT, false, RowLayoutN<H>::template type>(src, dst, smem_f2, smem_f2 + EX, a.tw, 1.f, false);
@@ -651,25 +769,35 @@ __global__ void __launch_bounds__(NT) rows_r2c_reg_kernel(const __grid_constant_
 
 // ---- R2C of an ODD length n: the n-point transform of the real row on the row kernel's stages, storing only
 // bins 0..n/2 (rows of n/2 + 1 bins). One read of 4 B and one write of ~4 B per input point.
+template <bool TAB = false>  // TAB: rows at base + rows[o] (strided layouts)
 struct GlobalHalfDst {
   float2* __restrict__ base;
   int bins;  // n/2 + 1 = output row stride
   int valid_o;
+  const long long* rows;
   __device__ __forceinline__ void store(int o, int i, int, float2 v) const {
     if (o >= valid_o || i >= bins) return;
-    base[(long long)o * bins + i] = v;
+    base[(TAB ? rows[o] : (long long)o * bins) + i] = v;
   }
 };
-template <int N, class RL, int C, int NT>
-__global__ void __launch_bounds__(NT) rows_r2c_odd_kernel(const __grid_constant__ HalfArgs a) {
+template <int N, class RL, int C, int NT, class Lay = DenseLay>
+__global__ void __launch_bounds__(NT) rows_r2c_odd_kernel(const __grid_constant__ typename Lay::template Args<HalfArgs> a) {
   static_assert(N % 2 == 1, "odd lengths only (even lengths run as an n/2-point complex transform)");
   extern __shared__ __align__(16) float2 smem_f2[];
   pdl_wait();
   constexpr int BUF = max_exchange_elems<RL, C, RowLayoutN<N>::template type>();
   const long long row0 = (long long)blockIdx.x * C;
   const int valid = (int)min((long long)C, a.nrows - row0);
+  if constexpr (Lay::strided) {
+    __shared__ long long rs[C], rd[C];
+    str_rows<NT>(a.g, row0, valid, rs, rd);
+    StrSrc<true, true> src{a.in, rs, 1, 0, valid, 1};
+    GlobalHalfDst<true> dst{reinterpret_cast<float2*>(a.out), N / 2 + 1, valid, rd};
+    run_axis<RL, N, C, 1, NT, false, RowLayoutN<N>::template type>(src, dst, smem_f2, smem_f2 + BUF, a.tw, 1.f, false);
+    return;
+  }
   GlobalSrc<true> src{reinterpret_cast<const in_scalar*>(a.in) + row0 * N, N, 1, valid, 1};
-  GlobalHalfDst dst{reinterpret_cast<float2*>(a.out) + row0 * (N / 2 + 1), N / 2 + 1, valid};
+  GlobalHalfDst<> dst{reinterpret_cast<float2*>(a.out) + row0 * (N / 2 + 1), N / 2 + 1, valid};
   run_axis<RL, N, C, 1, NT, false, RowLayoutN<N>::template type>(src, dst, smem_f2, smem_f2 + BUF, a.tw, 1.f, false);
 }
 
@@ -677,15 +805,17 @@ __global__ void __launch_bounds__(NT) rows_r2c_odd_kernel(const __grid_constant_
 // rows, so the second read of every element is an L1 / L2 hit, and the kernel needs no staging buffer, no staging
 // barrier and only the exchange buffer(s) of the H-point transform (rows_c2r_kernel used to stage the C x (H + 1) bins
 // in shared memory first: 100 KB per CTA for H = 512, two CTAs per SM, 100000 x 1024 C2R at 0.31 ms; now 3-6 CTAs).
-template <int H>
+template <int H, bool TAB = false>  // TAB: rows at xb + rows[o] (strided layouts)
 struct HermGlobalSrc {
   const in_vec2* __restrict__ xb;  // [rows][H+1] in global memory
   const float2* __restrict__ tw2;
   int valid_o;
+  const long long* rows;
   __device__ __forceinline__ float2 load(int o, int i, int) const {
     if (o >= valid_o) return make_float2(0.f, 0.f);
-    const in_vec2 a = __ldg(&xb[(long long)o * (H + 1) + i]);
-    const in_vec2 b = __ldg(&xb[(long long)o * (H + 1) + H - i]);
+    const long long r = TAB ? rows[o] : (long long)o * (H + 1);
+    const in_vec2 a = __ldg(&xb[r + i]);
+    const in_vec2 b = __ldg(&xb[r + H - i]);
     const float2 xk = make_float2((float)a.x, (float)a.y), xm = make_float2((float)b.x, -(float)b.y);
     const float2 s = make_float2(xk.x + xm.x, xk.y + xm.y), d = make_float2(xk.x - xm.x, xk.y - xm.y);
     const float2 t = cmulf(d, __ldg(&tw2[i]));  // W_n^{-i} * (X[i] - conj(X[H-i]))
@@ -694,8 +824,9 @@ struct HermGlobalSrc {
 };
 
 // (min 3 CTAs per SM for CTAs of up to 256 threads: <512, 32x16, 8, 256> sat at 83 registers = two CTAs)
-template <int H, class RL, int C, int NT>
-__global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) rows_c2r_kernel(const __grid_constant__ HalfArgs a) {
+// Lay = StrLay: the geometry's destination strides count real PAIRS (every real-side stride is even)
+template <int H, class RL, int C, int NT, class Lay = DenseLay>
+__global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) rows_c2r_kernel(const __grid_constant__ typename Lay::template Args<HalfArgs> a) {
   extern __shared__ __align__(16) float2 smem_f2[];
   pdl_wait();
   constexpr int EX = max_exchange_elems<RL, C, RowLayoutN<H>::template type>();
@@ -703,6 +834,14 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) rows_c2r_kernel(const _
   float2* buf1 = smem_f2 + EX;
   const long long row0 = (long long)blockIdx.x * C;
   const int valid = (int)min((long long)C, a.nrows - row0);
+  if constexpr (Lay::strided) {
+    __shared__ long long rs[C], rd[C];
+    str_rows<NT>(a.g, row0, valid, rs, rd);
+    HermGlobalSrc<H, true> src{reinterpret_cast<const in_vec2*>(a.in), a.tw2, valid, rs};
+    StrDst<true> dst{reinterpret_cast<float2*>(a.out), rd, 1, 0, valid, 1};
+    run_axis<RL, H, C, 1, NT, true, RowLayoutN<H>::template type>(src, dst, buf0, buf1, a.tw, a.scale, true);
+    return;
+  }
   HermGlobalSrc<H> src{reinterpret_cast<const in_vec2*>(a.in) + row0 * (H + 1), a.tw2, valid};
   GlobalDst dst{reinterpret_cast<float2*>(a.out) + row0 * H, H, 1, valid, 1};
   run_axis<RL, H, C, 1, NT, true, RowLayoutN<H>::template type>(src, dst, buf0, buf1, a.tw, a.scale, true);
@@ -710,35 +849,46 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 3 : 1) rows_c2r_kernel(const _
 
 // C2R of an ODD length n: the n-point inverse on the Hermitian-extended row (X[n - k] = conj X[k], read on the fly from
 // the n/2 + 1 stored bins), real parts stored. Mirror image of rows_r2c_odd_kernel.
-template <int N>
+template <int N, bool TAB = false>  // TAB: rows at xb + rows[o] (strided layouts)
 struct HermExtSrc {
   const in_vec2* __restrict__ xb;  // [rows][N/2+1]
   int valid_o;
+  const long long* rows;
   __device__ __forceinline__ float2 load(int o, int i, int) const {
     if (o >= valid_o) return make_float2(0.f, 0.f);
     constexpr int BINS = N / 2 + 1;
-    const in_vec2 v = __ldg(&xb[(long long)o * BINS + (i < BINS ? i : N - i)]);
+    const in_vec2 v = __ldg(&xb[(TAB ? rows[o] : (long long)o * BINS) + (i < BINS ? i : N - i)]);
     return make_float2((float)v.x, i < BINS ? (float)v.y : -(float)v.y);
   }
 };
+template <bool TAB = false>  // TAB: rows at base + rows[o] (strided layouts)
 struct RealDst {
   float* __restrict__ base;
   int n;
   int valid_o;
+  const long long* rows;
   __device__ __forceinline__ void store(int o, int i, int, float2 v) const {
-    if (o < valid_o) base[(long long)o * n + i] = v.x;
+    if (o < valid_o) base[(TAB ? rows[o] : (long long)o * n) + i] = v.x;
   }
 };
-template <int N, class RL, int C, int NT>
-__global__ void __launch_bounds__(NT) rows_c2r_odd_kernel(const __grid_constant__ HalfArgs a) {
+template <int N, class RL, int C, int NT, class Lay = DenseLay>
+__global__ void __launch_bounds__(NT) rows_c2r_odd_kernel(const __grid_constant__ typename Lay::template Args<HalfArgs> a) {
   static_assert(N % 2 == 1, "odd lengths only");
   extern __shared__ __align__(16) float2 smem_f2[];
   pdl_wait();
   constexpr int BUF = max_exchange_elems<RL, C, RowLayoutN<N>::template type>();
   const long long row0 = (long long)blockIdx.x * C;
   const int valid = (int)min((long long)C, a.nrows - row0);
+  if constexpr (Lay::strided) {
+    __shared__ long long rs[C], rd[C];
+    str_rows<NT>(a.g, row0, valid, rs, rd);
+    HermExtSrc<N, true> src{reinterpret_cast<const in_vec2*>(a.in), valid, rs};
+    RealDst<true> dst{reinterpret_cast<float*>(a.out), N, valid, rd};
+    run_axis<RL, N, C, 1, NT, true, RowLayoutN<N>::template type>(src, dst, smem_f2, smem_f2 + BUF, a.tw, a.scale, true);
+    return;
+  }
   HermExtSrc<N> src{reinterpret_cast<const in_vec2*>(a.in) + row0 * (N / 2 + 1), valid};
-  RealDst dst{reinterpret_cast<float*>(a.out) + row0 * N, N, valid};
+  RealDst<> dst{reinterpret_cast<float*>(a.out) + row0 * N, N, valid};
   run_axis<RL, N, C, 1, NT, true, RowLayoutN<N>::template type>(src, dst, smem_f2, smem_f2 + BUF, a.tw, a.scale, true);
 }
 template <int H, class RL, int C>
@@ -766,14 +916,29 @@ struct ColsArgs {
 
 // strided axis: tile = all N points of CW adjacent columns (CW*8 contiguous bytes per axis step);
 // the "transpose" the reference does with separate kernels happens in the tile addressing.
-template <int N, class RL, int CW, int NT, bool INV, bool REAL>
-__global__ void __launch_bounds__(NT) cols_kernel(const __grid_constant__ ColsArgs a) {
+// Lay = StrLay: `inner` columns along the dimension of stride g.s_col / g.d_col, tile origins from the geometry
+template <int N, class RL, int CW, int NT, bool INV, bool REAL, class Lay = DenseLay>
+__global__ void __launch_bounds__(NT) cols_kernel(const __grid_constant__ typename Lay::template Args<ColsArgs> a) {
   extern __shared__ __align__(16) float2 smem_f2[];
   constexpr int BUF = max_exchange_elems<RL, 1, DenseLayoutN<N, CW>::template type>();
   float2* buf0 = smem_f2;
   float2* buf1 = smem_f2 + BUF;
   pdl_wait();
   const unsigned bid = a.reverse ? gridDim.x - 1 - blockIdx.x : blockIdx.x;
+  if constexpr (Lay::strided) {
+    const long long t = bid / a.tiles_per_outer;
+    const long long c0 = (long long)(bid - t * a.tiles_per_outer) * CW;
+    long long so, dso;
+    str_origin(a.g, t, &so, &dso);
+    so += c0 * a.g.s_col;
+    const int valid_c = (int)min((long long)CW, a.inner - c0);
+    const void* in = REAL ? (const void*)(reinterpret_cast<const in_scalar*>(a.in) + so)
+                          : (const void*)(reinterpret_cast<const in_vec2*>(a.in) + so);
+    StrSrc<REAL, false> src{in, nullptr, a.g.s_ax, a.g.s_col, 1, valid_c};
+    StrDst<false> dst{a.out + dso + c0 * a.g.d_col, nullptr, a.g.d_ax, a.g.d_col, 1, valid_c};
+    run_axis<RL, N, 1, CW, NT, INV, DenseLayoutN<N, CW>::template type>(src, dst, buf0, buf1, a.tw, a.scale, a.do_scale != 0);
+    return;
+  }
   const long long o = bid / a.tiles_per_outer;
   const long long c0 = (long long)(bid - o * a.tiles_per_outer) * CW;
   const long long base = o * N * a.inner + c0;

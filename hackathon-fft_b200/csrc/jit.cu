@@ -135,7 +135,16 @@ std::string plane_args(const TileSpec& s) {  // "<NY, NX, Radices<y...>, Radices
 std::string shape_args(const TileSpec& s) {  // "<N, Radices<...>, tile" shared by every kernel and smem-size template
   return std::to_string(s.n) + ", b200fft::Radices<" + radix_list(s.radices) + ">, " + std::to_string(s.tile);
 }
+std::string dense_expression(const TileSpec& s);
 std::string expression(const TileSpec& s) {  // the template-id NVRTC instantiates
+  std::string e = dense_expression(s);
+  if (s.str) {  // the addressing policy, the last template parameter (rows_kernel: after VEC = false)
+    e.pop_back();
+    e += std::string(s.kind == TILE_ROWS ? ", false" : "") + ", b200fft::StrLay>";
+  }
+  return e;
+}
+std::string dense_expression(const TileSpec& s) {
   const std::string head = shape_args(s) + ", " + std::to_string(s.threads);
   const char* inv = s.inverse ? "true" : "false";
   const char* real = s.real_in ? "true" : "false";
@@ -203,7 +212,8 @@ std::string jit_name(const TileSpec& s) {
            radix_name(s.radices) + ";" + radix_name(s.radices2) + ")_inplace_t" + std::to_string(s.threads) + (s.f64 ? "_f64" : "");
   return std::string(tag[s.kind]) + std::to_string(s.n) + "_" + radix_name(s.radices) + (s.strided() ? "_w" : "_c") + std::to_string(s.tile) +
          "_t" + std::to_string(s.threads) + (s.f64 ? "_f64" : "") + ((s.kind == TILE_SPLIT_A || s.kind == TILE_SPLIT3_A) && s.real_in ? "_realin" : "") +
-         (s.in_dtype == B200FFT_U8 ? "_inu8" : s.in_dtype == (s.f64 ? B200FFT_F32 : B200FFT_F64) ? (s.f64 ? "_inf32" : "_inf64") : "");
+         (s.in_dtype == B200FFT_U8 ? "_inu8" : s.in_dtype == (s.f64 ? B200FFT_F32 : B200FFT_F64) ? (s.f64 ? "_inf32" : "_inf64") : "") +
+         (s.str ? "_str" : "");
 }
 std::string defines(const TileSpec& s) {  // rtc_prelude.cuh reads these
   std::string d;
@@ -1072,6 +1082,51 @@ std::unique_ptr<Pass> make_jit_pass(b200fft_plan& plan, int axis, const AxisView
   return pass;
 }
 
+// ---- strided layouts: every pass is one tile of this tier in its StrLay form (fast.cuh) ----------------------------------
+bool jit_strided_spec(const AxisSpec& ax, int64_t n, int64_t ncols, long long rows_hint, const IoSpec& src, bool inverse,
+                      HalfMode half, bool f64, TileSpec* spec) {
+  // rows up to the lengths the row kernels take (one-buffer rows included), column tiles up to 16384 points
+  const long long cap = ncols > 0 ? 16384 : 32768;
+  AxisView view;
+  view.n = n;
+  view.inner = ncols > 0 ? ncols : 1;
+  if (n > cap || !jit_plan_axis(ax, view, src, inverse, half, f64, spec, ncols > 0 ? 0 : rows_hint)) {
+    fail(B200FFT_ERR_UNSUPPORTED, "strided layouts are served on axes that fit one tile of the plan-time tier (%s up to %lld points, "
+         "radices up to %d); this axis of %lld points does not", ncols > 0 ? "column tiles" : "rows", cap, JIT_MAX_PRIME, (long long)n);
+    return false;
+  }
+  spec->str = true;
+  return true;
+}
+
+std::unique_ptr<StridedPass> make_jit_strided_pass(b200fft_plan& plan, int axis, const TileSpec& spec, int64_t n, HalfMode half,
+                                                   bool scale_inverse) {
+  std::shared_ptr<JitKernel> k = get_kernel(spec, plan.device);
+  if (!k) return nullptr;
+  auto pass = std::make_unique<StridedPass>();
+  pass->spec = spec;
+  pass->k = {nullptr, k->fn, jit_name(spec)};
+  pass->device = plan.device;
+  pass->do_scale = scale_inverse;
+  pass->scale = (scale_inverse || half == HALF_C2R) ? 1.0 / (double)n : 1.0;  // the half-spectrum inverse is always normalised
+  pass->smem = spec.smem();
+  const bool need_tw2 = half != HALF_NONE && spec.kind != TILE_R2C_ODD && spec.kind != TILE_C2R_ODD;
+  auto tables = [&](auto zero) {
+    using T2 = decltype(zero);
+    return (pass->tw = plan_upload(plan, build_twiddles<T2>(spec.radices, spec.inverse))) &&
+           (!need_tw2 || (pass->tw2 = plan_upload(plan, build_half_twiddles<T2>(n, half == HALF_C2R))));
+  };
+  if (!(spec.f64 ? tables(double2()) : tables(float2()))) {
+    fail(B200FFT_ERR_ALLOC, "axis %d: cannot allocate the twiddle tables of a strided pass", axis);
+    return nullptr;
+  }
+  char buf[300];
+  snprintf(buf, sizeof buf, "axis %d: %s n=%lld smem=%zuB regs=%d%s [NVRTC, %.0f ms]", axis, jit_name(spec).c_str(), (long long)n,
+           pass->smem, k->regs, k->local_bytes ? (" local=" + std::to_string(k->local_bytes) + "B").c_str() : "", k->compile_ms);
+  pass->text = buf;  // the caller appends the layout
+  return pass;
+}
+
 // ---- plane passes for plane sizes without a registered variant: the in-place plane kernels of plane.cuh specialised at
 // plan time (any NY x NX whose axes each split into two register stages and whose padded plane fits shared memory) ------
 namespace {
@@ -1216,6 +1271,21 @@ int jit_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bo
   TileSpec spec;
   if (!jit_plan_axis(ax, view, src, inverse, (HalfMode)half, out_dtype == B200FFT_F64, &spec))
     return fail(B200FFT_ERR_UNSUPPORTED, "the specialisation tier does not serve this axis (radix above %d, or no tile fits)", JIT_MAX_PRIME);
+  return probe_compile(spec, report);
+}
+
+// The same for the StrLay form of that kernel (strided layouts: b200fft_plan_create_strided)
+int jit_probe_strided(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bool inverse, bool real_in, int half,
+                      int in_dtype, int out_dtype, std::string* report) {
+  AxisSpec ax;
+  ax.n = n;
+  ax.ordered = ordered;
+  IoSpec src;
+  src.comps = real_in ? 1 : 2;
+  src.dtype = in_dtype;
+  TileSpec spec;
+  if (!jit_strided_spec(ax, n, inner > 1 ? inner : 0, 0, src, inverse, (HalfMode)half, out_dtype == B200FFT_F64, &spec))
+    return B200FFT_ERR_UNSUPPORTED;
   return probe_compile(spec, report);
 }
 

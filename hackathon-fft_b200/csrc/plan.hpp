@@ -90,6 +90,12 @@ struct b200fft_plan {
   size_t workspace_bytes = 0;
   size_t work_stride = 0;     // workspace bytes per batch item
   size_t in_align = 1, out_align = 1;  // least byte alignment of the input / output pointers the passes accept
+  // strided layouts (b200fft_plan_create_strided): per-buffer element strides over (batch, dims...), the bytes each buffer
+  // spans, and whether d_out == d_in maps every element onto itself (the only in-place call such a plan accepts)
+  bool strided = false;
+  std::vector<int64_t> in_strides, out_strides;
+  size_t in_span = 0, out_span = 0;
+  bool inplace_exact = false;
   // exec_host resources (lazily created)
   cudaStream_t hs[3] = {nullptr, nullptr, nullptr};
   void* h_dev_in[2] = {nullptr, nullptr};
@@ -132,6 +138,12 @@ std::unique_ptr<Pass> make_split_pass(b200fft_plan& plan, int axis, const AxisVi
 // runtime-length pass with compile-time codelets (rt.cu): any stage list with radices <= 32, f32 output
 std::unique_ptr<Pass> make_rt_pass(b200fft_plan& plan, int axis, const AxisView& view, const IoSpec& src,
                                    bool scale_inverse, HalfMode half = HALF_NONE);
+// strided layouts (strided.cu). strided_check: validate the strides of a validated problem and record them in `plan`, no
+// CUDA call (status 2 overlapping output / negative input strides, 1 offsets beyond int64, 4 a layout or axis this build does
+// not serve); *dense = both layouts are the dense ones, for which b200fft_plan_create's plan is built instead.
+// build_strided_passes: the passes of such a plan, one per transformed axis.
+int strided_check(b200fft_plan* plan, const int64_t* in_strides, const int64_t* out_strides, bool* dense);
+int build_strided_passes(b200fft_plan* plan);
 // fused N-d kernel (fused_registry.cu): one pass object that replaces ALL per-axis passes, or nullptr
 std::unique_ptr<Pass> make_fused_pass(b200fft_plan& plan);
 // half-spectrum inverse: the two innermost axes in one tile per plane (plane_registry.cu), or nullptr
@@ -146,6 +158,9 @@ std::unique_ptr<Pass> make_jit_pass(b200fft_plan& plan, int axis, const AxisView
                                     HalfMode half, int* status);
 int jit_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bool inverse, bool real_in, int half,
               int in_dtype, int out_dtype, std::string* report);
+// the StrLay form of that kernel, for strided layouts (same arguments; inner > 1: column tiles over `inner` columns)
+int jit_probe_strided(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bool inverse, bool real_in, int half,
+                      int in_dtype, int out_dtype, std::string* report);
 // the two passes the plan-time tier builds for an axis too long for one tile (same arguments)
 int jit_split_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bool inverse, bool real_in, int half,
                     int in_dtype, int out_dtype, std::string* report);

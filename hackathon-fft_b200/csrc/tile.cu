@@ -257,7 +257,62 @@ int split_launch(const SplitPass& p, const void* src, void* dst, long long outer
   return B200FFT_OK;
 }
 
+// the StrLay forms: the kernel's argument block followed by the pass's geometry (fast.cuh: StrLay::Args)
+template <bool F64>
+int strided_launch(const StridedPass& p, const void* src, void* dst, cudaStream_t stream) {
+  using T2 = typename Args<F64>::T2;
+  const TileSpec& s = p.spec;
+  const long long row_tiles = (p.count + s.tile - 1) / s.tile;
+  switch (s.kind) {
+    case TILE_ROWS:
+    case TILE_ROWS_IP: {
+      typename StrLay::template Args<typename Args<F64>::Rows> a;
+      memset(&a, 0, sizeof a);
+      a.in = src;
+      a.out = reinterpret_cast<T2*>(dst);
+      a.tw = reinterpret_cast<const T2*>(p.tw);
+      a.nrows = p.count;
+      a.scale = p.scale;
+      a.do_scale = p.do_scale;
+      a.g = p.geo;
+      void* params[1] = {&a};
+      return launch_tile(p.k, row_tiles, s.threads, p.smem, p.dependent, params, stream);
+    }
+    case TILE_COLS: {
+      typename StrLay::template Args<typename Args<F64>::Cols> a;
+      memset(&a, 0, sizeof a);
+      a.in = src;
+      a.out = reinterpret_cast<T2*>(dst);
+      a.tw = reinterpret_cast<const T2*>(p.tw);
+      a.inner = p.ncols;
+      a.tiles_per_outer = (int)((p.ncols + s.tile - 1) / s.tile);
+      a.scale = p.scale;
+      a.do_scale = p.do_scale;
+      a.g = p.geo;
+      void* params[1] = {&a};
+      return launch_tile(p.k, p.count * a.tiles_per_outer, s.threads, p.smem, p.dependent, params, stream);
+    }
+    default: {  // the half-spectrum row forms
+      typename StrLay::template Args<typename Args<F64>::Half> a;
+      memset(&a, 0, sizeof a);
+      a.in = src;
+      a.out = dst;
+      a.tw = reinterpret_cast<const T2*>(p.tw);
+      a.tw2 = reinterpret_cast<const T2*>(p.tw2);
+      a.nrows = p.count;
+      a.scale = p.scale;
+      a.g = p.geo;
+      void* params[1] = {&a};
+      return launch_tile(p.k, row_tiles, s.threads, p.smem, p.dependent, params, stream);
+    }
+  }
+}
+
 }  // namespace
+
+int StridedPass::launch(const void* src, void* dst, int64_t, cudaStream_t stream) {
+  return spec.f64 ? strided_launch<true>(*this, src, dst, stream) : strided_launch<false>(*this, src, dst, stream);
+}
 
 int TilePass::launch(const void* src, void* dst, int64_t nbatch, cudaStream_t stream) {
   const long long outer = nbatch * view.outer_per_batch;

@@ -8,6 +8,7 @@
 #include <string>
 #include <vector>
 
+#include "fast.cuh"
 #include "plan.hpp"
 
 namespace b200fft {
@@ -59,6 +60,7 @@ struct TileSpec {
   int in_dtype = B200FFT_F32;  // element type of the array the kernel READS (cast on load)
   int tile_divides = 0;        // geometry only: the tile must divide this (split pass B rows never straddle transforms)
   long long rows_hint = 0;     // geometry only: transforms per call when the planner knows it (few rows: more threads per row)
+  bool str = false;            // the StrLay form (fast.cuh): strided buffers, tile origins from a StrGeo (plan-time tier only)
 
   size_t esz() const { return f64 ? sizeof(double2) : sizeof(float2); }
   bool plane() const { return kind == TILE_PLANE_C2C || kind == TILE_PLANE_R2C; }
@@ -163,6 +165,28 @@ struct TilePass : Pass {
   std::string describe() const override { return text; }
   size_t min_align(bool src) const override { return tile_min_align({&spec}, src); }
 };
+
+// One pass of a plan over strided buffers (b200fft_plan_create_strided): a plan-time kernel in its StrLay form, tiles over
+// `count` rows (row kinds) or `count` x ceil(ncols / tile) column tiles (TILE_COLS), origins decomposed over `geo`.
+struct StridedPass : TilePass {
+  StrGeo geo{};
+  long long count = 0;
+  long long ncols = 0;
+  bool dependent = false;  // follows another pass of the plan (programmatic dependent launch)
+
+  int launch(const void* src, void* dst, int64_t nbatch, cudaStream_t stream) override;
+  int launch_scatter(const void*, const Scatter&, int64_t, cudaStream_t) override {
+    return fail(B200FFT_ERR_UNSUPPORTED, "strided plans have no scattering store");
+  }
+};
+
+// The plan-time kernel of one strided pass (jit.cu): n points along the axis, as rows (ncols == 0) or as column tiles over
+// ncols columns; rows_hint = rows per call. False, with the reason in last_error(), when no single tile serves it.
+bool jit_strided_spec(const AxisSpec& ax, int64_t n, int64_t ncols, long long rows_hint, const IoSpec& src, bool inverse,
+                      HalfMode half, bool f64, TileSpec* spec);
+// compile (or load) `spec` and make its pass, with the stage twiddles and W_n^{+-k} uploaded; nullptr when it fails
+std::unique_ptr<StridedPass> make_jit_strided_pass(b200fft_plan& plan, int axis, const TileSpec& spec, int64_t n, HalfMode half,
+                                                   bool scale_inverse);
 
 // An axis too long for one tile as two or three passes through one plan-owned temporary (fast.cuh: cols_split_a,
 // cols_split_b, rows_split_b, rows_split_c and their half-spectrum forms).

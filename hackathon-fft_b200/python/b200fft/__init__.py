@@ -72,6 +72,8 @@ _u32p = ctypes.POINTER(ctypes.c_uint32)
 _vp = ctypes.c_void_p
 SYMBOLS = [
     ("b200fft_plan_create", ctypes.c_int, [ctypes.POINTER(_vp), ctypes.POINTER(_Desc)]),
+    ("b200fft_plan_create_strided", ctypes.c_int, [ctypes.POINTER(_vp), ctypes.POINTER(_Desc), ctypes.POINTER(ctypes.c_int64),
+                                                    ctypes.POINTER(ctypes.c_int64)]),
     ("b200fft_exec", ctypes.c_int, [_vp, _vp, _vp, _vp]),
     ("b200fft_exec_host", ctypes.c_int, [_vp, _vp, _vp]),
     ("b200fft_stream_synchronize", ctypes.c_int, [_vp]),
@@ -117,6 +119,8 @@ SYMBOLS = [
     ("b200fft_plan_dry_run", ctypes.c_int, [ctypes.POINTER(_Desc), ctypes.c_char_p, ctypes.c_size_t]),
     ("b200fft_jit_probe", ctypes.c_int, [ctypes.c_int64, ctypes.c_int64, _u32p, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                           ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_char_p, ctypes.c_size_t]),
+    ("b200fft_jit_probe_strided", ctypes.c_int, [ctypes.c_int64, ctypes.c_int64, _u32p, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                                  ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_char_p, ctypes.c_size_t]),
     ("b200fft_jit_split_probe", ctypes.c_int, [ctypes.c_int64, ctypes.c_int64, _u32p, ctypes.c_int, ctypes.c_int, ctypes.c_int,
                                                 ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_char_p, ctypes.c_size_t]),
     ("b200fft_jit_split3_probe", ctypes.c_int, [ctypes.c_int64, ctypes.c_int64, _u32p, ctypes.c_int, ctypes.c_int, ctypes.c_int,
@@ -236,12 +240,16 @@ def schedule(phases, batch):
     return [tuple(int(out[4 * i + k]) for k in range(4)) for i in range(n)]
 
 
-def jit_probe(n, inner=1, bases=None, inverse=False, real_in=False, half=0, in_dtype="float32", out_dtype="float32"):
-    """Compile (NVRTC, no GPU needed) the specialised kernel the planner would pick for one axis; returns its report."""
+def jit_probe(n, inner=1, bases=None, inverse=False, real_in=False, half=0, in_dtype="float32", out_dtype="float32",
+              strided=False):
+    """Compile (NVRTC, no GPU needed) the specialised kernel the planner would pick for one axis; returns its report.
+    strided=True: the form a strided plan runs (b200fft_plan_create_strided), column tiles over `inner` columns when
+    inner > 1."""
     arr = (ctypes.c_uint32 * len(bases))(*bases) if bases else None
     buf = ctypes.create_string_buffer(1024)
-    _check(lib().b200fft_jit_probe(n, inner, arr, len(bases) if bases else 0, 1 if inverse else 0, 1 if real_in else 0, half,
-                                   _dtype_code(in_dtype), _dtype_code(out_dtype), buf, len(buf)))
+    probe = lib().b200fft_jit_probe_strided if strided else lib().b200fft_jit_probe
+    _check(probe(n, inner, arr, len(bases) if bases else 0, 1 if inverse else 0, 1 if real_in else 0, half,
+                 _dtype_code(in_dtype), _dtype_code(out_dtype), buf, len(buf)))
     return buf.value.decode()
 
 
@@ -372,10 +380,16 @@ class Plan:
     """Handle on a b200fft_plan: the runtime analogue of the reference's `_GPUPlan`
     (_ndim_fft_gpu.mojo:153-207): owns the device twiddle tables, built once, reused."""
 
-    def __init__(self, handle, in_layout, out_layout, in_dtype, out_dtype, inverse):
+    def __init__(self, handle, in_layout, out_layout, in_dtype, out_dtype, inverse, in_strides=None, out_strides=None):
         self._h = handle
         self.in_layout, self.out_layout = tuple(in_layout), tuple(out_layout)
         self.in_dtype, self.out_dtype, self.inverse = in_dtype, out_dtype, inverse
+        # element strides over (batch, dims...) of each buffer; None = dense (both None: a dense plan)
+        self.in_strides, self.out_strides = in_strides, out_strides
+
+    @property
+    def strided(self):
+        return self.in_strides is not None or self.out_strides is not None
 
     def exec(self, output, x, stream=None):
         _check(lib().b200fft_exec(self._h, _ptr(output), _ptr(x), _ptr(stream)))
@@ -537,8 +551,18 @@ class MgpuPlan:
             pass
 
 
+def _dense_strides(layout):
+    """Element strides over (batch, dims...) of a dense buffer of shape `layout` (last entry: 1 real / 2 complex)."""
+    out, s = [], 1
+    for v in reversed(tuple(layout)[:-1]):
+        out.append(s)
+        s *= int(v)
+    return tuple(reversed(out))
+
+
 def plan_fft(in_dtype, out_dtype, in_layout, out_layout, *, bases=None, inverse=False, runtime_twfs=True,
-             max_cluster_size=8, _test=None, real_mode=REAL_FULL, axis_mask=0, device=None, flags=0):
+             max_cluster_size=8, _test=None, real_mode=REAL_FULL, axis_mask=0, device=None, flags=0, in_strides=None,
+             out_strides=None):
     """Plan the FFT on GPU — the reference's `plan_fft[...](ctx=ctx)` (fft.mojo:160-210).
 
     in_layout / out_layout are the reference's layouts as shape tuples:
@@ -548,13 +572,26 @@ def plan_fft(in_dtype, out_dtype, in_layout, out_layout, *, bases=None, inverse=
     `max_cluster_size` are accepted for signature compatibility and ignored (twiddles always
     come from device tables here). `_test`: a GPUTest value forces a kernel tier (the role of the
     reference's `Optional[_GPUTest]`); any other non-None value forces the generic kernel.
+    `in_strides` / `out_strides`: strided buffers (b200fft_plan_create_strided), one stride per dimension of the layout
+    but the last, in ELEMENTS (complex pairs or real scalars) of that buffer; None = dense. A torch view `v` of complex
+    pairs has element strides `[s // 2 for s in v.stride()[:-1]]`.
     """
     if _test is not None:
         flags |= GPUTest.FLAGS.get(_test, FLAG_FORCE_GENERIC) if isinstance(_test, int) else FLAG_FORCE_GENERIC
     d, keep = _make_desc(in_dtype, out_dtype, in_layout, out_layout, bases, inverse, real_mode, axis_mask, device, flags)
     h = ctypes.c_void_p()
-    _check(lib().b200fft_plan_create(ctypes.byref(h), ctypes.byref(d)))
-    return Plan(h, in_layout, out_layout, in_dtype, out_dtype, inverse)
+    if in_strides is None and out_strides is None:
+        _check(lib().b200fft_plan_create(ctypes.byref(h), ctypes.byref(d)))
+        return Plan(h, in_layout, out_layout, in_dtype, out_dtype, inverse)
+    strides = []
+    for name, st, layout in (("in_strides", in_strides, in_layout), ("out_strides", out_strides, out_layout)):
+        st = _dense_strides(layout) if st is None else tuple(int(v) for v in st)
+        if len(st) != len(layout) - 1:
+            raise B200FFTError(2, "%s needs %d strides (batch and each axis), got %d" % (name, len(layout) - 1, len(st)))
+        strides.append(st)
+    arrs = [(ctypes.c_int64 * len(st))(*st) for st in strides]
+    _check(lib().b200fft_plan_create_strided(ctypes.byref(h), ctypes.byref(d), arrs[0], arrs[1]))
+    return Plan(h, in_layout, out_layout, in_dtype, out_dtype, inverse, strides[0], strides[1])
 
 
 def fft(output, x, ctx=None, *, plan):
@@ -564,10 +601,16 @@ def fft(output, x, ctx=None, *, plan):
     plan's layouts; `ctx` is the CUDA stream (torch.cuda.Stream, raw handle, or None for the
     current torch stream). Asynchronous; the caller synchronises (bench.mojo:51-52).
     """
-    for name, t, layout in (("output", output, plan.out_layout), ("x", x, plan.in_layout)):
+    for name, t, layout, st in (("output", output, plan.out_layout, plan.out_strides), ("x", x, plan.in_layout, plan.in_strides)):
         if hasattr(t, "shape") and tuple(t.shape) != tuple(layout):
             raise B200FFTError(2, "%s has shape %s, the plan was built for %s" % (name, tuple(t.shape), layout))
-        if hasattr(t, "is_contiguous") and not t.is_contiguous():
+        if plan.strided and hasattr(t, "stride"):
+            want = tuple(v * layout[-1] for v in (st or _dense_strides(layout))) + (1,)
+            got = tuple(t.stride())
+            # a dimension of extent 1 may carry any stride; the components of an element must be adjacent
+            if any(g != w for g, w, n in zip(got, want, t.shape) if n > 1) or (layout[-1] == 2 and got[-1] != 1):
+                raise B200FFTError(2, "%s has strides %s, the plan was built for %s" % (name, got, want))
+        elif hasattr(t, "is_contiguous") and not t.is_contiguous():
             raise B200FFTError(2, "%s must be dense row-major" % name)
         if hasattr(t, "is_cuda") and not t.is_cuda:
             raise B200FFTError(5, "%s is not a CUDA tensor: there is no CPU path (use Plan.exec_host for host buffers)" % name)

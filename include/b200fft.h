@@ -111,6 +111,26 @@ typedef struct b200fft_plan b200fft_plan;
  * Validates the layout and bases, chooses kernels, uploads the twiddle tables. */
 B200FFT_API int b200fft_plan_create(b200fft_plan** plan, const b200fft_desc* desc);
 
+/* The same transform over STRIDED buffers (the layouts of cuFFT's advanced plans, or of a torch view). Each array has
+ * rank + 1 strides, in ELEMENTS of that buffer, for the dimensions (batch, d0, ..., d_{rank-1}) of its own layout; one
+ * element is one complex pair (its two components stay adjacent) or one real scalar, and the complex side of a
+ * half-spectrum plan has n/2+1 elements along the last axis. NULL = the dense row-major strides; dense strides, given
+ * either way, make exactly b200fft_plan_create's plan. Checked before any CUDA call:
+ *   - input strides >= 0, output strides >= 1 and no two output elements at one offset: B200FFT_ERR_LAYOUT;
+ *   - an offset beyond int64: B200FFT_ERR_INVALID_ARG;
+ *   - REAL_HALF: stride 1 along the last axis on both sides (pitched rows), and for an even length every real-side stride
+ *     even (the kernels move real rows as pairs): B200FFT_ERR_UNSUPPORTED.
+ * Every transformed axis is one pass of the plan-time specialisation tier reading and writing the arrays through their
+ * strides (no copy pass): rows when the axis has the smallest stride of the buffer a pass reads, column tiles along the
+ * dimension that has it otherwise. An axis longer than one tile (rows above 32768 points, column tiles above 16384),
+ * FORCE_GENERIC, FORCE_RT and B200FFT_JIT=0 return B200FFT_ERR_UNSUPPORTED. b200fft_exec runs such a plan in place
+ * (d_out == d_in) only when that maps every element onto itself: equal strides and element types, or for REAL_HALF real
+ * strides twice the complex ones on every dimension but the last (the padded in-place R2C / C2R layout) with equal input
+ * and output precision; any other in-place call returns B200FFT_ERR_INVALID_ARG. b200fft_plan_in_bytes / out_bytes report
+ * the bytes each buffer spans; exec_host and exec_scatter(_at) take dense plans only (B200FFT_ERR_UNSUPPORTED). */
+B200FFT_API int b200fft_plan_create_strided(b200fft_plan** plan, const b200fft_desc* desc, const int64_t* in_strides,
+                                            const int64_t* out_strides);
+
 /* ---- fft(output, x, ctx, plan=plan)  (fft.mojo:262-323 -> _run_gpu_nd_fft, _ndim_fft_gpu.mojo:462-642)
  * Asynchronous on `cu_stream` (a CUstream / cudaStream_t; NULL = default stream);
  * the caller synchronises, as bench.mojo:51-52 does. `d_out` and `d_in` are device
@@ -259,6 +279,10 @@ B200FFT_API int b200fft_plan_dry_run(const b200fft_desc* desc, char* buf, size_t
 B200FFT_API int b200fft_jit_probe(int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in,
                                   int half /* 0 complex, 1 half-spectrum R2C rows, 2 C2R rows */, int in_dtype, int out_dtype,
                                   char* buf, size_t cap);
+/* The same for the strided form of that kernel (b200fft_plan_create_strided; inner > 1: column tiles over `inner` columns).
+ * Its variant name ends in "_str". No GPU needed. */
+B200FFT_API int b200fft_jit_probe_strided(int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in,
+                                          int half, int in_dtype, int out_dtype, char* buf, size_t cap);
 /* The same for an axis too long for one tile: compiles the two passes (pass A: N1-point strided transforms with the
  * twiddle fused into the store; pass B: N2-point rows with the natural-order, half-spectrum or real store) the
  * planner builds for it, and writes "<pass A report>; <pass B report>". Serves complex, real-input and half-spectrum

@@ -69,6 +69,9 @@ struct PlanOptions {
   uint32_t axis_mask = 0;          // 0 = all axes (reference)
   int device = -1;                 // -1 = current device
   uint32_t flags = 0;
+  // strided buffers (b200fft_plan_create_strided): one stride per dimension of the layout but the last, in ELEMENTS
+  // (complex pairs or real scalars) of that buffer; empty = dense
+  std::vector<int64_t> in_strides, out_strides;
 };
 
 namespace detail {
@@ -190,7 +193,15 @@ inline Plan plan_fft(DType in_dtype, DType out_dtype, const Layout& in_layout, c
   detail::Marshalled m;
   detail::marshal(in_dtype, out_dtype, in_layout, out_layout, options, &m);
   b200fft_plan* h = nullptr;
-  check(b200fft_plan_create(&h, &m.desc));
+  if (options.in_strides.empty() && options.out_strides.empty()) {
+    check(b200fft_plan_create(&h, &m.desc));
+  } else {
+    const size_t want = out_layout.rank() - 1;
+    if ((!options.in_strides.empty() && options.in_strides.size() != want) || (!options.out_strides.empty() && options.out_strides.size() != want))
+      throw Error(B200FFT_ERR_LAYOUT, "in_strides / out_strides need one stride per dimension of the layout but the last");
+    check(b200fft_plan_create_strided(&h, &m.desc, options.in_strides.empty() ? nullptr : options.in_strides.data(),
+                                      options.out_strides.empty() ? nullptr : options.out_strides.data()));
+  }
   return Plan(h, in_layout, out_layout);
 }
 

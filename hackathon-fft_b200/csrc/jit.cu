@@ -606,34 +606,40 @@ bool jit_enabled() {
   return !(e && atoi(e) == 0);
 }
 
-// kind + transform length + stage list for one axis; false when this tier does not serve it
+// kind + transform length + stage list for one axis; false when this tier does not serve it, with the reason in *why
 bool jit_plan_axis(const AxisSpec& ax, const AxisView& view, const IoSpec& src, bool inverse, HalfMode half, bool f64,
-                   TileSpec* spec, long long rows_hint = 0) {
+                   TileSpec* spec, long long rows_hint = 0, const char** why = nullptr) {
+  auto refuse = [&](const char* reason) {
+    if (why) *why = reason;
+    return false;
+  };
   spec->rows_hint = rows_hint;
   spec->inverse = inverse;
   spec->real_in = src.comps == 1;
   spec->f64 = f64;
   spec->in_dtype = src.dtype;
-  if (half == HALF_C2R && src.dtype != (f64 ? B200FFT_F64 : B200FFT_F32)) return false;  // the staged half spectrum is read as is
-  if (half != HALF_NONE && src.dtype == B200FFT_U8) return false;
+  static const char* const no_codelets = "the tier has no codelets for its stage list (primes up to 127, composites up to 64)";
+  if (half == HALF_C2R && src.dtype != (f64 ? B200FFT_F64 : B200FFT_F32))  // the staged half spectrum is read as is
+    return refuse("C2R reads the half spectrum in the working precision, and this input is not in it");
+  if (half != HALF_NONE && src.dtype == B200FFT_U8) return refuse("half-spectrum transforms take floating-point input");
   if (half == HALF_NONE) {
     spec->kind = view.inner != 1 ? TILE_COLS : TILE_ROWS;
     spec->n = (int)view.n;
-    if (!jit_group(ax.ordered, &spec->radices, f64)) return false;
+    if (!jit_group(ax.ordered, &spec->radices, f64)) return refuse(no_codelets);
   } else {
-    if (view.inner != 1) return false;  // half-spectrum handling is a row pass
+    if (view.inner != 1) return refuse("half-spectrum handling is a row pass");
     if (view.n % 2) {
       spec->kind = half == HALF_R2C ? TILE_R2C_ODD : TILE_C2R_ODD;
       spec->n = (int)view.n;
-      if (!jit_group(ax.ordered, &spec->radices, f64)) return false;
+      if (!jit_group(ax.ordered, &spec->radices, f64)) return refuse(no_codelets);
     } else {
       // n = 2H real points as an H-point complex transform: the user's stage list with one factor 2 removed
       spec->n = (int)(view.n / 2);
       bool ok = false;
       for (const auto& o : drop_factor_two(ax.ordered))
         if (jit_group(o, &spec->radices, f64)) { ok = true; break; }
-      if (!ok) return false;
-      if (spec->n == 1) return false;
+      if (!ok) return refuse(no_codelets);
+      if (spec->n == 1) return refuse("a 2-point half spectrum has no 1-point complex transform to run");
       spec->kind = half == HALF_C2R ? TILE_C2R : TILE_R2C;
       if (half == HALF_R2C && r2c_reg_shape_ok(*spec) && !getenv("B200FFT_R2C_SMEM")) spec->kind = TILE_R2C_REG;
     }
@@ -673,10 +679,11 @@ bool jit_plan_axis(const AxisSpec& ax, const AxisView& view, const IoSpec& src, 
     if (jit_rows_ip_geometry(spec)) return true;
     spec->kind = TILE_ROWS;
   }
+  static const char* const no_tile = "no tile fits the tier's 200 KB shared-memory budget (and 512 threads per CTA)";
   if (!jit_geometry(spec, view.inner)) {
-    if (spec->kind != TILE_R2C_REG) return false;
+    if (spec->kind != TILE_R2C_REG) return refuse(no_tile);
     spec->kind = TILE_R2C;  // no tile keeps whole warps per row group: the shared-memory unpack
-    if (!jit_geometry(spec, view.inner)) return false;
+    if (!jit_geometry(spec, view.inner)) return refuse(no_tile);
   }
   return true;
 }
@@ -1085,14 +1092,15 @@ std::unique_ptr<Pass> make_jit_pass(b200fft_plan& plan, int axis, const AxisView
 // ---- strided layouts: every pass is one tile of this tier in its StrLay form (fast.cuh) ----------------------------------
 bool jit_strided_spec(const AxisSpec& ax, int64_t n, int64_t ncols, long long rows_hint, const IoSpec& src, bool inverse,
                       HalfMode half, bool f64, TileSpec* spec) {
-  // rows up to the lengths the row kernels take (one-buffer rows included), column tiles up to 16384 points
-  const long long cap = ncols > 0 ? 16384 : 32768;
+  // the axis must fit one tile: what limits it is the shared memory of that tile (jit_geometry / jit_rows_ip_geometry), so
+  // the longest axis served depends on the precision, the stage count and, for column tiles, the number of columns
   AxisView view;
   view.n = n;
   view.inner = ncols > 0 ? ncols : 1;
-  if (n > cap || !jit_plan_axis(ax, view, src, inverse, half, f64, spec, ncols > 0 ? 0 : rows_hint)) {
-    fail(B200FFT_ERR_UNSUPPORTED, "strided layouts are served on axes that fit one tile of the plan-time tier (%s up to %lld points, "
-         "radices up to %d); this axis of %lld points does not", ncols > 0 ? "column tiles" : "rows", cap, JIT_MAX_PRIME, (long long)n);
+  const char* why = "";
+  if (!jit_plan_axis(ax, view, src, inverse, half, f64, spec, ncols > 0 ? 0 : rows_hint, &why)) {
+    fail(B200FFT_ERR_UNSUPPORTED, "strided layouts run every axis as one tile of the plan-time tier; for this %lld-point %s axis "
+         "(%s) %s", (long long)n, f64 ? "fp64" : "fp32", ncols > 0 ? "column tiles" : "rows", why);
     return false;
   }
   spec->str = true;
@@ -1285,7 +1293,7 @@ int jit_probe_strided(int64_t n, int64_t inner, const std::vector<uint32_t>& ord
   src.dtype = in_dtype;
   TileSpec spec;
   if (!jit_strided_spec(ax, n, inner > 1 ? inner : 0, 0, src, inverse, (HalfMode)half, out_dtype == B200FFT_F64, &spec))
-    return B200FFT_ERR_UNSUPPORTED;
+    return B200FFT_ERR_UNSUPPORTED;  // jit_strided_spec has set the reason
   return probe_compile(spec, report);
 }
 

@@ -162,6 +162,11 @@ int strided_check(b200fft_plan* plan, const int64_t* in_strides, const int64_t* 
   plan->out_strides.assign(dout.st, dout.st + nd);
   if (in_strides) plan->in_strides.assign(in_strides, in_strides + nd);
   if (out_strides) plan->out_strides.assign(out_strides, out_strides + nd);
+  // no kernel reads the stride of a dimension of extent 1 (a batch of 1, an axis of one point): any value is the dense one
+  for (int d = 0; d < nd; ++d) {
+    if (din.ext[d] == 1) plan->in_strides[(size_t)d] = din.st[d];
+    if (dout.ext[d] == 1) plan->out_strides[(size_t)d] = dout.st[d];
+  }
   *dense = std::equal(plan->in_strides.begin(), plan->in_strides.end(), din.st) &&
            std::equal(plan->out_strides.begin(), plan->out_strides.end(), dout.st);
   if (*dense) return B200FFT_OK;
@@ -217,7 +222,9 @@ int strided_check(b200fft_plan* plan, const int64_t* in_strides, const int64_t* 
     const std::vector<int64_t>& re = p.desc.inverse ? plan->out_strides : plan->in_strides;
     const std::vector<int64_t>& cx = p.desc.inverse ? plan->in_strides : plan->out_strides;
     plan->inplace_exact = p.desc.in_dtype == p.desc.out_dtype;
-    for (int d = 0; d + 1 < nd; ++d) plan->inplace_exact = plan->inplace_exact && re[(size_t)d] == 2 * cx[(size_t)d];
+    // (a dimension of extent 1 holds no second element: its strides, set to each side's dense value above, are not compared)
+    for (int d = 0; d + 1 < nd; ++d)
+      plan->inplace_exact = plan->inplace_exact && (din.ext[d] == 1 || re[(size_t)d] == 2 * cx[(size_t)d]);
   }
   return B200FFT_OK;
 }

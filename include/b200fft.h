@@ -115,15 +115,19 @@ B200FFT_API int b200fft_plan_create(b200fft_plan** plan, const b200fft_desc* des
  * rank + 1 strides, in ELEMENTS of that buffer, for the dimensions (batch, d0, ..., d_{rank-1}) of its own layout; one
  * element is one complex pair (its two components stay adjacent) or one real scalar, and the complex side of a
  * half-spectrum plan has n/2+1 elements along the last axis. NULL = the dense row-major strides; dense strides, given
- * either way, make exactly b200fft_plan_create's plan. Checked before any CUDA call:
+ * either way, make exactly b200fft_plan_create's plan. The stride of a dimension of extent 1 is never read: any value
+ * stands for the dense one, and no rule below applies to it. Checked before any CUDA call:
  *   - input strides >= 0, output strides >= 1 and no two output elements at one offset: B200FFT_ERR_LAYOUT;
  *   - an offset beyond int64: B200FFT_ERR_INVALID_ARG;
  *   - REAL_HALF: stride 1 along the last axis on both sides (pitched rows), and for an even length every real-side stride
  *     even (the kernels move real rows as pairs): B200FFT_ERR_UNSUPPORTED.
  * Every transformed axis is one pass of the plan-time specialisation tier reading and writing the arrays through their
  * strides (no copy pass): rows when the axis has the smallest stride of the buffer a pass reads, column tiles along the
- * dimension that has it otherwise. An axis longer than one tile (rows above 32768 points, column tiles above 16384),
- * FORCE_GENERIC, FORCE_RT and B200FFT_JIT=0 return B200FFT_ERR_UNSUPPORTED. b200fft_exec runs such a plan in place
+ * dimension that has it otherwise. One tile holds the whole axis in at most 200 KB of shared memory: rows up to 16384
+ * points in fp32 and 8192 in fp64 (some longer lengths fit, such as 20000 and 12500), column tiles over 8 or more
+ * columns up to 1024 points in fp32 and 512 in fp64 (two-stage fp32 lengths such as 2304 = 48 x 48 fit; tiles over
+ * fewer columns take longer axes). A longer axis, FORCE_GENERIC, FORCE_RT and B200FFT_JIT=0 return
+ * B200FFT_ERR_UNSUPPORTED, naming the case. b200fft_exec runs such a plan in place
  * (d_out == d_in) only when that maps every element onto itself: equal strides and element types, or for REAL_HALF real
  * strides twice the complex ones on every dimension but the last (the padded in-place R2C / C2R layout) with equal input
  * and output precision; any other in-place call returns B200FFT_ERR_INVALID_ARG. b200fft_plan_in_bytes / out_bytes report

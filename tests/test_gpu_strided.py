@@ -3,112 +3,16 @@
 Every case reads its input through a view of a larger random buffer and writes its output through a view of a larger
 NaN-filled buffer: afterwards the input buffer is unchanged and every output element outside the view is still NaN. The
 plan has one launch per transformed axis, names only plan-time `_str` kernels, and a second plan of the same problem
-gives the same bits."""
+gives the same bits (tests/_strided_forms.py: run_case; tests/test_gpu_strided_forms.py runs its table of every
+strided kernel form)."""
 import numpy as np
 import pytest
 import torch
 
 import b200fft
+from _strided_forms import check, dense, run_case, t2
 
 pytestmark = pytest.mark.gpu
-
-DT = {"float32": torch.float32, "float64": torch.float64, "uint8": torch.uint8}
-
-
-def dense(shape):
-    out, s = [], 1
-    for v in reversed(shape):
-        out.append(s)
-        s *= v
-    return list(reversed(out))
-
-
-def buffer_view(shape, strides, comps, dtype, fill, gen=None):
-    """A view of logical `shape` (batch, dims...) with element `strides` into a fresh buffer one element longer than
-    the span (so the view never ends at the buffer's end); `fill`: "rand" or "nan"."""
-    span = sum((n - 1) * s for n, s in zip(shape, strides)) + 2
-    dt = DT[dtype]
-    if fill == "nan":
-        buf = torch.full((span * comps,), float("nan"), dtype=dt, device="cuda")
-    elif dt == torch.uint8:
-        buf = torch.randint(0, 256, (span * comps,), dtype=dt, device="cuda", generator=gen)
-    else:
-        buf = torch.randn(span * comps, dtype=dt, device="cuda", generator=gen)
-    view = buf.as_strided(tuple(shape) + (comps,), tuple(s * comps for s in strides) + (1,))
-    return buf, view
-
-
-def as_complex64(t, comps):
-    t = t.double()
-    return torch.complex(t[..., 0], t[..., 1]) if comps == 2 else t[..., 0].to(torch.complex128)
-
-
-def check(got, ref, out_dtype):
-    got, ref = got.cpu(), ref.cpu()
-    err = (torch.linalg.vector_norm(got - ref) / torch.linalg.vector_norm(ref)).item()
-    if out_dtype == "float64":
-        assert err <= 1e-13, err
-    else:
-        assert err <= 2e-6, err
-        assert (got - ref).abs().max().item() <= 1e-5 * ref.abs().max().item()
-
-
-def run_case(shape, in_strides, out_strides, *, in_dtype="float32", out_dtype="float32", comps=2, half=False, inverse=False,
-             axis_mask=0):
-    """shape: logical (batch, dims...) of the real side for half-spectrum plans, of both sides otherwise."""
-    gen = torch.Generator(device="cuda").manual_seed(sum(shape))
-    rank = len(shape) - 1
-    axes = [a for a in range(rank) if not axis_mask or axis_mask >> a & 1]
-    cshape = list(shape[:-1]) + [shape[-1] // 2 + 1] if half else list(shape)
-    ishape, oshape = (cshape, shape) if half and inverse else (shape, cshape) if half else (shape, shape)
-    icomps = 2 if half and inverse else 1 if half else comps
-    ocomps = 1 if half and inverse else 2
-    in_buf, x = buffer_view(ishape, in_strides, icomps, in_dtype, "rand", gen)
-    if half and inverse:  # a Hermitian spectrum: the half spectrum of a real signal
-        real = torch.randn(tuple(shape), dtype=torch.float64, device="cuda", generator=gen)
-        spec = torch.fft.rfftn(real, dim=[a + 1 for a in axes])
-        x[..., 0].copy_(spec.real)
-        x[..., 1].copy_(spec.imag)
-    in_copy = in_buf.clone()
-    out_buf, y = buffer_view(oshape, out_strides, ocomps, out_dtype, "nan")
-    kw = dict(inverse=inverse, axis_mask=axis_mask, real_mode=b200fft.REAL_HALF if half else b200fft.REAL_FULL,
-              in_strides=in_strides, out_strides=out_strides)
-    plan = b200fft.plan_fft(in_dtype, out_dtype, tuple(ishape) + (icomps,), tuple(oshape) + (ocomps,), **kw)
-    assert plan.launches == len(axes), plan.describe()
-    lines = plan.describe().strip().split("\n")
-    assert len(lines) == len(axes) and all("_str" in ln and "NVRTC" in ln for ln in lines), lines
-    b200fft.fft(y, x, plan=plan)
-    torch.cuda.synchronize()
-    assert torch.equal(in_buf, in_copy), "the input was modified"
-    mask = torch.ones(out_buf.shape, dtype=torch.bool, device="cuda")
-    mask.as_strided(y.shape, y.stride()).fill_(False)
-    assert out_buf[mask].isnan().all(), "an element outside the output view was written"
-    assert not y.isnan().any(), "an output element was not written"
-    dims = [a + 1 for a in axes]
-    xd = as_complex64(x, icomps)
-    if half and inverse:
-        ref = torch.fft.irfftn(xd, s=[shape[a] for a in dims], dim=dims)
-        got = y[..., 0].double()
-    elif half:
-        ref = torch.fft.rfftn(x[..., 0].double(), dim=dims)
-        got = as_complex64(y, 2)
-    else:
-        ref = (torch.fft.ifftn if inverse else torch.fft.fftn)(xd, dim=dims)
-        got = as_complex64(y, 2)
-    check(got, ref, out_dtype)
-    # a second plan of the same problem: the same bits
-    out2_buf, y2 = buffer_view(oshape, out_strides, ocomps, out_dtype, "nan")
-    plan2 = b200fft.plan_fft(in_dtype, out_dtype, tuple(ishape) + (icomps,), tuple(oshape) + (ocomps,), **kw)
-    b200fft.fft(y2, x, plan=plan2)
-    torch.cuda.synchronize()
-    assert torch.equal(y, y2)
-
-
-def t2(shape, perm):
-    """element strides of a dense array of `shape` seen through the axis permutation `perm` (batch stays first)"""
-    st = dense(shape)
-    return [st[p] for p in perm]
-
 
 CASES = [
     # (id, logical shape, in strides, out strides, options)
@@ -145,9 +49,11 @@ def test_strided_view_matches_torch(shape, in_strides, out_strides, opts):
     run_case(shape, in_strides, out_strides, **opts)
 
 
-@pytest.mark.parametrize("shape", [(100000, 1024), (16, 128, 128, 128)], ids=["1d", "3d"])
-def test_in_place_padded_round_trip(shape):
-    """The classic in-place layout: real rows of pitch 2(n/2+1) sharing their bytes with the n/2+1 complex bins."""
+@pytest.mark.parametrize("shape,axis_mask", [((100000, 1024), 0), ((16, 128, 128, 128), 0), ((1, 64, 64, 64), 0),
+                                              ((4, 1, 64), 0b10)], ids=["1d", "3d", "3d-batch-1", "masked-axis-of-1"])
+def test_in_place_padded_round_trip(shape, axis_mask):
+    """The classic in-place layout: real rows of pitch 2(n/2+1) sharing their bytes with the n/2+1 complex bins. A
+    dimension of extent 1 (a batch of 1, a masked axis of one point) runs in place whatever its strides."""
     n = shape[-1]
     hb = n // 2 + 1
     cshape = shape[:-1] + (hb,)
@@ -160,9 +66,9 @@ def test_in_place_padded_round_trip(shape):
     x0 = real.clone()
     cplx = buf.as_strided(cshape + (2,), tuple(2 * s for s in cst) + (1,))
     fwd = b200fft.plan_fft("float32", "float32", shape + (1,), cshape + (2,), real_mode=b200fft.REAL_HALF,
-                           in_strides=rst, out_strides=cst)
+                           in_strides=rst, out_strides=cst, axis_mask=axis_mask)
     inv = b200fft.plan_fft("float32", "float32", cshape + (2,), shape + (1,), real_mode=b200fft.REAL_HALF, inverse=True,
-                           in_strides=cst, out_strides=rst)
+                           in_strides=cst, out_strides=rst, axis_mask=axis_mask)
     # out of place through the same layouts first
     sep = torch.full_like(buf, float("nan"))
     sep_c = sep.as_strided(cplx.shape, cplx.stride())
@@ -170,7 +76,7 @@ def test_in_place_padded_round_trip(shape):
     b200fft.fft(cplx, real, plan=fwd)  # in place
     torch.cuda.synchronize()
     assert torch.equal(cplx, sep_c), "in-place R2C differs from the out-of-place result"
-    dims = list(range(1, len(shape)))
+    dims = [a + 1 for a in range(len(shape) - 1) if not axis_mask or axis_mask >> a & 1]
     ref = torch.fft.rfftn(x0[..., 0].double(), dim=dims)
     check(torch.complex(cplx[..., 0].double(), cplx[..., 1].double()), ref, "float32")
     back = torch.full_like(buf, float("nan"))
@@ -204,7 +110,14 @@ def test_refusals_on_the_device():
     with pytest.raises(b200fft.B200FFTError) as e:  # in place, but input and output strides differ
         plan.exec(buf, buf)
     assert e.value.status == 1
-    # equal strides: in place is exact
+    # equal strides: in place is exact, the same bits as out of place, and the pitch padding is left alone
     same = b200fft.plan_fft("float32", "float32", shape, shape, in_strides=[1040, 1], out_strides=[1040, 1])
+    buf.copy_(torch.randn(buf.shape, generator=torch.Generator(device="cuda").manual_seed(2), device="cuda"))
+    sep = torch.full_like(buf, float("nan"))
+    same.exec(sep, buf)
+    before = buf.clone()
     same.exec(buf, buf)
     torch.cuda.synchronize()
+    rows = buf.view(64, 1040, 2)
+    assert torch.equal(rows[:, :1000], sep.view(64, 1040, 2)[:, :1000]), "in place differs from out of place"
+    assert torch.equal(rows[:, 1000:], before.view(64, 1040, 2)[:, 1000:]), "in place wrote into the pitch padding"

@@ -60,7 +60,8 @@ def test_strided_plans_refuse_without_the_plan_time_tier(monkeypatch):
 
 
 def test_axes_longer_than_one_tile_refuse():
-    # a column tile takes up to 16384 points: a 32768-point axis read across a transposed view has no plan
+    # far beyond one tile's shared memory (fp32 columns: 1024 points; rows: 16384), read across a transposed view and
+    # along pitched rows; tests/test_host_strided_forms.py pins the boundaries themselves
     shape = (1, 32768, 4, 2)
     status, msg = status_of("float32", "float32", shape, shape, in_strides=(4 * 32768, 1, 32768))
     assert status == 4 and "one tile" in msg, msg

@@ -1,62 +1,11 @@
-"""Runtime-length tier (csrc/rt.cu): axis lengths without a registered variant run on compile-time codelets
-selected at run time; parity against numpy float64 and the oracle, and that the tier is actually used."""
-import numpy as np
+"""Runtime-length tier (csrc/rt.cu): which stage lists stay on the generic kernel, and that the tier is much faster than
+it. The transforms of both kernels are checked against float64 by the form table (tests/_rt_generic_forms.py,
+tests/test_gpu_rt_generic_forms.py)."""
 import pytest
 
 import b200fft
 
 pytestmark = pytest.mark.gpu
-
-
-def c2(a):
-    a = np.asarray(a, dtype=np.float64)
-    return a[..., 0] + 1j * a[..., 1]
-
-
-CASES = [
-    # shape, bases, inverse, in dtype, comps
-    ((50, 1000), None, False, "float32", 2),
-    ((50, 1000), [[10, 10, 10]], True, "float32", 2),
-    ((33, 100), [[5, 2]], False, "float32", 2),
-    ((9, 343), None, False, "float32", 2),               # 7^3
-    ((6, 31 * 29), None, False, "float32", 2),           # two large primes, one stage each
-    ((4, 2187), [[3]], True, "float32", 2),              # 3^7 -> (27)(27)(3)
-    ((3, 30, 21), None, False, "float32", 2),
-    ((2, 12, 100, 18), None, True, "float32", 2),
-    ((5, 600), None, False, "float32", 1),               # real input, full spectrum
-    ((3, 50, 36), None, False, "uint8", 1),
-    ((4, 225), None, False, "float64", 2),               # f64 in, f32 out
-    ((2, 4000), None, False, "float32", 2),
-    ((1, 10000), None, False, "float32", 2),
-    ((7, 17, 1000), None, False, "float32", 2),          # long strided axis next to a long contiguous one
-]
-
-
-@pytest.mark.parametrize("shape,bases,inverse,in_dtype,comps", CASES)
-def test_rt_tier(oracle, shape, bases, inverse, in_dtype, comps):
-    import torch
-    rng = np.random.default_rng(17)
-    full = shape + (comps,)
-    x = rng.integers(0, 256, size=full).astype(np.uint8) if in_dtype == "uint8" else rng.standard_normal(full).astype(in_dtype)
-    # FORCE_RT: without it these lengths get a kernel specialised at plan time (csrc/jit.cu, tests/test_gpu_jit.py)
-    plan = b200fft.plan_fft(in_dtype, "float32", full, shape + (2,), bases=bases, inverse=inverse, flags=b200fft.FLAG_FORCE_RT)
-    desc = plan.describe()
-    assert "rt_" in desc and "generic" not in desc, desc
-    out = torch.full(shape + (2,), float("nan"), device="cuda")
-    b200fft.fft(out, torch.from_numpy(x).cuda(), plan=plan)
-    torch.cuda.synchronize()
-    got = c2(out.cpu().numpy())
-    xd = x.astype(np.float64)
-    xc = xd[..., 0] if comps == 1 else c2(xd)
-    axes = tuple(range(1, len(shape)))
-    want = np.fft.ifftn(xc, axes=axes) if inverse else np.fft.fftn(xc, axes=axes)
-    assert np.isfinite(got).all()
-    tol = 2e-6 * max(1.0, np.sqrt(len(axes)))
-    assert np.linalg.norm(got - want) <= tol * np.linalg.norm(want), desc
-    if in_dtype != "float64":
-        ref = c2(oracle.ref_fft(x, bases=bases, inverse=inverse))
-        assert np.linalg.norm(got - ref) <= 5e-6 * max(1.0, np.sqrt(len(axes))) * np.linalg.norm(want)
-    plan.destroy()
 
 
 def test_radix_above_64_stays_generic():

@@ -241,6 +241,18 @@ int build_passes(b200fft_plan* plan, bool dry, std::string* text) {
   return add(last, rows, any ? work_spec : in_spec, HALF_C2R, any ? BUF_WORK : BUF_INPUT, BUF_OUTPUT);
 }
 
+// the one pass of a scatter_z_plan_create plan: axis 0 of the user's input, stored into the peers' buffers
+int build_scatter_z_pass(b200fft_plan* plan) {
+  int status;
+  std::unique_ptr<Pass> pass = make_jit_scatter_z_pass(*plan, 0, view_of(plan->prob, 0), &status);
+  if (!pass) return status;
+  pass->src_sel = BUF_INPUT;
+  pass->dst_sel = BUF_OUTPUT;
+  pass->axis = 0;
+  plan->passes.push_back(std::move(pass));
+  return B200FFT_OK;
+}
+
 // The alignment b200fft_exec requires of the input and output pointers: one element of each buffer, raised to what the
 // kernels of every pass that touches it need (Pass::min_align), fallback passes included.
 void record_alignment(b200fft_plan* plan) {
@@ -344,10 +356,11 @@ namespace {
 // b200fft_jit_probe / b200fft_jit_split_probe / b200fft_jit_split3_probe: validate, order the bases, run the host-only probe
 using ProbeFn = int (*)(int64_t, int64_t, const std::vector<uint32_t>&, bool, bool, int, int, int, std::string*);
 int probe_entry(ProbeFn probe, int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in, int half,
-                int in_dtype, int out_dtype, char* buf, size_t cap) {
+                int in_dtype, int out_dtype, char* buf, size_t cap, int max_half = 2) {
   if (in_dtype < B200FFT_U8 || in_dtype > B200FFT_F64 || (out_dtype != B200FFT_F32 && out_dtype != B200FFT_F64))
     return fail(B200FFT_ERR_INVALID_ARG, "dtypes %d -> %d", in_dtype, out_dtype);
-  if (half < 0 || half > 2) return fail(B200FFT_ERR_INVALID_ARG, "half = %d (0 complex, 1 R2C, 2 C2R)", half);
+  if (half < 0 || half > max_half)  // 3, the scattering Z pass of a half-spectrum slab inverse: b200fft_jit_probe only
+    return fail(B200FFT_ERR_INVALID_ARG, "half = %d (0 complex, 1 R2C, 2 C2R%s)", half, max_half > 2 ? ", 3 slab Z scatter" : "");
   if (n < 2 || inner < 1) return fail(B200FFT_ERR_INVALID_ARG, "axis length %lld, inner %lld", (long long)n, (long long)inner);
   std::vector<uint32_t> ordered;
   if (bases && nbases > 0) {
@@ -371,7 +384,7 @@ extern "C" {
 
 int b200fft_jit_probe(int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in, int half,
                       int in_dtype, int out_dtype, char* buf, size_t cap) {
-  return probe_entry(jit_probe, n, inner, bases, nbases, inverse, real_in, half, in_dtype, out_dtype, buf, cap);
+  return probe_entry(jit_probe, n, inner, bases, nbases, inverse, real_in, half, in_dtype, out_dtype, buf, cap, 3);
 }
 
 int b200fft_jit_probe_strided(int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in, int half,
@@ -445,11 +458,13 @@ static int finish_plan(std::unique_ptr<b200fft_plan> plan, const b200fft_desc* d
   for (int a = 0; a < plan->prob.rank; ++a) {
     // the n-entry W_n table serves passes of at most SPLIT2_MAX_N points; a longer axis has twiddle tables of its own, and
     // the single-tile passes of a strided plan upload their own stage tables
-    if (plan->strided || !plan->prob.axes[a].transformed || plan->prob.axes[a].n > SPLIT2_MAX_N) continue;
+    if (plan->strided || plan->scatter_z || !plan->prob.axes[a].transformed || plan->prob.axes[a].n > SPLIT2_MAX_N) continue;
     rc = upload_twiddles(plan->prob.axes[a].n, desc->inverse != 0, f64, &plan->tw[a]);
     if (rc != B200FFT_OK) { b200fft_plan_destroy(plan.release()); return rc; }
   }
-  rc = plan->strided ? build_strided_passes(plan.get()) : build_passes(plan.get(), /*dry=*/false, nullptr);
+  rc = plan->strided     ? build_strided_passes(plan.get())
+       : plan->scatter_z ? build_scatter_z_pass(plan.get())
+                         : build_passes(plan.get(), /*dry=*/false, nullptr);
   if (rc != B200FFT_OK) { b200fft_plan_destroy(plan.release()); return rc; }
   record_alignment(plan.get());
   // The tables were uploaded with cudaMemcpy from pageable memory on the legacy stream: make sure they have landed
@@ -460,6 +475,24 @@ static int finish_plan(std::unique_ptr<b200fft_plan> plan, const b200fft_desc* d
   }
   *out = plan.release();
   return B200FFT_OK;
+}
+
+int b200fft::scatter_z_plan_create(b200fft_plan** out, const b200fft_desc* desc) {
+  if (!out) return fail(B200FFT_ERR_INVALID_ARG, "null plan pointer");
+  *out = nullptr;
+  std::unique_ptr<b200fft_plan> plan(new b200fft_plan());
+  int rc = validate(desc, &plan->prob);
+  if (rc != B200FFT_OK) return rc;
+  if (plan->prob.half || plan->prob.batch != 1 || plan->prob.rank < 2 || desc->axis_mask != 1)
+    return fail(B200FFT_ERR_INVALID_ARG, "the scattering Z pass takes one complex volume, axis 0 only");
+  plan->scatter_z = true;
+  return finish_plan(std::move(plan), desc, out);
+}
+
+int b200fft::plan_prepare_scatter(b200fft_plan* plan) {
+  if (plan->passes.empty() || plan->passes.back()->axis != 0)
+    return fail(B200FFT_ERR_UNSUPPORTED, "the last pass of the plan does not transform the split axis 0");
+  return plan->passes.back()->prepare_scatter();
 }
 
 extern "C" {
@@ -532,7 +565,11 @@ int b200fft_exec(b200fft_plan* plan, void* d_out, const void* d_in, void* cu_str
 static int exec_scatter_impl(b200fft_plan* plan, void* const* peer_out, int npeers, int my_rank, long long zbase, const void* d_in,
                              void* d_work, void* cu_stream) {
   if (!plan || !peer_out || !d_in || !d_work) return fail(B200FFT_ERR_INVALID_ARG, "null plan or buffer");
-  if (plan->prob.half) return fail(B200FFT_ERR_UNSUPPORTED, "exec_scatter takes a complex plan");
+  if (plan->prob.half && plan->prob.desc.inverse)
+    return fail(B200FFT_ERR_UNSUPPORTED, "exec_scatter takes complex or forward half-spectrum (R2C) plans; this one is C2R");
+  if (plan->prob.half && d_work == d_in)
+    return fail(B200FFT_ERR_INVALID_ARG, "exec_scatter of an R2C plan: d_work holds the half spectrum and cannot be the real "
+                                         "input d_in");
   if (plan->strided) return fail(B200FFT_ERR_UNSUPPORTED, "exec_scatter takes dense layouts; this plan is strided");
   if (my_rank < 0 || my_rank >= npeers) return fail(B200FFT_ERR_INVALID_ARG, "my_rank %d outside 0..%d", my_rank, npeers);
   if (plan->passes.empty() || plan->passes.back()->axis != 0)

@@ -973,10 +973,38 @@ struct ScatterDst {
     sa->peer[h][tile_off + r * inner + c] = v;
   }
 };
+__device__ __forceinline__ ScatterDst scatter_dst(const ScatterArgs& sa, long long o, long long c0, long long inner, int valid_c) {
+  return ScatterDst{&sa, ((sa.zbase + o) * sa.yl) * inner + c0, inner, valid_c};
+}
+// The reverse exchange (the inverse of a half-spectrum slab, mgpu.cu): the source is this rank's Y-slab viewed as
+// (outer, N = Z, inner = Y/G * W) and output k of column c belongs to peer h = k / rows, at row k - h * rows of that
+// peer's [Z/G][Y][W] slab. This rank's columns are one contiguous block of every such row, starting at col0; the rows
+// are `stride` = Y * W apart, not `inner` as in the forward exchange.
+struct ScatterZArgs {
+  float2* peer[16];
+  int rows;          // outputs of the transformed axis per peer (Z/G)
+  long long col0;    // this rank's first column inside a peer's row (g * Y/G * W)
+  long long stride;  // element stride between a peer's rows (Y * W)
+};
+struct ScatterZDst {
+  const ScatterZArgs* sa;
+  long long tile_off;  // o * rows * stride + col0 + c0
+  int valid_c;
+  __device__ __forceinline__ void store(int, int i, int c, float2 v) const {
+    if (c >= valid_c) return;
+    const int h = i / sa->rows;
+    const int r = i - h * sa->rows;
+    sa->peer[h][tile_off + r * sa->stride + c] = v;
+  }
+};
+__device__ __forceinline__ ScatterZDst scatter_dst(const ScatterZArgs& sa, long long o, long long c0, long long, int valid_c) {
+  return ScatterZDst{&sa, o * sa.rows * sa.stride + sa.col0 + c0, valid_c};
+}
 
-template <int N, class RL, int CW, int NT, bool INV>
+// SA: where the outputs go (ScatterArgs: the forward exchange, ScatterZArgs: the reverse one)
+template <int N, class RL, int CW, int NT, bool INV, class SA = ScatterArgs>
 __global__ void __launch_bounds__(NT) cols_scatter_kernel(const __grid_constant__ ColsArgs a,
-                                                          const __grid_constant__ ScatterArgs sa) {
+                                                          const __grid_constant__ SA sa) {
   extern __shared__ __align__(16) float2 smem_f2[];
   pdl_wait();
   constexpr int BUF = max_exchange_elems<RL, 1, DenseLayoutN<N, CW>::template type>();
@@ -988,7 +1016,7 @@ __global__ void __launch_bounds__(NT) cols_scatter_kernel(const __grid_constant_
   const long long base = o * N * a.inner + c0;
   const int valid_c = (int)min((long long)CW, a.inner - c0);
   GlobalSrc<false> src{reinterpret_cast<const float2*>(a.in) + base, 0, a.inner, 1, valid_c};
-  ScatterDst dst{&sa, ((sa.zbase + o) * sa.yl) * a.inner + c0, a.inner, valid_c};
+  const auto dst = scatter_dst(sa, o, c0, a.inner, valid_c);
   run_axis<RL, N, 1, CW, NT, INV, DenseLayoutN<N, CW>::template type>(src, dst, buf0, buf1, a.tw, a.scale,
                                                                       a.do_scale != 0);
 }

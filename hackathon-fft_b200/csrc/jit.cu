@@ -156,6 +156,7 @@ std::string dense_expression(const TileSpec& s) {
       return "b200fft::rows_ip_kernel<" + head + ", " + inv + ", " + real + ">";
     case TILE_COLS: return "b200fft::cols_kernel<" + head + ", " + inv + ", " + real + ">";
     case TILE_SCATTER: return "b200fft::cols_scatter_kernel<" + head + ", " + inv + ">";
+    case TILE_SCATTER_Z: return "b200fft::cols_scatter_kernel<" + head + ", " + inv + ", b200fft::ScatterZArgs>";
     case TILE_R2C: return "b200fft::rows_r2c_kernel<" + head + ">";
     case TILE_R2C_REG: return "b200fft::rows_r2c_reg_kernel<" + head + ">";
     case TILE_R2C_ODD: return "b200fft::rows_r2c_odd_kernel<" + head + ">";
@@ -195,7 +196,8 @@ std::string smem_expression(const TileSpec& s) {  // fast.cuh's own constexpr fo
     case TILE_SPLIT_A_C2R:
     case TILE_SPLIT_A_C2R_ODD:
     case TILE_SPLIT3_A:
-    case TILE_SCATTER: return "b200fft::cols_smem_bytes<" + shape_args(s) + ">()";
+    case TILE_SCATTER:
+    case TILE_SCATTER_Z: return "b200fft::cols_smem_bytes<" + shape_args(s) + ">()";
     case TILE_R2C:
     case TILE_SPLIT_B_R2C: return "b200fft::rows_r2c_smem_bytes<" + shape_args(s) + ">()";
     case TILE_R2C_REG: return "b200fft::rows_r2c_reg_smem_bytes<" + shape_args(s) + ">()";
@@ -206,7 +208,7 @@ std::string jit_name(const TileSpec& s) {
   static const char* const tag[] = {"jitrows", "jitcols", "jitscatter", "jitr2c", "jitr2creg", "jitr2codd", "jitc2r", "jitc2rodd",
                                     "jitsplitA", "jitsplitBcols", "jitsplitBrows", "jitplane", "jitr2cplane", "jitrowsIP",
                                     "jitsplitBr2c", "jitsplitAc2r", "jitsplitAc2rodd", "jitsplitBhalf", "jitsplitBreal",
-                                    "jitsplit3A", "jitsplit3C"};
+                                    "jitsplit3A", "jitsplit3C", "colsT" /* TILE_COLS_TMA: compiled-in only */, "jitscatterZ"};
   if (s.plane())
     return std::string(tag[s.kind]) + std::to_string(s.n) + "x" + std::to_string(s.kind == TILE_PLANE_R2C ? 2 * s.n2 : s.n2) + "(" +
            radix_name(s.radices) + ";" + radix_name(s.radices2) + ")_inplace_t" + std::to_string(s.threads) + (s.f64 ? "_f64" : "");
@@ -1036,6 +1038,26 @@ std::unique_ptr<Pass> make_jit_split3_pass(b200fft_plan& plan, int axis, const A
   return pass;
 }
 
+// The Z pass of a half-spectrum slab inverse with the reverse exchange in its stores (mgpu.cu): the column tile this tier
+// gives a plain n-point pass over `inner` columns of the working precision, with the ScatterZArgs store. No compiled-in
+// variant has that store, so it is built here whatever the length. False, with the reason in last_error(), when the axis
+// does not fit one column tile.
+bool jit_scatter_z_spec(const AxisSpec& ax, const AxisView& view, bool inverse, bool f64, TileSpec* spec) {
+  const IoSpec src{f64 ? B200FFT_F64 : B200FFT_F32, 2};
+  const char* why = nullptr;
+  if (!jit_enabled()) why = "B200FFT_JIT=0 turns that tier off";
+  else if (view.n > 16384) why = "it is longer than one column tile takes (16384 points)";
+  else if (view.inner < 2) why = "it has a single column";
+  else if (!jit_plan_axis(ax, view, src, inverse, HALF_NONE, f64, spec, 0, &why) && !why) why = "no column tile fits";
+  if (why) {
+    fail(B200FFT_ERR_UNSUPPORTED, "the scattering Z pass of a half-spectrum slab inverse is one column tile of the plan-time "
+         "tier; for this %lld-point %s axis %s", (long long)view.n, f64 ? "fp64" : "fp32", why);
+    return false;
+  }
+  spec->kind = TILE_SCATTER_Z;
+  return true;
+}
+
 }  // namespace
 
 std::unique_ptr<Pass> make_jit_pass(b200fft_plan& plan, int axis, const AxisView& view, const IoSpec& src, bool scale_inverse,
@@ -1085,6 +1107,41 @@ std::unique_ptr<Pass> make_jit_pass(b200fft_plan& plan, int axis, const AxisView
            half == HALF_R2C ? (spec.kind == TILE_R2C_ODD ? " r2c (real rows, bins 0..n/2 stored)" : " r2c")
            : half == HALF_C2R ? (spec.kind == TILE_C2R_ODD ? " c2r (Hermitian-extended load)" : " c2r") : spec.real_in ? " real-in" : "",
            k->compile_ms);
+  pass->text = buf;
+  return pass;
+}
+
+std::unique_ptr<Pass> make_jit_scatter_z_pass(b200fft_plan& plan, int axis, const AxisView& view, int* status) {
+  const Problem& p = plan.prob;
+  const bool f64 = p.desc.out_dtype == B200FFT_F64;
+  *status = B200FFT_ERR_UNSUPPORTED;
+  TileSpec spec;
+  if (!jit_scatter_z_spec(p.axes[axis], view, p.desc.inverse != 0, f64, &spec)) return nullptr;
+  std::shared_ptr<JitKernel> k = get_kernel(spec, plan.device);
+  if (!k) return nullptr;
+  auto pass = std::make_unique<TilePass>();
+  pass->spec = spec;
+  pass->k = {nullptr, k->fn, jit_name(spec)};
+  pass->view = view;
+  pass->device = plan.device;
+  pass->do_scale = p.desc.inverse != 0;
+  pass->scale = pass->do_scale ? 1.0 / (double)view.n : 1.0;
+  pass->smem = spec.smem();
+  auto tables = [&](auto zero) {
+    using T2 = decltype(zero);
+    return (pass->tw = plan_upload(plan, build_twiddles<T2>(spec.radices, spec.inverse))) != nullptr;
+  };
+  if (!(f64 ? tables(double2()) : tables(float2()))) {
+    *status = fail(B200FFT_ERR_ALLOC, "axis %d: cannot allocate the twiddle table of the scattering Z pass", axis);
+    return nullptr;
+  }
+  std::string stages;
+  for (uint32_t r : p.axes[axis].ordered) stages += (stages.empty() ? "" : ",") + std::to_string(r);
+  char buf[400];
+  snprintf(buf, sizeof buf, "axis %d: %s n=%lld inner=%lld smem=%zuB regs=%d%s user stages=[%s] fused as (%s), output k stored into the "
+           "Z-slab of peer k / (n/peers)%s [NVRTC, %.0f ms]", axis, jit_name(spec).c_str(), (long long)view.n, (long long)view.inner,
+           pass->smem, k->regs, k->local_bytes ? (" local=" + std::to_string(k->local_bytes) + "B").c_str() : "", stages.c_str(),
+           radix_name(spec.radices).c_str(), pass->do_scale ? ", 1/n" : "", k->compile_ms);
   pass->text = buf;
   return pass;
 }
@@ -1264,7 +1321,8 @@ int probe_compile(const TileSpec& spec, std::string* report) {
 }  // namespace
 
 // Host-only probe (no CUDA device needed): compile the kernel the planner would pick for one axis and report it.
-// half: 0 = complex / real-input full spectrum, 1 = R2C rows, 2 = C2R rows
+// half: 0 = complex / real-input full spectrum, 1 = R2C rows, 2 = C2R rows, 3 = the scattering Z pass of a half-spectrum
+// slab inverse (column tiles over `inner` columns, complex in the working precision)
 int jit_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bool inverse, bool real_in, int half,
               int in_dtype, int out_dtype, std::string* report) {
   AxisSpec ax;
@@ -1277,6 +1335,10 @@ int jit_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bo
   src.comps = real_in ? 1 : 2;
   src.dtype = in_dtype;
   TileSpec spec;
+  if (half == 3) {  // the scattering Z pass of a half-spectrum slab inverse (make_jit_scatter_z_pass)
+    if (!jit_scatter_z_spec(ax, view, inverse, out_dtype == B200FFT_F64, &spec)) return B200FFT_ERR_UNSUPPORTED;
+    return probe_compile(spec, report);
+  }
   if (!jit_plan_axis(ax, view, src, inverse, (HalfMode)half, out_dtype == B200FFT_F64, &spec))
     return fail(B200FFT_ERR_UNSUPPORTED, "the specialisation tier does not serve this axis (radix above %d, or no tile fits)", JIT_MAX_PRIME);
   return probe_compile(spec, report);

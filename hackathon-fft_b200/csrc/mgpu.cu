@@ -9,6 +9,10 @@
 //      (b200fft_exec_scatter over peer-mapped pointers: the all-to-all is the kernel's own NVLink stores);
 //   2. device-side barrier: every slot's stream waits for the "scatter done" event of every other slot;
 //   3. strided Z pass in place on the received [Z][Y/G][X] slab.
+// The forward half spectrum (R2C) is the same with the local (Y, X) R2C plan, over X/2+1 bins from step 1 on. Its inverse
+// (C2R) runs the other way round, Y-slab in, Z-slab out: 1. Z pass of the slot's [Z][Y/G][X/2+1] slab whose stores go to
+// the [Z/G][Y][X/2+1] receive buffer of the slot that owns z (the reverse exchange, make_jit_scatter_z_pass); 2. the
+// same barrier; 3. local (Y, X) C2R of the received planes.
 // What python/b200fft/slab.py does with one process per GPU, CUDA IPC and a one-word all-reduce, done here with peer
 // access and cross-device events: no NCCL, no host round trip between the steps.
 #include <cuda_runtime.h>
@@ -23,7 +27,7 @@
 #include <thread>
 #include <vector>
 
-#include "common.hpp"
+#include "plan.hpp"
 
 using namespace b200fft;
 
@@ -41,10 +45,11 @@ struct Slot {
   int device = 0;
   int64_t first = 0, count = 0;  // batch items (BATCH_SHARD) / z planes (SLAB)
   b200fft_plan* plan = nullptr;  // BATCH_SHARD: the shard's plan; SLAB: local (Y, X) transform of the slot's planes
-  b200fft_plan* planz = nullptr; // SLAB: Z pass over the received [Z][Y/G][X] slab
+  b200fft_plan* planz = nullptr; // SLAB: Z pass over the received [Z][Y/G][X] slab (inverse half spectrum: over the input)
   cudaStream_t stream = nullptr;
   cudaEvent_t scattered = nullptr, done = nullptr;
-  void* work = nullptr;          // SLAB: [Z/G][Y][X] intermediate of step 1
+  void* work = nullptr;          // SLAB: [Z/G][Y][X] (half spectrum: [Z/G][Y][X/2+1]) intermediate of step 1
+  void* recv = nullptr;          // SLAB inverse half spectrum: the [Z/G][Y][X/2+1] planes the peers' Z passes store into
   void* h_in = nullptr;          // SLAB exec_host: device staging, allocated on first use
   void* h_out = nullptr;
   size_t in_bytes = 0, out_bytes = 0;
@@ -73,6 +78,9 @@ struct b200fft_mgpu_plan {
   int mode = 0;
   int64_t batch = 0;
   int64_t Z = 0, Y = 0, X = 0;
+  bool half = false;                 // SLAB: B200FFT_REAL_HALF
+  bool yslab_in = false;             // SLAB inverse half spectrum: Y-slabs in, Z-slabs out
+  std::vector<void*> recv;           // SLAB inverse half spectrum: every slot's receive buffer, by slot
   size_t in_item = 0, out_item = 0;  // BATCH_SHARD: bytes per batch item
   bool executed = false;             // SLAB: `done` events have been recorded at least once
   std::vector<Slot> slots;
@@ -153,7 +161,7 @@ int b200fft_mgpu_plan_destroy(b200fft_mgpu_plan* m) {
     cudaSetDevice(s.device);
     if (s.plan) b200fft_plan_destroy(s.plan);
     if (s.planz) b200fft_plan_destroy(s.planz);
-    for (void* p : {s.work, s.h_in, s.h_out})
+    for (void* p : {s.work, s.recv, s.h_in, s.h_out})
       if (p) cudaFree(p);
     if (s.scattered) cudaEventDestroy(s.scattered);
     if (s.done) cudaEventDestroy(s.done);
@@ -212,9 +220,21 @@ int b200fft_mgpu_plan_create(b200fft_mgpu_plan** out, const b200fft_desc* desc, 
       }
     }
   } else {
-    if (desc->rank != 3 || desc->batch != 1 || desc->in_components != 2 || desc->in_dtype != B200FFT_F32 ||
-        desc->out_dtype != B200FFT_F32 || desc->real_mode != B200FFT_REAL_FULL || desc->axis_mask != 0)
-      return bail(fail(B200FFT_ERR_UNSUPPORTED, "slab mode takes ONE 3-D complex fp32 transform (batch 1, rank 3, all axes)"));
+    const bool half = desc->real_mode == B200FFT_REAL_HALF;
+    const bool fp32_c2c = !half && desc->in_components == 2 && desc->in_dtype == B200FFT_F32 && desc->out_dtype == B200FFT_F32;
+    if (desc->rank != 3)
+      return bail(fail(B200FFT_ERR_UNSUPPORTED, "slab mode takes ONE 3-D transform; rank %d is not served", desc->rank));
+    if (desc->batch != 1)
+      return bail(fail(B200FFT_ERR_UNSUPPORTED, "slab mode takes ONE 3-D transform; batch %lld is not served", (long long)desc->batch));
+    if (desc->axis_mask != 0)
+      return bail(fail(B200FFT_ERR_UNSUPPORTED, "slab mode transforms all three axes; axis_mask %u is not served", desc->axis_mask));
+    if (!half && desc->in_components != 2)
+      return bail(fail(B200FFT_ERR_UNSUPPORTED, "slab mode takes complex or half-spectrum (B200FFT_REAL_HALF) volumes; real "
+                                                "input with the full spectrum is not served"));
+    if (!half && !fp32_c2c && !(desc->in_dtype == B200FFT_F64 && desc->out_dtype == B200FFT_F64))
+      return bail(fail(B200FFT_ERR_UNSUPPORTED, "the complex slab takes fp32 or fp64, the same type in and out"));
+    m->half = half;
+    m->yslab_in = half && desc->inverse;
     m->Z = desc->dims[0];
     m->Y = desc->dims[1];
     m->X = desc->dims[2];
@@ -222,6 +242,7 @@ int b200fft_mgpu_plan_create(b200fft_mgpu_plan** out, const b200fft_desc* desc, 
       return bail(fail(B200FFT_ERR_INVALID_ARG, "slab decomposition needs Z = %lld and Y = %lld divisible by %d devices",
                        (long long)m->Z, (long long)m->Y, ngpu));
     const int64_t zl = m->Z / ngpu, yl = m->Y / ngpu;
+    const int64_t W = half ? m->X / 2 + 1 : m->X;  // complex values per row of the exchanged slabs
     if (yl < 2 && ngpu > 1) return bail(fail(B200FFT_ERR_INVALID_ARG, "fewer than 2 y rows per device"));
     if (int rc = enable_peers(m->slots)) return bail(rc);
     std::vector<uint32_t> b_yx, b_z;
@@ -230,37 +251,48 @@ int b200fft_mgpu_plan_create(b200fft_mgpu_plan** out, const b200fft_desc* desc, 
     slice_bases(*desc, 0, 1, &b_z, &c_z);
     for (int g = 0; g < ngpu; ++g) {
       Slot& s = m->slots[(size_t)g];
-      s.first = g * zl;
-      s.count = zl;
-      s.in_bytes = (size_t)zl * m->Y * m->X * 8;
-      s.out_bytes = (size_t)m->Z * yl * m->X * 8;
+      s.first = m->yslab_in ? g * yl : g * zl;
+      s.count = m->yslab_in ? yl : zl;
       b200fft_desc d2 = *desc;  // local 2-D transform of zl planes; exec_scatter drives its per-axis passes
       d2.rank = 2;
       d2.dims[0] = m->Y;
       d2.dims[1] = m->X;
       d2.batch = zl;
       d2.device = s.device;
-      d2.flags = (desc->flags | B200FFT_FLAG_NO_FUSED) & ~(uint32_t)B200FFT_FLAG_PREFER_FUSED;
+      if (!m->yslab_in)  // the C2R of the inverse half spectrum does not scatter: it keeps the plane kernel
+        d2.flags = (desc->flags | B200FFT_FLAG_NO_FUSED) & ~(uint32_t)B200FFT_FLAG_PREFER_FUSED;
       d2.bases = c_yx.empty() ? nullptr : b_yx.data();
       d2.bases_count = c_yx.empty() ? nullptr : c_yx.data();
       if (int rc = b200fft_plan_create(&s.plan, &d2)) return bail(rc);
-      b200fft_desc dz = *desc;  // Z pass over [Z][yl][X], only axis 0 transformed
+      b200fft_desc dz = *desc;  // Z pass over [Z][yl][W] in the working precision, only axis 0 transformed
       dz.rank = 3;
       dz.dims[0] = m->Z;
       dz.dims[1] = yl;
-      dz.dims[2] = m->X;
+      dz.dims[2] = W;
       dz.batch = 1;
       dz.axis_mask = 1;
       dz.device = s.device;
+      dz.real_mode = B200FFT_REAL_FULL;
+      dz.in_components = 2;
+      dz.in_dtype = desc->out_dtype;
       std::vector<int32_t> cz3;
       if (!c_z.empty()) cz3 = {c_z[0], 0, 0};
       dz.bases = cz3.empty() ? nullptr : b_z.data();
       dz.bases_count = cz3.empty() ? nullptr : cz3.data();
-      if (int rc = b200fft_plan_create(&s.planz, &dz)) return bail(rc);
-      if (cudaSetDevice(s.device) != cudaSuccess || cudaMalloc(&s.work, s.in_bytes) != cudaSuccess) {
+      if (int rc = m->yslab_in ? scatter_z_plan_create(&s.planz, &dz) : b200fft_plan_create(&s.planz, &dz)) return bail(rc);
+      // every form but the complex fp32 one checks here that its scattering Y pass is one column tile, and builds that
+      // pass's kernel now rather than on the first exec
+      if (!fp32_c2c && !m->yslab_in)
+        if (int rc = plan_prepare_scatter(s.plan)) return bail(rc);
+      s.in_bytes = b200fft_plan_in_bytes(m->yslab_in ? s.planz : s.plan);
+      s.out_bytes = b200fft_plan_out_bytes(m->yslab_in ? s.plan : s.planz);
+      void** buf = m->yslab_in ? &s.recv : &s.work;  // what the peers store into / what step 1 leaves for the scatter
+      const size_t bytes = m->yslab_in ? b200fft_plan_in_bytes(s.plan) : b200fft_plan_out_bytes(s.plan);
+      if (cudaSetDevice(s.device) != cudaSuccess || cudaMalloc(buf, bytes) != cudaSuccess) {
         cudaGetLastError();
-        return bail(fail(B200FFT_ERR_ALLOC, "cannot allocate %zu B of slab workspace on device %d", s.in_bytes, s.device));
+        return bail(fail(B200FFT_ERR_ALLOC, "cannot allocate %zu B of slab workspace on device %d", bytes, s.device));
       }
+      if (m->yslab_in) m->recv.push_back(s.recv);
     }
   }
   for (Slot& s : m->slots) {
@@ -274,26 +306,33 @@ int b200fft_mgpu_plan_create(b200fft_mgpu_plan** out, const b200fft_desc* desc, 
   char head[320];
   if (mode == B200FFT_MGPU_BATCH_SHARD)
     snprintf(head, sizeof head, "mgpu batch-shard over %d devices, batch %lld, no communication\n", ngpu, (long long)m->batch);
-  else
+  else if (!m->half)
     snprintf(head, sizeof head,
              "mgpu slab %lldx%lldx%lld over %d devices: local (Y,X) + peer-to-peer scattering Y stores -> event barrier -> Z pass\n",
              (long long)m->Z, (long long)m->Y, (long long)m->X, ngpu);
+  else if (!m->yslab_in)
+    snprintf(head, sizeof head,
+             "mgpu slab %lldx%lldx%lld over %d devices, half spectrum: local (Y,X) R2C + scattering Y stores -> event barrier -> "
+             "Z pass\n", (long long)m->Z, (long long)m->Y, (long long)m->X, ngpu);
+  else
+    snprintf(head, sizeof head,
+             "mgpu slab %lldx%lldx%lld over %d devices, half spectrum inverse (Y-slabs in, z planes out): Z pass with scattering "
+             "stores -> event barrier -> local (Y,X) C2R\n", (long long)m->Z, (long long)m->Y, (long long)m->X, ngpu);
   m->text = head;
   for (int g = 0; g < ngpu; ++g) {
     const Slot& s = m->slots[(size_t)g];
-    std::string t;
-    describe_plan(s.plan, &t);
     char line[160];
     snprintf(line, sizeof line, " slot %d (device %d): %s [%lld, %lld)\n", g, s.device,
-             mode == B200FFT_MGPU_SLAB ? "z planes" : "batch items", (long long)s.first, (long long)(s.first + s.count));
+             mode != B200FFT_MGPU_SLAB ? "batch items" : m->yslab_in ? "y rows" : "z planes", (long long)s.first,
+             (long long)(s.first + s.count));
     m->text += line;
-    if (g == 0) {
-      m->text += t;
-      if (s.planz) {
-        describe_plan(s.planz, &t);
+    if (g == 0)  // the slot's plans in the order they run
+      for (const b200fft_plan* p : {m->yslab_in ? s.planz : s.plan, m->yslab_in ? s.plan : s.planz}) {
+        if (!p) continue;
+        std::string t;
+        describe_plan(p, &t);
         m->text += t;
       }
-    }
   }
   {
     const char* e = getenv("B200FFT_MGPU_THREADS");
@@ -335,25 +374,30 @@ size_t b200fft_mgpu_describe(const b200fft_mgpu_plan* m, char* buf, size_t cap) 
 }
 
 // One slot's share of an exec call. phase 0: everything up to (and including) the record of `scattered`; phase 1: the Z
-// pass. Between the two every slot must have RECORDED its `scattered` event, or a wait on it would be a no-op.
+// pass (inverse half spectrum: the local C2R). Between the two every slot must have RECORDED its `scattered` event, or a
+// wait on it would be a no-op.
 static int slot_enqueue(b200fft_mgpu_plan* m, int g, int phase, void* const* d_out, const void* const* d_in) {
   const int G = (int)m->slots.size();
   Slot& s = m->slots[(size_t)g];
   B200_CUDA_CHECK(cudaSetDevice(s.device));
   if (m->mode == B200FFT_MGPU_BATCH_SHARD) return phase == 0 ? b200fft_exec(s.plan, d_out[g], d_in[g], s.stream) : B200FFT_OK;
   if (phase == 0) {
-    // a slot may not start scattering call k+1 into a peer's slab while that peer still runs the Z pass of call k
+    // a slot may not start scattering call k+1 into a peer's slab while that peer still runs phase 1 of call k on it
     if (m->executed)
       for (int h = 0; h < G; ++h)
         if (h != g) B200_CUDA_CHECK(cudaStreamWaitEvent(s.stream, m->slots[(size_t)h].done, 0));
-    if (int rc = b200fft_exec_scatter(s.plan, d_out, G, g, d_in[g], s.work, s.stream)) return rc;
+    // the inverse half spectrum scatters its Z pass into the peers' receive buffers; the one-pass plan reads d_in only
+    const int rc = m->yslab_in ? b200fft_exec_scatter(s.planz, m->recv.data(), G, g, d_in[g], const_cast<void*>(d_in[g]), s.stream)
+                               : b200fft_exec_scatter(s.plan, d_out, G, g, d_in[g], s.work, s.stream);
+    if (rc) return rc;
     B200_CUDA_CHECK(cudaSetDevice(s.device));
     B200_CUDA_CHECK(cudaEventRecord(s.scattered, s.stream));
     return B200FFT_OK;
   }
   for (int h = 0; h < G; ++h)
     if (h != g) B200_CUDA_CHECK(cudaStreamWaitEvent(s.stream, m->slots[(size_t)h].scattered, 0));
-  if (int rc = b200fft_exec(s.planz, d_out[g], d_out[g], s.stream)) return rc;
+  if (int rc = m->yslab_in ? b200fft_exec(s.plan, d_out[g], s.recv, s.stream) : b200fft_exec(s.planz, d_out[g], d_out[g], s.stream))
+    return rc;
   B200_CUDA_CHECK(cudaSetDevice(s.device));
   B200_CUDA_CHECK(cudaEventRecord(s.done, s.stream));
   return B200FFT_OK;
@@ -484,19 +528,27 @@ int b200fft_mgpu_exec_host(b200fft_mgpu_plan* m, void* h_out, const void* h_in) 
     if (!s.h_out) B200_CUDA_CHECK(cudaMalloc(&s.h_out, s.out_bytes));
     ins[(size_t)g] = s.h_in;
     outs[(size_t)g] = s.h_out;
-    B200_CUDA_CHECK(cudaMemcpyAsync(s.h_in, (const char*)h_in + (size_t)g * s.in_bytes, s.in_bytes, cudaMemcpyHostToDevice, s.stream));
+    if (m->yslab_in) {  // rows y in [g yl, (g+1) yl) of every z plane of the natural-order host spectrum -> slot g's Y-slab
+      const size_t row = s.in_bytes / (size_t)m->Z;
+      B200_CUDA_CHECK(cudaMemcpy2DAsync(s.h_in, row, (const char*)h_in + (size_t)g * row, (size_t)G * row, row, (size_t)m->Z,
+                                        cudaMemcpyHostToDevice, s.stream));
+    } else {
+      B200_CUDA_CHECK(cudaMemcpyAsync(s.h_in, (const char*)h_in + (size_t)g * s.in_bytes, s.in_bytes, cudaMemcpyHostToDevice, s.stream));
+    }
   }
   int rc = b200fft_mgpu_exec(m, outs.data(), ins.data());
-  if (rc == B200FFT_OK) {
-    // slot h's [Z][yl][X] slab -> rows y in [h yl, (h+1) yl) of every z plane of the natural-order host volume
-    const size_t yl = (size_t)(m->Y / G), row = yl * (size_t)m->X * 8, pitch = (size_t)m->Y * (size_t)m->X * 8;
-    for (int g = 0; g < G && rc == B200FFT_OK; ++g) {
-      Slot& s = m->slots[(size_t)g];
-      cudaSetDevice(s.device);
-      cudaError_t e = cudaMemcpy2DAsync((char*)h_out + (size_t)g * row, pitch, s.h_out, row, row, (size_t)m->Z,
-                                        cudaMemcpyDeviceToHost, s.stream);
-      if (e != cudaSuccess) rc = fail(B200FFT_ERR_CUDA, "device-to-host copy of slot %d: %s", g, cudaGetErrorString(e));
+  for (int g = 0; g < G && rc == B200FFT_OK; ++g) {
+    Slot& s = m->slots[(size_t)g];
+    cudaSetDevice(s.device);
+    cudaError_t e;
+    if (m->yslab_in) {  // slot g's z planes, contiguous in the natural-order host volume
+      e = cudaMemcpyAsync((char*)h_out + (size_t)g * s.out_bytes, s.h_out, s.out_bytes, cudaMemcpyDeviceToHost, s.stream);
+    } else {  // slot g's [Z][yl][W] slab -> rows y in [g yl, (g+1) yl) of every z plane of the natural-order host volume
+      const size_t row = s.out_bytes / (size_t)m->Z;
+      e = cudaMemcpy2DAsync((char*)h_out + (size_t)g * row, (size_t)G * row, s.h_out, row, row, (size_t)m->Z, cudaMemcpyDeviceToHost,
+                            s.stream);
     }
+    if (e != cudaSuccess) rc = fail(B200FFT_ERR_CUDA, "device-to-host copy of slot %d: %s", g, cudaGetErrorString(e));
   }
   // the caller may free its host buffers once we return: wait for every copy, also after an error
   for (Slot& s : m->slots) {

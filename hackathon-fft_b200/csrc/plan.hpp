@@ -56,6 +56,10 @@ struct Pass {
   virtual int launch_scatter(const void*, const Scatter&, int64_t, cudaStream_t) {
     return fail(B200FFT_ERR_UNSUPPORTED, "this pass has no scattering store (%s)", describe().c_str());
   }
+  // Whether launch_scatter can run, with whatever kernel it needs built now rather than on its first call.
+  virtual int prepare_scatter() {
+    return fail(B200FFT_ERR_UNSUPPORTED, "this pass has no scattering store (%s)", describe().c_str());
+  }
   int axis = -1;
   BufSel src_sel = BUF_OUTPUT, dst_sel = BUF_OUTPUT;
   // Serpentine pass order: every second pass of a per-axis plan walks its tiles back to front, starting on the part
@@ -96,6 +100,8 @@ struct b200fft_plan {
   std::vector<int64_t> in_strides, out_strides;
   size_t in_span = 0, out_span = 0;
   bool inplace_exact = false;
+  // the Z pass of a half-spectrum slab inverse (scatter_z_plan_create): one pass that only runs through exec_scatter
+  bool scatter_z = false;
   // exec_host resources (lazily created)
   cudaStream_t hs[3] = {nullptr, nullptr, nullptr};
   void* h_dev_in[2] = {nullptr, nullptr};
@@ -156,6 +162,9 @@ std::unique_ptr<Pass> make_jit_plane_pass(b200fft_plan& plan);
 // *status becomes B200FFT_ERR_ALLOC when an axis it would serve cannot get its device memory (stays as given otherwise)
 std::unique_ptr<Pass> make_jit_pass(b200fft_plan& plan, int axis, const AxisView& view, const IoSpec& src, bool scale_inverse,
                                     HalfMode half, int* status);
+// the Z pass of a half-spectrum slab inverse with the reverse exchange in its stores (TILE_SCATTER_Z), always through NVRTC;
+// nullptr with *status = B200FFT_ERR_UNSUPPORTED when the axis does not fit one column tile (B200FFT_ERR_ALLOC: no memory)
+std::unique_ptr<Pass> make_jit_scatter_z_pass(b200fft_plan& plan, int axis, const AxisView& view, int* status);
 int jit_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bool inverse, bool real_in, int half,
               int in_dtype, int out_dtype, std::string* report);
 // the StrLay form of that kernel, for strided layouts (same arguments; inner > 1: column tiles over `inner` columns)
@@ -167,6 +176,15 @@ int jit_split_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& order
 // the three passes it builds for a contiguous axis longer than SPLIT2_MAX_N points (same arguments)
 int jit_split3_probe(int64_t n, int64_t inner, const std::vector<uint32_t>& ordered, bool inverse, bool real_in, int half,
                      int in_dtype, int out_dtype, std::string* report);
+// Multi-device slab plumbing (mgpu.cu).
+// scatter_z_plan_create: a plan over (Z, Y/G, X/2+1) complex in the working precision, axis_mask 1, whose single pass is the
+// Z pass of a half-spectrum slab inverse with the reverse exchange in its stores; b200fft_exec_scatter(plan, peer_out, G, g,
+// d_in, d_in, stream) runs it, storing output z into the [Z/G][Y][X/2+1] buffer peer_out[z / (Z/G)]. Status 4 when Z does
+// not fit one column tile.
+int scatter_z_plan_create(b200fft_plan** out, const b200fft_desc* desc);
+// Whether b200fft_exec_scatter can run `plan`, with its scattering kernel built now: status 4 when the plan's last pass
+// (the split axis) is not one column tile with a scattering store.
+int plan_prepare_scatter(b200fft_plan* plan);
 // number of registered kernel variants per tier (host-only; triggers the one-time registration)
 size_t fast_variant_count();
 size_t fused_variant_count();

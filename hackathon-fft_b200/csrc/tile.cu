@@ -200,6 +200,7 @@ int tile_launch(const TilePass& p, const void* src, void* dst, long long outer, 
       void* params[3] = {&mi, &mo, &a};
       return launch_tile(p.k, outer * a.tiles_per_outer, s.threads, p.smem, false, params, stream);
     }
+    case TILE_SCATTER_Z: return fail(B200FFT_ERR_UNSUPPORTED, "%s only runs as a scattering store", p.text.c_str());
     default: {  // the half-spectrum row forms; the C2R pass is the last pass of its plan
       typename Args<F64>::Half a;
       a.in = src;
@@ -319,11 +320,10 @@ int TilePass::launch(const void* src, void* dst, int64_t nbatch, cudaStream_t st
   return spec.f64 ? tile_launch<true>(*this, src, dst, outer, stream) : tile_launch<false>(*this, src, dst, outer, stream);
 }
 
-int TilePass::launch_scatter(const void* src, const Scatter& sc, int64_t nbatch, cudaStream_t stream) {
+int TilePass::prepare_scatter() {
+  if (spec.kind == TILE_SCATTER_Z) return B200FFT_OK;  // the pass's own kernel, built with it (jit.cu: make_jit_scatter_z_pass)
   if (spec.kind != TILE_COLS || spec.real_in || spec.in_dtype != (spec.f64 ? B200FFT_F64 : B200FFT_F32) || (k.sym && !k_scatter.sym))
     return fail(B200FFT_ERR_UNSUPPORTED, "no scattering store for %s", text.c_str());
-  if (sc.npeers < 1 || sc.npeers > 16 || view.n % sc.npeers)
-    return fail(B200FFT_ERR_INVALID_ARG, "split axis length %lld is not divisible by %d peers", (long long)view.n, sc.npeers);
   if (!k.sym && !k_scatter.fn) {
     TileSpec sp = spec;
     sp.kind = TILE_SCATTER;
@@ -334,19 +334,43 @@ int TilePass::launch_scatter(const void* src, const Scatter& sc, int64_t nbatch,
     if (cur != device && cur >= 0) cudaSetDevice(cur);
     if (!k_scatter.fn) return fail(B200FFT_ERR_UNSUPPORTED, "could not specialise the scattering store for %s", text.c_str());
   }
-  ScatterArgs sa;  // pointers and integers only: the same block for both precisions
+  return B200FFT_OK;
+}
+
+namespace {
+// the scattering column kernel `k` with the store policy's argument block `sa` (pointers and integers only: the same block
+// for both precisions)
+template <class SA>
+int scatter_launch(const TilePass& p, const TileKernel& k, const void* src, SA sa, long long outer, cudaStream_t stream) {
+  if (p.spec.f64) {
+    ColsArgs64 ca = cols_args<true>(p, src, nullptr);
+    void* params[2] = {&ca, &sa};
+    return launch_tile(k, outer * ca.tiles_per_outer, p.spec.threads, p.smem, false, params, stream);
+  }
+  ColsArgs ca = cols_args<false>(p, src, nullptr);
+  void* params[2] = {&ca, &sa};
+  return launch_tile(k, outer * ca.tiles_per_outer, p.spec.threads, p.smem, false, params, stream);
+}
+}  // namespace
+
+int TilePass::launch_scatter(const void* src, const Scatter& sc, int64_t nbatch, cudaStream_t stream) {
+  if (int rc = prepare_scatter()) return rc;
+  if (sc.npeers < 1 || sc.npeers > 16 || view.n % sc.npeers)
+    return fail(B200FFT_ERR_INVALID_ARG, "split axis length %lld is not divisible by %d peers", (long long)view.n, sc.npeers);
+  const long long outer = nbatch * view.outer_per_batch;
+  if (spec.kind == TILE_SCATTER_Z) {  // this rank's columns are block my_rank of every row of a peer's slab
+    ScatterZArgs za;
+    for (int i = 0; i < 16; ++i) za.peer[i] = i < sc.npeers ? reinterpret_cast<float2*>(sc.peer_out[i]) : nullptr;
+    za.rows = (int)(view.n / sc.npeers);
+    za.col0 = (long long)sc.my_rank * view.inner;
+    za.stride = (long long)sc.npeers * view.inner;
+    return scatter_launch(*this, k, src, za, outer, stream);
+  }
+  ScatterArgs sa;
   for (int i = 0; i < 16; ++i) sa.peer[i] = i < sc.npeers ? reinterpret_cast<float2*>(sc.peer_out[i]) : nullptr;
   sa.yl = (int)(view.n / sc.npeers);
-  const long long outer = nbatch * view.outer_per_batch;
   sa.zbase = sc.zbase >= 0 ? sc.zbase : (long long)sc.my_rank * outer;
-  if (spec.f64) {
-    ColsArgs64 ca = cols_args<true>(*this, src, nullptr);
-    void* params[2] = {&ca, &sa};
-    return launch_tile(k_scatter, outer * ca.tiles_per_outer, spec.threads, smem, false, params, stream);
-  }
-  ColsArgs ca = cols_args<false>(*this, src, nullptr);
-  void* params[2] = {&ca, &sa};
-  return launch_tile(k_scatter, outer * ca.tiles_per_outer, spec.threads, smem, false, params, stream);
+  return scatter_launch(*this, k_scatter, src, sa, outer, stream);
 }
 
 int SplitPass::launch(const void* src, void* dst, int64_t nbatch, cudaStream_t stream) {

@@ -41,7 +41,9 @@ enum TileKind {
   // contiguous axes longer than 2^24 points as three passes, n = N1 * N2 * N3 (fast.cuh):
   TILE_SPLIT3_A,        // cols_split_a_kernel<N, RL, CW, NT, INV, REAL, true>: passes 1 and 2, the twiddle from two tables
   TILE_SPLIT3_C,        // rows_split_c_kernel<N3, RL, C, NT, INV>: pass 3, rows (k1, k2), natural-order store
-  TILE_COLS_TMA         // cols_tma_kernel<N, RL, CW, NT, INV>: strided tiles moved by TMA (compiled-in variants only)
+  TILE_COLS_TMA,        // cols_tma_kernel<N, RL, CW, NT, INV>: strided tiles moved by TMA (compiled-in variants only)
+  TILE_SCATTER_Z        // cols_scatter_kernel<N, RL, CW, NT, INV, ScatterZArgs>: the reverse exchange of the half-spectrum slab
+                        // inverse (mgpu.cu), stores into the peers' Z-slabs (plan-time tier only)
 };
 
 size_t in_scalar_bytes(int dtype);
@@ -66,7 +68,7 @@ struct TileSpec {
   bool plane() const { return kind == TILE_PLANE_C2C || kind == TILE_PLANE_R2C; }
   bool strided() const {
     return kind == TILE_COLS || kind == TILE_SCATTER || kind == TILE_SPLIT_A || kind == TILE_SPLIT_B_COLS || kind == TILE_SPLIT_A_C2R ||
-           kind == TILE_SPLIT_A_C2R_ODD || kind == TILE_SPLIT3_A || kind == TILE_COLS_TMA;
+           kind == TILE_SPLIT_A_C2R_ODD || kind == TILE_SPLIT3_A || kind == TILE_COLS_TMA || kind == TILE_SCATTER_Z;
   }
   // Host mirror of fast.cuh's shared-memory formulas for the kinds the plan-time tier builds: used to choose the tile
   // before anything is compiled, and checked against the value the compiled module reports.
@@ -150,7 +152,7 @@ std::vector<T2> build_half_twiddles(long long n, bool inverse);
 struct TilePass : Pass {
   TileSpec spec;
   TileKernel k;
-  TileKernel k_scatter;  // compiled-in: the variant's scatter instantiation (may be absent); NVRTC: built on first use
+  TileKernel k_scatter;  // compiled-in: the variant's scatter instantiation (may be absent); NVRTC: built by prepare_scatter
   size_t smem = 0;
   AxisView view;
   int device = 0;
@@ -162,6 +164,7 @@ struct TilePass : Pass {
 
   int launch(const void* src, void* dst, int64_t nbatch, cudaStream_t stream) override;
   int launch_scatter(const void* src, const Scatter& sc, int64_t nbatch, cudaStream_t stream) override;
+  int prepare_scatter() override;
   std::string describe() const override { return text; }
   size_t min_align(bool src) const override { return tile_min_align({&spec}, src); }
 };
@@ -178,6 +181,7 @@ struct StridedPass : TilePass {
   int launch_scatter(const void*, const Scatter&, int64_t, cudaStream_t) override {
     return fail(B200FFT_ERR_UNSUPPORTED, "strided plans have no scattering store");
   }
+  int prepare_scatter() override { return fail(B200FFT_ERR_UNSUPPORTED, "strided plans have no scattering store"); }
 };
 
 // The plan-time kernel of one strided pass (jit.cu): n points along the axis, as rows (ncols == 0) or as column tiles over

@@ -490,7 +490,16 @@ def mgpu_split(batch, ngpu, g):
 
 class MgpuPlan:
     """One host process driving several GPUs (b200fft_mgpu_*): batch sharding without communication, or the slab
-    decomposition of ONE 3-D transform with the exchange fused into the Y pass's peer-to-peer stores."""
+    decomposition of ONE 3-D transform with the exchange fused into the Y pass's peer-to-peer stores.
+
+    MGPU_SLAB over G devices, layouts (1, Z, Y, X, 2) complex (fp32 or fp64), or with real_mode=REAL_HALF the real
+    (1, Z, Y, X, 1) and the half spectrum (1, Z, Y, X//2+1, 2); W = X//2+1. Per slot g:
+      complex:               ins[g] (Z/G, Y, X, 2)  -> outs[g] (Z, Y/G, X, 2)
+      REAL_HALF forward:     ins[g] (Z/G, Y, X) real (fp32 or fp64) -> outs[g] (Z, Y/G, W, 2)
+      REAL_HALF inverse:     ins[g] (Z, Y/G, W, 2) -> outs[g] (Z/G, Y, X) real, scaled by 1/(Z*Y*X)
+    Forward outputs are Y-slabs (rows y of slot h: h*Y/G + y_local). The half-spectrum inverse takes exactly those
+    Y-slabs and returns z planes, so forward then inverse round-trips on the device buffers (the complex inverse keeps
+    z planes in and Y-slabs out). shard(g) reports z planes, or y rows for the half-spectrum inverse."""
 
     def __init__(self, in_dtype, out_dtype, in_layout, out_layout, *, devices, mode=MGPU_BATCH_SHARD, bases=None,
                  inverse=False, real_mode=REAL_FULL, flags=0):

@@ -176,7 +176,10 @@ B200FFT_API int b200fft_host_unregister(void* h_ptr);
  * i.e. into the [Z][Y/npeers][X] slab of the rank that owns row y. With peer_out[] mapped over
  * NVLink (b200fft_ipc_open) the all-to-all happens inside the kernel's stores; with local
  * pointers it is the pack step of an NCCL all-to-all. The caller synchronises the ranks (barrier)
- * before reading its slab and then runs the Z pass with a plan over (Z, Y/npeers, X), axis_mask=1. */
+ * before reading its slab and then runs the Z pass with a plan over (Z, Y/npeers, X), axis_mask=1.
+ * A forward half-spectrum (B200FFT_REAL_HALF, R2C) plan is served the same way: its last pass is the complex Y pass over
+ * the X/2+1 bins, so X above reads X/2+1, and d_work (which receives the half spectrum) must not be d_in (status 1).
+ * Inverse (C2R) plans are refused (status 4). */
 B200FFT_API int b200fft_exec_scatter(b200fft_plan* plan, void* const* peer_out, int npeers, int my_rank,
                                      const void* d_in, void* d_work, void* cu_stream);
 
@@ -223,17 +226,32 @@ B200FFT_API int b200fft_plan_destroy(b200fft_plan* plan);
  *   B200FFT_MGPU_BATCH_SHARD  `desc` describes the WHOLE job; slot g owns the contiguous batch items
  *                             [first_g, first_g + count_g) (the first batch % ngpu slots hold one more). No
  *                             communication. d_in[g] / d_out[g] hold only that slot's items.
- *   B200FFT_MGPU_SLAB         one 3-D complex fp32 transform (batch 1, dims (Z, Y, X), Z and Y divisible by ngpu). Slot g
- *                             holds the input z planes [g Z/G, (g+1) Z/G) as d_in[g][Z/G][Y][X]; after exec d_out[h] holds
- *                             out[z][y_local][x] for y = h Y/G + y_local, i.e. d_out[h][Z][Y/G][X] ("transposed out", as
- *                             the slab decomposition of north_star leaves it). Local (Y, X) transform with the exchange
- *                             fused into the Y pass's stores (peer-to-peer over NVLink, cudaDeviceEnablePeerAccess, no
- *                             pack buffer, no all-to-all), device-side event barrier, strided Z pass in place on d_out.
- *                             d_out[] must be peer-accessible device memory (cudaMalloc / b200fft_malloc).
+ *   B200FFT_MGPU_SLAB         one 3-D complex fp32 or fp64 transform (batch 1, dims (Z, Y, X), Z and Y divisible by ngpu,
+ *                             the same type in and out). Slot g holds the input z planes [g Z/G, (g+1) Z/G) as
+ *                             d_in[g][Z/G][Y][X]; after exec d_out[h] holds out[z][y_local][x] for y = h Y/G + y_local,
+ *                             i.e. d_out[h][Z][Y/G][X] ("transposed out", as the slab decomposition of north_star leaves
+ *                             it). Local (Y, X) transform with the exchange fused into the Y pass's stores (peer-to-peer
+ *                             over NVLink, cudaDeviceEnablePeerAccess, no pack buffer, no all-to-all), device-side event
+ *                             barrier, strided Z pass in place on d_out. The inverse keeps this orientation (z planes in,
+ *                             Y-slabs out). d_out[] must be peer-accessible device memory (cudaMalloc / b200fft_malloc).
+ *                             With real_mode = B200FFT_REAL_HALF (W = X/2+1, X even or odd):
+ *                             forward (R2C): d_in[g][Z/G][Y][X] real (fp32 or fp64, cast on load) -> d_out[h]
+ *                               [Z][Y/G][W] complex in out_dtype (fp32 or fp64): the same Y-slabs over the half spectrum,
+ *                               which halves the bytes the exchange moves.
+ *                             inverse (C2R): the OTHER orientation, so that forward then inverse round-trips on the device
+ *                               buffers: d_in[g][Z][Y/G][W] is the Y-slab the forward leaves (rows y = g Y/G + y_local, in
+ *                               the working precision) -> d_out[g][Z/G][Y][X] real z planes, scaled by 1 / (Z Y X). A Z
+ *                               pass whose stores go to the owning peers' receive buffers (allocated by the plan),
+ *                               the event barrier, then the local (Y, X) C2R. d_in is not written.
+ *                             Refused with status 4: batch > 1, axis_mask != 0, real input with B200FFT_REAL_FULL, uint8
+ *                             input (as by the single-device half-spectrum plans), and a
+ *                             half-spectrum plan whose scattering axis (Y forward, Z inverse) is too long for one column
+ *                             tile (checked at plan creation).
  *
  * exec enqueues on every slot's stream and returns; b200fft_mgpu_synchronize waits for all of them.
  * b200fft_mgpu_stream(plan, g) is that stream (a cudaStream_t) for callers that order their own work against it.
- * exec_host takes the WHOLE job in host memory, natural order (SLAB: h_in[Z][Y][X] -> h_out[Z][Y][X]): every slot
+ * exec_host takes the WHOLE job in host memory, natural order (SLAB: h_in[Z][Y][X] -> h_out[Z][Y][X]; half spectrum:
+ * real [Z][Y][X] -> complex [Z][Y][X/2+1], the inverse the reverse): every slot
  * copies its share in, runs, and copies its share out (one host thread per slot for BATCH_SHARD, each running the
  * chunked 3-stream pipeline of b200fft_exec_host); returns when h_out is complete. */
 enum { B200FFT_MGPU_BATCH_SHARD = 0, B200FFT_MGPU_SLAB = 1 };
@@ -242,7 +260,8 @@ B200FFT_API int b200fft_mgpu_plan_create(b200fft_mgpu_plan** plan, const b200fft
                                          int mode);
 B200FFT_API int b200fft_mgpu_plan_destroy(b200fft_mgpu_plan* plan);
 B200FFT_API int b200fft_mgpu_ngpu(const b200fft_mgpu_plan* plan);
-/* what slot g holds on input: batch items (BATCH_SHARD) or z planes (SLAB) [*first, *first + *count) */
+/* what slot g holds on input: batch items (BATCH_SHARD), z planes (SLAB) or, for the SLAB half-spectrum inverse, y rows
+ * [*first, *first + *count). in_bytes / out_bytes: the sizes of slot g's d_in[g] / d_out[g]. */
 B200FFT_API int b200fft_mgpu_shard(const b200fft_mgpu_plan* plan, int g, int64_t* first, int64_t* count);
 B200FFT_API size_t b200fft_mgpu_in_bytes(const b200fft_mgpu_plan* plan, int g);
 B200FFT_API size_t b200fft_mgpu_out_bytes(const b200fft_mgpu_plan* plan, int g);
@@ -281,7 +300,9 @@ B200FFT_API int b200fft_plan_dry_run(const b200fft_desc* desc, char* buf, size_t
  * planner would pick for ONE axis (length n, element stride `inner`, user bases or NULL for the default rule) and
  * writes "<variant>: <template-id>, smem, cubin size, compile time, symbol" into buf. Needs libnvrtc but no GPU. */
 B200FFT_API int b200fft_jit_probe(int64_t n, int64_t inner, const uint32_t* bases, int nbases, int inverse, int real_in,
-                                  int half /* 0 complex, 1 half-spectrum R2C rows, 2 C2R rows */, int in_dtype, int out_dtype,
+                                  int half /* 0 complex, 1 half-spectrum R2C rows, 2 C2R rows, 3 the scattering Z pass of a
+                                              half-spectrum slab inverse (B200FFT_MGPU_SLAB) over `inner` columns */,
+                                  int in_dtype, int out_dtype,
                                   char* buf, size_t cap);
 /* The same for the strided form of that kernel (b200fft_plan_create_strided; inner > 1: column tiles over `inner` columns).
  * Its variant name ends in "_str". No GPU needed. */

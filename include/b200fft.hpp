@@ -210,7 +210,9 @@ inline Plan plan_fft(DType in_dtype, DType out_dtype, const Layout& in_layout, c
 inline void fft(void* output, const void* x, void* stream, const Plan& plan) { plan.exec(output, x, stream); }
 
 // One host process, several GPUs (b200fft_mgpu_*): batch sharding without communication, or the slab decomposition of ONE
-// 3-D complex fp32 transform (dims (Z, Y, X); slot g holds z planes [g Z/G, (g+1) Z/G), the result is Y-slab distributed).
+// 3-D complex fp32 / fp64 transform (dims (Z, Y, X); slot g holds z planes [g Z/G, (g+1) Z/G), the result is Y-slab
+// distributed), or of a real one with options.real_mode = half spectrum: R2C forward as above over X/2+1 bins, C2R inverse
+// from those Y-slabs back to z planes (include/b200fft.h, B200FFT_MGPU_SLAB).
 enum class MultiGpuMode { batch_shard = B200FFT_MGPU_BATCH_SHARD, slab = B200FFT_MGPU_SLAB };
 
 class MultiGpuPlan {
